@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — batched Waveform.sample throughput (GSa/s) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1], SURVEY.md §8d-2): the 20-qubit XY+Z control
@@ -242,6 +242,23 @@ def run_cpu(chans, steps, warmup, procs):
     return n, dt, kind
 
 
+def dump_outputs(d, out, batch, n_channels=16, n_scattered=1 << 20, seed=20260020):
+    """Writes what one step returns, sampled so that it stays under 64 MB: `n_channels` whole channels
+    drawn with `seed` (ch<index>.npy, the index into the batch's channel list) and `n_scattered`
+    single samples at seeded positions over the whole output, in ascending order (scattered.npy).
+    The dtype is the step's.  The same arguments pick the same channels and positions, so two
+    builds can be compared file by file."""
+    import torch
+    d.mkdir(parents=True, exist_ok=True)
+    rng = np.random.default_rng(seed)
+    n_ch = len(batch.chan_n)
+    for r in np.sort(rng.choice(n_ch, size=min(n_channels, n_ch), replace=False)):
+        off, cnt = int(batch.chan_off[r]), int(batch.chan_n[r])
+        np.save(d / f'ch{r:05d}.npy', out[off:off + cnt].cpu().numpy())
+    pos = np.sort(rng.integers(0, out.numel(), size=min(n_scattered, out.numel())))
+    np.save(d / 'scattered.npy', out[torch.from_numpy(pos).to(out.device)].cpu().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
@@ -254,7 +271,11 @@ def main():
     ap.add_argument('--no-cpu', action='store_true')
     ap.add_argument('--no-extras', action='store_true', help='skip configs / pipeline_cfg4 / fp32 / calibration (N = 1 sections)')
     ap.add_argument('--quick', action='store_true', help='extras at reduced size (smoke runs)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write a fixed, seeded sample of the last timed step\'s output to DIR/*.npy (rank 0)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get('RANK', '0'))
@@ -351,6 +372,8 @@ def main():
     per_launch_ms = [ev[k].elapsed_time(ev[k + 1]) for k in range(args.steps)]
     launches = prog.launch_count - launches0
     n_kernel_clock = len(clock_lines)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(Path(args.dump_outputs), out, batch)
 
     # ---- in-run parity (BASELINE.md 4.3): rows of THIS step's output against the reference evaluator
     parity = None

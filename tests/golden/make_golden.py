@@ -7,13 +7,14 @@ into this repository).  Run:
 
     python oracle/build_ref.py && python tests/golden/make_golden.py
 
-Output (committed): tests/golden/sampling.pkl  — per case: the reference object's
+Output (committed): tests/golden/sampling.pkl.gz  — per case: the reference object's
 wire format (``tolist()``), the grid, and the reference's sampled output;
 tests/golden/dsp.pkl — distortion.py vectors (parity of that module is unpinned
 by the reference's own tests, SURVEY §4, so these are the only pins).
 """
 from __future__ import annotations
 
+import gzip
 import os
 import pickle
 import shutil
@@ -69,7 +70,8 @@ def main():
         out[name] = rec
         print(f'{name:28s} {rec["kind"]:9s} n={len(rec["expect"]):6d} '
               f'dtype={rec["expect"].dtype} max|y|={np.abs(rec["expect"]).max():.4g}')
-    with open(HERE / 'sampling.pkl', 'wb') as f:
+    # gzip keeps the file under 1 MB; mtime=0 makes the same vectors give the same bytes
+    with gzip.GzipFile(HERE / 'sampling.pkl.gz', 'wb', compresslevel=9, mtime=0) as f:
         pickle.dump({'reference_version': ref.__version__,
                      'numpy': np.__version__, 'cases': out}, f, protocol=4)
 

@@ -2,6 +2,7 @@
 record, and evaluation of the same record through waveforms_b200 (CUDA)."""
 from __future__ import annotations
 
+import gzip
 import pickle
 import types
 import warnings
@@ -16,7 +17,7 @@ FP32_TOL = 1e-6   # 1e-6 (fp32)
 
 
 def load_golden():
-    with open(GOLDEN / 'sampling.pkl', 'rb') as f:
+    with gzip.open(GOLDEN / 'sampling.pkl.gz', 'rb') as f:
         return pickle.load(f)['cases']
 
 

@@ -1,5 +1,5 @@
 """Full-size units of every BASELINE.json config against the reference's own compiled
-evaluator (oracle/_ref; the oracle port where the reference is Python: multi-DRAG ids
+evaluator (oracle/_ref, else the oracle port; the oracle port where the reference is Python: multi-DRAG ids
 16 / 17, scipy / numpy for the DSP stages), fp64 1e-12 and fp32 1e-6 (VERDICT r1, item 1;
 reference: waveforms/waveform.py:173-207, distortion.py:213-223, :289-337)."""
 import warnings
@@ -23,10 +23,10 @@ def pair_small_batches(monkeypatch):
 
 @pytest.fixture(scope='module')
 def X():
+    """cpu_sample() evaluates with the reference's compiled evaluator when oracle/_ref holds it and
+    with the oracle port otherwise; the port is pinned to the reference's stored outputs
+    (tests/test_oracle_golden.py), so a checkout without the reference still runs these tests."""
     from tools import bench_extras
-    calc, kind = bench_extras.ref_calc()
-    if calc is None:
-        pytest.skip('oracle/_ref is not built')
     return bench_extras
 
 
