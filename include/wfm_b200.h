@@ -262,7 +262,7 @@ int  wfm_sample_host(wfm_program_t prog, const WfmLaunch* launch);
  * [n_sig][n_sections][2] initial / final states (either may be NULL: zero
  * initial state / final state not returned; a non-NULL zf makes the call
  * synchronous).
- *   WFM_IIR_EXACT  one thread per signal, sequential in time: bit-identical to
+ *   WFM_IIR_EXACT  one warp per signal, sequential in time: bit-identical to
  *                  scipy (parallelism = n_sig).
  *   WFM_IIR_SCAN   block-parallel associative scan over time (one CTA per
  *                  signal, 4096-sample tiles): the throughput path; equals the
@@ -277,16 +277,18 @@ int  wfm_sosfilt(const double* sos, int32_t n_sections, double initial,
 
 /* scipy.signal.lfilter(b, a, x, zi=zi) — one direct-form-II-transposed section of
  * order max(nb, na) - 1 <= 16 (distortion.py:321, the polynomial products built by
- * combine_filters).  One thread per signal, sequential in time, bit-identical to
- * scipy.  b, a, zi, zf are HOST arrays (zi/zf: [n_sig][order], may be NULL). */
+ * combine_filters).  One warp per signal, sequential in time, bit-identical to
+ * scipy.  b, a, zi, zf are HOST arrays (zi/zf: [n_sig][order], may be NULL; a
+ * non-NULL zf makes the call synchronous). */
 int  wfm_lfilter(const double* b, int32_t nb, const double* a, int32_t na,
                  const double* x, double* y, int64_t n_sig, int64_t n,
                  int64_t stride, const double* zi, double* zf, void* stream);
 
-/* The same with a mode: WFM_IIR_EXACT = wfm_lfilter; WFM_IIR_SCAN = block-parallel (orders 1..4: the DF2T state is a
- * linear system, carries by M x M matrix powers, the samples themselves by scipy's own recurrence from the carried-in
- * state) — equal to the sequential result up to the filter's rounding-noise gain, at the cost of a read and a write
- * (cfg4: 13.4 ms -> 0.3 ms).  Orders above 4 run the sequential kernel whatever the mode. */
+/* The same with a mode: WFM_IIR_EXACT = wfm_lfilter; WFM_IIR_SCAN = block-parallel, the scan kernel of wfm_sosfilt
+ * (orders 1..4: the DF2T state is a linear system, carries by M x M matrix powers, the samples themselves by scipy's
+ * own recurrence from the carried-in state) — equal to the sequential result up to the filter's rounding-noise gain,
+ * at the cost of a read and a write (cfg4: 13.4 ms -> 0.3 ms).  Orders above 4 and order 0 run the sequential kernel
+ * whatever the mode. */
 int  wfm_lfilter_mode(const double* b, int32_t nb, const double* a, int32_t na,
                       const double* x, double* y, int64_t n_sig, int64_t n,
                       int64_t stride, const double* zi, double* zf, int32_t mode, void* stream);

@@ -237,6 +237,14 @@ def test_lfilter_scan_on_unaligned_rows_and_high_orders():
     want = lfilter(b, a, x.cpu().numpy(), axis=-1)
     y, _ = lfilter_device(b, a, x, mode='scan')
     assert rel_err(y.cpu().numpy(), want) <= FP64_TOL
+    # sosfilt's scan runs the same kernel: the same odd-offset rows, 1 and 2 sections in one launch, 3 as a chain
+    from waveforms_b200.dsp import sosfilt_device
+    for nsec, initial in ((1, 0.0), (2, 0.0), (3, 0.0), (2, 0.3), (3, 0.3)):
+        sos = tf2sos(*butter(2 * nsec, 0.3))
+        xs = base.clone()[1:].view(3, 5001)
+        want = sosfilt(sos, xs.cpu().numpy() - initial, axis=-1) + initial
+        y, _ = sosfilt_device(sos, xs, initial=initial, mode='scan')
+        assert rel_err(y.cpu().numpy(), want) <= FP64_TOL, (nsec, initial)
     b6, a6 = butter(6, 0.25)             # order 6: no scan kernel, the sequential one answers (bit-identical)
     x6 = rng.standard_normal((2, 3000))
     y6, _ = lfilter_device(b6, a6, _dev(x6), mode='scan')
@@ -299,6 +307,12 @@ def test_lfilter_scan_degenerate_inputs():
     zi = np.array([[0.3, -0.1]])
     y, zf = lfilter_device(b, a, torch.zeros(1, 0, dtype=torch.float64, device='cuda'), zi=zi, want_zf=True, mode='scan')
     assert y.shape == (1, 0) and np.array_equal(zf, zi)
+    from waveforms_b200.dsp import sosfilt_device
+    sos = tf2sos(*butter(4, 0.2))
+    szi = np.array([[[0.3, -0.1], [0.2, 0.05]]])
+    for mode in ('exact', 'scan'):
+        y, zf = sosfilt_device(sos, torch.zeros(1, 0, dtype=torch.float64, device='cuda'), zi=szi, want_zf=True, mode=mode)
+        assert y.shape == (1, 0) and np.array_equal(zf, szi), mode
     x = np.linspace(-1, 1, 1000)
     y, _ = lfilter_device([2.5], [1.0], _dev(x), mode='scan')
     assert np.array_equal(y.cpu().numpy(), lfilter([2.5], [1.0], x))

@@ -12,12 +12,12 @@ python tools/bench_dsp.py --cpu > $o/${tag}_dsp_cfg4.json 2> $o/${tag}_dsp.err
 # launch lists (cold-cache, serialised: shares of the step, not absolute times)
 ncu --metrics gpu__time_duration.sum --clock-control none -c 600 --csv --log-file $o/${tag}_launches_bench.csv \
     python bench.py --steps 2 --warmup 3 --no-cpu --no-e2e > /dev/null 2>&1
-# full captures: K1 sparse (one launch of the bench kernel, 16 frames), K1 dense (cfg3), K2 joint scan, K3 passes
+# full captures: K1 sparse (one launch of the bench kernel, 16 frames), K1 dense (cfg3), K2 scan, K3 passes
 ncu --set full --clock-control none --import-source on -k regex:sample_kernel -s 3 -c 1 -o $o/${tag}_k1_cfg2 \
     python bench.py --steps 2 --warmup 3 --frames 16 --no-cpu --no-e2e --no-extras > /dev/null 2>&1
 ncu --set full --clock-control none --import-source on -k regex:sample_dense -s 2 -c 1 -o $o/${tag}_k1_cfg3 \
     python tools/bench_configs.py --only cfg3 --reps 2 > /dev/null 2>&1
-ncu --set full --clock-control none --import-source on -k regex:'fft_|sosfilt_scan|lfilter_scan' -s 4 -c 5 -o $o/${tag}_dsp \
+ncu --set full --clock-control none --import-source on -k regex:'fft_|iir_scan' -s 4 -c 5 -o $o/${tag}_dsp \
     python tools/bench_dsp.py --reps 1 > /dev/null 2>&1
 # the reports stay on the box (gpurun returns at most 64 MiB): keep their text pages
 for r in k1_cfg2 k1_cfg3 dsp; do

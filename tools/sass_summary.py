@@ -63,7 +63,8 @@ def main():
     print('# columns: registers, stack bytes, static shared bytes, SASS instructions, then mnemonic counts (static, per kernel)')
     hot = re.compile(r'sample_kernel<double, false, 1, 4, false, false>|sample_kernel<double, false, 2, 4, (true|false), false>'
                      r'|sample_kernel<float, false, 1, 0, false, (true|false)>|sample_dense_kernel<double, false, 4, (true|false), false>'
-                     r'|sample_dense_kernel<float, false, 4, true, (true|false)>|sosfilt_scan_joint_kernel<2, true>|sosfilt_scan_kernel'
+                     r'|sample_dense_kernel<float, false, 4, true, (true|false)>|iir_scan_kernel<wfm::BiquadForm<2>, true>'
+                     r'|iir_scan_kernel<wfm::DirectForm<2>, true>'
                      r'|sosfilt_exact|lfilter_exact|fft_cols_kernel|fft_rows_kernel<true>|fft_filter_single|prepare_|fill_packets'
                      r'|dfma_kernel|reflection_response')
     for n in names:
@@ -72,7 +73,7 @@ def main():
             continue
         reg, stack, shared, local = usage[n]
         c = counts.get(n, {})
-        short = re.sub(r'\(wfm::DevProgram.*|\(wfm::FftPlan.*|\(wfm::IirParams.*', '', d).replace('void ', '')
+        short = re.sub(r'\(wfm::DevProgram.*|\(wfm::FftPlan.*|\(wfm::IirParams.*|\(wfm::LfilterParams.*|\(wfm::\w+<\d+>::Params.*', '', d).replace('void ', '')
         print('%-110s reg %3d stack %4d smem %6d inst %6d  %s' % (short[:110], reg, stack, shared, size.get(n, 0),
               ' '.join('%s=%d' % (k, c[k]) for k in MNEMONICS if c.get(k))))
     print('# %d kernels in the library; --all lists every template instantiation' % len(names))

@@ -1,5 +1,8 @@
-import sys, numpy as np, torch
-sys.path.insert(0, '/root/repo')
+import sys
+from pathlib import Path
+
+import numpy as np, torch
+sys.path.insert(0, str(Path(__file__).resolve().parent.parent))
 from scipy.signal import butter, tf2sos
 from waveforms_b200.dsp import sosfilt_device
 x = torch.randn(256, 400000, dtype=torch.float64, device='cuda')

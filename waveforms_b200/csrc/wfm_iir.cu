@@ -1,62 +1,45 @@
-// wfm_iir.cu — K2: cascaded-biquad IIR, scipy.signal.sosfilt semantics.
+// wfm_iir.cu — K2: IIR filters with the semantics of scipy.signal.sosfilt and scipy.signal.lfilter.
 //
-// Replaces the sosfilt call sites /root/reference/waveforms/waveform.py:200-203,
-// :249 and (through first/second-order sections) lfilter in
-// /root/reference/waveforms/distortion.py:321.  Per section, direct form II
-// transposed, exactly the recurrence scipy runs (scipy/signal/_sosfilt.pyx):
+// Replaces the sosfilt call sites of the reference's waveforms/waveform.py:200-203 and :249 and the lfilter of its
+// waveforms/distortion.py:321.  Per biquad section, direct form II transposed, exactly the recurrence scipy runs
+// (scipy/signal/_sosfilt.pyx):
 //     y  = b0*x + z0
 //     z0 = b1*x - a1*y + z1
 //     z1 = b2*x - a2*y
-// with every product and sum rounded separately (no FMA; built with -fmad=false
-// and written with __dmul_rn/__dadd_rn).
+// and for lfilter scipy's direct-form loop (lfilter_step below), with every product and sum rounded separately
+// (no FMA; built with -fmad=false and written with __dmul_rn/__dadd_rn).
 //
-// Two kernels:
+// Three kernels:
 //
-//  * WFM_IIR_EXACT — one thread per signal walks time sequentially with the
-//    recurrence above.  Bit-identical to scipy.  Parallelism = n_sig.
+//  * sosfilt_exact_kernel, lfilter_exact_kernel (WFM_IIR_EXACT) — one warp per signal walks time sequentially with
+//    scipy's recurrence.  Bit-identical to scipy.
 //
-//  * WFM_IIR_SCAN — block-parallel associative scan.  One CTA per signal walks
-//    4096-sample tiles; inside a tile each of 256 threads owns 16 consecutive
-//    samples.  The biquad is the affine map z' = A z + B x, A = [[-a1,1],[-a2,0]]
-//    on its state z = (z0, z1); because A is the same for every sample, the scan
-//    over thread chunks only has to carry 2-vectors and uses the precomputed
-//    powers A^(16*2^d):
-//       pass a: every thread runs its chunk from the zero state -> f_i
-//               (thread 0 starts from the tile's carry-in state);
-//       scan  : E_i = sum_{j<i} A^(16 (i-1-j)) f_j  (warp shuffles, then 8 warp
-//               totals through shared memory);
-//       pass c: every thread re-runs its chunk from E_i with the faithful
-//               recurrence and writes y.
-//    Cascaded sections are processed one after the other on the register-resident
-//    tile.  The result differs from the sequential one only through the rounding
-//    of the carried states: ~1e-16 * (filter noise gain).  For poles within 5e-3
-//    of the unit circle (the exp-decay predistortion filters) that noise gain
-//    makes scipy's OWN sequential result uncertain at the 3e-12 level, which no
-//    re-association can track (DESIGN.md §K2); for well-conditioned filters the
-//    two modes agree to ~1e-15.
+//  * iir_scan_kernel<Form, kAligned> (WFM_IIR_SCAN) — block-parallel associative scan, shared by both filters.  Each
+//    is a linear system on its D state words, s' = M s + g x: a cascade of one or two biquads on the joint state of
+//    its sections (BiquadForm, D = 2 S; longer cascades run as a chain of launches) or lfilter's direct form of
+//    order 1..4 (DirectForm, D = M).  One CTA per signal walks 4096-sample tiles; inside a tile each of 256 threads
+//    owns 16 consecutive samples:
+//       pass a: every thread runs its chunk from the zero state in state-space form (one FMA per step on the
+//               critical path) -> its end state f_i (thread 0 starts from the tile's carry-in state);
+//       scan  : E_i = sum_{j<i} (M^16)^(i-1-j) f_j  (warp shuffles, then 8 warp totals through shared memory; the
+//               D x D powers of M^16 come from the host, computed in long double);
+//       pass c: every thread re-runs its chunk from E_i with scipy's own recurrence and writes y.
+//    The result differs from the sequential one only through the rounding of the carried states: ~1e-16 * (filter
+//    noise gain).  For poles within 5e-3 of the unit circle (the exp-decay predistortion filters) that noise gain
+//    makes scipy's OWN sequential result uncertain at the 3e-12 level, which no re-association can track
+//    (DESIGN.md §K2); for well-conditioned filters the two modes agree to ~1e-15.
 #include <cuda_runtime.h>
 #include <algorithm>
-#include <cstdlib>
 #include <cstring>
-#include <vector>
 #include "wfm_internal.h"
 #include "wfm_math.cuh"
 
 namespace wfm {
 
-#ifndef WFM_IIR_THREADS
-#define WFM_IIR_THREADS 256
-#endif
-#ifndef WFM_IIR_T
-#define WFM_IIR_T 16
-#endif
-#ifndef WFM_IIR_MINB
-#define WFM_IIR_MINB 2
-#endif
-constexpr int kIirThreads = WFM_IIR_THREADS;
-constexpr int kIirT = WFM_IIR_T;                   // samples per thread per tile
+constexpr int kIirThreads = 256;
+constexpr int kIirT = 16;                          // samples per thread per tile
 constexpr int kIirTile = kIirThreads * kIirT;      // 4096
-constexpr int kIirRow = kIirT + 1;                 // padded smem row (bank spread)
+constexpr int kIirMinBlocks = 2;                   // CTAs per SM the scan kernel is compiled for
 constexpr int kMaxSections = 8;
 
 struct Biquad {
@@ -65,16 +48,9 @@ struct Biquad {
 
 struct IirParams {
   int n_sections;
-  int shift_in, shift_out;  // joint scan only: subtract `initial` at the input / add it at the output of THIS launch
+  int shift_in, shift_out;  // scan only: subtract `initial` at the input / add it at the output of THIS launch
   double initial;
   Biquad sec[kMaxSections];
-};
-
-// powers of A used by the scan, per section; 2x2 row-major
-struct IirScanTables {
-  double lane[kMaxSections][32][4];  // A^(T*l), l = 0..31
-  double lvl[kMaxSections][5][4];    // A^(T*2^d), d = 0..4
-  double warp[kMaxSections][4];      // A^(T*32)
 };
 
 __device__ __forceinline__ void biquad_step(const Biquad& q, double x, double& z0, double& z1, double& y) {
@@ -177,428 +153,21 @@ __global__ void __launch_bounds__(32 * kExactWarps) sosfilt_exact_kernel(const _
 }
 
 // ---------------------------------------------------------------------------
-// scan: one CTA per signal, tiles of 4096 samples
-// ---------------------------------------------------------------------------
-__device__ __forceinline__ void matvec(const double* __restrict__ M, double a, double b, double& ra, double& rb) {
-  ra = fma(M[0], a, M[1] * b);
-  rb = fma(M[2], a, M[3] * b);
-}
-
-__global__ void __launch_bounds__(kIirThreads, WFM_IIR_MINB) sosfilt_scan_kernel(const __grid_constant__ IirParams P,
-                                                                        const __grid_constant__ IirScanTables TT,
-                                                                        const double* __restrict__ x, double* y,
-                                                                     int64_t n, int64_t stride,
-                                                                     const double* __restrict__ zi,
-                                                                     double* __restrict__ zf) {
-  const IirScanTables* __restrict__ T = &TT;  // ~10 KB of kernel parameters (constant bank): no table upload per call
-  __shared__ double s_tile[kIirThreads * kIirRow];
-  __shared__ double s_tot[kIirThreads / 32][2];
-  __shared__ double s_carry[kMaxSections][2];
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int64_t sig = blockIdx.x;
-  const double* __restrict__ xs = x + sig * stride;
-  double* ys = y + sig * stride;
-  const int S = P.n_sections;
-  const bool shift = P.initial != 0.0;
-  if (tid < S) {
-    s_carry[tid][0] = zi ? zi[(sig * S + tid) * 2 + 0] : 0.0;
-    s_carry[tid][1] = zi ? zi[(sig * S + tid) * 2 + 1] : 0.0;
-  }
-  __syncthreads();
-
-  for (int64_t base = 0; base < n; base += kIirTile) {
-    const int cnt = (int)min((int64_t)kIirTile, n - base);
-    // coalesced load -> padded rows (thread r owns row r)
-#pragma unroll
-    for (int k = 0; k < kIirT; ++k) {
-      const int e = k * kIirThreads + tid;
-      double v = 0.0;
-      if (e < cnt) {
-        v = xs[base + e];
-        if (shift) v = sub(v, P.initial);
-      }
-      s_tile[(e / kIirT) * kIirRow + (e % kIirT)] = v;
-    }
-    __syncthreads();
-    double v[kIirT];
-#pragma unroll
-    for (int k = 0; k < kIirT; ++k) v[k] = s_tile[tid * kIirRow + k];
-    const int valid = max(0, min(kIirT, cnt - tid * kIirT));  // my valid samples
-
-    for (int sct = 0; sct < S; ++sct) {
-      const Biquad q = P.sec[sct];
-      const double c0 = s_carry[sct][0], c1 = s_carry[sct][1];
-      // pass a: zero-state response of my chunk (thread 0 carries the tile state)
-      double f0 = tid == 0 ? c0 : 0.0, f1 = tid == 0 ? c1 : 0.0;
-#pragma unroll
-      for (int k = 0; k < kIirT; ++k) {
-        double out;
-        biquad_step(q, v[k], f0, f1, out);
-      }
-      // inclusive warp scan of the affine maps (constant matrix per level)
-#pragma unroll
-      for (int d = 0; d < 5; ++d) {
-        const double p0 = __shfl_up_sync(0xffffffffu, f0, 1 << d);
-        const double p1 = __shfl_up_sync(0xffffffffu, f1, 1 << d);
-        if (lane >= (1 << d)) {
-          double r0, r1;
-          matvec(T->lvl[sct][d], p0, p1, r0, r1);
-          f0 += r0;
-          f1 += r1;
-        }
-      }
-      if (lane == 31) {
-        s_tot[warp][0] = f0;
-        s_tot[warp][1] = f1;
-      }
-      // state entering my chunk from the lanes before me in this warp
-      double e0 = __shfl_up_sync(0xffffffffu, f0, 1);
-      double e1 = __shfl_up_sync(0xffffffffu, f1, 1);
-      if (lane == 0) e0 = e1 = 0.0;
-      __syncthreads();
-      // carry entering my warp: C_w = Q C_{w-1} + tot_{w-1}
-      double w0 = 0.0, w1 = 0.0;
-      for (int k = 0; k < warp; ++k) {
-        double r0, r1;
-        matvec(T->warp[sct], w0, w1, r0, r1);
-        w0 = r0 + s_tot[k][0];
-        w1 = r1 + s_tot[k][1];
-      }
-      if (warp > 0) {
-        double r0, r1;
-        matvec(T->lane[sct][lane], w0, w1, r0, r1);
-        e0 += r0;
-        e1 += r1;
-      }
-      if (tid == 0) { e0 = c0; e1 = c1; }
-      // pass c: faithful recurrence from the carried-in state
-      double z0 = e0, z1 = e1;
-#pragma unroll
-      for (int k = 0; k < kIirT; ++k) {
-        if (k == valid && valid < kIirT && (tid * kIirT + k == cnt)) {
-          // first padded sample of the signal's tail: this is the final state
-          s_carry[sct][0] = z0;
-          s_carry[sct][1] = z1;
-        }
-        double out;
-        biquad_step(q, v[k], z0, z1, out);
-        v[k] = out;
-      }
-      __syncthreads();  // all reads of s_carry/s_tot for this section are done
-      if (cnt == kIirTile && tid == kIirThreads - 1) {
-        s_carry[sct][0] = z0;
-        s_carry[sct][1] = z1;
-      }
-      __syncthreads();
-    }
-    // registers -> padded rows -> coalesced store
-#pragma unroll
-    for (int k = 0; k < kIirT; ++k) s_tile[tid * kIirRow + k] = v[k];
-    __syncthreads();
-#pragma unroll
-    for (int k = 0; k < kIirT; ++k) {
-      const int e = k * kIirThreads + tid;
-      if (e < cnt) {
-        double o = s_tile[(e / kIirT) * kIirRow + (e % kIirT)];
-        ys[base + e] = shift ? add(o, P.initial) : o;
-      }
-    }
-    __syncthreads();
-  }
-  if (zf && tid < S) {
-    zf[(sig * S + tid) * 2 + 0] = s_carry[tid][0];
-    zf[(sig * S + tid) * 2 + 1] = s_carry[tid][1];
-  }
-}
-
-// ---------------------------------------------------------------------------
-// scan, all sections at once (S <= 2): the cascade is ONE linear system on the joint state
-// s = (z0, z1) of every section (D = 2S components): s' = M s + g x.  Per tile
-//   pass a: every thread runs its 16 samples from the zero state in the STATE-SPACE form
-//           z0' = -a1 z0 + (z1 + c1 x), z1' = -a2 z0 + c2 x  (c1 = b1 - a1 b0, c2 = b2 - a2 b0):
-//           one FMA per step on the critical path instead of the four dependent operations of
-//           the faithful recurrence; only the chunk's END state f_i leaves this pass, and f_i
-//           only feeds the carries, whose rounding is the same noise as before;
-//   scan  : E_i = sum_{j<i} (M^16)^(i-1-j) f_j with D x D powers of M^16 (host, long double);
-//           the per-lane powers sit in shared memory;
-//   pass c: the FAITHFUL recurrence from E_i, the sections software-pipelined (section 1 of
-//           sample k+1 next to section 2 of sample k: two independent chains).
-// One scan and two passes per tile instead of two scans and four passes, and a shorter chain
-// in pass a: 0.63 -> ~0.3 ms on cfg4 (256 x 400 000 samples; its two exponential decays make ONE biquad section; a
-// two-section cascade of the same size takes 0.50 ms).
-// ---------------------------------------------------------------------------
-constexpr int kMaxJoint = 4;  // D = 2 S, S <= 2
-struct IirJointTables {
-  double lane[32][kMaxJoint * kMaxJoint];  // (M^16)^l, l = 0..31, row-major D x D
-  double lvl[5][kMaxJoint * kMaxJoint];    // (M^16)^(2^d)
-  double warp[kMaxJoint * kMaxJoint];      // (M^16)^32
-  double c1[2], c2[2];                     // state-space input gains per section
-};
-
-template <int D>
-__device__ __forceinline__ void matvec_d(const double* __restrict__ M, const double (&a)[D], double (&r)[D]) {
-#pragma unroll
-  for (int i = 0; i < D; ++i) {
-    double acc = M[i * D] * a[0];
-#pragma unroll
-    for (int j = 1; j < D; ++j) acc = fma(M[i * D + j], a[j], acc);
-    r[i] = acc;
-  }
-}
-
-// Tile staging of the joint kernel: rows of 16 samples at a pitch of 18 doubles (144 B): thread r reads / writes its
-// row with 16-byte accesses without bank conflicts, and 16-byte chunks stay aligned for cp.async.  Two buffers: the
-// NEXT tile is already on its way (cp.async, no registers held) while this one is filtered — the one-buffer kernel
-// spent three quarters of its time waiting for its own loads (ncu: long-scoreboard stalls on the first use of every
-// loaded sample).
-constexpr int kJointPitch = kIirT + 2;                                       // doubles per staged row
-constexpr int kJointTileBytes = kIirThreads * kJointPitch * (int)sizeof(double);  // 36 864
-extern __shared__ __align__(16) unsigned char iir_smem[];
-
-__device__ __forceinline__ void cp_async16_zfill(void* dst_smem, const void* src, int src_bytes) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"((uint32_t)__cvta_generic_to_shared(dst_smem)), "l"(src),
-               "r"(src_bytes)
-               : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-
-// kAligned: x and y rows start on 16-byte boundaries (cp.async loads, 16-byte stores); else plain 8-byte accesses
-template <int S, bool kAligned>
-__global__ void __launch_bounds__(kIirThreads, WFM_IIR_MINB) sosfilt_scan_joint_kernel(
-    const __grid_constant__ IirParams P, const __grid_constant__ IirJointTables TT, const double* __restrict__ x, double* y,
-    int64_t n, int64_t stride, const double* __restrict__ zi, double* __restrict__ zf, int zs) {
-  // zs: state words between two signals in zi / zf (2 x the sections of the WHOLE cascade: a long cascade runs as a chain
-  // of launches over its sections two by two, each on its slice of the states)
-  constexpr int D = 2 * S;
-  double* s_buf0 = reinterpret_cast<double*>(iir_smem);
-  double* s_buf1 = reinterpret_cast<double*>(iir_smem + kJointTileBytes);
-  __shared__ double s_lane[D * D][32];  // (M^16)^lane, entry-major: conflict-free
-  __shared__ double s_tot[kIirThreads / 32][D];
-  __shared__ double s_carry[D];
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int64_t sig = blockIdx.x;
-  const double* __restrict__ xs = x + sig * stride;
-  double* ys = y + sig * stride;
-  const bool shift_in = P.initial != 0.0 && P.shift_in, shift_out = P.initial != 0.0 && P.shift_out;
-  for (int e = tid; e < D * D * 32; e += kIirThreads) s_lane[e / 32][e % 32] = TT.lane[e % 32][(e / 32) / D * kMaxJoint + (e / 32) % D];
-  if (tid < D) s_carry[tid] = zi ? zi[sig * zs + tid] : 0.0;  // zi[sig][section][2] is the joint state in order
-  Biquad q[S];
-  double c1[S], c2[S];
-#pragma unroll
-  for (int k = 0; k < S; ++k) {
-    q[k] = P.sec[k];
-    c1[k] = TT.c1[k];
-    c2[k] = TT.c2[k];
-  }
-
-  // tile `base` -> buffer: 2048 chunks of two samples, chunk c of the tile at row c / 8, column 2 (c % 8)
-  auto load_tile = [&](double* buf, int64_t base) {
-    const int cnt = (int)min((int64_t)kIirTile, n - base);
-#pragma unroll
-    for (int j = 0; j < kIirT / 2; ++j) {
-      const int c = j * kIirThreads + tid;
-      double* dst = buf + (c >> 3) * kJointPitch + 2 * (c & 7);
-      if (kAligned) {
-        const int left = cnt - 2 * c;  // samples of this chunk that exist: the rest is zero-filled
-        cp_async16_zfill(dst, left > 0 ? xs + base + 2 * c : xs + base, left >= 2 ? 16 : (left == 1 ? 8 : 0));
-      } else {
-        dst[0] = 2 * c < cnt ? xs[base + 2 * c] : 0.0;
-        dst[1] = 2 * c + 1 < cnt ? xs[base + 2 * c + 1] : 0.0;
-      }
-    }
-  };
-  if (n > 0) load_tile(s_buf0, 0);
-  if (kAligned) cp_async_commit();
-  __syncthreads();
-
-  int it = 0;
-  for (int64_t base = 0; base < n; base += kIirTile, ++it) {
-    const int cnt = (int)min((int64_t)kIirTile, n - base);
-    double* buf = (it & 1) ? s_buf1 : s_buf0;
-    if (base + kIirTile < n) load_tile((it & 1) ? s_buf0 : s_buf1, base + kIirTile);
-    if (kAligned) {
-      cp_async_commit();
-      cp_async_wait<1>();  // everything but the tile just requested has landed
-    }
-    __syncthreads();
-    double v[kIirT];
-    {
-      const double2* row = reinterpret_cast<const double2*>(buf + tid * kJointPitch);
-#pragma unroll
-      for (int k = 0; k < kIirT / 2; ++k) {
-        const double2 d = row[k];
-        v[2 * k] = d.x;
-        v[2 * k + 1] = d.y;
-      }
-    }
-    const int valid = max(0, min(kIirT, cnt - tid * kIirT));  // my valid samples
-    if (shift_in) {
-#pragma unroll
-      for (int k = 0; k < kIirT; ++k) v[k] = k < valid ? sub(v[k], P.initial) : 0.0;
-    }
-
-    double carry[D];
-#pragma unroll
-    for (int i = 0; i < D; ++i) carry[i] = s_carry[i];
-    // ---- pass a: end state of my chunk from the zero state (thread 0: from the tile's carry-in), state-space form
-    double f[D];
-#pragma unroll
-    for (int i = 0; i < D; ++i) f[i] = tid == 0 ? carry[i] : 0.0;
-#pragma unroll
-    for (int k = 0; k < kIirT; ++k) {
-      double in = v[k];
-#pragma unroll
-      for (int sct = 0; sct < S; ++sct) {
-        const double z0 = f[2 * sct], z1 = f[2 * sct + 1];
-        const double out = fma(q[sct].b0, in, z0);
-        f[2 * sct] = fma(-q[sct].a1, z0, fma(c1[sct], in, z1));
-        f[2 * sct + 1] = fma(-q[sct].a2, z0, c2[sct] * in);
-        in = out;
-      }
-    }
-    // ---- scan over the threads: inclusive warp scan with constant matrices per level
-#pragma unroll
-    for (int d = 0; d < 5; ++d) {
-      double p[D], r[D];
-#pragma unroll
-      for (int i = 0; i < D; ++i) p[i] = __shfl_up_sync(0xffffffffu, f[i], 1 << d);
-      if (lane >= (1 << d)) {
-        double m[D * D];
-#pragma unroll
-        for (int i = 0; i < D; ++i)
-#pragma unroll
-          for (int j = 0; j < D; ++j) m[i * D + j] = TT.lvl[d][i * kMaxJoint + j];
-        matvec_d<D>(m, p, r);
-#pragma unroll
-        for (int i = 0; i < D; ++i) f[i] += r[i];
-      }
-    }
-    if (lane == 31) {
-#pragma unroll
-      for (int i = 0; i < D; ++i) s_tot[warp][i] = f[i];
-    }
-    double e[D];
-#pragma unroll
-    for (int i = 0; i < D; ++i) {
-      e[i] = __shfl_up_sync(0xffffffffu, f[i], 1);
-      if (lane == 0) e[i] = 0.0;
-    }
-    __syncthreads();
-    // carry entering my warp: C_w = Q C_{w-1} + tot_{w-1}, Q = (M^16)^32
-    if (warp > 0) {
-      double w[D], r[D], mq[D * D];
-#pragma unroll
-      for (int i = 0; i < D; ++i) w[i] = 0.0;
-#pragma unroll
-      for (int i = 0; i < D; ++i)
-#pragma unroll
-        for (int j = 0; j < D; ++j) mq[i * D + j] = TT.warp[i * kMaxJoint + j];
-      for (int k = 0; k < warp; ++k) {
-        matvec_d<D>(mq, w, r);
-#pragma unroll
-        for (int i = 0; i < D; ++i) w[i] = r[i] + s_tot[k][i];
-      }
-      double ml[D * D];
-#pragma unroll
-      for (int i = 0; i < D * D; ++i) ml[i] = s_lane[i][lane];
-      matvec_d<D>(ml, w, r);
-#pragma unroll
-      for (int i = 0; i < D; ++i) e[i] += r[i];
-    }
-    if (tid == 0) {
-#pragma unroll
-      for (int i = 0; i < D; ++i) e[i] = carry[i];
-    }
-    // ---- pass c: the faithful recurrence from the carried-in state; section 2 runs one sample behind section 1
-    double z[D];
-#pragma unroll
-    for (int i = 0; i < D; ++i) z[i] = e[i];
-    const bool tail_here = valid < kIirT && tid * kIirT + valid == cnt;  // the signal ends inside my chunk
-    double fin[D];
-#pragma unroll
-    for (int i = 0; i < D; ++i) fin[i] = 0.0;
-    if (S == 1) {
-#pragma unroll
-      for (int k = 0; k < kIirT; ++k) {
-        if (tail_here && k == valid) { fin[0] = z[0]; fin[1] = z[1]; }
-        double out;
-        biquad_step(q[0], v[k], z[0], z[1], out);
-        v[k] = out;
-      }
-    } else {
-      double o1_prev;
-      {
-        if (tail_here && valid == 0) { fin[0] = z[0]; fin[1] = z[1]; }
-        biquad_step(q[0], v[0], z[0], z[1], o1_prev);
-      }
-#pragma unroll
-      for (int k = 1; k <= kIirT; ++k) {
-        double o1 = 0.0, o2;
-        if (k < kIirT) {
-          if (tail_here && k == valid) { fin[0] = z[0]; fin[1] = z[1]; }
-          biquad_step(q[0], v[k], z[0], z[1], o1);
-        }
-        if (tail_here && k - 1 == valid) { fin[2 % D] = z[2 % D]; fin[3 % D] = z[3 % D]; }
-        biquad_step(q[S - 1], o1_prev, z[2 % D], z[3 % D], o2);
-        v[k - 1] = o2;
-        o1_prev = o1;
-      }
-    }
-    if (shift_out) {
-#pragma unroll
-      for (int k = 0; k < kIirT; ++k) v[k] = add(v[k], P.initial);
-    }
-    // my row back into the buffer (nobody else reads it before the barrier), then coalesced 16-byte stores
-    {
-      double2* row = reinterpret_cast<double2*>(buf + tid * kJointPitch);
-#pragma unroll
-      for (int k = 0; k < kIirT / 2; ++k) row[k] = make_double2(v[2 * k], v[2 * k + 1]);
-    }
-    __syncthreads();  // rows complete; all reads of s_carry / s_tot are done
-    if (tail_here) {
-#pragma unroll
-      for (int i = 0; i < D; ++i) s_carry[i] = fin[i];
-    }
-    if (cnt == kIirTile && tid == kIirThreads - 1) {
-#pragma unroll
-      for (int i = 0; i < D; ++i) s_carry[i] = z[i];
-    }
-#pragma unroll
-    for (int j = 0; j < kIirT / 2; ++j) {
-      const int c = j * kIirThreads + tid;
-      const double2 d = *reinterpret_cast<const double2*>(buf + (c >> 3) * kJointPitch + 2 * (c & 7));
-      if (kAligned && 2 * c + 1 < cnt) {
-        *reinterpret_cast<double2*>(ys + base + 2 * c) = d;
-      } else {
-        if (2 * c < cnt) ys[base + 2 * c] = d.x;
-        if (2 * c + 1 < cnt) ys[base + 2 * c + 1] = d.y;
-      }
-    }
-    __syncthreads();  // the buffer may be refilled (tile t + 2) and s_carry read (tile t + 1)
-  }
-  if (kAligned) cp_async_wait<0>();
-  if (zf && tid < D) zf[sig * zs + tid] = s_carry[tid];
-}
-
-// ---------------------------------------------------------------------------
 // lfilter: single high-order section, scipy.signal.lfilter's DF2T loop
 // (scipy/signal/_lfilter.c.src): y = z[0] + b[0]*x;
 // z[k] = (z[k+1] + x*b[k+1]) - y*a[k+1];  z[M-1] = x*b[M] - y*a[M].
-// One thread per signal, sequential in time, bit-faithful (note the different
-// association from sosfilt's (b1*x - a1*y) + z1).
+// Bit-faithful (note the different association from sosfilt's (b1*x - a1*y) + z1).
 // ---------------------------------------------------------------------------
 constexpr int kMaxOrder = 16;
 struct LfilterParams {
   int order;  // M = max(len(a), len(b)) - 1
-  double b[kMaxOrder + 1];
+  double b[kMaxOrder + 1];  // normalised by a[0]
   double a[kMaxOrder + 1];
 };
 
-// one lfilter step on the replicated state (M = order)
-template <int M>
-__device__ __forceinline__ double lfilter_step(const LfilterParams& P, double xv, double (&z)[kMaxOrder]) {
+// one lfilter step of order M on the state z[0..M-1] (the exact kernel's replicated state, the scan's chunk state)
+template <int M, int N>
+__device__ __forceinline__ double lfilter_step(const LfilterParams& P, double xv, double (&z)[N]) {
   if (M == 0) return mul(P.b[0], xv);
   const double yv = add(z[0], mul(P.b[0], xv));
 #pragma unroll
@@ -669,36 +238,181 @@ __global__ void __launch_bounds__(32 * kExactWarps) lfilter_exact_kernel(const _
   }
 }
 
-
 // ---------------------------------------------------------------------------
-// lfilter, block-parallel (orders 1..4): the DF2T recurrence above is a linear system on its M state words,
-// z' = A z + g x with A[i][0] = -a[i+1], A[i][i+1] = 1, so the machinery of the joint sosfilt scan applies unchanged:
-//   pass a: every thread runs its 16 samples from the zero state in the state-space form
-//           z_i' = -a_{i+1} z_0 + (z_{i+1} + c_{i+1} x), c_j = b_j - a_j b_0 (one FMA per step on the critical path);
-//   scan  : carries with M x M powers of A^16 (host, long double);
-//   pass c: scipy's own recurrence (lfilter_step: same operations, same association) from the carried-in state.
-// predistort() (distortion.py:289-337) filters every flux channel with ONE combined high-order (b, a): the sequential
-// kernel needs 13.4 ms for cfg4's 256 x 400 000 samples, this one the time of a read and a write.
+// scan: one CTA per signal, tiles of 4096 samples (see the top of the file)
 // ---------------------------------------------------------------------------
-struct LfScanParams {
-  double b[kMaxJoint + 1], a[kMaxJoint + 1], c[kMaxJoint + 1];  // normalised by a[0]; c[j] = b[j] - a[j] b[0]
+constexpr int kMaxJoint = 4;  // largest D: two biquad sections, or lfilter of order 4
+struct IirJointTables {
+  double lane[32][kMaxJoint * kMaxJoint];  // (M^16)^l, l = 0..31, row-major D x D
+  double lvl[5][kMaxJoint * kMaxJoint];    // (M^16)^(2^d)
+  double warp[kMaxJoint * kMaxJoint];      // (M^16)^32
+  double c[kMaxJoint];                     // state-space input gain of every state word (pass a)
 };
-template <int M>
-__device__ __forceinline__ double lfilter_step_scan(const LfScanParams& P, double xv, double (&z)[M]) {
-  const double yv = add(z[0], mul(P.b[0], xv));
+
+template <int D>
+__device__ __forceinline__ void matvec_d(const double* __restrict__ M, const double (&a)[D], double (&r)[D]) {
 #pragma unroll
-  for (int k = 0; k < M - 1; ++k) z[k] = sub(add(z[k + 1], mul(xv, P.b[k + 1])), mul(yv, P.a[k + 1]));
-  z[M - 1] = sub(mul(xv, P.b[M]), mul(yv, P.a[M]));
-  return yv;
+  for (int i = 0; i < D; ++i) {
+    double acc = M[i * D] * a[0];
+#pragma unroll
+    for (int j = 1; j < D; ++j) acc = fma(M[i * D + j], a[j], acc);
+    r[i] = acc;
+  }
 }
-template <int M, bool kAligned>
-__global__ void __launch_bounds__(kIirThreads, WFM_IIR_MINB) lfilter_scan_kernel(
-    const __grid_constant__ LfScanParams P, const __grid_constant__ IirJointTables TT, const double* __restrict__ x, double* y,
-    int64_t n, int64_t stride, const double* __restrict__ zi, double* __restrict__ zf) {
-  constexpr int D = M;
+
+// What the two filters do differently inside the scan kernel, each a small device-side type:
+//   D                          state words per signal;
+//   enter(v, valid), leave(v)  the input / output offset of the chunk's samples;
+//   state_step(x, f)           pass a: one sample through the state-space form, z' = A z + c x (c in the tables);
+//   filter(v, z, ...)          pass c: scipy's recurrence over the chunk from the carried-in state z, in place on v;
+//                              where the signal ends inside the chunk (tail_here) `fin` takes the state at sample
+//                              `valid`, the final state;
+//   state_stride(zs)           state words between two signals in zi / zf: a biquad launch may work on a slice of a
+//                              longer cascade's states (zs), a direct form owns all of its D words (a compile-time
+//                              stride keeps the order-4 kernel clear of spills);
+//   Params                     the kernel parameter block of the coefficients; kMax the largest template argument.
+
+// Cascade of S = 1 or 2 biquads on the joint state (z0, z1) of its sections, D = 2 S.  Section k's state-space step
+// is z0' = -a1 z0 + (z1 + c1 u), z1' = -a2 z0 + c2 u (c1 = b1 - a1 b0, c2 = b2 - a2 b0) on its input u, the output of
+// section k - 1.  Pass c runs the sections software-pipelined: section 1 of sample k+1 next to section 2 of sample k,
+// two independent dependency chains.
+template <int S>
+struct BiquadForm {
+  static constexpr int D = 2 * S, kMax = 2;
+  using Params = IirParams;
+  __device__ static constexpr int state_stride(int zs) { return zs; }
+  Biquad q[S];
+  double c1[S], c2[S];
+  double initial;
+  bool shift_in, shift_out;
+
+  __device__ __forceinline__ BiquadForm(const IirParams& P, const IirJointTables& T)
+      : initial(P.initial), shift_in(P.initial != 0.0 && P.shift_in), shift_out(P.initial != 0.0 && P.shift_out) {
+#pragma unroll
+    for (int k = 0; k < S; ++k) {
+      q[k] = P.sec[k];
+      c1[k] = T.c[2 * k];
+      c2[k] = T.c[2 * k + 1];
+    }
+  }
+  __device__ __forceinline__ void enter(double (&v)[kIirT], int valid) const {
+    if (shift_in) {
+#pragma unroll
+      for (int k = 0; k < kIirT; ++k) v[k] = k < valid ? sub(v[k], initial) : 0.0;
+    }
+  }
+  __device__ __forceinline__ void leave(double (&v)[kIirT]) const {
+    if (shift_out) {
+#pragma unroll
+      for (int k = 0; k < kIirT; ++k) v[k] = add(v[k], initial);
+    }
+  }
+  __device__ __forceinline__ void state_step(double in, double (&f)[D]) const {
+#pragma unroll
+    for (int sct = 0; sct < S; ++sct) {
+      const double z0 = f[2 * sct], z1 = f[2 * sct + 1];
+      const double out = fma(q[sct].b0, in, z0);
+      f[2 * sct] = fma(-q[sct].a1, z0, fma(c1[sct], in, z1));
+      f[2 * sct + 1] = fma(-q[sct].a2, z0, c2[sct] * in);
+      in = out;
+    }
+  }
+  __device__ __forceinline__ void filter(double (&v)[kIirT], double (&z)[D], bool tail_here, int valid,
+                                         double (&fin)[D]) const {
+    if constexpr (S == 1) {
+#pragma unroll
+      for (int k = 0; k < kIirT; ++k) {
+        if (tail_here && k == valid) { fin[0] = z[0]; fin[1] = z[1]; }
+        double out;
+        biquad_step(q[0], v[k], z[0], z[1], out);
+        v[k] = out;
+      }
+    } else {
+      double o1_prev;
+      {
+        if (tail_here && valid == 0) { fin[0] = z[0]; fin[1] = z[1]; }
+        biquad_step(q[0], v[0], z[0], z[1], o1_prev);
+      }
+#pragma unroll
+      for (int k = 1; k <= kIirT; ++k) {
+        double o1 = 0.0, o2;
+        if (k < kIirT) {
+          if (tail_here && k == valid) { fin[0] = z[0]; fin[1] = z[1]; }
+          biquad_step(q[0], v[k], z[0], z[1], o1);
+        }
+        if (tail_here && k - 1 == valid) { fin[2] = z[2]; fin[3] = z[3]; }
+        biquad_step(q[1], o1_prev, z[2], z[3], o2);
+        v[k - 1] = o2;
+        o1_prev = o1;
+      }
+    }
+  }
+};
+
+// lfilter's direct form of order M = 1..4, D = M: its DF2T state is z' = A z + c x with A[i][0] = -a[i+1],
+// A[i][i+1] = 1 and c[i] = b[i+1] - a[i+1] b[0]; pass c is lfilter_step, the operations of the exact kernel.
+template <int M>
+struct DirectForm {
+  static constexpr int D = M, kMax = 4;
+  using Params = LfilterParams;
+  __device__ static constexpr int state_stride(int) { return D; }
+  const LfilterParams& P;
+  const double* c;
+
+  __device__ __forceinline__ DirectForm(const LfilterParams& P_, const IirJointTables& T) : P(P_), c(T.c) {}
+  __device__ __forceinline__ void enter(double (&)[kIirT], int) const {}
+  __device__ __forceinline__ void leave(double (&)[kIirT]) const {}
+  __device__ __forceinline__ void state_step(double in, double (&f)[D]) const {
+    const double z0 = f[0];
+#pragma unroll
+    for (int i = 0; i < D - 1; ++i) f[i] = fma(-P.a[i + 1], z0, fma(c[i], in, f[i + 1]));
+    f[D - 1] = fma(-P.a[D], z0, c[D - 1] * in);
+  }
+  __device__ __forceinline__ void filter(double (&v)[kIirT], double (&z)[D], bool tail_here, int valid,
+                                         double (&fin)[D]) const {
+#pragma unroll
+    for (int k = 0; k < kIirT; ++k) {
+      if (tail_here && k == valid) {
+#pragma unroll
+        for (int i = 0; i < D; ++i) fin[i] = z[i];
+      }
+      v[k] = lfilter_step<M>(P, v[k], z);
+    }
+  }
+};
+
+// Tile staging: rows of 16 samples at a pitch of 18 doubles (144 B): thread r reads / writes its row with 16-byte
+// accesses without bank conflicts, and 16-byte chunks stay aligned for cp.async.  Two buffers: the NEXT tile is
+// already on its way (cp.async, no registers held) while this one is filtered — a one-buffer kernel spent three
+// quarters of its time waiting for its own loads (ncu: long-scoreboard stalls on the first use of every loaded sample).
+constexpr int kJointPitch = kIirT + 2;                                            // doubles per staged row
+constexpr int kJointTileBytes = kIirThreads * kJointPitch * (int)sizeof(double);  // 36 864
+static_assert(kIirT == 16, "staging puts two-sample chunk c at row c >> 3, column 2 (c & 7): 8 chunks per row");
+static_assert(kJointPitch % 2 == 0 && (kJointPitch / 2) % 2 == 1,
+              "rows start on 16-byte boundaries at an odd number of 16-byte words apart (no bank conflicts)");
+extern __shared__ __align__(16) unsigned char iir_smem[];
+
+__device__ __forceinline__ void cp_async16_zfill(void* dst_smem, const void* src, int src_bytes) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"((uint32_t)__cvta_generic_to_shared(dst_smem)), "l"(src),
+               "r"(src_bytes)
+               : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N>
+__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
+
+// kAligned: x and y rows start on 16-byte boundaries (cp.async loads, 16-byte stores); else plain 8-byte accesses.
+// zi / zf: signal s's state is zi[s * Form::state_stride(zs) + 0 .. D - 1]; a long biquad cascade runs as a chain of
+// launches over its sections two by two, each on its slice of the states of the whole cascade (zs = 2 x all its
+// sections).
+template <class Form, bool kAligned>
+__global__ void __launch_bounds__(kIirThreads, kIirMinBlocks) iir_scan_kernel(
+    const __grid_constant__ typename Form::Params P, const __grid_constant__ IirJointTables TT, const double* __restrict__ x,
+    double* y, int64_t n, int64_t stride, const double* __restrict__ zi, double* __restrict__ zf, int zs) {
+  constexpr int D = Form::D;
   double* s_buf0 = reinterpret_cast<double*>(iir_smem);
   double* s_buf1 = reinterpret_cast<double*>(iir_smem + kJointTileBytes);
-  __shared__ double s_lane[D * D][32];  // (A^16)^lane, entry-major: conflict-free
+  __shared__ double s_lane[D * D][32];  // (M^16)^lane, entry-major: conflict-free
   __shared__ double s_tot[kIirThreads / 32][D];
   __shared__ double s_carry[D];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -706,8 +420,10 @@ __global__ void __launch_bounds__(kIirThreads, WFM_IIR_MINB) lfilter_scan_kernel
   const double* __restrict__ xs = x + sig * stride;
   double* ys = y + sig * stride;
   for (int e = tid; e < D * D * 32; e += kIirThreads) s_lane[e / 32][e % 32] = TT.lane[e % 32][(e / 32) / D * kMaxJoint + (e / 32) % D];
-  if (tid < D) s_carry[tid] = zi ? zi[sig * D + tid] : 0.0;
+  if (tid < D) s_carry[tid] = zi ? zi[sig * Form::state_stride(zs) + tid] : 0.0;
+  const Form form(P, TT);
 
+  // tile `base` -> buffer: 2048 chunks of two samples, chunk c of the tile at row c / 8, column 2 (c % 8)
   auto load_tile = [&](double* buf, int64_t base) {
     const int cnt = (int)min((int64_t)kIirTile, n - base);
 #pragma unroll
@@ -715,7 +431,7 @@ __global__ void __launch_bounds__(kIirThreads, WFM_IIR_MINB) lfilter_scan_kernel
       const int c = j * kIirThreads + tid;
       double* dst = buf + (c >> 3) * kJointPitch + 2 * (c & 7);
       if (kAligned) {
-        const int left = cnt - 2 * c;
+        const int left = cnt - 2 * c;  // samples of this chunk that exist: the rest is zero-filled
         cp_async16_zfill(dst, left > 0 ? xs + base + 2 * c : xs + base, left >= 2 ? 16 : (left == 1 ? 8 : 0));
       } else {
         dst[0] = 2 * c < cnt ? xs[base + 2 * c] : 0.0;
@@ -734,7 +450,7 @@ __global__ void __launch_bounds__(kIirThreads, WFM_IIR_MINB) lfilter_scan_kernel
     if (base + kIirTile < n) load_tile((it & 1) ? s_buf0 : s_buf1, base + kIirTile);
     if (kAligned) {
       cp_async_commit();
-      cp_async_wait<1>();
+      cp_async_wait<1>();  // everything but the tile just requested has landed
     }
     __syncthreads();
     double v[kIirT];
@@ -747,22 +463,19 @@ __global__ void __launch_bounds__(kIirThreads, WFM_IIR_MINB) lfilter_scan_kernel
         v[2 * k + 1] = d.y;
       }
     }
-    const int valid = max(0, min(kIirT, cnt - tid * kIirT));
+    const int valid = max(0, min(kIirT, cnt - tid * kIirT));  // my valid samples
+    form.enter(v, valid);
+
     double carry[D];
 #pragma unroll
     for (int i = 0; i < D; ++i) carry[i] = s_carry[i];
-    // ---- pass a: end state of my chunk from the zero state (thread 0: from the tile's carry-in)
+    // ---- pass a: end state of my chunk from the zero state (thread 0: from the tile's carry-in), state-space form
     double f[D];
 #pragma unroll
     for (int i = 0; i < D; ++i) f[i] = tid == 0 ? carry[i] : 0.0;
 #pragma unroll
-    for (int k = 0; k < kIirT; ++k) {
-      const double in = v[k], z0 = f[0];
-#pragma unroll
-      for (int i = 0; i < D - 1; ++i) f[i] = fma(-P.a[i + 1], z0, fma(P.c[i + 1], in, f[i + 1]));
-      f[D - 1] = fma(-P.a[D], z0, P.c[D] * in);
-    }
-    // ---- scan over the threads
+    for (int k = 0; k < kIirT; ++k) form.state_step(v[k], f);
+    // ---- scan over the threads: inclusive warp scan with constant matrices per level
 #pragma unroll
     for (int d = 0; d < 5; ++d) {
       double p[D], r[D];
@@ -790,6 +503,7 @@ __global__ void __launch_bounds__(kIirThreads, WFM_IIR_MINB) lfilter_scan_kernel
       if (lane == 0) e[i] = 0.0;
     }
     __syncthreads();
+    // carry entering my warp: C_w = Q C_{w-1} + tot_{w-1}, Q = (M^16)^32
     if (warp > 0) {
       double w[D], r[D], mq[D * D];
 #pragma unroll
@@ -814,7 +528,7 @@ __global__ void __launch_bounds__(kIirThreads, WFM_IIR_MINB) lfilter_scan_kernel
 #pragma unroll
       for (int i = 0; i < D; ++i) e[i] = carry[i];
     }
-    // ---- pass c: scipy's recurrence from the carried-in state
+    // ---- pass c: the faithful recurrence from the carried-in state
     double z[D];
 #pragma unroll
     for (int i = 0; i < D; ++i) z[i] = e[i];
@@ -822,20 +536,15 @@ __global__ void __launch_bounds__(kIirThreads, WFM_IIR_MINB) lfilter_scan_kernel
     double fin[D];
 #pragma unroll
     for (int i = 0; i < D; ++i) fin[i] = 0.0;
-#pragma unroll
-    for (int k = 0; k < kIirT; ++k) {
-      if (tail_here && k == valid) {
-#pragma unroll
-        for (int i = 0; i < D; ++i) fin[i] = z[i];
-      }
-      v[k] = lfilter_step_scan<M>(P, v[k], z);
-    }
+    form.filter(v, z, tail_here, valid, fin);
+    form.leave(v);
+    // my row back into the buffer (nobody else reads it before the barrier), then coalesced 16-byte stores
     {
       double2* row = reinterpret_cast<double2*>(buf + tid * kJointPitch);
 #pragma unroll
       for (int k = 0; k < kIirT / 2; ++k) row[k] = make_double2(v[2 * k], v[2 * k + 1]);
     }
-    __syncthreads();
+    __syncthreads();  // rows complete; all reads of s_carry / s_tot are done
     if (tail_here) {
 #pragma unroll
       for (int i = 0; i < D; ++i) s_carry[i] = fin[i];
@@ -855,33 +564,13 @@ __global__ void __launch_bounds__(kIirThreads, WFM_IIR_MINB) lfilter_scan_kernel
         if (2 * c + 1 < cnt) ys[base + 2 * c + 1] = d.y;
       }
     }
-    __syncthreads();
+    __syncthreads();  // the buffer may be refilled (tile t + 2) and s_carry read (tile t + 1)
   }
   if (kAligned) cp_async_wait<0>();
-  if (zf && tid < D) zf[sig * D + tid] = s_carry[tid];
+  if (zf && tid < D) zf[sig * Form::state_stride(zs) + tid] = s_carry[tid];
 }
 
-// host: 2x2 matrix powers in long double
-struct M2 {
-  long double a, b, c, d;
-};
-static M2 mm(const M2& x, const M2& y) {
-  return {x.a * y.a + x.b * y.c, x.a * y.b + x.b * y.d, x.c * y.a + x.d * y.c, x.c * y.b + x.d * y.d};
-}
-static M2 mpow(M2 base, long e) {
-  M2 r{1, 0, 0, 1};
-  while (e) {
-    if (e & 1) r = mm(r, base);
-    base = mm(base, base);
-    e >>= 1;
-  }
-  return r;
-}
-static void put(double* dst, const M2& m) {
-  dst[0] = (double)m.a; dst[1] = (double)m.b; dst[2] = (double)m.c; dst[3] = (double)m.d;
-}
-
-// D x D matrices in long double (joint state of the cascade)
+// D x D matrices in long double (the scan's one-step matrix and its powers)
 struct MD {
   long double m[kMaxJoint][kMaxJoint];
 };
@@ -927,8 +616,8 @@ static void joint_tables(const IirParams& P, IirJointTables* tab) {
   for (int k = 0; k < S; ++k) {
     const long double a1 = P.sec[k].a1, a2 = P.sec[k].a2, b0 = P.sec[k].b0, b1 = P.sec[k].b1, b2 = P.sec[k].b2;
     const long double c1 = b1 - a1 * b0, c2 = b2 - a2 * b0;
-    tab->c1[k] = (double)c1;
-    tab->c2[k] = (double)c2;
+    tab->c[2 * k] = (double)c1;
+    tab->c[2 * k + 1] = (double)c2;
     M.m[2 * k][2 * k] = -a1;
     M.m[2 * k][2 * k + 1] = 1;
     M.m[2 * k + 1][2 * k] = -a2;
@@ -943,13 +632,33 @@ static void joint_tables(const IirParams& P, IirJointTables* tab) {
   power_tables(M, D, tab);
 }
 // one-step matrix of lfilter's DF2T state (order Mo): z_i' = -a_{i+1} z_0 + z_{i+1}
-static void lfilter_tables(const LfScanParams& P, int Mo, IirJointTables* tab) {
+static void lfilter_tables(const LfilterParams& P, IirJointTables* tab) {
+  const int Mo = P.order;
   MD M{};
   for (int i = 0; i < Mo; ++i) {
+    tab->c[i] = (double)((long double)P.b[i + 1] - (long double)P.a[i + 1] * (long double)P.b[0]);
     M.m[i][0] = -(long double)P.a[i + 1];
     if (i + 1 < Mo) M.m[i][i + 1] = 1;
   }
   power_tables(M, Mo, tab);
+}
+
+// The scan kernel of Form<k> (k = sections or order, 1..Form::kMax) over n_sig signals, with 16-byte accesses when
+// every row of x and y starts on a 16-byte boundary.
+template <template <int> class Form, int K = 1>
+static cudaError_t launch_scan(int k, const typename Form<K>::Params& P, const IirJointTables& T, const double* x,
+                               double* y, int64_t n_sig, int64_t n, int64_t stride, const double* zi, double* zf,
+                               int zs, cudaStream_t st) {
+  if constexpr (K < Form<K>::kMax) {
+    if (k > K) return launch_scan<Form, K + 1>(k, P, T, x, y, n_sig, n, stride, zi, zf, zs, st);
+  }
+  const bool aligned = ((uintptr_t)x % 16 == 0) && ((uintptr_t)y % 16 == 0) && (stride % 2 == 0 || n_sig == 1);
+  const auto kern = aligned ? iir_scan_kernel<Form<K>, true> : iir_scan_kernel<Form<K>, false>;
+  const int smem = 2 * kJointTileBytes;
+  const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+  if (e != cudaSuccess) return e;
+  kern<<<(unsigned)n_sig, kIirThreads, smem, st>>>(P, T, x, y, n, stride, zi, zf, zs);
+  return cudaGetLastError();
 }
 
 // Host -> device copy of a small table (the initial states) that does NOT stall the stream: cudaMemcpyAsync from
@@ -991,6 +700,34 @@ static cudaError_t upload_small(void* dst, const void* src, size_t bytes, cudaSt
   return e;
 }
 
+// One filter call's states on the device: `words` doubles of HOST zi / zf (either may be NULL) in stream-ordered
+// scratch, zi uploaded, then run(d_zi, d_zf) filters; zf is copied back and the stream synchronised before the call
+// returns, because the caller reads zf then.  An empty signal (n = 0) passes the state through: zf = zi, or zeros
+// without zi.
+template <class Run>
+static int with_states(const double* zi, double* zf, size_t words, int64_t n, cudaStream_t st, Run run) {
+  const size_t bytes = sizeof(double) * words;
+  double *d_zi = nullptr, *d_zf = nullptr;
+  cudaError_t e = cudaSuccess;
+  if (zi && words) {
+    e = cudaMallocAsync(&d_zi, bytes, st);
+    if (e == cudaSuccess) e = upload_small(d_zi, zi, bytes, st);
+  }
+  if (e == cudaSuccess && zf && words) e = cudaMallocAsync(&d_zf, bytes, st);
+  if (e == cudaSuccess && n > 0) {
+    e = run(d_zi, d_zf);
+  } else if (e == cudaSuccess && d_zf) {
+    e = d_zi ? cudaMemcpyAsync(d_zf, d_zi, bytes, cudaMemcpyDeviceToDevice, st) : cudaMemsetAsync(d_zf, 0, bytes, st);
+  }
+  if (e == cudaSuccess && d_zf) {
+    e = cudaMemcpyAsync(zf, d_zf, bytes, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+  }
+  if (d_zi) cudaFreeAsync(d_zi, st);
+  if (d_zf) cudaFreeAsync(d_zf, st);
+  return e == cudaSuccess ? WFM_OK : WFM_ECUDA;
+}
+
 }  // namespace wfm
 
 extern "C" int wfm_sosfilt(const double* sos, int32_t n_sections, double initial, const double* x, double* y,
@@ -1012,78 +749,29 @@ extern "C" int wfm_sosfilt(const double* sos, int32_t n_sections, double initial
     // scipy normalises by a0 when it is not 1
     P.sec[k] = {c[0] / a0, c[1] / a0, c[2] / a0, c[4] / a0, c[5] / a0};
   }
-  const size_t state_bytes = sizeof(double) * 2 * (size_t)n_sections * (size_t)n_sig;
-  double *d_zi = nullptr, *d_zf = nullptr;
-  cudaError_t e = cudaSuccess;
-  // stream-ordered scratch for the states (pageable host sources are staged by the driver
-  // before cudaMemcpyAsync returns, so no synchronisation is needed for them)
-  if (zi) {
-    e = cudaMallocAsync(&d_zi, state_bytes, st);
-    if (e == cudaSuccess) e = upload_small(d_zi, zi, state_bytes, st);
-  }
-  if (e == cudaSuccess && zf) e = cudaMallocAsync(&d_zf, state_bytes, st);
-  if (e == cudaSuccess && n > 0) {
+  return with_states(zi, zf, 2 * (size_t)n_sections * (size_t)n_sig, n, st, [&](const double* d_zi, double* d_zf) {
     if (mode == WFM_IIR_EXACT) {
       const unsigned blocks = (unsigned)((n_sig + kExactWarps - 1) / kExactWarps);
       sosfilt_exact_kernel<<<blocks, 32 * kExactWarps, 0, st>>>(P, x, y, n_sig, n, stride, d_zi, d_zf);
-      e = cudaGetLastError();
-    } else if (!getenv("WFM_IIR_OLD_SCAN")) {
-      // the joint kernel takes the sections two by two: a cascade of S sections is ceil(S / 2) launches, each a read and
-      // a write of the signal; `initial` is subtracted by the first launch and added back by the last one only
-      const bool aligned = ((uintptr_t)x % 16 == 0) && ((uintptr_t)y % 16 == 0) && (stride % 2 == 0 || n_sig == 1);
-      const size_t smem = 2 * (size_t)kJointTileBytes;
-      for (int k0 = 0; k0 < n_sections && e == cudaSuccess; k0 += 2) {
-        IirParams Pk{};
-        Pk.n_sections = std::min(2, n_sections - k0);
-        Pk.initial = P.initial;
-        Pk.shift_in = k0 == 0;
-        Pk.shift_out = k0 + 2 >= n_sections;
-        for (int k = 0; k < Pk.n_sections; ++k) Pk.sec[k] = P.sec[k0 + k];
-        static thread_local IirJointTables jt;
-        joint_tables(Pk, &jt);
-        const double* xin = k0 == 0 ? x : y;
-        auto launch = [&](auto kern) {
-          cudaError_t ee = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-          if (ee != cudaSuccess) return ee;
-          kern<<<(unsigned)n_sig, kIirThreads, smem, st>>>(Pk, jt, xin, y, n, stride, d_zi ? d_zi + 2 * k0 : nullptr,
-                                                           d_zf ? d_zf + 2 * k0 : nullptr, 2 * n_sections);
-          return cudaGetLastError();
-        };
-        if (Pk.n_sections == 1) e = aligned ? launch(sosfilt_scan_joint_kernel<1, true>) : launch(sosfilt_scan_joint_kernel<1, false>);
-        else e = aligned ? launch(sosfilt_scan_joint_kernel<2, true>) : launch(sosfilt_scan_joint_kernel<2, false>);
-      }
-    } else {
-      static thread_local IirScanTables tab;
-      for (int k = 0; k < n_sections; ++k) {
-        const M2 A{-(long double)P.sec[k].a1, 1.0L, -(long double)P.sec[k].a2, 0.0L};
-        const M2 AT = mpow(A, kIirT);
-        M2 pw{1, 0, 0, 1};
-        for (int l = 0; l < 32; ++l) {
-          put(tab.lane[k][l], pw);
-          pw = mm(pw, AT);
-        }
-        put(tab.warp[k], pw);  // AT^32
-        M2 sq = AT;
-        for (int d = 0; d < 5; ++d) {
-          put(tab.lvl[k][d], sq);
-          sq = mm(sq, sq);
-        }
-      }
-      sosfilt_scan_kernel<<<(unsigned)n_sig, kIirThreads, 0, st>>>(P, tab, x, y, n, stride, d_zi, d_zf);
-      e = cudaGetLastError();
+      return cudaGetLastError();
     }
-  } else if (e == cudaSuccess && zf && zi) {
-    e = cudaMemcpyAsync(d_zf, d_zi, state_bytes, cudaMemcpyDeviceToDevice, st);
-  } else if (e == cudaSuccess && zf) {
-    e = cudaMemsetAsync(d_zf, 0, state_bytes, st);
-  }
-  if (e == cudaSuccess && zf) {
-    e = cudaMemcpyAsync(zf, d_zf, state_bytes, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);  // the caller reads zf on return
-  }
-  if (d_zi) cudaFreeAsync(d_zi, st);
-  if (d_zf) cudaFreeAsync(d_zf, st);
-  return e == cudaSuccess ? WFM_OK : WFM_ECUDA;
+    // the scan takes the sections two by two: a cascade of S sections is ceil(S / 2) launches, each a read and a write
+    // of the signal; `initial` is subtracted by the first launch and added back by the last one only
+    cudaError_t e = cudaSuccess;
+    for (int k0 = 0; k0 < n_sections && e == cudaSuccess; k0 += 2) {
+      IirParams Pk{};
+      Pk.n_sections = std::min(2, n_sections - k0);
+      Pk.initial = P.initial;
+      Pk.shift_in = k0 == 0;
+      Pk.shift_out = k0 + 2 >= n_sections;
+      for (int k = 0; k < Pk.n_sections; ++k) Pk.sec[k] = P.sec[k0 + k];
+      static thread_local IirJointTables jt;
+      joint_tables(Pk, &jt);
+      e = launch_scan<BiquadForm>(Pk.n_sections, Pk, jt, k0 == 0 ? x : y, y, n_sig, n, stride,
+                                  d_zi ? d_zi + 2 * k0 : nullptr, d_zf ? d_zf + 2 * k0 : nullptr, 2 * n_sections, st);
+    }
+    return e;
+  });
 }
 
 extern "C" int wfm_lfilter(const double* b, int32_t nb, const double* a, int32_t na, const double* x, double* y,
@@ -1108,48 +796,15 @@ extern "C" int wfm_lfilter_mode(const double* b, int32_t nb, const double* a, in
     P.b[k] = k < nb ? b[k] / a[0] : 0.0;
     P.a[k] = k < na ? a[k] / a[0] : 0.0;
   }
-  const size_t state_bytes = sizeof(double) * (size_t)std::max(M, 1) * (size_t)n_sig;
-  double *d_zi = nullptr, *d_zf = nullptr;
-  cudaError_t e = cudaSuccess;
-  if (zi && M > 0) {
-    e = cudaMallocAsync(&d_zi, state_bytes, st);
-    if (e == cudaSuccess) e = upload_small(d_zi, zi, sizeof(double) * M * n_sig, st);
-  }
-  if (e == cudaSuccess && zf && M > 0) e = cudaMallocAsync(&d_zf, state_bytes, st);
-  if (e == cudaSuccess && mode == WFM_IIR_SCAN && M >= 1 && M <= kMaxJoint && n > 0) {
-    LfScanParams S{};
-    for (int k = 0; k <= M; ++k) {
-      S.b[k] = P.b[k];
-      S.a[k] = P.a[k];
-      S.c[k] = (double)((long double)P.b[k] - (long double)P.a[k] * (long double)P.b[0]);
+  return with_states(zi, zf, (size_t)M * (size_t)n_sig, n, st, [&](const double* d_zi, double* d_zf) {
+    if (mode == WFM_IIR_SCAN && M >= 1 && M <= kMaxJoint) {
+      static thread_local IirJointTables jt;
+      lfilter_tables(P, &jt);
+      return launch_scan<DirectForm>(M, P, jt, x, y, n_sig, n, stride, d_zi, d_zf, M, st);
     }
-    static thread_local IirJointTables jt;
-    lfilter_tables(S, M, &jt);
-    const bool aligned = ((uintptr_t)x % 16 == 0) && ((uintptr_t)y % 16 == 0) && (stride % 2 == 0 || n_sig == 1);
-    const size_t smem = 2 * (size_t)kJointTileBytes;
-    auto launch = [&](auto kern) {
-      cudaError_t ee = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      if (ee != cudaSuccess) return ee;
-      kern<<<(unsigned)n_sig, kIirThreads, smem, st>>>(S, jt, x, y, n, stride, d_zi, d_zf);
-      return cudaGetLastError();
-    };
-    switch (M) {
-      case 1: e = aligned ? launch(lfilter_scan_kernel<1, true>) : launch(lfilter_scan_kernel<1, false>); break;
-      case 2: e = aligned ? launch(lfilter_scan_kernel<2, true>) : launch(lfilter_scan_kernel<2, false>); break;
-      case 3: e = aligned ? launch(lfilter_scan_kernel<3, true>) : launch(lfilter_scan_kernel<3, false>); break;
-      default: e = aligned ? launch(lfilter_scan_kernel<4, true>) : launch(lfilter_scan_kernel<4, false>); break;
-    }
-  } else if (e == cudaSuccess) {
-    // (orders above 4, order 0 and empty signals: the sequential kernel, whatever the mode)
+    // (orders above 4 and order 0: the sequential kernel, whatever the mode)
     lfilter_exact_kernel<<<(unsigned)((n_sig + kExactWarps - 1) / kExactWarps), 32 * kExactWarps, 0, st>>>(
         P, x, y, n_sig, n, stride, d_zi, d_zf);
-    e = cudaGetLastError();
-  }
-  if (e == cudaSuccess && d_zf) {
-    e = cudaMemcpyAsync(zf, d_zf, sizeof(double) * M * n_sig, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);  // the caller reads zf on return
-  }
-  if (d_zi) cudaFreeAsync(d_zi, st);
-  if (d_zf) cudaFreeAsync(d_zf, st);
-  return e == cudaSuccess ? WFM_OK : WFM_ECUDA;
+    return cudaGetLastError();
+  });
 }

@@ -67,9 +67,7 @@ def sosfilt_device(sos, x, initial=0.0, zi=None, want_zf=False, out=None,
                          zi_arr.ctypes.data if zi_arr is not None else None,
                          zf.ctypes.data if zf is not None else None,
                          _IIR_MODES[mode], _stream(torch, x.device))
-    engine._check(rc)
-    if zf is not None:
-        torch.cuda.current_stream(x.device).synchronize()
+    engine._check(rc)  # (with zf requested the call has synchronised the stream: zf is filled)
     return (y if x.dim() == 2 else y[0]), zf
 
 
