@@ -65,7 +65,7 @@ def main():
                      r'|sample_kernel<float, false, 1, 0, false, (true|false)>|sample_dense_kernel<double, false, 4, (true|false), false>'
                      r'|sample_dense_kernel<float, false, 4, true, (true|false)>|iir_scan_kernel<wfm::BiquadForm<2>, true>'
                      r'|iir_scan_kernel<wfm::DirectForm<2>, true>'
-                     r'|sosfilt_exact|lfilter_exact|fft_cols_kernel|fft_rows_kernel<true>|fft_filter_single|prepare_|fill_packets'
+                     r'|sosfilt_exact|lfilter_exact|fft_cols_kernel|fft_rows_tma_kernel|fft_rows_kernel<true>|fft_filter_single|prepare_|fill_packets'
                      r'|dfma_kernel|reflection_response')
     for n in names:
         d = dm.get(n, n)

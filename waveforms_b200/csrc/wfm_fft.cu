@@ -36,7 +36,6 @@
 #include <cmath>
 #include <complex>
 #include <cstdint>
-#include <cstdlib>
 #include <cstring>
 #include <map>
 #include <mutex>
@@ -46,35 +45,25 @@
 
 namespace wfm {
 
-#ifndef WFM_FFT_MAX_RADIX
-#define WFM_FFT_MAX_RADIX 8  // largest power-of-two butterfly: 4, 8 or 16 (measured on cfg4: 6.11 / 5.90 / 6.30 ms)
-#endif
-#ifndef WFM_FFT_BIG_RADIX
-#define WFM_FFT_BIG_RADIX 1  // composite butterflies held in registers: 1 = 10 (2x5), 2 = also 25 (5x5)
-#endif
-#ifndef WFM_FFT_CT_COLS_640
-#define WFM_FFT_CT_COLS_640 1
-#endif
-#ifndef WFM_FFT_CT
-#define WFM_FFT_CT 1  // compile-time plans for the tile shapes of cfg4 (625 x 4 columns, 640 x 2 rows)
-#endif
-#ifndef WFM_FFT_THREADS
-#define WFM_FFT_THREADS 512
-#endif
-constexpr int kFftThreads = WFM_FFT_THREADS;
+// ---- tile geometry: fixed, every alternative below was measured on cfg4 and rejected (DESIGN §K3) --------------------
+// Radices: the largest power-of-two butterfly is 8 (4 / 8 / 16: 6.11 / 5.90 / 6.30 ms); the one composite butterfly
+// is 10 = 2 x 5 (25 = 5 x 5 in the column passes: 2.19-2.20 against 2.19 ms).  The shared-memory buffers are unpadded
+// (a 16-byte pad per 32 / 16 elements: 2.24 / 2.26 against 2.20 ms: the reads pay what the writes gain), and the
+// transform direction is a run-time argument of the stages (compile-time: 2.21 against 2.19 ms).
+constexpr int kFftThreads = 512;  // one-level kernels: one CTA per transform
 // the row pass has the radix-10 stage and reads contiguous rows, so its tile can be small: 2 rows per CTA, 160 threads
 // (the 160 radix-8 / 128 radix-10 butterflies of a 640-point x 2 tile), three CTAs per SM at up to 136 registers.  More,
 // smaller CTAs overlap the load / butterfly / store phases that block barriers serialise inside one CTA.  Measured on
 // cfg4 (fft_filter, ms): 4 rows x 320 threads x 2 CTAs 2.19 (512 / 448 / 384 threads: 2.27 / 2.21 / 2.20);
 // 2 rows x 160 x 3 CTAs 2.08; x 4 CTAs 2.13; x 2 CTAs 2.24; 2 rows x 128 x 3: 2.16; x 192 x 3: 2.12; 1 row x 96 x 6: 2.19
-#ifndef WFM_FFT_ROWS_THREADS
-#define WFM_FFT_ROWS_THREADS 160
-#endif
-constexpr int kFftRowsThreads = WFM_FFT_ROWS_THREADS;
-#ifndef WFM_FFT_COLS_THREADS
-#define WFM_FFT_COLS_THREADS WFM_FFT_THREADS
-#endif
-constexpr int kFftColsThreads = WFM_FFT_COLS_THREADS;
+constexpr int kFftRowsThreads = 160;
+constexpr int kFftRowsMinBlocks = 3;
+constexpr int kFftRowsLogC = 1;
+// column pass: 4 interleaved columns per CTA and two CTAs per SM (32 warps) measured 14 % faster than 8 columns and one
+// CTA (cfg4, n = 625 x 640)
+constexpr int kFftColsThreads = 512;
+constexpr int kFftColsMinBlocks = 2;
+constexpr int kFftColsLogC = 2;
 constexpr int kMaxPoints = 6144;  // complex points per shared-memory buffer (2 buffers = 192 KB)
 constexpr int kMaxStages = 20;
 constexpr int kSmemBudget = 227 * 1024 - 1024;
@@ -201,66 +190,39 @@ __device__ __forceinline__ void dft_small<8>(double2 (&v)[8], double sgn) {
   dft_composite<2, 4>(v, sgn, cs, sn);
 }
 template <>
-__device__ __forceinline__ void dft_small<16>(double2 (&v)[16], double sgn) {
-  constexpr double cs[16] = {1.0, 0.9238795325112867, 0.7071067811865476, 0.38268343236508984, 6.123233995736766e-17, -0.3826834323650897, -0.7071067811865475, -0.9238795325112867, -1.0, -0.9238795325112868, -0.7071067811865477, -0.38268343236509034, -1.8369701987210297e-16, 0.38268343236509, 0.7071067811865474, 0.9238795325112865};
-  constexpr double sn[16] = {0.0, 0.3826834323650898, 0.7071067811865475, 0.9238795325112867, 1.0, 0.9238795325112867, 0.7071067811865476, 0.3826834323650899, 1.2246467991473532e-16, -0.38268343236508967, -0.7071067811865475, -0.9238795325112865, -1.0, -0.9238795325112866, -0.7071067811865477, -0.3826834323650904};
-  dft_composite<4, 4>(v, sgn, cs, sn);
-}
-
-#if WFM_FFT_BIG_RADIX
-template <>
 __device__ __forceinline__ void dft_small<10>(double2 (&v)[10], double sgn) {
   constexpr double cs[10] = {1.0, 0.8090169943749475, 0.30901699437494745, -0.30901699437494734, -0.8090169943749473, -1.0, -0.8090169943749476, -0.30901699437494756, 0.30901699437494723, 0.8090169943749473};
   constexpr double sn[10] = {0.0, 0.5877852522924731, 0.9510565162951535, 0.9510565162951536, 0.5877852522924732, 1.2246467991473532e-16, -0.587785252292473, -0.9510565162951535, -0.9510565162951536, -0.5877852522924734};
   dft_composite<2, 5>(v, sgn, cs, sn);
 }
-template <>
-__device__ __forceinline__ void dft_small<25>(double2 (&v)[25], double sgn) {
-  constexpr double cs[25] = {1.0, 0.9685831611286311, 0.8763066800438636, 0.7289686274214116, 0.5358267949789965, 0.30901699437494745, 0.06279051952931353, -0.1873813145857246, -0.4257792915650727, -0.6374239897486897, -0.8090169943749473, -0.9297764858882513, -0.9921147013144778, -0.9921147013144779, -0.9297764858882515, -0.8090169943749478, -0.6374239897486895, -0.42577929156507216, -0.18738131458572463, 0.06279051952931283, 0.30901699437494723, 0.5358267949789968, 0.7289686274214112, 0.8763066800438631, 0.968583161128631};
-  constexpr double sn[25] = {0.0, 0.2486898871648548, 0.4817536741017153, 0.6845471059286886, 0.8443279255020151, 0.9510565162951535, 0.9980267284282716, 0.9822872507286887, 0.9048270524660195, 0.7705132427757893, 0.5877852522924732, 0.36812455268467814, 0.12533323356430454, -0.12533323356430429, -0.3681245526846779, -0.5877852522924727, -0.7705132427757894, -0.9048270524660198, -0.9822872507286887, -0.9980267284282716, -0.9510565162951536, -0.844327925502015, -0.684547105928689, -0.4817536741017161, -0.24868988716485535};
-  dft_composite<5, 5>(v, sgn, cs, sn);
-}
-#endif
 
 // ---- Stockham stages ------------------------------------------------------------------
 // C = 2^logc interleaved transforms live in shared memory, point p of transform c at
-// [p*C + c].  A stage reads its R inputs through `in(p, c)` and hands its R outputs to
-// `out(p, c, v)`: the middle stages use the shared-memory accessors below, the FIRST stage
-// of a transform reads global memory directly and the LAST one writes global memory (or
-// multiplies by the response on the way to shared memory), so loading, filtering and storing
-// cost no passes of their own over shared memory — the shared-memory data pipe is what
-// bounds these kernels (ncu: 75 % of its peak, profiles/r1o_k3_ncu_details.txt).
+// [p*C + c].  A stage reads its R inputs through `in(p, c, e)` and hands its R outputs to
+// `out(p, c, e, v)`, e = (p << logc) + c the element's index in a shared-memory buffer: the
+// middle stages use the shared-memory accessors below, the FIRST stage of a transform reads
+// global memory directly and the LAST one writes global memory (or multiplies by the response
+// on the way to shared memory), so loading, filtering and storing cost no passes of their own
+// over shared memory — the shared-memory data pipe is what bounds these kernels (ncu: 75 % of
+// its peak, profiles/r1o_k3_ncu_details.txt).  An accessor uses what it needs of (p, c, e).
 // accessors that have no inter-pass twiddle carry this no-op (a member, so they stay aggregates)
 #define WFM_NO_RUN_TWIDDLE \
   template <int R>         \
   __device__ __forceinline__ void twiddle_run(double2 (&)[R], int, int, int) const {}
-// Shared-memory index of element i of a ping-pong buffer: one 16-byte pad after every 2^WFM_FFT_PAD elements.  A Stockham
-// stage WRITES its outputs at a lane stride of R * C elements (a multiple of 8 for every radix / interleave used here:
-// all lanes of a quarter warp on the same bank group, 4..8-way conflicts; ncu counted 15 M conflicts per row pass); the
-// pad rotates the bank group every 2^WFM_FFT_PAD elements and costs 3 % of the buffer.  0 = unpadded.
-#ifndef WFM_FFT_PAD
-#define WFM_FFT_PAD 0  // measured on cfg4 (625 x 640): 2.24 ms padded (5) / 2.26 (4) against 2.20 unpadded: the reads pay what the writes gain
-#endif
-__host__ __device__ __forceinline__ constexpr int spad(int i) { return WFM_FFT_PAD ? i + (i >> WFM_FFT_PAD) : i; }
-__host__ __device__ __forceinline__ constexpr size_t padded_points(size_t points) {
-  return WFM_FFT_PAD ? points + (points >> WFM_FFT_PAD) + 1 : points;
-}
 struct SmemIn {
   WFM_NO_RUN_TWIDDLE
   const double2* a;
-  int logc;
-  __device__ __forceinline__ double2 operator()(int p, int c) const { return a[spad((p << logc) + c)]; }
+  __device__ __forceinline__ double2 operator()(int, int, int e) const { return a[e]; }
 };
 struct SmemOut {
   WFM_NO_RUN_TWIDDLE
   double2* b;
-  int logc;
-  __device__ __forceinline__ void operator()(int p, int c, double2 v) const { b[spad((p << logc) + c)] = v; }
+  __device__ __forceinline__ void operator()(int, int, int e, double2 v) const { b[e] = v; }
 };
 
 // twiddles W^(k r), r = 1..R-1, of one butterfly: ONE look-up, W^k from the stage's slice of the compact table
-// (FftPlan.twc: consecutive k at consecutive addresses — in a full W_L^p table a stage's twiddles sit tstep * 16 bytes
-// apart, a multiple of the bank period for the early stages of even lengths: up to 16-way conflicts), the powers by
+// (FftPlan.twc: consecutive k at consecutive addresses — in a full W_L^p table a stage's twiddles sit L / (Ns R) * 16
+// bytes apart, a multiple of the bank period for the early stages of even lengths: up to 16-way conflicts), the powers by
 // products of depth <= log2 R (a few roundings more; the FP64 pipe idles in these kernels, the shared-memory pipe does not)
 template <int R>
 __device__ __forceinline__ void load_twiddles(double2 (&w)[R], const double2* __restrict__ tw_k, double sgn) {
@@ -282,7 +244,7 @@ __device__ __forceinline__ void stockham_stage(In in, Out out, int L, int logc, 
     const int k = j - q * Ns;
     double2 v[R];
 #pragma unroll
-    for (int r = 0; r < R; ++r) v[r] = in(j + r * nb, c);
+    for (int r = 0; r < R; ++r) v[r] = in(j + r * nb, c, ((j + r * nb) << logc) + c);
     in.template twiddle_run<R>(v, j, nb, c);  // inter-pass twiddles of the run j, j+nb, ... (column passes)
     if (k > 0) {
       double2 w[R];
@@ -294,7 +256,7 @@ __device__ __forceinline__ void stockham_stage(In in, Out out, int L, int logc, 
     const int j0 = q * Ns * R + k;
     out.template twiddle_run<R>(v, j0, Ns, c);
 #pragma unroll
-    for (int r = 0; r < R; ++r) out(j0 + r * Ns, c, v[r]);
+    for (int r = 0; r < R; ++r) out(j0 + r * Ns, c, ((j0 + r * Ns) << logc) + c, v[r]);
   }
 }
 
@@ -306,18 +268,8 @@ __device__ __forceinline__ void stage_any(int R, In in, Out out, int L, int logc
     case 3: stockham_stage<3>(in, out, L, logc, Ns, inv, toff, tw, sgn); break;
     case 4: stockham_stage<4>(in, out, L, logc, Ns, inv, toff, tw, sgn); break;
     case 5: stockham_stage<5>(in, out, L, logc, Ns, inv, toff, tw, sgn); break;
-#if WFM_FFT_MAX_RADIX >= 8
     case 8: stockham_stage<8>(in, out, L, logc, Ns, inv, toff, tw, sgn); break;
-#endif
-#if WFM_FFT_MAX_RADIX >= 16
-    case 16: stockham_stage<16>(in, out, L, logc, Ns, inv, toff, tw, sgn); break;
-#endif
-#if WFM_FFT_BIG_RADIX
     case 10: stockham_stage<10>(in, out, L, logc, Ns, inv, toff, tw, sgn); break;
-#endif
-#if WFM_FFT_BIG_RADIX >= 2
-    case 25: stockham_stage<25>(in, out, L, logc, Ns, inv, toff, tw, sgn); break;
-#endif
     default: stockham_stage<7>(in, out, L, logc, Ns, inv, toff, tw, sgn); break;
   }
 }
@@ -327,29 +279,11 @@ __device__ __forceinline__ void stage_any(int R, In in, Out out, int L, int logc
 // writes through `out` instead.  `in` may read buf1 (never buf0).  Ends with a block
 // barrier, so what `out` wrote to shared memory is visible.  All threads must call it.
 template <class In, class Out>
-__device__ __forceinline__ void smem_fft_rt(const FftPlan& P, int logc, double sgn, const double2* __restrict__ tw, In in,
-                                            Out out, double2* buf0, double2* buf1);
-#ifndef WFM_FFT_CT_SGN
-#define WFM_FFT_CT_SGN 0  // 1: the direction is a compile-time constant inside the stages (two copies of the code)
-#endif
-template <class In, class Out>
 __device__ __forceinline__ void smem_fft(const FftPlan& P, int logc, double sgn, const double2* __restrict__ tw, In in,
                                          Out out, double2* buf0, double2* buf1) {
-#if WFM_FFT_CT_SGN
-  if (sgn < 0.0)
-    smem_fft_rt(P, logc, -1.0, tw, in, out, buf0, buf1);
-  else
-    smem_fft_rt(P, logc, 1.0, tw, in, out, buf0, buf1);
-#else
-  smem_fft_rt(P, logc, sgn, tw, in, out, buf0, buf1);
-#endif
-}
-template <class In, class Out>
-__device__ __forceinline__ void smem_fft_rt(const FftPlan& P, int logc, double sgn, const double2* __restrict__ tw, In in,
-                                            Out out, double2* buf0, double2* buf1) {
   const int S = P.n_stage;
   if (S == 0) {  // L == 1: the transform is the identity
-    for (int c = threadIdx.x; c < (1 << logc); c += blockDim.x) out(0, c, in(0, c));
+    for (int c = threadIdx.x; c < (1 << logc); c += blockDim.x) out(0, c, c, in(0, c, c));
     __syncthreads();
     return;
   }
@@ -358,18 +292,18 @@ __device__ __forceinline__ void smem_fft_rt(const FftPlan& P, int logc, double s
     __syncthreads();
     return;
   }
-  stage_any(P.radix[0], in, SmemOut{buf0, logc}, P.L, logc, 1, P.inv_ns[0], 0, tw, sgn);
+  stage_any(P.radix[0], in, SmemOut{buf0}, P.L, logc, 1, P.inv_ns[0], 0, tw, sgn);
   __syncthreads();
   int Ns = P.radix[0], toff = 1;
   double2 *src = buf0, *dst = buf1;
   for (int s = 1; s < S - 1; ++s) {
-    stage_any(P.radix[s], SmemIn{src, logc}, SmemOut{dst, logc}, P.L, logc, Ns, P.inv_ns[s], toff, tw, sgn);
+    stage_any(P.radix[s], SmemIn{src}, SmemOut{dst}, P.L, logc, Ns, P.inv_ns[s], toff, tw, sgn);
     __syncthreads();
     double2* t = src; src = dst; dst = t;
     toff += Ns;
     Ns *= P.radix[s];
   }
-  stage_any(P.radix[S - 1], SmemIn{src, logc}, out, P.L, logc, Ns, P.inv_ns[S - 1], toff, tw, sgn);
+  stage_any(P.radix[S - 1], SmemIn{src}, out, P.L, logc, Ns, P.inv_ns[S - 1], toff, tw, sgn);
   __syncthreads();
 }
 // the buffer the last stage of smem_fft(.., buf0, buf1) may write through `out` (the one it
@@ -411,7 +345,7 @@ struct PairIn {
   const double* xa;
   const double* xb;  // nullptr: odd tail
   int nv;
-  __device__ __forceinline__ double2 operator()(int p, int) const {
+  __device__ __forceinline__ double2 operator()(int p, int, int) const {
     return p < nv ? make_double2(xa[p], xb ? xb[p] : 0.0) : make_double2(0.0, 0.0);
   }
 };
@@ -421,7 +355,7 @@ struct PairOut {
   double* yb;
   double scale;
   int nv;
-  __device__ __forceinline__ void operator()(int p, int, double2 v) const {
+  __device__ __forceinline__ void operator()(int p, int, int, double2 v) const {
     if (p >= nv) return;
     ya[p] = v.x * scale;
     if (yb) yb[p] = v.y * scale;
@@ -431,30 +365,31 @@ struct MulHOut {
   WFM_NO_RUN_TWIDDLE  // spectrum x response on the way to shared memory
   double2* z;
   const double2* __restrict__ H;
-  __device__ __forceinline__ void operator()(int p, int, double2 v) const { z[spad(p)] = cmul(v, __ldg(H + p)); }
+  __device__ __forceinline__ void operator()(int p, int, int, double2 v) const { z[p] = cmul(v, __ldg(H + p)); }
 };
 __global__ void __launch_bounds__(kFftThreads) fft_filter_single_kernel(FftPlan P, const double* __restrict__ x,
                                                                         double* __restrict__ y, int64_t stride,
                                                                         int64_t y_stride, int64_t n_sig,
                                                                         const double2* __restrict__ H, int nv) {
   double2* a = reinterpret_cast<double2*>(fft_smem_raw);
-  double2* b = a + padded_points(P.L);
-  const double2* tw = stage_twiddles(P, b + padded_points(P.L));
+  double2* b = a + P.L;
+  const double2* tw = stage_twiddles(P, b + P.L);
   const int64_t s0 = 2 * (int64_t)blockIdx.x;
   const bool two = s0 + 1 < n_sig;
   const double* xs = x + s0 * stride;
   double* ys = y + s0 * y_stride;
   double2* z = last_stage_target(P, a, b);
   smem_fft(P, 0, -1.0, tw, PairIn{xs, two ? xs + stride : nullptr, nv}, MulHOut{z, H}, a, b);
-  smem_fft(P, 0, +1.0, tw, SmemIn{z, 0}, PairOut{ys, two ? ys + y_stride : nullptr, 1.0 / (double)P.L, nv}, z == a ? b : a, z);
+  smem_fft(P, 0, +1.0, tw, SmemIn{z}, PairOut{ys, two ? ys + y_stride : nullptr, 1.0 / (double)P.L, nv}, z == a ? b : a, z);
 }
 
 // ---- compile-time plans -------------------------------------------------------------------------------------------------
 // The generic stages take the transform length, the interleave, the radix sequence and the strides at run time: two
 // thirds of their instructions are index arithmetic (ncu: 88 M fp64 of 365 M warp instructions per column pass of cfg4).
 // For the tile shapes that matter the whole plan is a template argument: element indices become immediate offsets, the
-// butterfly count per thread is a constant, j / Ns is a multiply-shift by a constant.  CtIn / CtOut accessors get the
-// point, the column and the element index e = (point << LOGC) + column.
+// butterfly count per thread is a constant, j / Ns is a multiply-shift by a constant.  The accessors are those of the
+// generic stages.  The inverse twiddle product conjugates inside its fma arrangement, where stockham_stage conjugates W
+// and calls cmul: the two round differently in the last bit, so the two stage bodies stay separate.
 template <int R, int L, int LOGC, int NS, int TOFF, bool kFwd, int T, class In, class Out>
 __device__ __forceinline__ void stage_ct(In in, Out out, const double2* __restrict__ tw) {
   constexpr double sgn = kFwd ? -1.0 : 1.0;
@@ -473,7 +408,7 @@ __device__ __forceinline__ void stage_ct(In in, Out out, const double2* __restri
     in.template twiddle_run<R>(v, j, nb, c);
     if (NS > 1 && k > 0) {
       // ONE look-up per butterfly, W^k from the stage's own compact table (consecutive k: consecutive addresses, no bank
-      // conflicts — in the full table a stage's twiddles are tstep * 16 bytes apart, a multiple of the 128-byte bank
+      // conflicts — in the full table a stage's twiddles are L / (NS R) * 16 bytes apart, a multiple of the 128-byte bank
       // period for the early stages); W^(k r) by products of depth <= 3.  The shared-memory pipe, not the FP64 pipe, is
       // what these passes saturate.
       double2 w[R];
@@ -493,31 +428,6 @@ __device__ __forceinline__ void stage_ct(In in, Out out, const double2* __restri
     for (int r = 0; r < R; ++r) out(j0 + r * NS, c, e0 + r * NsC, v[r]);
   }
 }
-// the (point, column) accessors of the generic stages behind the compile-time interface
-template <class A>
-struct CtWrapIn {
-  A a;
-  __device__ __forceinline__ double2 operator()(int p, int c, int) const { return a(p, c); }
-  template <int R>
-  __device__ __forceinline__ void twiddle_run(double2 (&v)[R], int r0, int step, int c) const { a.template twiddle_run<R>(v, r0, step, c); }
-};
-template <class A>
-struct CtWrapOut {
-  A a;
-  __device__ __forceinline__ void operator()(int p, int c, int, double2 v) const { a(p, c, v); }
-  template <int R>
-  __device__ __forceinline__ void twiddle_run(double2 (&v)[R], int r0, int step, int c) const { a.template twiddle_run<R>(v, r0, step, c); }
-};
-struct CtSmemIn {
-  WFM_NO_RUN_TWIDDLE
-  const double2* a;
-  __device__ __forceinline__ double2 operator()(int, int, int e) const { return a[e]; }
-};
-struct CtSmemOut {
-  WFM_NO_RUN_TWIDDLE
-  double2* b;
-  __device__ __forceinline__ void operator()(int, int, int e, double2 v) const { b[e] = v; }
-};
 // stages 0 .. S-1 of the radix pack; stage s reads `in` (s = 0) or the buffer stage s-1 wrote, and writes `out`
 // (s = S-1) or buf[s & 1]
 struct CtNoHook {
@@ -534,53 +444,43 @@ __device__ __forceinline__ void stages_ct_impl(int s, In in, Out out, const doub
     hook();
     __syncthreads();
   } else {
-    stage_ct<R0, L, LOGC, NS, TOFF, kFwd, T>(in, CtSmemOut{dst}, tw);
+    stage_ct<R0, L, LOGC, NS, TOFF, kFwd, T>(in, SmemOut{dst}, tw);
     hook();
     __syncthreads();
-    stages_ct_impl<L, LOGC, kFwd, T, NS * R0, TOFF + NS>(s + 1, CtSmemIn{dst}, out, tw, buf0, buf1, CtNoHook{},
+    stages_ct_impl<L, LOGC, kFwd, T, NS * R0, TOFF + NS>(s + 1, SmemIn{dst}, out, tw, buf0, buf1, CtNoHook{},
                                                          std::integer_sequence<int, Rest...>{});
   }
 }
 // same contract as smem_fft: `in` may read buf1, the last stage writes through `out` (last_stage_target is the buffer it
-// does not read)
-template <int L, int LOGC, bool kFwd, int T, int... Rs, class In, class Out, class Hook = CtNoHook>
-__device__ __forceinline__ void smem_fft_ct(In in, Out out, const double2* __restrict__ tw, double2* buf0, double2* buf1,
-                                            Hook hook = Hook{}) {
-  stages_ct_impl<L, LOGC, kFwd, T, 1, 0>(0, in, out, tw, buf0, buf1, hook, std::integer_sequence<int, Rs...>{});
+// does not read).  The transform length is the product of the radices.
+template <int LOGC, bool kFwd, int T, int... Rs, class In, class Out, class Hook = CtNoHook>
+__device__ __forceinline__ void smem_fft_ct(std::integer_sequence<int, Rs...> radices, In in, Out out,
+                                            const double2* __restrict__ tw, double2* buf0, double2* buf1, Hook hook = Hook{}) {
+  stages_ct_impl<(Rs * ...), LOGC, kFwd, T, 1, 0>(0, in, out, tw, buf0, buf1, hook, radices);
 }
-struct CtRowsTileIn {
-  WFM_NO_RUN_TWIDDLE
-  const double2* t;  // [c][p]
-  int N2;
-  __device__ __forceinline__ double2 operator()(int p, int c, int) const { return t[c * N2 + p]; }
-};
-struct CtRowsTileOut {
-  WFM_NO_RUN_TWIDDLE
-  double2* t;  // [c][p]
-  int N2;
-  __device__ __forceinline__ void operator()(int p, int c, int, double2 v) const { t[c * N2 + p] = v; }
-};
-struct CtRowsTileMulHOut {
-  WFM_NO_RUN_TWIDDLE
-  double2* z;        // interleaved
-  const double2* h;  // [c][p]
-  int N2;
-  __device__ __forceinline__ void operator()(int p, int c, int e, double2 v) const { z[e] = cmul(v, h[c * N2 + p]); }
-};
+// the compile-time plans: 625 = 5^4 (column passes of n = 400 000) and 640 = 10 x 8 x 8 (the passes of n = 409 600)
+using Radices625 = std::integer_sequence<int, 5, 5, 5, 5>;
+using Radices640 = std::integer_sequence<int, 10, 8, 8>;
+// entries of a plan's compact twiddle table: the sum of the stage strides 1, R0, R0 R1, ...
+template <int... Rs>
+__host__ __device__ constexpr int ct_twiddle_count(std::integer_sequence<int, Rs...>) {
+  int n = 0, ns = 1;
+  ((n += ns, ns *= Rs), ...);
+  return n;
+}
+// stride of a plan's last stage: L / last radix
+template <int... Rs>
+__host__ __device__ constexpr int ct_last_stride(std::integer_sequence<int, Rs...>) {
+  int ns = 1, last = 1;
+  ((ns *= Rs, last = Rs), ...);
+  return ns / last;
+}
 
 // ---- four-step, kernel A / C: column transforms of length N1 -----------------------
 // element (r, n2) of the [N1][N2] view; C = 2^logc adjacent columns per CTA.  The inter-pass
 // twiddle W_n^(sgn * r * n2) (r * n2 < n: no reduction needed) is applied after the
 // transform (first pass of a forward-structured transform) or before it (last pass of the
 // fused filter, undoing the forward pass)
-// column pass: 4 interleaved columns per CTA and two CTAs per SM (32 warps) measured 14 % faster
-// than 8 columns and one CTA (cfg4, n = 625 x 640)
-#ifndef WFM_FFT_COLS_MINB
-#define WFM_FFT_COLS_MINB 2
-#endif
-#ifndef WFM_FFT_COLS_LOGC
-#define WFM_FFT_COLS_LOGC 2
-#endif
 // kRealIn / kRealOut: the signal index is a PAIR of real signals packed as the real and
 // imaginary part of one complex signal (the filter's response is Hermitian); pb == nullptr
 // for the odd tail
@@ -592,7 +492,7 @@ struct ColsIn {
   int N2, c0, cw;
   double sgn;
   int64_t nv;  // real input: samples the signals hold (zeros beyond)
-  __device__ __forceinline__ double2 operator()(int r, int c) const {
+  __device__ __forceinline__ double2 operator()(int r, int c, int) const {
     double2 v = make_double2(0.0, 0.0);
     if (c < cw) {
       const int64_t idx = (int64_t)r * N2 + c0 + c;
@@ -638,7 +538,7 @@ struct ColsOut {
     if (!kTwAfter || c >= cw) return;
     if (pre_w) {
       double2 w = pre_w[threadIdx.x];
-      const double2 ws = pre_w[blockDim.x + c];
+      const double2 ws = pre_w[kFftColsThreads + c];
 #pragma unroll
       for (int q = 0; q < R; ++q) {
         v[q] = cmul(v[q], w);
@@ -654,7 +554,7 @@ struct ColsOut {
       if (q + 1 < R) w = cmul(w, ws);
     }
   }
-  __device__ __forceinline__ void operator()(int r, int c, double2 v) const {
+  __device__ __forceinline__ void operator()(int r, int c, int, double2 v) const {
     if (c >= cw) return;
     const int64_t idx = (int64_t)r * N2 + c0 + c;
     if (kRealOut) {
@@ -667,18 +567,17 @@ struct ColsOut {
   }
 };
 template <bool kTwAfter, bool kRealIn, bool kRealOut>
-__global__ void __launch_bounds__(kFftColsThreads, WFM_FFT_COLS_MINB) fft_cols_kernel(FftPlan P, BigTwiddle T, int N2, int logc,
+__global__ void __launch_bounds__(kFftColsThreads, kFftColsMinBlocks) fft_cols_kernel(FftPlan P, BigTwiddle T, int N2, int logc,
                                                                const void* __restrict__ in, void* __restrict__ out,
                                                                int64_t in_stride, int64_t out_stride, double sgn,
                                                                double scale, int64_t n_real, int64_t nv) {
   const int N1 = P.L, C = 1 << logc;
   double2* a = reinterpret_cast<double2*>(fft_smem_raw);
-  double2* b = a + padded_points((size_t)N1 << logc);
-  const bool ct = WFM_FFT_CT && (P.L == 625 || (WFM_FFT_CT_COLS_640 && P.L == 640)) && logc == 2 && P.tw_in_smem && blockDim.x == 512 &&
-                  (kTwAfter ? sgn < 0.0 : sgn > 0.0);
+  double2* b = a + ((size_t)N1 << logc);
+  const bool ct = (P.L == 625 || P.L == 640) && logc == kFftColsLogC && P.tw_in_smem && (kTwAfter ? sgn < 0.0 : sgn > 0.0);
   // (the compile-time path parks its tables behind the first stage's barrier instead of staging them in a phase of
   // their own: one barrier-bounded phase less in a tile that lives for 8 us)
-  const double2* tw = ct ? P.twc : stage_twiddles(P, b + padded_points((size_t)N1 << logc));
+  const double2* tw = ct ? P.twc : stage_twiddles(P, b + ((size_t)N1 << logc));
   const int c0 = blockIdx.x << logc;
   const int cw = min(C, N2 - c0);
   const int64_t sig = blockIdx.y;
@@ -708,33 +607,39 @@ __global__ void __launch_bounds__(kFftColsThreads, WFM_FFT_COLS_MINB) fft_cols_k
     // twiddles and, for the pass that applies the inter-pass twiddles at its END, this thread's W^(j col) with the four
     // per-column steps W^(Ns col).  (By source line 24 % of the stall samples of these passes were first uses of such
     // look-ups, L1 misses behind the streaming signal.)
-    double2* tws = b + padded_points((size_t)N1 << logc);  // compact twiddles (<= 160), then blockDim + C run twiddles
-    double2* pre = tws + 160;
+    // Thread t fetches compact twiddle t; in the last stage thread t runs butterfly t (column t % kCols, first output row
+    // t / kCols, step Ns) and the last kCols threads fetch the per-column steps.
+    constexpr int kCols = 1 << kFftColsLogC;
+    constexpr int kTwSlot = 160;                         // compact twiddles, then kFftColsThreads + kCols run twiddles
+    constexpr int kStepThread = kFftColsThreads - kCols;  // thread kStepThread + c fetches the step of column c
+    static_assert(ct_twiddle_count(Radices625{}) <= kTwSlot && ct_twiddle_count(Radices640{}) <= kTwSlot, "twiddle slot");
+    static_assert(kCols * ct_last_stride(Radices625{}) <= kStepThread && kCols * ct_last_stride(Radices640{}) <= kStepThread,
+                  "one last-stage butterfly per thread, below the step threads");
+    double2* tws = b + ((size_t)N1 << logc);
+    double2* pre = tws + kTwSlot;
     const int tid = (int)threadIdx.x;
     const bool l625 = P.L == 625;
-    const int n_tw = l625 ? 156 : 91, ns_last = l625 ? 125 : 80;  // last stage: radix 5 resp. 8, butterfly tid of ns_last * 4
+    const int n_tw = l625 ? ct_twiddle_count(Radices625{}) : ct_twiddle_count(Radices640{});
+    const int ns_last = l625 ? ct_last_stride(Radices625{}) : ct_last_stride(Radices640{});
     double2 twv = make_double2(0.0, 0.0), wv = make_double2(0.0, 0.0);
     if (tid < n_tw) twv = __ldg(P.twc + tid);
     if (kTwAfter) {
-      // last stage: butterfly tid -> column tid & 3, first output row tid >> 2 (< Ns), step Ns
-      const int c = tid & 3, j = tid >> 2;
-      if (tid < 4 * ns_last && c < cw) wv = big_twiddle(T, (int64_t)j * (c0 + c), sgn);
-      else if (tid >= 508 && tid - 508 < cw) wv = big_twiddle(T, (int64_t)ns_last * (c0 + tid - 508), sgn);
+      const int c = tid & (kCols - 1), j = tid >> kFftColsLogC;
+      if (tid < kCols * ns_last && c < cw) wv = big_twiddle(T, (int64_t)j * (c0 + c), sgn);
+      else if (tid >= kStepThread && tid - kStepThread < cw) wv = big_twiddle(T, (int64_t)ns_last * (c0 + tid - kStepThread), sgn);
       dst.pre_w = pre;
     }
     auto park = [&]() {
       if (tid < n_tw) tws[tid] = twv;
       if (kTwAfter) {
-        if (tid < 4 * ns_last) pre[tid] = wv;
-        else if (tid >= 508) pre[kFftColsThreads + tid - 508] = wv;
+        if (tid < kCols * ns_last) pre[tid] = wv;
+        else if (tid >= kStepThread) pre[kFftColsThreads + tid - kStepThread] = wv;
       }
     };
     if (l625)
-      smem_fft_ct<625, 2, kTwAfter, kFftColsThreads, 5, 5, 5, 5>(CtWrapIn<ColsIn<!kTwAfter, kRealIn>>{src},
-                                                                       CtWrapOut<ColsOut<kTwAfter, kRealOut>>{dst}, tws, a, b, park);
+      smem_fft_ct<kFftColsLogC, kTwAfter, kFftColsThreads>(Radices625{}, src, dst, tws, a, b, park);
     else
-      smem_fft_ct<640, 2, kTwAfter, kFftColsThreads, 10, 8, 8>(CtWrapIn<ColsIn<!kTwAfter, kRealIn>>{src},
-                                                                     CtWrapOut<ColsOut<kTwAfter, kRealOut>>{dst}, tws, a, b, park);
+      smem_fft_ct<kFftColsLogC, kTwAfter, kFftColsThreads>(Radices640{}, src, dst, tws, a, b, park);
     return;
   }
   smem_fft(P, logc, sgn, tw, src, dst, a, b);
@@ -744,17 +649,11 @@ __global__ void __launch_bounds__(kFftColsThreads, WFM_FFT_COLS_MINB) fft_cols_k
 // C = 2^logc adjacent rows per CTA.
 // kFilter: FFT -> * Hp[k1*N2 + k2] -> IFFT, in place (spectrum stays transposed)
 // else   : FFT (sgn) and scatter to natural order out[k1 + N1*k2], scaled
-#ifndef WFM_FFT_ROWS_MINB
-#define WFM_FFT_ROWS_MINB 3
-#endif
-#ifndef WFM_FFT_ROWS_LOGC
-#define WFM_FFT_ROWS_LOGC 1
-#endif
 struct RowsIn {
   WFM_NO_RUN_TWIDDLE
   const double2* rows;  // first row of the tile
   int N2, rw;
-  __device__ __forceinline__ double2 operator()(int p, int c) const {
+  __device__ __forceinline__ double2 operator()(int p, int c, int) const {
     return c < rw ? rows[(int64_t)c * N2 + p] : make_double2(0.0, 0.0);
   }
 };
@@ -762,7 +661,7 @@ struct RowsOut {
   WFM_NO_RUN_TWIDDLE
   double2* rows;
   int N2, rw;
-  __device__ __forceinline__ void operator()(int p, int c, double2 v) const {
+  __device__ __forceinline__ void operator()(int p, int c, int, double2 v) const {
     if (c < rw) rows[(int64_t)c * N2 + p] = v;
   }
 };
@@ -770,10 +669,10 @@ struct RowsMulHOut {
   WFM_NO_RUN_TWIDDLE
   double2* z;
   const double2* __restrict__ hrows;  // Hp at the tile's first row
-  int N2, rw, logc;
-  __device__ __forceinline__ void operator()(int p, int c, double2 v) const {
+  int N2, rw;
+  __device__ __forceinline__ void operator()(int p, int c, int e, double2 v) const {
     if (c < rw) v = cmul(v, __ldg(hrows + (int64_t)c * N2 + p));
-    z[spad((p << logc) + c)] = v;
+    z[e] = v;
   }
 };
 struct NaturalOut {
@@ -781,33 +680,31 @@ struct NaturalOut {
   double2* o;
   int N1, rw;
   double scale;
-  __device__ __forceinline__ void operator()(int p, int c, double2 v) const {
+  __device__ __forceinline__ void operator()(int p, int c, int, double2 v) const {
     if (c < rw) o[(int64_t)c + (int64_t)N1 * p] = cscale(v, scale);
   }
 };
 template <bool kFilter>
-__global__ void __launch_bounds__(kFftRowsThreads, WFM_FFT_ROWS_MINB) fft_rows_kernel(FftPlan P, int N1, int logc, double2* __restrict__ data,
+__global__ void __launch_bounds__(kFftRowsThreads, kFftRowsMinBlocks) fft_rows_kernel(FftPlan P, int N1, int logc, double2* __restrict__ data,
                                                                double2* __restrict__ out, int64_t stride,
                                                                int64_t out_stride, const double2* __restrict__ Hp,
                                                                double sgn, double scale) {
   const int N2 = P.L, C = 1 << logc;
   double2* a = reinterpret_cast<double2*>(fft_smem_raw);
-  double2* b = a + padded_points((size_t)N2 << logc);
-  const double2* tw = stage_twiddles(P, b + padded_points((size_t)N2 << logc));
+  double2* b = a + ((size_t)N2 << logc);
+  const double2* tw = stage_twiddles(P, b + ((size_t)N2 << logc));
   const int r0 = blockIdx.x << logc;
   const int rw = min(C, N1 - r0);
   const int64_t sig = blockIdx.y;
   double2* rows = data + sig * stride + (int64_t)r0 * N2;
   if (kFilter) {
     double2* z = last_stage_target(P, a, b);
-    smem_fft(P, logc, -1.0, tw, RowsIn{rows, N2, rw}, RowsMulHOut{z, Hp + (int64_t)r0 * N2, N2, rw, logc}, a, b);
-    smem_fft(P, logc, +1.0, tw, SmemIn{z, logc}, RowsOut{rows, N2, rw}, z == a ? b : a, z);
+    smem_fft(P, logc, -1.0, tw, RowsIn{rows, N2, rw}, RowsMulHOut{z, Hp + (int64_t)r0 * N2, N2, rw}, a, b);
+    smem_fft(P, logc, +1.0, tw, SmemIn{z}, RowsOut{rows, N2, rw}, z == a ? b : a, z);
   } else {
     smem_fft(P, logc, sgn, tw, RowsIn{rows, N2, rw}, NaturalOut{out + sig * out_stride + r0, N1, rw, scale}, a, b);
   }
 }
-
-
 
 // ---- kernel B with TMA: the tile's rows are ONE contiguous span of the scratch ---------------------------------------
 // C adjacent rows of the [N1][N2] scratch are rw * N2 consecutive complex numbers, and so are the rows of the permuted
@@ -853,22 +750,27 @@ struct RowsTileIn {
   WFM_NO_RUN_TWIDDLE
   const double2* t;  // [c][p]
   int N2;
-  __device__ __forceinline__ double2 operator()(int p, int c) const { return t[c * N2 + p]; }
+  __device__ __forceinline__ double2 operator()(int p, int c, int) const { return t[c * N2 + p]; }
 };
 struct RowsTileOut {
   WFM_NO_RUN_TWIDDLE
   double2* t;  // [c][p]
   int N2;
-  __device__ __forceinline__ void operator()(int p, int c, double2 v) const { t[c * N2 + p] = v; }
+  __device__ __forceinline__ void operator()(int p, int c, int, double2 v) const { t[c * N2 + p] = v; }
 };
 struct RowsTileMulHOut {
   WFM_NO_RUN_TWIDDLE
-  double2* z;          // interleaved [(p << logc) + c]
+  double2* z;          // interleaved [e]
   const double2* h;    // the response rows of the tile in shared memory, [c][p]
-  int N2, logc;
-  __device__ __forceinline__ void operator()(int p, int c, double2 v) const { z[spad((p << logc) + c)] = cmul(v, h[c * N2 + p]); }
+  int N2;
+  __device__ __forceinline__ void operator()(int p, int c, int e, double2 v) const { z[e] = cmul(v, h[c * N2 + p]); }
 };
-__global__ void __launch_bounds__(kFftRowsThreads, WFM_FFT_ROWS_MINB) fft_rows_tma_kernel(FftPlan P, int N1, int logc,
+// dynamic shared memory of fft_rows_tma_kernel: what the row plan's buffers and table take (plan_smem, from get_plan),
+// the tile's response rows, kRowPad elements behind every row of the three, and the two mbarriers
+static size_t rows_tma_smem(size_t plan_smem, int L, int logc) {
+  return plan_smem + sizeof(double2) * (((size_t)L << logc) + 3 * ((size_t)kRowPad << logc)) + 16;
+}
+__global__ void __launch_bounds__(kFftRowsThreads, kFftRowsMinBlocks) fft_rows_tma_kernel(FftPlan P, int N1, int logc,
                                                                                          double2* __restrict__ data, int64_t stride,
                                                                                          const double2* __restrict__ Hp) {
   const int N2 = P.L, C = 1 << logc;
@@ -893,7 +795,7 @@ __global__ void __launch_bounds__(kFftRowsThreads, WFM_FFT_ROWS_MINB) fft_rows_t
     fft_mbar_expect_tx(bar + 1, row_bytes * rw);
     for (int c = 0; c < rw; ++c) fft_bulk_g2s(h + (size_t)c * RS, Hp + (int64_t)(r0 + c) * N2, row_bytes, bar + 1);
   }
-  const bool ct = WFM_FFT_CT && P.L == 640 && logc == 1;
+  const bool ct = P.L == 640 && logc == kFftRowsLogC;
   const double2* tw = stage_twiddles(P, twp);  // (the launch requires the table in shared memory)
   __syncthreads();  // the barriers are initialised (and the twiddles staged) for every thread
   fft_mbar_wait(bar, 0);
@@ -903,15 +805,16 @@ __global__ void __launch_bounds__(kFftRowsThreads, WFM_FFT_ROWS_MINB) fft_rows_t
   double2* o = b;
   if (ct) {
     // 640 = 10 x 8 x 8, two rows: b -> a -> b -> (x H) a;  a -> b -> a -> b
-    smem_fft_ct<640, 1, true, kFftRowsThreads, 10, 8, 8>(CtRowsTileIn{b, 640 + kRowPad}, CtRowsTileMulHOut{a, h, 640 + kRowPad}, twp, a, b);
-    smem_fft_ct<640, 1, false, kFftRowsThreads, 10, 8, 8>(CtSmemIn{a}, CtRowsTileOut{b, 640 + kRowPad}, twp, b, a);
+    smem_fft_ct<kFftRowsLogC, true, kFftRowsThreads>(Radices640{}, RowsTileIn{b, 640 + kRowPad}, RowsTileMulHOut{a, h, 640 + kRowPad},
+                                                     twp, a, b);
+    smem_fft_ct<kFftRowsLogC, false, kFftRowsThreads>(Radices640{}, SmemIn{a}, RowsTileOut{b, 640 + kRowPad}, twp, b, a);
   } else {
     // (either buffer may end up holding the padded output rows: both have room for them)
     double2* z = last_stage_target(P, a, b);
-    smem_fft(P, logc, -1.0, tw, RowsTileIn{b, RS}, RowsTileMulHOut{z, h, RS, logc}, a, b);
+    smem_fft(P, logc, -1.0, tw, RowsTileIn{b, RS}, RowsTileMulHOut{z, h, RS}, a, b);
     double2* w0 = z == a ? b : a;
     double2* oo = last_stage_target(P, w0, z);
-    smem_fft(P, logc, +1.0, tw, SmemIn{z, logc}, RowsTileOut{oo, RS}, w0, z);
+    smem_fft(P, logc, +1.0, tw, SmemIn{z}, RowsTileOut{oo, RS}, w0, z);
     o = oo;
   }
   asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // this thread's tile writes -> the async proxy
@@ -926,19 +829,19 @@ __global__ void __launch_bounds__(kFftRowsThreads, WFM_FFT_ROWS_MINB) fft_rows_t
 struct PlainIn {
   WFM_NO_RUN_TWIDDLE
   const double2* d;
-  __device__ __forceinline__ double2 operator()(int p, int) const { return d[p]; }
+  __device__ __forceinline__ double2 operator()(int p, int, int) const { return d[p]; }
 };
 struct PlainOut {
   WFM_NO_RUN_TWIDDLE
   double2* d;
   double scale;
-  __device__ __forceinline__ void operator()(int p, int, double2 v) const { d[p] = cscale(v, scale); }
+  __device__ __forceinline__ void operator()(int p, int, int, double2 v) const { d[p] = cscale(v, scale); }
 };
 __global__ void __launch_bounds__(kFftThreads) fft_c2c_single_kernel(FftPlan P, double2* __restrict__ data,
                                                                      int64_t stride, double sgn, double scale) {
   double2* a = reinterpret_cast<double2*>(fft_smem_raw);
-  double2* b = a + padded_points(P.L);
-  const double2* tw = stage_twiddles(P, b + padded_points(P.L));
+  double2* b = a + P.L;
+  const double2* tw = stage_twiddles(P, b + P.L);
   double2* d = data + (int64_t)blockIdx.x * stride;
   smem_fft(P, 0, sgn, tw, PlainIn{d}, PlainOut{d, scale}, a, b);
 }
@@ -1003,57 +906,24 @@ __global__ void complex_to_real_kernel(const double2* __restrict__ c, int64_t n,
 }
 
 // =============================== host side =============================================
+// the radix sequence of a length-n transform (distortion._fft_radices mirrors it): false if n is not 7-smooth.  The
+// plan fixes the rounding of the transform, so the sequence must not change.
 static bool factor_smooth(int64_t n, int* radix, int* n_stage) {
   int k = 0;
-#if WFM_FFT_BIG_RADIX >= 2
-  while (n % 25 == 0) {
-    if (k >= kMaxStages) return false;
-    radix[k++] = 25;
-    n /= 25;
-  }
-#endif
-#if WFM_FFT_BIG_RADIX
-  if (n % 10 == 0) {  // a 5 takes the lone 2 the larger power-of-two butterflies would leave over
+  if (n % 10 == 0) {  // a 5 takes the lone 2 the radix-8 stages would leave over
     int e = 0;
     for (int64_t m = n; m % 2 == 0; m /= 2) ++e;
-    const int per = WFM_FFT_MAX_RADIX >= 16 ? 4 : (WFM_FFT_MAX_RADIX >= 8 ? 3 : 2);
-    if (e % per == 1) {
-      if (k >= kMaxStages) return false;
+    if (e % 3 == 1) {
       radix[k++] = 10;
       n /= 10;
     }
   }
-#endif
-  for (int r : {7, 5, 3}) {
+  for (int r : {7, 5, 3, 8, 4, 2}) {
     while (n % r == 0) {
       if (k >= kMaxStages) return false;
       radix[k++] = r;
       n /= r;
     }
-  }
-#if WFM_FFT_MAX_RADIX >= 16
-  while (n % 16 == 0) {
-    if (k >= kMaxStages) return false;
-    radix[k++] = 16;
-    n /= 16;
-  }
-#endif
-#if WFM_FFT_MAX_RADIX >= 8
-  while (n % 8 == 0) {
-    if (k >= kMaxStages) return false;
-    radix[k++] = 8;
-    n /= 8;
-  }
-#endif
-  while (n % 4 == 0) {
-    if (k >= kMaxStages) return false;
-    radix[k++] = 4;
-    n /= 4;
-  }
-  while (n % 2 == 0) {
-    if (k >= kMaxStages) return false;
-    radix[k++] = 2;
-    n /= 2;
   }
   *n_stage = k;
   return n == 1;
@@ -1087,7 +957,7 @@ static cudaError_t get_plan(int L, int64_t points, FftPlan* plan, size_t* smem) 
     plan->inv_ns[s] = (uint32_t)(((uint64_t(1) << 32) + ns - 1) / ns);  // exact quotient for j < 2^16
     ns *= plan->radix[s];
   }
-  const size_t buffers = 2 * sizeof(double2) * padded_points((size_t)points) + kPlanSlackBytes;
+  const size_t buffers = 2 * sizeof(double2) * (size_t)points + kPlanSlackBytes;
   plan->tw_in_smem = buffers + sizeof(double2) * (size_t)L <= (size_t)kSmemBudget;
   *smem = buffers + (plan->tw_in_smem ? sizeof(double2) * (size_t)L : 0);
   int dev = 0;
@@ -1162,6 +1032,16 @@ static bool split_two_level(int64_t n, int* N1, int* N2) {
   return true;
 }
 
+// how a length-n transform runs: one CTA per transform, four-step over the split n = N1 * N2, or (a prime factor > 7, or
+// no split) through Bluestein's 7-smooth transforms
+enum FftPath { kPathSingle, kPathTwoLevel, kPathGeneric };
+static FftPath choose_path(int64_t n, int* N1, int* N2) {
+  const bool smooth = is_smooth(n);
+  if (smooth && n <= kMaxPoints) return kPathSingle;
+  if (smooth && split_two_level(n, N1, N2)) return kPathTwoLevel;
+  return kPathGeneric;
+}
+
 static int64_t next_smooth(int64_t m) {
   while (!is_smooth(m)) ++m;
   return m;
@@ -1197,11 +1077,42 @@ static int tile_logc(int L, int want_log) {
   return lc;
 }
 
+// What the four-step transform of length n = N1 * N2 (choose_path) needs for n_tr transforms: the plans of the column
+// pass (length N1) and of the row pass (length N2), the inter-pass twiddles, a scratch of n complex points per
+// transform and both grids.  On success the caller owns the scratch and cudaFreeAsync's it on the stream.
+struct TwoLevel {
+  int lc1, lc2;  // log2 of the columns / rows per CTA
+  FftPlan P1, P2;
+  size_t smem1, smem2;
+  BigTwiddle T;
+  dim3 g1, g2;
+  double2* scratch;
+};
+static cudaError_t two_level_setup(int64_t n, int N1, int N2, int64_t n_tr, cudaStream_t st, TwoLevel* t) {
+  cudaError_t e;
+  t->lc1 = tile_logc(N1, kFftColsLogC);
+  t->lc2 = tile_logc(N2, kFftRowsLogC);
+  if ((e = get_plan(N1, (int64_t)N1 << t->lc1, &t->P1, &t->smem1)) != cudaSuccess) return e;
+  if ((e = get_plan(N2, (int64_t)N2 << t->lc2, &t->P2, &t->smem2)) != cudaSuccess) return e;
+  if ((e = get_big_twiddle(n, &t->T)) != cudaSuccess) return e;
+  const int C1 = 1 << t->lc1, C2 = 1 << t->lc2;
+  t->g1 = dim3((unsigned)((N2 + C1 - 1) / C1), (unsigned)n_tr);
+  t->g2 = dim3((unsigned)((N1 + C2 - 1) / C2), (unsigned)n_tr);
+  // (Measured and rejected: running the three passes of the filter group by group of signal pairs so that a group's
+  // scratch stays in the 126 MB L2 — 2.39 ms at 22 pairs per group .. 3.87 ms at 2 against 2.19 ms for one group: the
+  // passes are bound on the SM (L1TEX 63-76 %, issue 43-52 %), not by HBM, and smaller grids add tails.)
+  keep_pool_memory();
+  t->scratch = nullptr;
+  return cudaMallocAsync(&t->scratch, sizeof(double2) * (size_t)n * (size_t)n_tr, st);
+}
+
 // plain complex transform of n_sig signals, natural order, in place; n 7-smooth
 static cudaError_t c2c_smooth(double2* data, int64_t n_sig, int64_t n, int64_t stride, double sgn, double scale,
                               cudaStream_t st) {
   cudaError_t e;
-  if (n <= kMaxPoints) {
+  int N1 = 0, N2 = 0;
+  const FftPath path = choose_path(n, &N1, &N2);
+  if (path == kPathSingle) {
     FftPlan P;
     size_t smem;
     if ((e = get_plan((int)n, n, &P, &smem)) != cudaSuccess) return e;
@@ -1209,28 +1120,18 @@ static cudaError_t c2c_smooth(double2* data, int64_t n_sig, int64_t n, int64_t s
     fft_c2c_single_kernel<<<(unsigned)n_sig, kFftThreads, smem, st>>>(P, data, stride, sgn, scale);
     return cudaGetLastError();
   }
-  int N1, N2;
-  if (!split_two_level(n, &N1, &N2)) return cudaErrorNotSupported;
-  const int lc1 = tile_logc(N1, WFM_FFT_COLS_LOGC), lc2 = tile_logc(N2, WFM_FFT_ROWS_LOGC);
-  FftPlan P1, P2;
-  BigTwiddle T;
-  size_t smem1, smem2;
-  if ((e = get_plan(N1, (int64_t)N1 << lc1, &P1, &smem1)) != cudaSuccess) return e;
-  if ((e = get_plan(N2, (int64_t)N2 << lc2, &P2, &smem2)) != cudaSuccess) return e;
-  if ((e = get_big_twiddle(n, &T)) != cudaSuccess) return e;
-  keep_pool_memory();
-  double2* scratch = nullptr;
-  if ((e = cudaMallocAsync(&scratch, sizeof(double2) * (size_t)n * (size_t)n_sig, st)) != cudaSuccess) return e;
-  const int C1 = 1 << lc1, C2 = 1 << lc2;
-  dim3 g1((unsigned)((N2 + C1 - 1) / C1), (unsigned)n_sig), g2((unsigned)((N1 + C2 - 1) / C2), (unsigned)n_sig);
-  if ((e = set_smem(fft_cols_kernel<true, false, false>, smem1)) != cudaSuccess) goto done;
-  fft_cols_kernel<true, false, false><<<g1, kFftColsThreads, smem1, st>>>(P1, T, N2, lc1, data, scratch, stride, n, sgn, 1.0, 0, n);
+  if (path != kPathTwoLevel) return cudaErrorNotSupported;
+  TwoLevel t;
+  if ((e = two_level_setup(n, N1, N2, n_sig, st, &t)) != cudaSuccess) return e;
+  if ((e = set_smem(fft_cols_kernel<true, false, false>, t.smem1)) != cudaSuccess) goto done;
+  fft_cols_kernel<true, false, false><<<t.g1, kFftColsThreads, t.smem1, st>>>(t.P1, t.T, N2, t.lc1, data, t.scratch, stride, n,
+                                                                             sgn, 1.0, 0, n);
   if ((e = cudaGetLastError()) != cudaSuccess) goto done;
-  if ((e = set_smem(fft_rows_kernel<false>, smem2)) != cudaSuccess) goto done;
-  fft_rows_kernel<false><<<g2, kFftRowsThreads, smem2, st>>>(P2, N1, lc2, scratch, data, n, stride, nullptr, sgn, scale);
+  if ((e = set_smem(fft_rows_kernel<false>, t.smem2)) != cudaSuccess) goto done;
+  fft_rows_kernel<false><<<t.g2, kFftRowsThreads, t.smem2, st>>>(t.P2, N1, t.lc2, t.scratch, data, n, stride, nullptr, sgn, scale);
   e = cudaGetLastError();
 done:
-  cudaFreeAsync(scratch, st);
+  cudaFreeAsync(t.scratch, st);
   return e;
 }
 
@@ -1238,14 +1139,10 @@ done:
 static cudaError_t c2c_any(double2* data, int64_t n_sig, int64_t n, int64_t stride, double sgn, double scale,
                            cudaStream_t st) {
   if (n <= 1) return cudaSuccess;
-  if (is_smooth(n) && (n <= kMaxPoints || [&] { int a, b; return split_two_level(n, &a, &b); }())) {
-    return c2c_smooth(data, n_sig, n, stride, sgn, scale, st);
-  }
+  int N1, N2;
+  if (choose_path(n, &N1, &N2) != kPathGeneric) return c2c_smooth(data, n_sig, n, stride, sgn, scale, st);
   const int64_t M = next_smooth(2 * n - 1);
-  {
-    int a, b;
-    if (M > kMaxPoints && !split_two_level(M, &a, &b)) return cudaErrorNotSupported;
-  }
+  if (choose_path(M, &N1, &N2) == kPathGeneric) return cudaErrorNotSupported;
   double2 *A = nullptr, *B = nullptr;
   cudaError_t e;
   if ((e = cudaMallocAsync(&A, sizeof(double2) * (size_t)M * (size_t)n_sig, st)) != cudaSuccess) return e;
@@ -1267,6 +1164,13 @@ done:
   return e;
 }
 
+// the library's status for what the transforms return: cudaErrorNotSupported stands for a length or layout they do not
+// handle
+static int fft_status(cudaError_t e) {
+  if (e == cudaErrorNotSupported) return WFM_EUNSUPPORTED;
+  return e == cudaSuccess ? WFM_OK : WFM_ECUDA;
+}
+
 }  // namespace wfm
 
 extern "C" int wfm_fft_c2c(double* data, int64_t n_sig, int64_t n, int64_t stride, int32_t sign, void* stream) {
@@ -1274,9 +1178,7 @@ extern "C" int wfm_fft_c2c(double* data, int64_t n_sig, int64_t n, int64_t strid
   if (!data || n_sig < 0 || n < 0 || (sign != 1 && sign != -1) || (n_sig > 1 && stride < n)) return WFM_EINVAL;
   if (n_sig == 0 || n == 0) return WFM_OK;
   const double scale = sign > 0 ? 1.0 / (double)n : 1.0;
-  cudaError_t e = c2c_any(reinterpret_cast<double2*>(data), n_sig, n, stride, (double)sign, scale, (cudaStream_t)stream);
-  if (e == cudaErrorNotSupported) return WFM_EUNSUPPORTED;
-  return e == cudaSuccess ? WFM_OK : WFM_ECUDA;
+  return fft_status(c2c_any(reinterpret_cast<double2*>(data), n_sig, n, stride, (double)sign, scale, (cudaStream_t)stream));
 }
 
 namespace wfm {
@@ -1335,13 +1237,6 @@ static thread_local HStage g_hstage;
 // single-CTA and generic paths: the Hermitian part in natural order; two-level path: the
 // Hermitian part in the transposed order the row pass produces.
 namespace wfm {
-enum FilterPath { kPathSingle, kPathTwoLevel, kPathGeneric };
-static FilterPath choose_path(int64_t n, int* N1, int* N2) {
-  const bool smooth = is_smooth(n);
-  if (smooth && n <= kMaxPoints) return kPathSingle;
-  if (smooth && split_two_level(n, N1, N2)) return kPathTwoLevel;
-  return kPathGeneric;
-}
 // dH: natural-order response on the device -> ready (n complex, caller-allocated)
 static cudaError_t prepare_response(const double2* dH, double2* ready, int64_t n, cudaStream_t st) {
   int N1 = 0, N2 = 0;
@@ -1355,83 +1250,61 @@ static cudaError_t prepare_response(const double2* dH, double2* ready, int64_t n
 // y = real(ifft(fft(x) * H)) with the response already prepared (prepare_response)
 // n: transform length; nv <= n: samples the signals hold (the rest of the circular grid is zero padding that is never
 // read or written: x and y are n_sig rows of nv samples at their pitches)
-static int run_filter(const double* x, double* y, int64_t n_sig, int64_t n, int64_t x_stride, int64_t y_stride,
-                      const double2* ready, cudaStream_t st, int64_t nv = -1) {
+static cudaError_t run_filter(const double* x, double* y, int64_t n_sig, int64_t n, int64_t x_stride, int64_t y_stride,
+                              const double2* ready, cudaStream_t st, int64_t nv = -1) {
   if (nv < 0) nv = n;
-  cudaError_t e = cudaSuccess;
-  int rc = WFM_OK;
+  cudaError_t e;
   int N1 = 0, N2 = 0;
-  const FilterPath path = choose_path(n, &N1, &N2);
+  const FftPath path = choose_path(n, &N1, &N2);
   const int64_t n_pair = (n_sig + 1) / 2;  // two real signals per complex transform
-  const int T = 256;
-  const unsigned gH = (unsigned)((n + T - 1) / T);
   if (path == kPathSingle) {
     FftPlan P;
     size_t smem;
-    e = get_plan((int)n, n, &P, &smem);
-    if (e == cudaSuccess) e = set_smem(fft_filter_single_kernel, smem);
-    if (e == cudaSuccess) {
-      fft_filter_single_kernel<<<(unsigned)n_pair, kFftThreads, smem, st>>>(P, x, y, x_stride, y_stride, n_sig, ready, (int)nv);
-      e = cudaGetLastError();
-    }
-  } else if (path == kPathTwoLevel) {
-    const int lc1 = tile_logc(N1, WFM_FFT_COLS_LOGC), lc2 = tile_logc(N2, WFM_FFT_ROWS_LOGC);
-    FftPlan P1, P2;
-    BigTwiddle BT;
-    size_t smem1 = 0, smem2 = 0;
-    double2* scratch = nullptr;
-    e = get_plan(N1, (int64_t)N1 << lc1, &P1, &smem1);
-    if (e == cudaSuccess) e = get_plan(N2, (int64_t)N2 << lc2, &P2, &smem2);
-    if (e == cudaSuccess) e = get_big_twiddle(n, &BT);
-    // (Measured and rejected: running the three passes group by group of signal pairs so that a group's scratch stays in
-    // the 126 MB L2 — 2.39 ms at 22 pairs per group .. 3.87 ms at 2 against 2.19 ms for one group: the passes are bound
-    // on the SM (L1TEX 63-76 %, issue 43-52 %), not by HBM, and smaller grids add tails.)
-    if (e == cudaSuccess) e = cudaMallocAsync(&scratch, sizeof(double2) * (size_t)n * (size_t)n_pair, st);
-    const int C1 = 1 << lc1, C2 = 1 << lc2;
-    dim3 g1((unsigned)((N2 + C1 - 1) / C1), (unsigned)n_pair), g2((unsigned)((N1 + C2 - 1) / C2), (unsigned)n_pair);
-    if (e == cudaSuccess) e = set_smem(fft_cols_kernel<true, true, false>, smem1);
-    if (e == cudaSuccess) e = set_smem(fft_cols_kernel<false, false, true>, smem1);
-    if (e == cudaSuccess) e = set_smem(fft_rows_kernel<true>, smem2);
-    // the TMA row pass needs the response rows of the tile next to the two buffers and the twiddle table
-    const size_t smem2t = smem2 + sizeof(double2) * (((size_t)N2 << lc2) + 3 * ((size_t)kRowPad << lc2)) + 16;
-    static const bool no_tma = std::getenv("WFM_FFT_NO_TMA") != nullptr;
-    const bool rows_tma = !no_tma && P2.tw_in_smem && WFM_FFT_PAD == 0 && smem2t <= (size_t)kSmemBudget && P2.n_stage >= 1;
-    if (e == cudaSuccess && rows_tma) e = set_smem(fft_rows_tma_kernel, smem2t);
-    if (e == cudaSuccess) {
-      fft_cols_kernel<true, true, false><<<g1, kFftColsThreads, smem1, st>>>(P1, BT, N2, lc1, x, scratch, x_stride, n, -1.0, 1.0,
-                                                                         n_sig, nv);
-      if (rows_tma)
-        fft_rows_tma_kernel<<<g2, kFftRowsThreads, smem2t, st>>>(P2, N1, lc2, scratch, n, ready);
-      else
-        fft_rows_kernel<true><<<g2, kFftRowsThreads, smem2, st>>>(P2, N1, lc2, scratch, nullptr, n, 0, ready, -1.0, 1.0);
-      fft_cols_kernel<false, false, true><<<g1, kFftColsThreads, smem1, st>>>(P1, BT, N2, lc1, scratch, y, n, y_stride, +1.0,
-                                                                          1.0 / (double)n, n_sig, nv);
-      e = cudaGetLastError();
-    }
-    if (scratch) cudaFreeAsync(scratch, st);
-  } else {
-    // generic: complex copy, forward, * H, inverse, real part
-    if (nv != n) return WFM_EUNSUPPORTED;  // padded grids are chosen 7-smooth by the callers
-    double2* c = nullptr;
-    e = cudaMallocAsync(&c, sizeof(double2) * (size_t)n * (size_t)n_pair, st);
-    dim3 gn(gH, (unsigned)n_pair);
-    if (e == cudaSuccess) {
-      real_to_complex_kernel<<<gn, T, 0, st>>>(x, x_stride, c, n, n_sig);
-      e = c2c_any(c, n_pair, n, n, -1.0, 1.0, st);
-    }
-    if (e == cudaSuccess) {
-      pointwise_mul_kernel<<<gn, T, 0, st>>>(c, ready, n, n);
-      e = c2c_any(c, n_pair, n, n, +1.0, 1.0 / (double)n, st);
-    }
-    if (e == cudaSuccess) {
-      complex_to_real_kernel<<<gn, T, 0, st>>>(c, n, y, y_stride, n_sig);
-      e = cudaGetLastError();
-    }
-    if (c) cudaFreeAsync(c, st);
-    if (e == cudaErrorNotSupported) rc = WFM_EUNSUPPORTED;
+    if ((e = get_plan((int)n, n, &P, &smem)) != cudaSuccess) return e;
+    if ((e = set_smem(fft_filter_single_kernel, smem)) != cudaSuccess) return e;
+    fft_filter_single_kernel<<<(unsigned)n_pair, kFftThreads, smem, st>>>(P, x, y, x_stride, y_stride, n_sig, ready, (int)nv);
+    return cudaGetLastError();
   }
-  if (rc != WFM_OK) return rc;
-  return e == cudaSuccess ? WFM_OK : WFM_ECUDA;
+  if (path == kPathTwoLevel) {
+    TwoLevel t;
+    if ((e = two_level_setup(n, N1, N2, n_pair, st, &t)) != cudaSuccess) return e;
+    // the TMA row pass when its tile fits: the plan's table in shared memory and the response rows next to it
+    const size_t smem2t = rows_tma_smem(t.smem2, N2, t.lc2);
+    const bool rows_tma = t.P2.tw_in_smem && smem2t <= (size_t)kSmemBudget && t.P2.n_stage >= 1;
+    if ((e = set_smem(fft_cols_kernel<true, true, false>, t.smem1)) == cudaSuccess &&
+        (e = set_smem(fft_cols_kernel<false, false, true>, t.smem1)) == cudaSuccess &&
+        (e = rows_tma ? set_smem(fft_rows_tma_kernel, smem2t) : set_smem(fft_rows_kernel<true>, t.smem2)) == cudaSuccess) {
+      fft_cols_kernel<true, true, false><<<t.g1, kFftColsThreads, t.smem1, st>>>(t.P1, t.T, N2, t.lc1, x, t.scratch, x_stride, n,
+                                                                                 -1.0, 1.0, n_sig, nv);
+      if (rows_tma)
+        fft_rows_tma_kernel<<<t.g2, kFftRowsThreads, smem2t, st>>>(t.P2, N1, t.lc2, t.scratch, n, ready);
+      else
+        fft_rows_kernel<true><<<t.g2, kFftRowsThreads, t.smem2, st>>>(t.P2, N1, t.lc2, t.scratch, nullptr, n, 0, ready, -1.0, 1.0);
+      fft_cols_kernel<false, false, true><<<t.g1, kFftColsThreads, t.smem1, st>>>(t.P1, t.T, N2, t.lc1, t.scratch, y, n, y_stride,
+                                                                                  +1.0, 1.0 / (double)n, n_sig, nv);
+      e = cudaGetLastError();
+    }
+    cudaFreeAsync(t.scratch, st);
+    return e;
+  }
+  // generic: complex copy, forward, * H, inverse, real part
+  if (nv != n) return cudaErrorNotSupported;  // padded grids are chosen 7-smooth by the callers
+  const int T = 256;
+  const dim3 gn((unsigned)((n + T - 1) / T), (unsigned)n_pair);
+  double2* c = nullptr;
+  if ((e = cudaMallocAsync(&c, sizeof(double2) * (size_t)n * (size_t)n_pair, st)) != cudaSuccess) return e;
+  real_to_complex_kernel<<<gn, T, 0, st>>>(x, x_stride, c, n, n_sig);
+  e = c2c_any(c, n_pair, n, n, -1.0, 1.0, st);
+  if (e == cudaSuccess) {
+    pointwise_mul_kernel<<<gn, T, 0, st>>>(c, ready, n, n);
+    e = c2c_any(c, n_pair, n, n, +1.0, 1.0 / (double)n, st);
+  }
+  if (e == cudaSuccess) {
+    complex_to_real_kernel<<<gn, T, 0, st>>>(c, n, y, y_stride, n_sig);
+    e = cudaGetLastError();
+  }
+  cudaFreeAsync(c, st);
+  return e;
 }
 
 // H(f) = (1 - A) / (1 - A exp(-2 pi i f tau)) (distortion.py:188-205) or its reciprocal, on the np.fft.fftfreq(n, d)
@@ -1526,7 +1399,7 @@ extern "C" int wfm_fft_filter_prepared(const double* x, double* y, int64_t n_sig
     return WFM_EINVAL;
   if (n_sig == 0 || n_valid == 0) return WFM_OK;
   keep_pool_memory();
-  return run_filter(x, y, n_sig, r->n, x_stride, y_stride, r->ready, (cudaStream_t)stream, n_valid);
+  return fft_status(run_filter(x, y, n_sig, r->n, x_stride, y_stride, r->ready, (cudaStream_t)stream, n_valid));
 }
 
 extern "C" int wfm_fft_filter(const double* x, double* y, int64_t n_sig, int64_t n, int64_t stride, const double* H,
@@ -1547,7 +1420,7 @@ extern "C" int wfm_fft_filter(const double* x, double* y, int64_t n_sig, int64_t
   if (e == cudaSuccess) e = cudaEventRecord(g_hstage.used, st);
   if (e == cudaSuccess) e = cudaMallocAsync(&ready, h_bytes, st);
   if (e == cudaSuccess) e = prepare_response(dH, ready, n, st);
-  int rc = e == cudaSuccess ? run_filter(x, y, n_sig, n, stride, stride, ready, st) : WFM_ECUDA;
+  int rc = e == cudaSuccess ? fft_status(run_filter(x, y, n_sig, n, stride, stride, ready, st)) : WFM_ECUDA;
   if (ready) cudaFreeAsync(ready, st);
   cudaFreeAsync(dH, st);
   return rc;
@@ -1611,5 +1484,5 @@ extern "C" int wfm_reflection_filter(const double* x, double* y, int64_t n_sig, 
       ready = en.ready;
     }
   }
-  return run_filter(x, y, n_sig, n, x_stride, y_stride, ready, st);
+  return fft_status(run_filter(x, y, n_sig, n, x_stride, y_stride, ready, st));
 }
