@@ -246,10 +246,11 @@ int64_t wfm_program_launch_count(wfm_program_t prog);
  *  table_arena_bytes, samples_per_lane_unit, shared_bytes_per_cta}, n <= 8 */
 int  wfm_program_info(wfm_program_t prog, int64_t* out, int32_t n);
 
-/* Asynchronous on `stream`.  Large fp64 launches deal their tiles dynamically from a
- * per-launch device counter (zeroed on `stream`, guarded by an event of the library):
- * results do not depend on the deal.  Environment WFM_K1_DEAL=static|dynamic overrides;
- * use `static` when capturing the call into a CUDA graph. */
+/* Asynchronous on `stream`.  Large launches of fp64 sparse programs and of every dense
+ * program (mostly active samples) deal their tiles dynamically from a per-launch device
+ * counter (zeroed on `stream`, guarded by an event of the library): results do not depend
+ * on the deal.  Environment WFM_K1_DEAL=static|dynamic overrides for every launch; use
+ * `static` when capturing the call into a CUDA graph. */
 int  wfm_sample(wfm_program_t prog, const WfmLaunch* launch, void* stream);
 int  wfm_sample_host(wfm_program_t prog, const WfmLaunch* launch);
 

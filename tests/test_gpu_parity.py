@@ -340,13 +340,20 @@ def test_unit_sizes_on_pairs_and_accumulate(unit, ns, monkeypatch):
     assert rel_err(acc - 0.5, O.waveform_call(ws[0].bounds, ws[0].seq, x)) <= 1e-11  # (y + 0.5) - 0.5 rounds once more
 
 
-@pytest.mark.parametrize('name', ['readme_x_sample', 'cfg2_xy_stack', 'cfg2_z', 'cfg3_rb_I', 'cfg4_flux', 'cfg5_drag_sin',
-                                  'complex_amp', 'boundary_hits'])
-def test_dynamic_deal_equals_static_deal(name, golden, monkeypatch):
+_DEAL_CASES = ['readme_x_sample', 'cfg2_xy_stack', 'cfg2_z', 'cfg3_rb_I', 'cfg4_flux', 'cfg5_drag_sin', 'complex_amp',
+               'boundary_hits']
+
+
+# unit 1 is what these small programs get by default: its cases keep the plain case name as their id
+@pytest.mark.parametrize('name,unit', [pytest.param(n, u, id=n if u == '1' else f'{n}-unit{u}')
+                                       for u in ('1', '2', '4') for n in _DEAL_CASES])
+def test_dynamic_deal_equals_static_deal(name, unit, golden, monkeypatch):
     """WFM_K1_DEAL=dynamic hands the tiles out in batches from a device counter instead of the
-    static round-robin: which warp computes a tile must not change a single bit of it."""
+    static round-robin: which warp computes a tile must not change a single bit of it, in the
+    one- and two-sample sparse kernels and in the dense kernel (fp64 and fast fp32 evaluators)."""
     if name not in golden:
         pytest.skip('case not in the golden set')
+    monkeypatch.setenv('WFM_K1_UNIT', unit)
     rec = golden[name]
     monkeypatch.setenv('WFM_K1_DEAL', 'static')
     static = b200_eval(rec)
@@ -354,6 +361,14 @@ def test_dynamic_deal_equals_static_deal(name, golden, monkeypatch):
     dynamic = b200_eval(rec)
     assert np.array_equal(static, dynamic)
     assert rel_err(dynamic, rec['expect']) <= FP64_TOL
+    if not name.startswith('complex') and rec['grid'][0] == 'sample':
+        from waveforms_b200 import sample_batch
+        fast = {}
+        for deal in ('static', 'dynamic'):
+            monkeypatch.setenv('WFM_K1_DEAL', deal)
+            fast[deal] = sample_batch([b200_object(rec)], dtype=np.float32, fast_fp32=True).numpy()[0]
+        assert np.array_equal(fast['static'], fast['dynamic'])
+        assert rel_err(fast['dynamic'].astype(np.float64), rec['expect']) <= FP32_TOL
 
 
 def test_dynamic_deal_many_tiles_and_subranges(ns, monkeypatch):

@@ -1,5 +1,5 @@
 #!/bin/bash
-# A/B the kernel variants built by `python waveforms_b200/csrc/build.py --out=... -D...` on one box:
+# A/B library builds (`python -m waveforms_b200.csrc.build --out=...`, e.g. of two source trees) on one box:
 #   tools/ab.sh <lib> [<lib> ...]   -> GSa/s and roofline fraction per library, two rounds
 for round in 1 2; do
   for lib in "$@"; do

@@ -1,5 +1,5 @@
 #!/bin/bash
-# A/B the K2/K3 variants built by `python -m waveforms_b200.csrc.build --out=... -D...` on one box:
+# A/B the K2/K3 variants built by `python -m waveforms_b200.csrc.build --out=...` (e.g. of two source trees) on one box:
 #   tools/ab_dsp.sh <lib> [<lib> ...]   -> ms of the cfg4 DSP stages per library, two rounds
 for round in 1 2; do
   for lib in "$@"; do

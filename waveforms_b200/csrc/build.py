@@ -41,9 +41,9 @@ def stale():
     return any(d.stat().st_mtime > t for d in deps)
 
 
-def build(force=False, verbose=False, defines=(), out=None):
-    """``defines``/``out``: experiment builds (e.g. -DWFM_K1_MIN_BLOCKS=2 into
-    another file name, selected at run time with WFM_LIB=<path>)."""
+def build(force=False, verbose=False, out=None):
+    """``out``: build into another file name (e.g. another source tree's library,
+    selected at run time with WFM_LIB=<path> for an A/B)."""
     lib = LIB if out is None else Path(out)
     if out is None and not force and not stale():
         return LIB
@@ -51,8 +51,7 @@ def build(force=False, verbose=False, defines=(), out=None):
 
     def compile_one(src):
         obj = HERE / (Path(src).stem + ('' if out is None else '.' + lib.stem) + '.o')
-        cmd = [nvcc_path(), *NVCC_FLAGS, *PER_SOURCE_FLAGS.get(src, []),
-               *[f'-D{d}' for d in defines], '-c', str(HERE / src), '-o', str(obj)]
+        cmd = [nvcc_path(), *NVCC_FLAGS, *PER_SOURCE_FLAGS.get(src, []), '-c', str(HERE / src), '-o', str(obj)]
         if verbose:
             cmd.insert(1, '-Xptxas')
             cmd.insert(2, '-v')
@@ -70,8 +69,7 @@ def build(force=False, verbose=False, defines=(), out=None):
 
 
 if __name__ == '__main__':
-    defs = [a[2:] for a in sys.argv[1:] if a.startswith('-D')]
     outs = [a[6:] for a in sys.argv[1:] if a.startswith('--out=')]
     path = build(force='--force' in sys.argv, verbose='--verbose' in sys.argv,
-                 defines=defs, out=outs[0] if outs else None)
+                 out=outs[0] if outs else None)
     print(path)

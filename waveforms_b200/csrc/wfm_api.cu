@@ -561,12 +561,7 @@ int wfm_program_create(const WfmProgramDesc* d, int device, wfm_program_t* out) 
   wfm::PrepareCounts pc{d->n_waves, d->n_segs, d->n_facs, d->n_terms, 0};
   p->dev.unit = 1;
   uint32_t* d_stats = (uint32_t*)(base + o_stats);
-  auto cap_of = [&](int ts) {
-    const int fixed = wfm::warp_fixed_bytes(p->dev.n_slots, p->dev.unit);
-    // (an I/Q pair program keeps one tile buffer per output row; the dense kernel keeps none)
-    if (p->dev.dense) return ((wfm::kDenseSliceBytes - fixed) / 2) & ~15;
-    return ((wfm::kWarpSliceBytes - fixed - ts * 8 * p->dev.planes) / 2) & ~15;
-  };
+  auto cap_of = [&](int ts) { return wfm::packet_capacity(p->dev, ts); };
   // the largest tile the average packet density allows (the device then measures every tile)
   auto estimate_tile = [&]() {
     int ts = wfm::kMaxTileSamples;

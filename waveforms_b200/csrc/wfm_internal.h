@@ -10,15 +10,8 @@ namespace wfm {
 // private slice of shared memory (tile_samples x 8 B) and stored with one TMA bulk
 // copy.  Chosen per program from the table density: dense programs take smaller
 // tiles so that the tile's packet fits the warp's slice.
-#ifndef WFM_K1_MIN_BLOCKS
-#define WFM_K1_MIN_BLOCKS 2  // resident 8-warp CTAs per SM the kernel is sized for
-#endif
-#ifndef WFM_K1_WARPS
-#define WFM_K1_WARPS 8  // autonomous warps per CTA
-#endif
-#ifndef WFM_K1_MAX_TILE
-#define WFM_K1_MAX_TILE 1536
-#endif
+constexpr int kMinBlocks = 2;  // resident 8-warp CTAs per SM the kernel is sized for
+constexpr int kWarps = 8;      // autonomous warps per CTA
 // Samples one lane evaluates together (a UNIT: consecutive samples of one active segment),
 // chosen per program (DevProgram::unit).  Two samples per lane run as independent dependency
 // chains and pay the row decoding once: the dense case (RB batches: every sample active,
@@ -26,24 +19,16 @@ namespace wfm {
 // and half the slot memory: the sparse case (control frames: at most ~2 rounds per tile;
 // +4.5 % measured on cfg2).
 constexpr int kMinTileSamples = 128;
-constexpr int kMaxTileSamples = WFM_K1_MAX_TILE;
-// shared memory per warp: 8 * WFM_K1_MIN_BLOCKS warps share the SM's 227 KB (1 KB per CTA is reserved
-// by the driver, 2.5 KB hold the CTA's copy of the erf coefficient table)
-// 1: the CTA keeps a shared-memory copy of the erf coefficient table (2.5 KB).  Measured
-// within noise of reading it through L1 (610 vs 616 GSa/s on cfg2), so the default leaves
-// the shared memory to the packet buffers.
-#ifndef WFM_K1_ERF_SMEM
-#define WFM_K1_ERF_SMEM 0
-#endif
-constexpr int kWarpSliceBytes = ((227 * 1024 / WFM_K1_MIN_BLOCKS - 1024 - (WFM_K1_ERF_SMEM ? 2560 : 0)) / WFM_K1_WARPS) & ~127;
+constexpr int kMaxTileSamples = 1536;
+// shared memory per warp: 8 * kMinBlocks warps share the SM's 227 KB (1 KB per CTA is reserved by the
+// driver).  The erf coefficient table is read through L1: a shared-memory copy per CTA (2.5 KB) was
+// measured within noise of it (610 vs 616 GSa/s on cfg2), so the shared memory goes to the packet buffers.
+constexpr int kWarpSliceBytes = ((227 * 1024 / kMinBlocks - 1024) / kWarps) & ~127;
 
 // The DENSE kernel (programs whose samples are mostly active, e.g. randomized-benchmarking batches): one CTA of 12
 // autonomous warps per SM at up to 168 registers, four samples per lane unit, results stored straight from registers
 // (no tile buffer): its warp slice holds the value slots and the two packet buffers only.
-#ifndef WFM_K1_DENSE_WARPS
-#define WFM_K1_DENSE_WARPS 12
-#endif
-constexpr int kDenseWarps = WFM_K1_DENSE_WARPS;
+constexpr int kDenseWarps = 12;
 constexpr int kDenseUnit = 4;
 constexpr int kDenseSliceBytes = ((227 * 1024 - 1024) / kDenseWarps) & ~127;
 
@@ -52,6 +37,23 @@ constexpr int kDenseSliceBytes = ((227 * 1024 - 1024) / kDenseWarps) & ~127;
 // k * slot_stride(unit) + l * 8 * unit: conflict-free).  Slot 0 always holds 1.0.
 constexpr int kMaxSlots = 12;
 __host__ __device__ constexpr int slot_stride(int unit) { return 32 * 8 * unit; }  // bytes between consecutive slots
+
+// One warp's slice of the sampling kernels' dynamic shared memory (every part 16-byte aligned):
+//   [tile buffers: planes x tile_samples x element][value slots: n_slots x slot_stride(unit)][packet buffer 0]
+//   [packet buffer 1][2 mbarriers]
+// planes = 2 when the program holds I/Q pairs (one tile buffer per output row); the dense kernel keeps none (0).
+struct WarpSlice {
+  size_t tile_bytes, slot_bytes, pkt_cap;
+  __host__ __device__ size_t slots() const { return tile_bytes; }
+  __host__ __device__ size_t packets() const { return tile_bytes + slot_bytes; }
+  __host__ __device__ size_t barriers() const { return packets() + 2 * pkt_cap; }
+  __host__ __device__ size_t bytes() const { return (barriers() + 16 + 127) & ~(size_t)127; }
+  // the largest packet buffer (16-byte multiple) whose slice fits `budget` bytes; may be negative
+  int max_pkt_cap(int budget) const { return ((budget - (int)tile_bytes - ((int)slot_bytes + 16 + 128)) / 2) & ~15; }
+};
+__host__ __device__ inline WarpSlice warp_slice(int planes, int tile_samples, int elem_bytes, int n_slots, int unit, int pkt_cap) {
+  return WarpSlice{(size_t)planes * tile_samples * elem_bytes, (size_t)n_slots * slot_stride(unit), (size_t)pkt_cap};
+}
 
 // ---- the device program of ONE active segment (built on the device at upload) ------------
 // The ABI factor rows of a segment are regrouped so that the interpreter decodes no opcode
@@ -177,7 +179,7 @@ struct DevProgram {
   const int32_t* seg_wave;   // [n_segs] owning channel (host-built; pre-pass only)
   const uint32_t* pkt_off;       // [n_tiles + 1] packet offsets in 16-byte units
   const unsigned char* packets;  // the tile packets
-  int unit;          // samples per lane unit: 1 or 2
+  int unit;          // samples per lane unit: 1 or 2 (sparse kernel), kDenseUnit = 4 (dense kernel)
   int tile_samples;  // kMinTileSamples .. kMaxTileSamples, multiple of 128
   int n_slots;       // value slots per lane in shared memory: 1 (the constant 1.0) + max rows per segment
   int pkt_cap;       // bytes of ONE packet buffer in a warp's shared slice (two buffers per warp)
@@ -230,8 +232,16 @@ cudaError_t launch_scan(const uint32_t* pkt_size, uint32_t* pkt_off, uint32_t* s
 // pass 2: write the packets
 cudaError_t launch_fill_packets(const DevProgram& P, const TileDesc* tiles, int64_t n_tiles, unsigned char* packets,
                                 cudaStream_t stream);
-// shared memory per warp besides the output tile and the two packet buffers
-int warp_fixed_bytes(int n_slots, int unit);
+// a warp's shared-memory slice for the program's kernel, with tiles of tile_samples elements of elem_bytes
+inline WarpSlice program_slice(const DevProgram& P, int tile_samples, int elem_bytes, int pkt_cap) {
+  if (P.dense) return warp_slice(0, 0, 0, P.n_slots, kDenseUnit, pkt_cap);
+  return warp_slice(P.planes == 2 ? 2 : 1, tile_samples, elem_bytes, P.n_slots, P.unit, pkt_cap);
+}
+// the packet buffer capacity of tiles of tile_samples: the largest that fits the kernel's warp slice when the
+// tile buffers hold fp64 (fp32 output uses a smaller slice with the same buffers)
+inline int packet_capacity(const DevProgram& P, int tile_samples) {
+  return program_slice(P, tile_samples, 8, 0).max_pkt_cap(P.dense ? kDenseSliceBytes : kWarpSliceBytes);
+}
 size_t sample_smem_bytes(const DevProgram& P, int dtype);
 
 cudaError_t launch_sample(const DevProgram& P, const TileDesc* tiles, int64_t tile_begin, int64_t n_tiles, int dtype,

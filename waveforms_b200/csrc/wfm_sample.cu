@@ -48,18 +48,15 @@
 #include <cstdlib>
 #include <stdint.h>
 #include <algorithm>
+#include <type_traits>
 #include "wfm_basis.cuh"
 #include "wfm_multidrag.cuh"
 #include "wfm_internal.h"
 
 
-#ifndef WFM_K1_SKIP_UNIT_REFS
-#define WFM_K1_SKIP_UNIT_REFS 1  // +3.5 % on the dense RB batch, neutral on sparse frames
-#endif
-
 namespace wfm {
 
-constexpr int kThreads = 32 * WFM_K1_WARPS;  // autonomous warps per CTA
+constexpr int kThreads = 32 * kWarps;  // autonomous warps per CTA
 constexpr int kWarpsPerCta = kThreads / 32;
 
 template <typename T> struct OutVec;
@@ -284,19 +281,14 @@ static __device__ __noinline__ double term_product_ext(const DevProgram& P, int 
 // ---- the hot evaluator: one UNIT (U samples of one active segment) per call ------------------
 // blk: the segment's rows in the staged packet ({SRow CRow..}.. GRow.. CTerm..); sl: this
 // lane's value slots (slot k at sl + k * kSlotStride, slot 0 holds 1.0).
-struct NoSwitch {
-  template <typename T>
-  __device__ __forceinline__ void operator()(const T&) const {}
-};
 // kPair: the segment may belong to an I/Q pair.  Its terms list the first row's groups, then the second row's; the
 // first second-row term carries kCTermPlaneSwitch: the first row's sum is complete there, `on_switch(total)` hands it
 // to the caller (who stores it) and the accumulation restarts from offset1.  `plane1` tells which row the returned
 // total belongs to.
 template <int U, bool kPair, typename Switch>
 __device__ __forceinline__ Val<U> eval_unit(const unsigned char* __restrict__ blk, int n_sc, int n_rot, int n_gen, int n_term,
-                                         bool has_ext, const DevProgram& P, int gseg, const WaveEval& w,
-                                         const double (&x)[U], unsigned char* __restrict__ sl,
-                                         const double* __restrict__ erf_s, bool affine, const double* offset1, bool& plane1,
+                                         const DevProgram& P, int gseg, const WaveEval& w, const double (&x)[U],
+                                         unsigned char* __restrict__ sl, bool affine, const double* offset1, bool& plane1,
                                          Switch on_switch) {
   constexpr int kSlotStride = slot_stride(U);
   unsigned char* dst = sl + kSlotStride;  // slot 1
@@ -378,7 +370,7 @@ __device__ __forceinline__ Val<U> eval_unit(const unsigned char* __restrict__ bl
       for (int u = 0; u < U; ++u) r.v[u] = f_gaussian(sub(x[u], shift), a0);
     } else if (func == WFM_ERF) {
 #pragma unroll
-      for (int u = 0; u < U; ++u) r.v[u] = erf_tab(dvd(sub(x[u], shift), a0), erf_s);
+      for (int u = 0; u < U; ++u) r.v[u] = erf_tab(dvd(sub(x[u], shift), a0));
     } else {
       const FacArgs fa{func, gr[k].arg_off, shift, a0, gr[k].a1};
 #pragma unroll
@@ -411,15 +403,15 @@ __device__ __forceinline__ Val<U> eval_unit(const unsigned char* __restrict__ bl
           for (int u = 0; u < U; ++u) total.v[u] = *offset1;  // the packet header in shared memory: not held in registers
         }
       }
-      ext = has_ext && (fl & kCTermExt);
+      ext = fl & kCTermExt;
     }
     Val<U> prod;
     if (ext) {
 #pragma unroll
       for (int u = 0; u < U; ++u) prod.v[u] = term_product_ext(P, gseg, it, sl, u);
     } else {
-#if WFM_K1_SKIP_UNIT_REFS
-      // only the references the term has (an absent one is slot 0 = 1.0: the product is the same)
+      // only the references the term has (an absent one is slot 0 = 1.0: the product is the same; loading all three
+      // and multiplying was measured 3.5 % slower on the dense RB batch, neutral on sparse frames)
       prod = ld_slot<U>(sl + (c.z & 0xffffu));
       if (c.z >> 16) {
         const Val<U> f1 = ld_slot<U>(sl + (c.z >> 16));
@@ -431,12 +423,6 @@ __device__ __forceinline__ Val<U> eval_unit(const unsigned char* __restrict__ bl
           for (int u = 0; u < U; ++u) prod.v[u] = mul(prod.v[u], f2.v[u]);
         }
       }
-#else
-      const Val<U> f0 = ld_slot<U>(sl + (c.z & 0xffffu)), f1 = ld_slot<U>(sl + (c.z >> 16)),
-                   f2 = ld_slot<U>(sl + (c.w & 0xffffu));
-#pragma unroll
-      for (int u = 0; u < U; ++u) prod.v[u] = mul(mul(f0.v[u], f1.v[u]), f2.v[u]);
-#endif
     }
 #pragma unroll
     for (int u = 0; u < U; ++u) grp.v[u] = add(grp.v[u], mul(amp, prod.v[u]));
@@ -1110,6 +1096,7 @@ __device__ __forceinline__ void fill_tile(unsigned char* p, int n_rows, double v
       v.y = v.w = (uint32_t)__double2hiint(val);
     }
   }
+  static_assert(kMaxTileSamples * 8 / 512 == 24, "the largest tile (fp64) is the first case");
   switch (n_rows) {  // tile_samples is a multiple of 128: 2 rows each in fp64, 1 row in fp32
     case 24: fill_rows<24>(p, v); break;
     case 22: fill_rows<22>(p, v); break;
@@ -1133,12 +1120,10 @@ __device__ __forceinline__ void fill_tile(unsigned char* p, int n_rows, double v
   }
 }
 
-// per-warp shared-memory slice (dynamic shared memory; all sub-arrays 16-byte aligned):
-//   [out: planes x tile_samples x OutT][slots: n_slots x slot_stride(unit)][packet buffer 0][packet buffer 1][2 mbarriers]
-// (planes = 2 when the program holds I/Q pairs: one tile buffer per output row)
-__host__ __device__ inline size_t warp_slice_bytes(int tile_samples, int n_slots, int unit, int pkt_cap, size_t esz, int planes) {
-  size_t b = (size_t)planes * tile_samples * esz + (size_t)n_slots * slot_stride(unit) + 2 * (size_t)pkt_cap + 16;
-  return (b + 127) & ~(size_t)127;
+// this lane's fp64 value slots (four-sample slots: two 16-byte halves 512 bytes apart, lane l at l * 16 in each)
+template <int U>
+__device__ __forceinline__ unsigned char* lane_slots(unsigned char* s_slots, int lane) {
+  return s_slots + lane * (U == 4 ? 16 : 8 * U);
 }
 
 // the cold path of a tile (its packet would not fit the warp's buffers): per-sample
@@ -1170,59 +1155,29 @@ __device__ __noinline__ void sample_tile_cold(const DevProgram& P, const TileDes
   }
 }
 
-// Tiles per warp of a launch: 0 = persistent grid (CTAs per SM x SMs), k > 0 = a grid of short-lived CTAs
-// whose warps take about k tiles each, handed out by the hardware CTA scheduler (dynamic balance).
-#ifndef WFM_K1_TILES_PER_WARP
-#define WFM_K1_TILES_PER_WARP 0
-#endif
-// batch size of the dynamic deal (WFM_K1_DEAL=dynamic at run time; the default deal is static)
-#ifndef WFM_K1_DYNAMIC
-#define WFM_K1_DYNAMIC 4
-#endif
+// batch size of the dynamic deal (WFM_K1_DEAL=dynamic at run time, or a large launch: dynamic_deal)
+constexpr int kDealBatch = 4;
 // the dense kernel's tiles are long (hundreds of active samples each): smaller batches balance the tail of a launch
-#ifndef WFM_K1_DENSE_DYNAMIC
-#define WFM_K1_DENSE_DYNAMIC 2
-#endif
+constexpr int kDenseDealBatch = 2;
 extern __shared__ __align__(128) unsigned char k1_smem[];
 
-// kF32Eval (float output only): the fp32 EVALUATOR (eval_unit_f32) instead of the fp64 one rounded at the store.
-// Faster, but its error is ~1e-7 x (sum of the term magnitudes), so segments whose terms cancel (a DRAG scaling with
-// w * s >> 1) leave the 1e-6 tolerance: WFM_F32_FAST is opt-in, WFM_F32 always evaluates in fp64.
-template <typename OutT, bool kAccumulate, int U, int kBatch, bool kPair, bool kF32Eval>
-__global__ void __launch_bounds__(kThreads, WFM_K1_MIN_BLOCKS)
-    sample_kernel(const __grid_constant__ DevProgram P, const TileDesc* __restrict__ tiles, int tile_begin, int tile_end,
-                  OutT* __restrict__ out, unsigned int* __restrict__ tile_counter) {
-  constexpr int V = OutVec<OutT>::N;
-  constexpr int kPlanes = kPair ? 2 : 1;
-  const int lane = threadIdx.x & 31;
-  const int warp_in_cta = threadIdx.x >> 5;
-  // this warp's private slice
-  unsigned char* slice =
-      k1_smem + (size_t)warp_in_cta * warp_slice_bytes(P.tile_samples, P.n_slots, U, P.pkt_cap, sizeof(OutT), kPlanes);
-  OutT* s_out = reinterpret_cast<OutT*>(slice);
-  unsigned char* s_slots = slice + (size_t)kPlanes * P.tile_samples * sizeof(OutT);
-  constexpr int kSlotStride = slot_stride(U);
-  unsigned char* s_pkt = s_slots + (size_t)P.n_slots * kSlotStride;
-  uint64_t* s_bar = reinterpret_cast<uint64_t*>(s_pkt + 2 * (size_t)P.pkt_cap);
-  unsigned char* sl = s_slots + lane * 8 * U;  // this lane's value slots
-
-  // the erf coefficient table next to the tile buffers (global / L1 latency showed up as
-  // long-scoreboard stalls in the generic rows); the only block-level barrier of the kernel
-#if WFM_K1_ERF_SMEM
-  __shared__ double s_erf[kErfIntervals * (kErfDegree + 1)];
-  for (int i = threadIdx.x; i < kErfIntervals * (kErfDegree + 1); i += kThreads) s_erf[i] = (&kErfTab[0][0])[i];
-  __syncthreads();
-#else
-  const double* s_erf = &kErfTab[0][0];
-#endif
-
-  // kBatch == 0: the static deal, warp w of the persistent grid walks tiles w, w+G, ...
-  // kBatch >= 2: the dynamic deal, tiles are handed out in aligned batches of kBatch consecutive tiles from a device
-  // counter (zeroed before the launch): warps on slower SMs simply take fewer batches.  nb = the batch this warp takes
-  // next; the one after is drawn one batch early by lane 0 (fetch), so nobody waits for the atomic's round trip and
-  // the packet pipeline can still look two tiles on
+// ---- the tile pipeline of both sampling kernels ---------------------------------------------------------------------
+// The warp walks its tiles and calls body(pk, flags) with every hot tile's packet in shared memory and its flags (a
+// cold tile is sampled by sample_tile_cold instead); s_slots, s_pkt and s_bar are the warp's value slots, packet
+// buffers and mbarriers.  Slot 0, the mbarriers, the packet double buffer and the drain of the last bulk store are
+// the pipeline's.
+// kBatch == 0: the static deal, warp w of the persistent grid walks tiles w, w+G, ...
+// kBatch >= 2: the dynamic deal, tiles are handed out in aligned batches of kBatch consecutive tiles from a device
+// counter (zeroed before the launch): warps on slower SMs simply take fewer batches.  nb = the batch this warp takes
+// next; the one after is drawn one batch early by lane 0 (fetch), so nobody waits for the atomic's round trip and
+// the packet pipeline can still look two tiles on
+template <int kCtaWarps, int kBatch, int U, bool kF32Eval, typename OutT, bool kAccumulate, bool kPair, typename Body>
+__device__ __forceinline__ void for_each_tile(const DevProgram& P, const TileDesc* tiles, int tile_begin, int tile_end,
+                                              OutT* out, unsigned int* tile_counter,
+                                              unsigned char* s_slots, unsigned char* s_pkt, uint64_t* s_bar, const Body& body) {
   static_assert(kBatch == 0 || (kBatch >= 2 && (kBatch & (kBatch - 1)) == 0), "batch: 0 or a power of two >= 2");
-  const int n_warps = gridDim.x * kWarpsPerCta;
+  const int lane = threadIdx.x & 31;
+  const int n_warps = gridDim.x * kCtaWarps;
   int t, nb = 0;
   unsigned int fetch = 0;
   if constexpr (kBatch > 0) {
@@ -1232,7 +1187,7 @@ __global__ void __launch_bounds__(kThreads, WFM_K1_MIN_BLOCKS)
     nb = t + kBatch;
     if (lane == 0) fetch = atomicAdd(tile_counter, (unsigned int)kBatch);
   } else {
-    t = tile_begin + blockIdx.x * kWarpsPerCta + warp_in_cta;
+    t = tile_begin + blockIdx.x * kCtaWarps + (threadIdx.x >> 5);
   }
   auto next1 = [&](int tt) -> int {
     if constexpr (kBatch > 0) return (((tt) - tile_begin) & (kBatch - 1)) < kBatch - 1 ? tt + 1 : nb;
@@ -1253,26 +1208,25 @@ __global__ void __launch_bounds__(kThreads, WFM_K1_MIN_BLOCKS)
     mbar_init(s_bar + 1, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
-  {
-    if constexpr (kF32Eval) {
-      ValF<U> one;  // slot 0: the unit a missing term reference multiplies by (fp32 evaluator: float slots)
+  // slot 0: the unit a missing term reference multiplies by (the fp32 evaluator keeps float slots)
+  if constexpr (kF32Eval) {
+    ValF<U> one;
 #pragma unroll
-      for (int u = 0; u < U; ++u) one.v[u] = 1.0f;
-      st_slot_f(s_slots + lane * 4 * U, one);
-    } else {
-      Val<U> one;
+    for (int u = 0; u < U; ++u) one.v[u] = 1.0f;
+    st_slot_f(s_slots + lane * 4 * U, one);
+  } else {
+    Val<U> one;
 #pragma unroll
-      for (int u = 0; u < U; ++u) one.v[u] = 1.0;
-      st_slot(sl, one);
-    }
+    for (int u = 0; u < U; ++u) one.v[u] = 1.0;
+    st_slot(lane_slots<U>(s_slots, lane), one);
   }
   __syncwarp();
 
   // packet pipeline: tile t's packet is in flight into buffer 0, tile t+G's offsets sit in
-  // registers (its packet goes into the other buffer at the top of iteration t).  The kernel
+  // registers (its packet goes into the other buffer at the top of iteration t).  The sparse kernel
   // sits exactly at its 128-register budget: a third pipeline stage (L2 prefetch of tile
   // t+2G) or a hoisted L2 policy register spill in this loop and cost 4-9 % (measured)
-  uint32_t off_next = 0, end_next = 0;    // packet of tile t + G, 16-byte units
+  uint32_t off_next = 0, end_next = 0;  // packet of tile t + G, 16-byte units
   {
     const uint32_t o0 = P.pkt_off[t], o1 = P.pkt_off[t + 1];
     if (lane == 0) {
@@ -1286,8 +1240,6 @@ __global__ void __launch_bounds__(kThreads, WFM_K1_MIN_BLOCKS)
   }
   // it = tiles this warp has started: packet buffer it & 1, whose mbarrier completes its (it >> 1)-th phase
   uint32_t it = 0;
-#define buf ((int)(it & 1u))
-
   auto advance = [&]() {
     if constexpr (kBatch > 0) {
       // leaving the last tile of a batch: this warp moves into batch nb and draws the one after the next
@@ -1303,6 +1255,7 @@ __global__ void __launch_bounds__(kThreads, WFM_K1_MIN_BLOCKS)
   };
 #pragma unroll 1
   for (; t < tile_end; advance()) {
+    const int buf = (int)(it & 1u);
     const unsigned char* pk = s_pkt + (size_t)buf * P.pkt_cap;
     // prefetch: the next tile's packet into the other buffer (its previous tile is done:
     // every lane passed the __syncwarp that ends an iteration), the offsets of the tile after.
@@ -1320,153 +1273,175 @@ __global__ void __launch_bounds__(kThreads, WFM_K1_MIN_BLOCKS)
     }
     mbar_wait(s_bar + buf, (it >> 1) & 1u);
 
-    const PacketHeader* __restrict__ h = reinterpret_cast<const PacketHeader*>(pk);
-    const int cnt = h->cnt;
-    const uint32_t flags = h->flags;
-    const int n_arows = h->n_arows, n_patch = h->n_patch, n_units = h->n_units;
-    const double base = h->base;
-    OutT* __restrict__ dst = out + h->out0;
-
+    // (the cold tile ends its iteration on its own: one shared tail for both paths costs the sparse kernel 4-16 bytes
+    // of spills at its 128-register budget, ptxas -v)
+    const uint32_t flags = reinterpret_cast<const PacketHeader*>(pk)->flags;
     if (flags & kPacketCold) {
       sample_tile_cold<OutT, kAccumulate, kPair>(P, tiles[t], out, lane);
       __syncwarp();
       ++it;
       continue;
     }
-
-    // the previous tile's bulk store must have finished READING the tile buffer
-    if (lane == 0) bulk_wait_read_all();  // returns at once when no store is outstanding
-    __syncwarp();
-
-    // base fill: the whole tile BUFFER (tile_samples, a multiple of 128) <- the zero-segment
-    // value; flat segments with another value and the active samples overwrite it below
-    fill_tile(reinterpret_cast<unsigned char*>(s_out) + lane * 16, P.tile_samples * (int)sizeof(OutT) / 512, base,
-              sizeof(OutT) == 4);
-    if constexpr (kPair) {
-      if (flags & WFM_WAVE_PAIR)
-        fill_tile(reinterpret_cast<unsigned char*>(s_out + P.tile_samples) + lane * 16, P.tile_samples * (int)sizeof(OutT) / 512,
-                  h->base1, sizeof(OutT) == 4);
-    }
-    __syncwarp();
-
-    const ARow* __restrict__ arows = reinterpret_cast<const ARow*>(pk + sizeof(PacketHeader));
-    const PatchRow* __restrict__ patches = reinterpret_cast<const PatchRow*>(arows + (n_arows ? n_arows + 1 : 0));
-    // ---- flat segments with their own value ----------------------------------------------
-    for (int i = 0; i < n_patch; ++i)
-      fill_run(kPair && patches[i].plane ? s_out + P.tile_samples : s_out, (int)patches[i].a, (int)patches[i].b, patches[i].val,
-               lane);
-
-    // ---- the tile's ACTIVE samples: units dealt round-robin to the lanes -------------------
-    if (n_units > 0) {
-      const WaveEval we{base, flags, h->wave};
-      const double t0 = h->t0, delta = h->delta;
-      const int64_t j0 = h->j0;
-      const bool plain_grid = !(flags & (WFM_WAVE_EXPLICIT_X | WFM_WAVE_LAST_OVERRIDE | WFM_WAVE_PRESHIFT));
-      int lo = 0;
-#pragma unroll 1
-      for (int i = lane; i < n_units; i += 32) {
-        while ((int)arows[lo + 1].first <= i) ++lo;  // the active segment holding unit i (i grows monotonically)
-        const uint4 rw = reinterpret_cast<const uint4*>(arows)[lo];  // ARow: start first | rel len | n_sc n_rot n_gen n_term | gseg
-        const int start = rw.x & 0xffffu, first = rw.x >> 16, rel = rw.y & 0xfffu, len = rw.y >> 16;
-        const uint32_t sflags = (rw.y >> 12) & 0xfu;
-        const int jj = start + (i - first) * U;
-        const int n_valid = min(U, start + len - jj);
-        double x[U];
-        if (plain_grid) {
-          // the tile's sample index fits 32 bits (channels hold < 2^31 samples)
-          const int jg = (int)j0 + jj;
-#pragma unroll
-          for (int u = 0; u < U; ++u) x[u] = add(t0, mul((double)(jg + u), delta));
-        } else {
-#pragma unroll
-          for (int u = 0; u < U; ++u) x[u] = abscissa(P.waves[h->wave], P.x, j0 + min(jj + u, cnt - 1));
-        }
-        Val<U> r;
-        if constexpr (kPair) {
-          bool plane1 = false;
-          // the first row of an I/Q pair is complete when its last term has been added: into the first tile buffer
-          auto first_row = [&](const Val<U>& v) {
-#pragma unroll
-            for (int u = 0; u < U; ++u)
-              if (u < n_valid) s_out[jj + u] = (OutT)v.v[u];
-          };
-          if (sflags & kSegWide) {
-            const bool two = flags & WFM_WAVE_PAIR;
-#pragma unroll
-            for (int u = 0; u < U; ++u) r.v[u] = eval_segment_slow_row(P, (int)rw.w, we.offset, we.flags, we.wave, x[u], 0, 0.0);
-            if (two) {
-              first_row(r);
-              plane1 = true;
-#pragma unroll
-              for (int u = 0; u < U; ++u) r.v[u] = eval_segment_slow_row(P, (int)rw.w, we.offset, we.flags, we.wave, x[u], 1, h->base1);
-            }
-          } else if constexpr (kF32Eval) {
-            r = eval_unit_f32<U, true>(pk + rel * 16, rw.z & 0xffu, (rw.z >> 8) & 0xffu, (rw.z >> 16) & 0xffu, rw.z >> 24, P,
-                                       (int)rw.w, we, x, s_slots + lane * 4 * U, &h->base1, plane1, first_row);
-          } else {
-            r = eval_unit<U, true>(pk + rel * 16, rw.z & 0xffu, (rw.z >> 8) & 0xffu, (rw.z >> 16) & 0xffu, rw.z >> 24, true, P,
-                                   (int)rw.w, we, x, sl, s_erf, !(flags & WFM_WAVE_EXPLICIT_X), &h->base1, plane1, first_row);
-          }
-          OutT* row_buf = plane1 ? s_out + P.tile_samples : s_out;
-#pragma unroll
-          for (int u = 0; u < U; ++u)
-            if (u < n_valid) row_buf[jj + u] = (OutT)r.v[u];
-        } else {
-          NoSwitch none;
-          bool unused;
-          if (sflags & kSegWide) {
-#pragma unroll
-            for (int u = 0; u < U; ++u) r.v[u] = eval_segment_slow(P, (int)rw.w, we.offset, we.flags, we.wave, x[u]);
-          } else if constexpr (kF32Eval) {
-            r = eval_unit_f32<U, false>(pk + rel * 16, rw.z & 0xffu, (rw.z >> 8) & 0xffu, (rw.z >> 16) & 0xffu, rw.z >> 24, P,
-                                        (int)rw.w, we, x, s_slots + lane * 4 * U, nullptr, unused, none);
-          } else {
-            r = eval_unit<U, false>(pk + rel * 16, rw.z & 0xffu, (rw.z >> 8) & 0xffu, (rw.z >> 16) & 0xffu, rw.z >> 24, true, P,
-                                    (int)rw.w, we, x, sl, s_erf, !(flags & WFM_WAVE_EXPLICIT_X), nullptr, unused, none);
-          }
-#pragma unroll
-          for (int u = 0; u < U; ++u)
-            if (u < n_valid) s_out[jj + u] = (OutT)r.v[u];
-        }
-      }
-    }
-
-    // ---- store ---------------------------------------------------------------------------
-    if (kAccumulate) {
-      // out += tile (Waveform.__call__(..., accumulate=True)): read-modify-write epilogue
-      __syncwarp();
-      for (int p = lane; p < cnt; p += 32) dst[p] = (OutT)add((double)dst[p], (double)s_out[p]);
-      if constexpr (kPair) {
-        if (flags & WFM_WAVE_PAIR) {
-          OutT* __restrict__ dst1 = out + h->out1;
-          for (int p = lane; p < cnt; p += 32) dst1[p] = (OutT)add((double)dst1[p], (double)s_out[P.tile_samples + p]);
-        }
-      }
-    } else {
-      // the whole tile as one TMA bulk copy (an I/Q pair: one per row)
-      fence_proxy_async_smem();
-      __syncwarp();
-      const int n_bulk = cnt & ~(V - 1);  // 16-byte multiple; the ragged tail goes out as scalars
-      if (lane == 0 && n_bulk > 0) {
-        const uint64_t policy = l2_evict_first_policy();
-        bulk_s2g_evict_first(dst, s_out, (uint32_t)n_bulk * sizeof(OutT), policy);
-        if constexpr (kPair) {
-          if (flags & WFM_WAVE_PAIR)
-            bulk_s2g_evict_first(out + h->out1, s_out + P.tile_samples, (uint32_t)n_bulk * sizeof(OutT), policy);
-        }
-      }
-      if (n_bulk + lane < cnt) {
-        dst[n_bulk + lane] = s_out[n_bulk + lane];
-        if constexpr (kPair) {
-          if (flags & WFM_WAVE_PAIR) (out + h->out1)[n_bulk + lane] = s_out[P.tile_samples + n_bulk + lane];
-        }
-      }
-    }
-    __syncwarp();  // all reads of the packet and of the tail of s_out are done
+    body(pk, flags);
+    __syncwarp();  // all reads of the packet are done: its buffer may be refilled
     ++it;
   }
-  if (lane == 0) bulk_wait_read_all();  // shared memory must outlive the copy's reads
-#undef buf
+  if (lane == 0) bulk_wait_read_all();  // shared memory must outlive the reads of a tile's bulk store
+}
+
+// ---- the active samples of a tile, shared by both sampling kernels -------------------------------------------------
+// The tile's units are dealt round-robin to the lanes.  Per unit: its abscissae, the evaluator (the slow one for a wide
+// segment, else the fp32 or the fp64 interpreter) and, in an I/Q pair, the switch to the second row.  The results go
+// to sink(plane1, jj, n_valid, r): samples jj .. jj + n_valid - 1 of the tile in row plane1 of the pair.
+// s_slots: the warp's value slots, sl: this lane's (lane_slots).
+template <int U, bool kPair, bool kF32Eval, typename Sink>
+__device__ __forceinline__ void eval_units(const DevProgram& P, const unsigned char* pk, double base,
+                                           uint32_t flags, int cnt, int n_units, unsigned char* s_slots, unsigned char* sl,
+                                           int lane, const Sink& sink) {
+  if (n_units <= 0) return;
+  const PacketHeader* __restrict__ h = reinterpret_cast<const PacketHeader*>(pk);
+  const ARow* __restrict__ arows = reinterpret_cast<const ARow*>(pk + sizeof(PacketHeader));
+  const WaveEval we{base, flags, h->wave};
+  const double t0 = h->t0, delta = h->delta;
+  const int64_t j0 = h->j0;
+  const bool plain_grid = !(flags & (WFM_WAVE_EXPLICIT_X | WFM_WAVE_LAST_OVERRIDE | WFM_WAVE_PRESHIFT));
+  int lo = 0;
+#pragma unroll 1
+  for (int i = lane; i < n_units; i += 32) {
+    while ((int)arows[lo + 1].first <= i) ++lo;  // the active segment holding unit i (i grows monotonically)
+    const uint4 rw = reinterpret_cast<const uint4*>(arows)[lo];  // ARow: start first | rel len | n_sc n_rot n_gen n_term | gseg
+    const int start = rw.x & 0xffffu, first = rw.x >> 16, rel = rw.y & 0xfffu, len = rw.y >> 16;
+    const uint32_t sflags = (rw.y >> 12) & 0xfu;
+    const int jj = start + (i - first) * U;
+    const int n_valid = min(U, start + len - jj);
+    double x[U];
+    if (plain_grid) {
+      // the tile's sample index fits 32 bits (channels hold < 2^31 samples)
+      const int jg = (int)j0 + jj;
+#pragma unroll
+      for (int u = 0; u < U; ++u) x[u] = add(t0, mul((double)(jg + u), delta));
+    } else {
+#pragma unroll
+      for (int u = 0; u < U; ++u) x[u] = abscissa(P.waves[h->wave], P.x, j0 + min(jj + u, cnt - 1));
+    }
+    Val<U> r;
+    bool plane1 = false;
+    // the first row of an I/Q pair is complete when its last term has been added
+    auto first_row = [&](const Val<U>& v) { sink(false, jj, n_valid, v); };
+    if (sflags & kSegWide) {
+      if constexpr (kPair) {
+#pragma unroll
+        for (int u = 0; u < U; ++u) r.v[u] = eval_segment_slow_row(P, (int)rw.w, we.offset, we.flags, we.wave, x[u], 0, 0.0);
+        if (flags & WFM_WAVE_PAIR) {
+          first_row(r);
+          plane1 = true;
+#pragma unroll
+          for (int u = 0; u < U; ++u) r.v[u] = eval_segment_slow_row(P, (int)rw.w, we.offset, we.flags, we.wave, x[u], 1, h->base1);
+        }
+      } else {
+#pragma unroll
+        for (int u = 0; u < U; ++u) r.v[u] = eval_segment_slow(P, (int)rw.w, we.offset, we.flags, we.wave, x[u]);
+      }
+    } else if constexpr (kF32Eval) {
+      r = eval_unit_f32<U, kPair>(pk + rel * 16, rw.z & 0xffu, (rw.z >> 8) & 0xffu, (rw.z >> 16) & 0xffu, rw.z >> 24, P,
+                                  (int)rw.w, we, x, s_slots + lane * 4 * U, &h->base1, plane1, first_row);
+    } else {
+      r = eval_unit<U, kPair>(pk + rel * 16, rw.z & 0xffu, (rw.z >> 8) & 0xffu, (rw.z >> 16) & 0xffu, rw.z >> 24, P,
+                              (int)rw.w, we, x, sl, !(flags & WFM_WAVE_EXPLICIT_X), &h->base1, plane1, first_row);
+    }
+    sink(plane1, jj, n_valid, r);
+  }
+}
+
+// kF32Eval (float output only): the fp32 EVALUATOR (eval_unit_f32) instead of the fp64 one rounded at the store.
+// Faster, but its error is ~1e-7 x (sum of the term magnitudes), so segments whose terms cancel (a DRAG scaling with
+// w * s >> 1) leave the 1e-6 tolerance: WFM_F32_FAST is opt-in, WFM_F32 always evaluates in fp64.
+template <typename OutT, bool kAccumulate, int U, int kBatch, bool kPair, bool kF32Eval>
+__global__ void __launch_bounds__(kThreads, kMinBlocks)
+    sample_kernel(const __grid_constant__ DevProgram P, const TileDesc* __restrict__ tiles, int tile_begin, int tile_end,
+                  OutT* __restrict__ out, unsigned int* __restrict__ tile_counter) {
+  constexpr int V = OutVec<OutT>::N;
+  const int lane = threadIdx.x & 31;
+  // this warp's private slice
+  const WarpSlice ws = warp_slice(kPair ? 2 : 1, P.tile_samples, sizeof(OutT), P.n_slots, U, P.pkt_cap);
+  unsigned char* slice = k1_smem + (size_t)(threadIdx.x >> 5) * ws.bytes();
+  OutT* s_out = reinterpret_cast<OutT*>(slice);
+  unsigned char* s_slots = slice + ws.slots();
+  unsigned char* sl = lane_slots<U>(s_slots, lane);
+
+  // a unit's results -> the tile buffer of its row
+  auto to_tile = [&](bool plane1, int jj, int n_valid, const Val<U>& r) {
+    OutT* row_buf = plane1 ? s_out + P.tile_samples : s_out;
+#pragma unroll
+    for (int u = 0; u < U; ++u)
+      if (u < n_valid) row_buf[jj + u] = (OutT)r.v[u];
+  };
+  for_each_tile<kWarpsPerCta, kBatch, U, kF32Eval, OutT, kAccumulate, kPair>(
+      P, tiles, tile_begin, tile_end, out, tile_counter, s_slots, slice + ws.packets(),
+      reinterpret_cast<uint64_t*>(slice + ws.barriers()), [&](const unsigned char* pk, uint32_t flags) {
+        const PacketHeader* __restrict__ h = reinterpret_cast<const PacketHeader*>(pk);
+        const int cnt = h->cnt;
+        const int n_arows = h->n_arows, n_patch = h->n_patch, n_units = h->n_units;
+        const double base = h->base;
+        OutT* __restrict__ dst = out + h->out0;
+
+        // the previous tile's bulk store must have finished READING the tile buffer
+        if (lane == 0) bulk_wait_read_all();  // returns at once when no store is outstanding
+        __syncwarp();
+
+        // base fill: the whole tile BUFFER (tile_samples, a multiple of 128) <- the zero-segment
+        // value; flat segments with another value and the active samples overwrite it below
+        fill_tile(reinterpret_cast<unsigned char*>(s_out) + lane * 16, P.tile_samples * (int)sizeof(OutT) / 512, base,
+                  sizeof(OutT) == 4);
+        if constexpr (kPair) {
+          if (flags & WFM_WAVE_PAIR)
+            fill_tile(reinterpret_cast<unsigned char*>(s_out + P.tile_samples) + lane * 16,
+                      P.tile_samples * (int)sizeof(OutT) / 512, h->base1, sizeof(OutT) == 4);
+        }
+        __syncwarp();
+
+        const ARow* __restrict__ arows = reinterpret_cast<const ARow*>(pk + sizeof(PacketHeader));
+        const PatchRow* __restrict__ patches = reinterpret_cast<const PatchRow*>(arows + (n_arows ? n_arows + 1 : 0));
+        // ---- flat segments with their own value ----------------------------------------------
+        for (int i = 0; i < n_patch; ++i)
+          fill_run(kPair && patches[i].plane ? s_out + P.tile_samples : s_out, (int)patches[i].a, (int)patches[i].b,
+                   patches[i].val, lane);
+
+        // ---- the tile's ACTIVE samples ---------------------------------------------------------
+        eval_units<U, kPair, kF32Eval>(P, pk, base, flags, cnt, n_units, s_slots, sl, lane, to_tile);
+
+        // ---- store ---------------------------------------------------------------------------
+        if (kAccumulate) {
+          // out += tile (Waveform.__call__(..., accumulate=True)): read-modify-write epilogue
+          __syncwarp();
+          for (int p = lane; p < cnt; p += 32) dst[p] = (OutT)add((double)dst[p], (double)s_out[p]);
+          if constexpr (kPair) {
+            if (flags & WFM_WAVE_PAIR) {
+              OutT* __restrict__ dst1 = out + h->out1;
+              for (int p = lane; p < cnt; p += 32) dst1[p] = (OutT)add((double)dst1[p], (double)s_out[P.tile_samples + p]);
+            }
+          }
+        } else {
+          // the whole tile as one TMA bulk copy (an I/Q pair: one per row)
+          fence_proxy_async_smem();
+          __syncwarp();
+          const int n_bulk = cnt & ~(V - 1);  // 16-byte multiple; the ragged tail goes out as scalars
+          if (lane == 0 && n_bulk > 0) {
+            const uint64_t policy = l2_evict_first_policy();
+            bulk_s2g_evict_first(dst, s_out, (uint32_t)n_bulk * sizeof(OutT), policy);
+            if constexpr (kPair) {
+              if (flags & WFM_WAVE_PAIR)
+                bulk_s2g_evict_first(out + h->out1, s_out + P.tile_samples, (uint32_t)n_bulk * sizeof(OutT), policy);
+            }
+          }
+          if (n_bulk + lane < cnt) {
+            dst[n_bulk + lane] = s_out[n_bulk + lane];
+            if constexpr (kPair) {
+              if (flags & WFM_WAVE_PAIR) (out + h->out1)[n_bulk + lane] = s_out[P.tile_samples + n_bulk + lane];
+            }
+          }
+        }
+      });
 }
 
 // ---- the DENSE sampling kernel -------------------------------------------------------------
@@ -1483,11 +1458,6 @@ __global__ void __launch_bounds__(kThreads, WFM_K1_MIN_BLOCKS)
 //   * writes flat runs (zero / constant segments, ALL listed as patch rows in dense programs) directly as well.
 // Packets, the pre-pass, the deal of the tiles and the evaluator are the sparse kernel's.
 constexpr int kDenseThreads = 32 * kDenseWarps;
-
-__host__ __device__ inline size_t dense_slice_bytes(int n_slots, int pkt_cap) {
-  size_t b = (size_t)n_slots * slot_stride(kDenseUnit) + 2 * (size_t)pkt_cap + 16;
-  return (b + 127) & ~(size_t)127;
-}
 
 // U consecutive results -> global memory (16-byte stores when the address allows)
 template <typename OutT, bool kAccumulate, int U>
@@ -1544,184 +1514,30 @@ __global__ void __launch_bounds__(kDenseThreads, 1)
                         OutT* __restrict__ out, unsigned int* __restrict__ tile_counter) {
   constexpr int U = kDenseUnit;
   const int lane = threadIdx.x & 31;
-  const int warp_in_cta = threadIdx.x >> 5;
-  unsigned char* slice = k1_smem + (size_t)warp_in_cta * dense_slice_bytes(P.n_slots, P.pkt_cap);
-  unsigned char* s_slots = slice;
-  constexpr int kSlotStride = slot_stride(U);
-  unsigned char* s_pkt = s_slots + (size_t)P.n_slots * kSlotStride;
-  uint64_t* s_bar = reinterpret_cast<uint64_t*>(s_pkt + 2 * (size_t)P.pkt_cap);
-  unsigned char* sl = s_slots + lane * 16;  // this lane's value slots (two 16-byte halves per slot, see ld_slot)
-  const double* s_erf = &kErfTab[0][0];
-
-  static_assert(kBatch == 0 || (kBatch >= 2 && (kBatch & (kBatch - 1)) == 0), "batch: 0 or a power of two >= 2");
-  const int n_warps = gridDim.x * kDenseWarps;
-  int t, nb = 0;
-  unsigned int fetch = 0;
-  if constexpr (kBatch > 0) {
-    unsigned int b0 = 0;
-    if (lane == 0) b0 = atomicAdd(tile_counter, 2u * kBatch);
-    t = tile_begin + (int)__shfl_sync(0xffffffffu, b0, 0);
-    nb = t + kBatch;
-    if (lane == 0) fetch = atomicAdd(tile_counter, (unsigned int)kBatch);
-  } else {
-    t = tile_begin + blockIdx.x * kDenseWarps + warp_in_cta;
-  }
-  auto next1 = [&](int tt) -> int {
-    if constexpr (kBatch > 0) return (((tt) - tile_begin) & (kBatch - 1)) < kBatch - 1 ? tt + 1 : nb;
-    else return tt + n_warps;
-  };
-  auto next2 = [&](int tt) -> int {
-    if constexpr (kBatch > 0) {
-      const int pos = (tt - tile_begin) & (kBatch - 1);
-      return pos < kBatch - 2 ? tt + 2 : (pos == kBatch - 2 ? nb : nb + 1);
-    } else {
-      return tt + 2 * n_warps;
-    }
-  };
-  if (t >= tile_end) return;
-  if (lane == 0) {
-    mbar_init(s_bar, 1);
-    mbar_init(s_bar + 1, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if constexpr (kF32Eval) {
-    ValF<U> one;
-#pragma unroll
-    for (int u = 0; u < U; ++u) one.v[u] = 1.0f;
-    st_slot_f(s_slots + lane * 4 * U, one);
-  } else {
-    Val<U> one;
-#pragma unroll
-    for (int u = 0; u < U; ++u) one.v[u] = 1.0;
-    st_slot(sl, one);
-  }
-  __syncwarp();
-
-  uint32_t off_next = 0, end_next = 0;
-  {
-    const uint32_t o0 = P.pkt_off[t], o1 = P.pkt_off[t + 1];
-    if (lane == 0) {
-      mbar_expect_tx(s_bar, (o1 - o0) * 16u);
-      bulk_g2s(s_pkt, P.packets + (size_t)o0 * 16, (o1 - o0) * 16u, s_bar);
-    }
-    if (next1(t) < tile_end) {
-      off_next = P.pkt_off[next1(t)];
-      end_next = P.pkt_off[next1(t) + 1];
-    }
-  }
-  uint32_t it = 0;
-  auto advance = [&]() {
-    if constexpr (kBatch > 0) {
-      const bool last = ((t - tile_begin) & (kBatch - 1)) == kBatch - 1;
-      t = next1(t);
-      if (last) {
-        nb = tile_begin + (int)__shfl_sync(0xffffffffu, fetch, 0);
-        if (lane == 0) fetch = atomicAdd(tile_counter, (unsigned int)kBatch);
-      }
-    } else {
-      t += n_warps;
-    }
-  };
-#pragma unroll 1
-  for (; t < tile_end; advance()) {
-    const int buf = (int)(it & 1u);
-    const unsigned char* pk = s_pkt + (size_t)buf * P.pkt_cap;
-    if (next1(t) < tile_end) {
-      if (lane == 0) {
-        mbar_expect_tx(s_bar + (buf ^ 1), (end_next - off_next) * 16u);
-        bulk_g2s(s_pkt + (size_t)(buf ^ 1) * P.pkt_cap, P.packets + (size_t)off_next * 16, (end_next - off_next) * 16u,
-                 s_bar + (buf ^ 1));
-      }
-      if (next2(t) < tile_end) {
-        off_next = P.pkt_off[next2(t)];
-        end_next = P.pkt_off[next2(t) + 1];
-      }
-    }
-    mbar_wait(s_bar + buf, (it >> 1) & 1u);
-
-    const PacketHeader* __restrict__ h = reinterpret_cast<const PacketHeader*>(pk);
-    const uint32_t flags = h->flags;
-    if (flags & kPacketCold) {
-      sample_tile_cold<OutT, kAccumulate, kPair>(P, tiles[t], out, lane);
-      __syncwarp();
-      ++it;
-      continue;
-    }
-    const int n_arows = h->n_arows, n_patch = h->n_patch, n_units = h->n_units;
-    OutT* __restrict__ dst0 = out + h->out0;
-    OutT* dst1 = dst0;
-    if constexpr (kPair) dst1 = out + h->out1;
-    const ARow* __restrict__ arows = reinterpret_cast<const ARow*>(pk + sizeof(PacketHeader));
-    const PatchRow* __restrict__ patches = reinterpret_cast<const PatchRow*>(arows + (n_arows ? n_arows + 1 : 0));
-    // ---- flat runs: every zero / constant segment of the tile is listed (dense programs) ----------------------------
-    for (int i = 0; i < n_patch; ++i)
-      fill_global<OutT, kAccumulate>((kPair && patches[i].plane) ? dst1 : dst0, (int)patches[i].a, (int)patches[i].b, patches[i].val,
-                                     lane);
-    // ---- active samples: units of four, results straight to global memory ------------------------------------------
-    if (n_units > 0) {
-      const WaveEval we{h->base, flags, h->wave};
-      const double t0 = h->t0, delta = h->delta;
-      const int j0 = (int)h->j0, cnt = h->cnt;
-      const bool plain_grid = !(flags & (WFM_WAVE_EXPLICIT_X | WFM_WAVE_LAST_OVERRIDE | WFM_WAVE_PRESHIFT));
-      int lo = 0;
-#pragma unroll 1
-      for (int i = lane; i < n_units; i += 32) {
-        while ((int)arows[lo + 1].first <= i) ++lo;
-        const uint4 rw = reinterpret_cast<const uint4*>(arows)[lo];
-        const int start = rw.x & 0xffffu, first = rw.x >> 16, rel = rw.y & 0xfffu, len = rw.y >> 16;
-        const uint32_t sflags = (rw.y >> 12) & 0xfu;
-        const int jj = start + (i - first) * U;
-        const int n_valid = min(U, start + len - jj);
-        double x[U];
-        if (plain_grid) {
-          const int jg = j0 + jj;
-#pragma unroll
-          for (int u = 0; u < U; ++u) x[u] = add(t0, mul((double)(jg + u), delta));
-        } else {
-#pragma unroll
-          for (int u = 0; u < U; ++u) x[u] = abscissa(P.waves[h->wave], P.x, h->j0 + min(jj + u, cnt - 1));
-        }
-        Val<U> r;
-        if constexpr (kPair) {
-          bool plane1 = false;
-          auto first_row = [&](const Val<U>& v) { store_unit<OutT, kAccumulate, U>(dst0 + jj, v, n_valid); };
-          if (sflags & kSegWide) {
-#pragma unroll
-            for (int u = 0; u < U; ++u) r.v[u] = eval_segment_slow_row(P, (int)rw.w, we.offset, we.flags, we.wave, x[u], 0, 0.0);
-            if (flags & WFM_WAVE_PAIR) {
-              first_row(r);
-              plane1 = true;
-#pragma unroll
-              for (int u = 0; u < U; ++u) r.v[u] = eval_segment_slow_row(P, (int)rw.w, we.offset, we.flags, we.wave, x[u], 1, h->base1);
-            }
-          } else if constexpr (kF32Eval) {
-            r = eval_unit_f32<U, true>(pk + rel * 16, rw.z & 0xffu, (rw.z >> 8) & 0xffu, (rw.z >> 16) & 0xffu, rw.z >> 24, P,
-                                       (int)rw.w, we, x, s_slots + lane * 4 * U, &h->base1, plane1, first_row);
-          } else {
-            r = eval_unit<U, true>(pk + rel * 16, rw.z & 0xffu, (rw.z >> 8) & 0xffu, (rw.z >> 16) & 0xffu, rw.z >> 24, true, P,
-                                   (int)rw.w, we, x, sl, s_erf, !(flags & WFM_WAVE_EXPLICIT_X), &h->base1, plane1, first_row);
-          }
-          store_unit<OutT, kAccumulate, U>((plane1 ? dst1 : dst0) + jj, r, n_valid);
-        } else {
-          NoSwitch none;
-          bool unused;
-          if (sflags & kSegWide) {
-#pragma unroll
-            for (int u = 0; u < U; ++u) r.v[u] = eval_segment_slow(P, (int)rw.w, we.offset, we.flags, we.wave, x[u]);
-          } else if constexpr (kF32Eval) {
-            r = eval_unit_f32<U, false>(pk + rel * 16, rw.z & 0xffu, (rw.z >> 8) & 0xffu, (rw.z >> 16) & 0xffu, rw.z >> 24, P,
-                                        (int)rw.w, we, x, s_slots + lane * 4 * U, nullptr, unused, none);
-          } else {
-            r = eval_unit<U, false>(pk + rel * 16, rw.z & 0xffu, (rw.z >> 8) & 0xffu, (rw.z >> 16) & 0xffu, rw.z >> 24, true, P,
-                                    (int)rw.w, we, x, sl, s_erf, !(flags & WFM_WAVE_EXPLICIT_X), nullptr, unused, none);
-          }
-          store_unit<OutT, kAccumulate, U>(dst0 + jj, r, n_valid);
-        }
-      }
-    }
-    __syncwarp();  // all reads of the packet are done: its buffer may be refilled
-    ++it;
-  }
+  const WarpSlice ws = warp_slice(0, 0, 0, P.n_slots, U, P.pkt_cap);
+  unsigned char* slice = k1_smem + (size_t)(threadIdx.x >> 5) * ws.bytes();
+  unsigned char* s_slots = slice + ws.slots();
+  unsigned char* sl = lane_slots<U>(s_slots, lane);
+  for_each_tile<kDenseWarps, kBatch, U, kF32Eval, OutT, kAccumulate, kPair>(
+      P, tiles, tile_begin, tile_end, out, tile_counter, s_slots, slice + ws.packets(),
+      reinterpret_cast<uint64_t*>(slice + ws.barriers()), [&](const unsigned char* pk, uint32_t flags) {
+        const PacketHeader* __restrict__ h = reinterpret_cast<const PacketHeader*>(pk);
+        const int n_arows = h->n_arows, n_patch = h->n_patch, n_units = h->n_units;
+        OutT* __restrict__ dst0 = out + h->out0;
+        OutT* dst1 = dst0;
+        if constexpr (kPair) dst1 = out + h->out1;
+        const ARow* __restrict__ arows = reinterpret_cast<const ARow*>(pk + sizeof(PacketHeader));
+        const PatchRow* __restrict__ patches = reinterpret_cast<const PatchRow*>(arows + (n_arows ? n_arows + 1 : 0));
+        // ---- flat runs: every zero / constant segment of the tile is listed (dense programs) --------------------------
+        for (int i = 0; i < n_patch; ++i)
+          fill_global<OutT, kAccumulate>((kPair && patches[i].plane) ? dst1 : dst0, (int)patches[i].a, (int)patches[i].b,
+                                         patches[i].val, lane);
+        // ---- active samples: units of four, results straight to global memory ----------------------------------------
+        eval_units<U, kPair, kF32Eval>(P, pk, h->base, flags, h->cnt, n_units, s_slots, sl, lane,
+                                       [&](bool plane1, int jj, int n_valid, const Val<U>& r) {
+                                         store_unit<OutT, kAccumulate, U>((plane1 ? dst1 : dst0) + jj, r, n_valid);
+                                       });
+      });
 }
 
 // complex128 output: the real and the imaginary PLANE are sampled by the real-valued kernel
@@ -1818,11 +1634,8 @@ cudaError_t launch_fill_packets(const DevProgram& P, const TileDesc* tiles, int6
   return cudaGetLastError();
 }
 
-int warp_fixed_bytes(int n_slots, int unit) { return n_slots * slot_stride(unit) + 16 + 128; }
-
 size_t sample_smem_bytes(const DevProgram& P, int dtype) {
-  if (P.dense) return kDenseWarps * dense_slice_bytes(P.n_slots, P.pkt_cap);
-  return kWarpsPerCta * warp_slice_bytes(P.tile_samples, P.n_slots, P.unit, P.pkt_cap, dtype == WFM_F32 ? 4 : 8, P.planes == 2 ? 2 : 1);
+  return (size_t)(P.dense ? kDenseWarps : kWarpsPerCta) * program_slice(P, P.tile_samples, dtype == WFM_F32 ? 4 : 8, P.pkt_cap).bytes();
 }
 
 // tile counters of the dynamic deal: one ring per device, never freed
@@ -1887,22 +1700,22 @@ static cudaError_t launch_cfg(K k, LaunchCfg* table, std::mutex& mu, size_t smem
   return cudaSuccess;
 }
 
-template <typename OutT, int kBatch, typename K>
-static cudaError_t launch_kernel(K k, int threads, const DevProgram& P, const TileDesc* tiles, int64_t tile_begin, int64_t n_tiles,
-                                 int dtype, void* out, cudaStream_t stream, LaunchCfg* cfg_table, std::mutex& cfg_mu) {
-  const int warps = threads / 32;
+// One launch of a sampling kernel: the persistent grid (every warp walks tiles w, w+G, ... or draws batches of kBatch
+// tiles), at most one warp per tile.  The shared-memory attribute and occupancy table is per kernel instantiation.
+template <auto kKernel, int kThreadsPerCta, int kBatch, typename OutT>
+static cudaError_t launch_kernel(const DevProgram& P, const TileDesc* tiles, int64_t tile_begin, int64_t n_tiles, int dtype,
+                                 void* out, cudaStream_t stream) {
+  static LaunchCfg cfg_table[64];
+  static std::mutex cfg_mu;
+  const int warps = kThreadsPerCta / 32;
   const size_t smem = sample_smem_bytes(P, dtype);
   int dev = 0, sms = 0, per_sm = 0;
-  cudaError_t e = launch_cfg(k, cfg_table, cfg_mu, smem, &sms, &per_sm, threads);
+  cudaError_t e = launch_cfg(kKernel, cfg_table, cfg_mu, smem, &sms, &per_sm, kThreadsPerCta);
   if (e != cudaSuccess) return e;
   if (per_sm < 1) return cudaErrorInvalidConfiguration;
-  const int64_t want = (n_tiles + warps - 1) / warps;
-  int64_t cap = (int64_t)sms * per_sm;  // persistent: every warp walks tiles w, w+G, ...
-  static const int tiles_per_warp = [] { const char* v = getenv("WFM_K1_TILES_PER_WARP"); return v ? atoi(v) : WFM_K1_TILES_PER_WARP; }();
-  if (tiles_per_warp > 0) cap = std::max<int64_t>(cap, (want + tiles_per_warp - 1) / tiles_per_warp);
-  const unsigned grid = (unsigned)std::min<int64_t>(want, cap);
+  const unsigned grid = (unsigned)std::min<int64_t>((n_tiles + warps - 1) / warps, (int64_t)sms * per_sm);
   if (kBatch == 0) {
-    k<<<grid, threads, smem, stream>>>(P, tiles, (int)tile_begin, (int)(tile_begin + n_tiles), (OutT*)out, nullptr);
+    kKernel<<<grid, kThreadsPerCta, smem, stream>>>(P, tiles, (int)tile_begin, (int)(tile_begin + n_tiles), (OutT*)out, nullptr);
     return cudaGetLastError();
   }
   // the tile counter of this launch: the next slot of a per-device ring (allocated once), zeroed on the launch's
@@ -1921,49 +1734,29 @@ static cudaError_t launch_kernel(K k, int threads, const DevProgram& P, const Ti
   }
   unsigned int* counter = ring->counters + slot;
   if ((e = cudaMemsetAsync(counter, 0, sizeof(unsigned int), stream)) != cudaSuccess) return e;
-  k<<<grid, threads, smem, stream>>>(P, tiles, (int)tile_begin, (int)(tile_begin + n_tiles), (OutT*)out, counter);
+  kKernel<<<grid, kThreadsPerCta, smem, stream>>>(P, tiles, (int)tile_begin, (int)(tile_begin + n_tiles), (OutT*)out, counter);
   if ((e = cudaGetLastError()) != cudaSuccess) return e;
   return cudaEventRecord(ring->used[slot], stream);
 }
 
-template <typename OutT, bool kAcc, int U, int kBatch, bool kPair, bool kF32Eval = false>
-static cudaError_t launch_deal(const DevProgram& P, const TileDesc* tiles, int64_t tile_begin, int64_t n_tiles,
-                               int dtype, void* out, cudaStream_t stream) {
-  static LaunchCfg cfg_table[64];
-  static std::mutex cfg_mu;
-  return launch_kernel<OutT, kBatch>(sample_kernel<OutT, kAcc, U, kBatch, kPair, kF32Eval>, kThreads, P, tiles, tile_begin, n_tiles, dtype,
-                                     out, stream, cfg_table, cfg_mu);
-}
-
-template <typename OutT, bool kAcc, int kBatch, bool kPair, bool kF32Eval = false>
-static cudaError_t launch_dense(const DevProgram& P, const TileDesc* tiles, int64_t tile_begin, int64_t n_tiles,
-                                int dtype, void* out, cudaStream_t stream) {
-  static LaunchCfg cfg_table[64];
-  static std::mutex cfg_mu;
-  return launch_kernel<OutT, kBatch>(sample_dense_kernel<OutT, kAcc, kBatch, kPair, kF32Eval>, kDenseThreads, P, tiles, tile_begin, n_tiles,
-                                     dtype, out, stream, cfg_table, cfg_mu);
-}
-
-// The deal of a launch.  Dynamic (batches of WFM_K1_DYNAMIC tiles drawn from a counter) is the default whenever the warps
-// have several batches each to draw: measured +7..10 % on near-pure-store programs (cfg4) and on very uneven tiles (cfg5),
-// +2 % on dense cfg3, +-1 % on the control frames (cfg2), DESIGN.md; small launches keep the static deal (no counter to
-// allocate and zero).  WFM_K1_DEAL=static|dynamic overrides.
-template <typename OutT, bool kAcc, int U, bool kF32Eval = false>
-static cudaError_t launch_persistent(const DevProgram& P, const TileDesc* tiles, int64_t tile_begin, int64_t n_tiles,
-                                     int dtype, void* out, cudaStream_t stream) {
+// The deal of a launch.  Dynamic (batches of tiles drawn from a counter) is the default whenever the warps have several
+// batches each to draw: measured +7..10 % on near-pure-store programs (cfg4) and on very uneven tiles (cfg5), +2 % on
+// dense cfg3, +-1 % on the control frames (cfg2), DESIGN.md; small launches keep the static deal (no counter to allocate
+// and zero).  Sparse: >= ~7 tiles per warp of a full persistent grid, fp64 output only (fp32 tiles are half as long,
+// the counter traffic doubles: 856 static against 811-822 GSa/s dynamic on cfg2).  Dense: >= 8192 tiles.
+// WFM_K1_DEAL=static|dynamic overrides, for every launch.
+static bool dynamic_deal(const DevProgram& P, int64_t n_tiles, int dtype) {
   const char* dv = getenv("WFM_K1_DEAL");  // a scan of environ (~0.1 us); read per launch so that tests can flip it
   const char deal = dv ? dv[0] : '\0';
-  // >= ~7 tiles per warp of a full persistent grid; fp32 output keeps the static deal (its tiles are half as long, the
-  // counter traffic doubles: 856 static against 811-822 GSa/s dynamic on cfg2)
-  bool dynamic = n_tiles >= (int64_t)16 * 1024 && sizeof(OutT) == 8;
-  if (deal == 'd') dynamic = true;
-  if (deal == 's') dynamic = false;
-  if (P.planes == 2) {
-    if (dynamic) return launch_deal<OutT, kAcc, U, WFM_K1_DYNAMIC, true, kF32Eval>(P, tiles, tile_begin, n_tiles, dtype, out, stream);
-    return launch_deal<OutT, kAcc, U, 0, true, kF32Eval>(P, tiles, tile_begin, n_tiles, dtype, out, stream);
-  }
-  if (dynamic) return launch_deal<OutT, kAcc, U, WFM_K1_DYNAMIC, false, kF32Eval>(P, tiles, tile_begin, n_tiles, dtype, out, stream);
-  return launch_deal<OutT, kAcc, U, 0, false, kF32Eval>(P, tiles, tile_begin, n_tiles, dtype, out, stream);
+  if (deal == 'd') return true;
+  if (deal == 's') return false;
+  return P.dense ? n_tiles >= (int64_t)8 * 1024 : n_tiles >= (int64_t)16 * 1024 && dtype == WFM_F64;
+}
+
+// f(std::true_type) or f(std::false_type): a run-time flag as a compile-time one
+template <typename F>
+static cudaError_t with_bool(bool b, F&& f) {
+  return b ? f(std::true_type{}) : f(std::false_type{});
 }
 
 cudaError_t launch_sample(const DevProgram& P, const TileDesc* tiles, int64_t tile_begin, int64_t n_tiles, int dtype,
@@ -1973,64 +1766,36 @@ cudaError_t launch_sample(const DevProgram& P, const TileDesc* tiles, int64_t ti
   // WFM_F32_FAST: float output by the fp32 evaluator (not with accumulate: that is the careful path anyway)
   const bool fast32 = dtype == WFM_F32_FAST && !accumulate;
   if (dtype == WFM_F32_FAST) dtype = WFM_F32;
-  if (fast32) {
-    if (P.dense) {
-      const bool dyn = n_tiles >= (int64_t)8 * 1024;
-      if (P.planes == 2) return dyn ? launch_dense<float, false, WFM_K1_DENSE_DYNAMIC, true, true>(P, tiles, tile_begin, n_tiles, dtype, out, stream)
-                                    : launch_dense<float, false, 0, true, true>(P, tiles, tile_begin, n_tiles, dtype, out, stream);
-      return dyn ? launch_dense<float, false, WFM_K1_DENSE_DYNAMIC, false, true>(P, tiles, tile_begin, n_tiles, dtype, out, stream)
-                 : launch_dense<float, false, 0, false, true>(P, tiles, tile_begin, n_tiles, dtype, out, stream);
-    }
-    if (P.unit == 2) return launch_persistent<float, false, 2, true>(P, tiles, tile_begin, n_tiles, dtype, out, stream);
-    return launch_persistent<float, false, 1, true>(P, tiles, tile_begin, n_tiles, dtype, out, stream);
-  }
-#ifdef WFM_K1_ONLY  // register-allocation experiments: one instantiation only (compiles in seconds)
-  return launch_deal<double, false, 1, WFM_K1_DYNAMIC, false>(P, tiles, tile_begin, n_tiles, dtype, out, stream);
-#else
-  if (P.dense && (dtype == WFM_F64 || dtype == WFM_F32)) {
-    const char* dv = getenv("WFM_K1_DEAL");
-    const char deal = dv ? dv[0] : '\0';
-    bool dynamic = n_tiles >= (int64_t)8 * 1024;
-    if (deal == 'd') dynamic = true;
-    if (deal == 's') dynamic = false;
-    const int sel = (dtype == WFM_F32 ? 8 : 0) | (accumulate ? 4 : 0) | (P.planes == 2 ? 2 : 0) | (dynamic ? 1 : 0);
-    switch (sel) {
-#define WFM_DENSE_CASE(n, T, acc, batch, pair) \
-  case n: return launch_dense<T, acc, batch, pair>(P, tiles, tile_begin, n_tiles, dtype, out, stream);
-      WFM_DENSE_CASE(0, double, false, 0, false)
-      WFM_DENSE_CASE(1, double, false, WFM_K1_DENSE_DYNAMIC, false)
-      WFM_DENSE_CASE(2, double, false, 0, true)
-      WFM_DENSE_CASE(3, double, false, WFM_K1_DENSE_DYNAMIC, true)
-      WFM_DENSE_CASE(4, double, true, 0, false)
-      WFM_DENSE_CASE(5, double, true, WFM_K1_DENSE_DYNAMIC, false)
-      WFM_DENSE_CASE(6, double, true, 0, true)
-      WFM_DENSE_CASE(7, double, true, WFM_K1_DENSE_DYNAMIC, true)
-      WFM_DENSE_CASE(8, float, false, 0, false)
-      WFM_DENSE_CASE(9, float, false, WFM_K1_DENSE_DYNAMIC, false)
-      WFM_DENSE_CASE(10, float, false, 0, true)
-      WFM_DENSE_CASE(11, float, false, WFM_K1_DENSE_DYNAMIC, true)
-      WFM_DENSE_CASE(12, float, true, 0, false)
-      WFM_DENSE_CASE(13, float, true, WFM_K1_DENSE_DYNAMIC, false)
-      WFM_DENSE_CASE(14, float, true, 0, true)
-      default: return launch_dense<float, true, WFM_K1_DENSE_DYNAMIC, true>(P, tiles, tile_begin, n_tiles, dtype, out, stream);
-#undef WFM_DENSE_CASE
-    }
-  }
-  if (dtype == WFM_F64 || dtype == WFM_F32) {
-    const int sel = (dtype == WFM_F32 ? 4 : 0) | (accumulate ? 2 : 0) | (P.unit == 2 ? 1 : 0);
-    switch (sel) {
-      case 0: return launch_persistent<double, false, 1>(P, tiles, tile_begin, n_tiles, dtype, out, stream);
-      case 1: return launch_persistent<double, false, 2>(P, tiles, tile_begin, n_tiles, dtype, out, stream);
-      case 2: return launch_persistent<double, true, 1>(P, tiles, tile_begin, n_tiles, dtype, out, stream);
-      case 3: return launch_persistent<double, true, 2>(P, tiles, tile_begin, n_tiles, dtype, out, stream);
-      case 4: return launch_persistent<float, false, 1>(P, tiles, tile_begin, n_tiles, dtype, out, stream);
-      case 5: return launch_persistent<float, false, 2>(P, tiles, tile_begin, n_tiles, dtype, out, stream);
-      case 6: return launch_persistent<float, true, 1>(P, tiles, tile_begin, n_tiles, dtype, out, stream);
-      default: return launch_persistent<float, true, 2>(P, tiles, tile_begin, n_tiles, dtype, out, stream);
-    }
-  }
-  return cudaErrorInvalidValue;  // WFM_C128 is assembled from two real planes (wfm_api.cu)
-#endif
+  if (dtype != WFM_F64 && dtype != WFM_F32) return cudaErrorInvalidValue;  // WFM_C128 is assembled from two real planes (wfm_api.cu)
+  const bool dynamic = dynamic_deal(P, n_tiles, dtype);
+  return with_bool(fast32, [&](auto fast) {
+    return with_bool(dtype == WFM_F64 && !fast32, [&](auto f64) {
+      return with_bool(accumulate && !fast32, [&](auto acc) {
+        return with_bool(P.planes == 2, [&](auto pair) {
+          return with_bool(dynamic, [&](auto dyn) {
+            constexpr bool kFast = decltype(fast)::value, kAcc = decltype(acc)::value;
+            using OutT = std::conditional_t<decltype(f64)::value, double, float>;
+            if constexpr (kFast && (sizeof(OutT) == 8 || kAcc)) {
+              return cudaErrorInvalidValue;  // not reached: the fp32 evaluator writes float and never accumulates
+            } else {
+              constexpr bool kPair = decltype(pair)::value;
+              if (P.dense) {
+                constexpr int kBatch = decltype(dyn)::value ? kDenseDealBatch : 0;
+                return launch_kernel<sample_dense_kernel<OutT, kAcc, kBatch, kPair, kFast>, kDenseThreads, kBatch, OutT>(
+                    P, tiles, tile_begin, n_tiles, dtype, out, stream);
+              }
+              constexpr int kBatch = decltype(dyn)::value ? kDealBatch : 0;
+              return with_bool(P.unit == 2, [&](auto u2) {
+                constexpr int U = decltype(u2)::value ? 2 : 1;
+                return launch_kernel<sample_kernel<OutT, kAcc, U, kBatch, kPair, kFast>, kThreads, kBatch, OutT>(
+                    P, tiles, tile_begin, n_tiles, dtype, out, stream);
+              });
+            }
+          });
+        });
+      });
+    });
+  });
 }
 
 }  // namespace wfm
