@@ -17,6 +17,10 @@
  *                          multy_drag.py:158-232) + np.clip + _fill_parts.
  *   wfm_sample_host      – same, with HOST output buffers (device->host copy
  *                          inside the call): the end-to-end path.
+ *   wfm_sample_quant(_host), wfm_quantize
+ *                        – no reference counterpart: 16-bit DAC codes
+ *                          (gain, offset, round, saturate) converted in the
+ *                          kernel's store instead of NumPy on the host.
  *   wfm_sosfilt          – scipy.signal.sosfilt call sites
  *                          waveforms/waveform.py:200-203, :249.
  *   wfm_lfilter,
@@ -216,11 +220,12 @@ typedef struct WfmProgram* wfm_program_t;
                           peak unless large terms cancel (e.g. a DRAG scaling with w * s >> 1).  Opt-in. */
 #define WFM_C128 2  /* interleaved (re, im) doubles; assembled from two real planes in scratch that
                        belongs to the program: WFM_C128 launches of ONE program must be stream-ordered */
+#define WFM_I16 4   /* 16-bit DAC codes, through wfm_sample_quant / wfm_sample_quant_host only (see there) */
 
 typedef struct WfmLaunch {
   int64_t first_wave;  /* channels [first_wave, first_wave + n_wave) */
   int64_t n_wave;      /* 0 = all from first_wave                    */
-  int32_t dtype;       /* WFM_F64 | WFM_F32 | WFM_F32_FAST | WFM_C128 */
+  int32_t dtype;       /* WFM_F64 | WFM_F32 | WFM_F32_FAST | WFM_C128 | WFM_I16 */
   int32_t accumulate;  /* 0: out = value; 1: out += value            */
   void*   out;         /* DEVICE pointer (wfm_sample) / HOST pointer (wfm_sample_host) */
   int64_t out_elems;   /* capacity of out, in elements of dtype      */
@@ -253,6 +258,28 @@ int  wfm_program_info(wfm_program_t prog, int64_t* out, int32_t n);
  * `static` when capturing the call into a CUDA graph. */
 int  wfm_sample(wfm_program_t prog, const WfmLaunch* launch, void* stream);
 int  wfm_sample_host(wfm_program_t prog, const WfmLaunch* launch);
+
+/* ---- 16-bit DAC codes (WFM_I16) ---------------------------------------------------------------------------------
+ * Every sample v of an output row with gain g and offset o becomes
+ *   code = clamp(rint(v * g + o), -32768, 32767)    multiply, then add (never fused); rint rounds half to even
+ *   NaN -> 0;  +inf -> 32767;  -inf -> -32768
+ * where v is, bit for bit, the value the WFM_F64 launch of the same program writes (fp64 evaluator, the channel's
+ * min / max clip applied first).  Flat segments are converted too: an offset reaches the zero runs.  The conversion
+ * runs in the store of the sampling kernel: 2 bytes per sample leave the GPU instead of 8.
+ * row_gain_offset is a DEVICE pointer to [n_waves][2 rows][2] doubles (gain, offset), indexed by the program's
+ * absolute channel index (first_wave / n_wave sub-launches read their own rows); row 1 is read for WFM_WAVE_PAIR
+ * channels only (the second row of the pair).  launch->dtype must be WFM_I16, accumulate 0; complex channels are
+ * rejected (WFM_EINVAL), and so is a program whose rows (out_off, out_off2) are not multiples of 8 samples (the
+ * 16-byte bulk stores of 2-byte samples; lower such batches with align=8). */
+typedef struct WfmQuant {
+  const double* row_gain_offset;
+} WfmQuant;
+int  wfm_sample_quant(wfm_program_t prog, const WfmLaunch* launch, const WfmQuant* quant, void* stream);
+int  wfm_sample_quant_host(wfm_program_t prog, const WfmLaunch* launch, const WfmQuant* quant);
+/* The same conversion on f64 rows: y[s][j] = code(x[s][j]) with gain_offset[s] = (gain, offset), a DEVICE
+ * [n_sig][2] table; x (f64) and y (int16) are DEVICE pointers with their own row strides (in elements). */
+int  wfm_quantize(const double* x, int16_t* y, int64_t n_sig, int64_t n, int64_t x_stride, int64_t y_stride,
+                  const double* gain_offset, void* stream);
 
 /* Cascaded biquads, direct form II transposed, exactly scipy.signal.sosfilt:
  *   y = b0*x + z0;  z0 = b1*x - a1*y + z1;  z1 = b2*x - a2*y

@@ -80,8 +80,36 @@ class BatchResult:
         return [host[dev][off:off + n] for dev, off, n in self.table]
 
 
+def dac_rows(dtype, dac_gain, dac_offset, n, fast_fp32=False):
+    """The per-channel (gain, offset) arrays of a request for 16-bit DAC codes (``dtype=np.int16``), or None for
+    any other dtype.  Checked on the host before any device work: ``dac_gain`` is required for int16 and refused
+    otherwise, both are scalars or ``n`` values, and codes come from the fp64 evaluator only (no ``fast_fp32``)."""
+    if np.dtype(dtype) != np.dtype(np.int16):
+        if dac_gain is not None or np.any(np.asarray(dac_offset) != 0.0):
+            raise ValueError('dac_gain / dac_offset convert to 16-bit DAC codes: they need dtype=np.int16')
+        return None
+    if dac_gain is None:
+        raise ValueError('dtype=np.int16 (DAC codes) needs dac_gain: code = clamp(rint(v * dac_gain + dac_offset))')
+    if fast_fp32:
+        raise ValueError('fast_fp32 is a float32 option: DAC codes are converted from the fp64 evaluator')
+    try:
+        g = np.broadcast_to(np.asarray(dac_gain, dtype=np.float64), (n,))
+        o = np.broadcast_to(np.asarray(dac_offset, dtype=np.float64), (n,))
+    except ValueError:
+        raise ValueError(f'dac_gain / dac_offset: a scalar or one value per channel ({n})') from None
+    return np.ascontiguousarray(g), np.ascontiguousarray(o)
+
+
+def _codes(prog, batch, dev, gain, offset):
+    """The program's samples as DAC codes (WFM_I16) with per-channel gain and offset."""
+    import torch
+    table = torch.from_numpy(engine.quant_table(batch, gain, offset)).to(f'cuda:{dev}')
+    return prog.sample_device(dtype=engine.WFM_I16, quant=table)
+
+
 def sample_batch(waveforms, sample_rate=None, dtype=np.float64, devices=None,
-                 filters='own', iir_mode='auto', pair_iq='auto', fast_fp32=False):
+                 filters='own', iir_mode='auto', pair_iq='auto', fast_fp32=False,
+                 dac_gain=None, dac_offset=0.0):
     """Sample every waveform in ``waveforms`` on its own start/stop/sample_rate
     grid.  ``dtype``: np.float64 (reference parity, 1e-12) or np.float32
     (fp32 output, 1e-6).  ``devices``: list of CUDA device indices to shard the
@@ -99,6 +127,14 @@ def sample_batch(waveforms, sample_rate=None, dtype=np.float64, devices=None,
     segment's terms, see include/wfm_b200.h) instead of fp64 arithmetic rounded at
     the store, which meets 1e-6 on every program.
 
+    ``dtype=np.int16``: 16-bit DAC codes, ``clamp(rint(v * dac_gain + dac_offset), -32768,
+    32767)`` (multiply, then add; half to even; NaN -> 0, +-inf saturate) of the float64
+    samples ``v`` this call returns for ``dtype=np.float64`` — exactly, converted in the
+    kernel's store (2 bytes per sample leave the GPU).  ``dac_gain`` (required) and
+    ``dac_offset`` are scalars or one value per channel in the order of ``waveforms``; the
+    I and Q of a pair keep their own.  Filtered batches are sampled and filtered in float64
+    and then converted (``dsp.quantize_device``).  Complex channels have no single code.
+
     (Batches below ``PAIR_MIN_SAMPLES`` samples stay unpaired under 'auto': a pair is one
     work item per tile instead of two, and a launch that cannot fill the GPU is bound by
     the latency of its longest item — the README example is 1.8 x slower paired.)
@@ -109,6 +145,7 @@ def sample_batch(waveforms, sample_rate=None, dtype=np.float64, devices=None,
     computed once and feeds both outputs (the second row's cosines are rotated from
     the shared sincos: equal to unpaired sampling to a few ulp); ``False`` keeps every channel
     on its own; ``True`` requires channels (0, 1), (2, 3) ... to pair."""
+    dac = dac_rows(dtype, dac_gain, dac_offset, len(waveforms), fast_fp32)
     import torch
     engine.require_gpu()
     items = [channel_grid(w, sample_rate) for w in waveforms]
@@ -117,14 +154,15 @@ def sample_batch(waveforms, sample_rate=None, dtype=np.float64, devices=None,
     np_dtype = np.dtype(dtype)
     code = {np.dtype(np.float64): engine.WFM_F64,
             np.dtype(np.float32): engine.WFM_F32,
-            np.dtype(np.complex128): engine.WFM_C128}[np_dtype]
+            np.dtype(np.complex128): engine.WFM_C128,
+            np.dtype(np.int16): engine.WFM_I16}[np_dtype]
     filtered = filters == 'own' and any(w.filters is not None for w in waveforms)
     if filtered and code == engine.WFM_C128:
         raise TypeError('sample_batch(filters=\'own\') filters real channels; sample complex '
                         'channels one by one (Waveform.sample) or pass filters=None')
-    # the IIR runs on float64 samples: an fp32 batch with filters is sampled and filtered in
-    # float64 and cast at the end
-    run_code = engine.WFM_F64 if (filtered and code == engine.WFM_F32) else code
+    # the IIR runs on float64 samples: an fp32 or int16 batch with filters is sampled and filtered in
+    # float64 and converted at the end
+    run_code = engine.WFM_F64 if (filtered and code in (engine.WFM_F32, engine.WFM_I16)) else code
     if run_code == engine.WFM_F32 and fast_fp32:
         run_code = engine.WFM_F32_FAST
     ranges = shard_ranges([g.n for _, g in items], len(devices))
@@ -135,7 +173,11 @@ def sample_batch(waveforms, sample_rate=None, dtype=np.float64, devices=None,
         ranges = [(lo + (lo & 1) if lo < len(items) else lo, hi + (hi & 1) if hi < len(items) else hi)
                   for lo, hi in ranges]
 
-    shards = [(dev, lo, hi, lower(plan_pairs(items[lo:hi], pair_iq))) for dev, (lo, hi) in zip(devices, ranges)]
+    # 16-bit codes: rows at multiples of 8 samples (16-byte bulk stores of 2-byte samples)
+    align = 8 if dac is not None else 4
+    shards = [(dev, lo, hi, lower(plan_pairs(items[lo:hi], pair_iq), align)) for dev, (lo, hi) in zip(devices, ranges)]
+    if dac is not None and any(batch.any_complex for _, _, _, batch in shards):
+        raise ValueError('dtype=np.int16: a channel with complex amplitudes has no single DAC code')
 
     def run(shard):
         # one host thread per device: upload, pre-pass, K1 and the filters of every device run
@@ -143,12 +185,17 @@ def sample_batch(waveforms, sample_rate=None, dtype=np.float64, devices=None,
         dev, lo, hi, batch = shard
         with torch.cuda.device(dev):
             prog = engine.Program(batch, dev)
+            if run_code == engine.WFM_I16:
+                return prog, _codes(prog, batch, dev, dac[0][lo:hi], dac[1][lo:hi])
             out = prog.sample_device(dtype=run_code)
             if filtered:
                 from .dsp import apply_channel_filters
                 apply_channel_filters(out, batch, waveforms[lo:hi], mode=iir_mode)
             if run_code == engine.WFM_F64 and code == engine.WFM_F32:
                 out = out.to(torch.float32)
+            if code == engine.WFM_I16:
+                from .dsp import quantize_batch
+                out = quantize_batch(out, batch, dac[0][lo:hi], dac[1][lo:hi])
         return prog, out
 
     results = _run_shards(run, shards)
@@ -199,7 +246,8 @@ def sample_wire(records, kinds=None, **kw):
 
 
 def sample_pulse_trains(templates, tmpl_idx, t0, start, stop, sample_rate,
-                        dtype=np.float64, devices=None, params=None, compact='auto'):
+                        dtype=np.float64, devices=None, params=None, compact='auto',
+                        dac_gain=None, dac_offset=0.0):
     """Channels given as PARAMETER ARRAYS instead of objects: channel ``c`` is the
     stack of pulses ``templates[tmpl_idx[c][k]]`` started at ``t0[c][k]``
     (``builder.PulseTemplate.trace`` / ``builder.pulse_train_batch``), sampled on
@@ -208,7 +256,11 @@ def sample_pulse_trains(templates, tmpl_idx, t0, start, stop, sample_rate,
     Same sharding and result type as ``sample_batch``; the tables are those the
     object API would have produced.  ``compact``: upload templates + per-pulse payloads and write the per-pulse rows
     on the device (``builder.CompactBatch``, ``wfm_expand_templates``) — 'auto' = whenever the channels allow it
-    (time-ordered, non-overlapping pulses), True = insist, False = build the full tables on the host."""
+    (time-ordered, non-overlapping pulses), True = insist, False = build the full tables on the host.
+    ``dtype=np.int16`` with ``dac_gain`` / ``dac_offset``: 16-bit DAC codes as in ``sample_batch``; per-channel
+    values follow the result's channels (pair templates: the I and Q rows of every ``t0`` row)."""
+    rows = 2 if templates and templates[0].pair else 1
+    dac = dac_rows(dtype, dac_gain, dac_offset, len(t0) * rows)
     import torch
     from .builder import pulse_train_batch
     engine.require_gpu()
@@ -216,14 +268,15 @@ def sample_pulse_trains(templates, tmpl_idx, t0, start, stop, sample_rate,
         devices = [torch.cuda.current_device()]
     code = {np.dtype(np.float64): engine.WFM_F64,
             np.dtype(np.float32): engine.WFM_F32,
-            np.dtype(np.complex128): engine.WFM_C128}[np.dtype(dtype)]
+            np.dtype(np.complex128): engine.WFM_C128,
+            np.dtype(np.int16): engine.WFM_I16}[np.dtype(dtype)]
     ranges = shard_ranges([max(len(r), 1) for r in t0], len(devices))
     shards = [(dev, lo, hi) for dev, (lo, hi) in zip(devices, ranges)]
 
     def run(shard):
         dev, lo, hi = shard
         args = (templates, tmpl_idx[lo:hi], t0[lo:hi], start, stop, sample_rate)
-        kw = dict(params={k: v[lo:hi] for k, v in (params or {}).items()})
+        kw = dict(params={k: v[lo:hi] for k, v in (params or {}).items()}, align=8 if dac is not None else 4)
         if compact == 'auto':
             try:
                 batch = pulse_train_batch(*args, compact=True, **kw)
@@ -233,8 +286,12 @@ def sample_pulse_trains(templates, tmpl_idx, t0, start, stop, sample_rate,
                 batch = pulse_train_batch(*args, **kw)
         else:
             batch = pulse_train_batch(*args, compact=bool(compact), **kw)
+        if dac is not None and batch.any_complex:
+            raise ValueError('dtype=np.int16: a channel with complex amplitudes has no single DAC code')
         with torch.cuda.device(dev):
             prog = engine.Program(batch, dev)
+            if dac is not None:
+                return prog, _codes(prog, batch, dev, dac[0][lo * rows:hi * rows], dac[1][lo * rows:hi * rows]), batch
             out = prog.sample_device(dtype=code)
         return prog, out, batch
 

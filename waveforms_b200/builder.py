@@ -31,7 +31,7 @@ import numpy as np
 from . import _algebra as A
 from . import engine
 from .lowering import (PACKERS, FACTOR_DT, REF_DT, SEGPTR_DT, TERM_DT, WAVE_COMPLEX, WAVE_PAIR,
-                       WAVE_DT, LoweredBatch, TracedFloat, _Pools, _lower_segment, _plan_slots)
+                       WAVE_DT, LoweredBatch, TracedFloat, _Pools, _lower_segment, _plan_slots, row_pitch)
 
 
 class UntraceablePulse(ValueError):
@@ -541,7 +541,7 @@ class CompactBatch:
 
 
 def pulse_train_batch(templates, tmpl_idx, t0, start, stop, sample_rate, params=None,
-                      spot_check=4, compact=False) -> LoweredBatch:
+                      spot_check=4, compact=False, align=4) -> LoweredBatch:
     """One channel per row: channel ``c`` is the stack of pulses ``templates[tmpl_idx[c][k]]`` started at
     ``t0[c][k]``.  Channels whose pulses are time-ordered and do not overlap — gate sequences — are assembled
     by NumPy scatter (``_pulse_train_disjoint``); a channel with OVERLAPPING (or unordered) pulses — flux
@@ -553,11 +553,13 @@ def pulse_train_batch(templates, tmpl_idx, t0, start, stop, sample_rate, params=
 
     ``compact=True`` (all channels disjoint): a ``CompactBatch`` — the templates' tables once plus a few
     doubles per pulse; the per-pulse rows are written on the device (``wfm_expand_templates``), so the host
-    neither builds nor uploads them."""
+    neither builds nor uploads them.
+
+    ``align``: rows start at multiples of this many samples (``lowering.row_pitch``; 8 for 16-bit DAC codes)."""
     n_ch = len(t0)
     params = params or {}
     if n_ch == 0 or not templates:
-        return _pulse_train_disjoint(templates, tmpl_idx, t0, start, stop, sample_rate, params, spot_check, compact)
+        return _pulse_train_disjoint(templates, tmpl_idx, t0, start, stop, sample_rate, params, spot_check, compact, align)
     # first / last edge of every pulse: the templates' outer bounds over the parameter arrays
     general = []
     for c in range(n_ch):
@@ -581,7 +583,7 @@ def pulse_train_batch(templates, tmpl_idx, t0, start, stop, sample_rate, params=
         if np.any(first[1:] < last[:-1]):
             general.append(c)
     if not general:
-        return _pulse_train_disjoint(templates, tmpl_idx, t0, start, stop, sample_rate, params, spot_check, compact)
+        return _pulse_train_disjoint(templates, tmpl_idx, t0, start, stop, sample_rate, params, spot_check, compact, align)
     if compact:
         raise ValueError('compact=True needs channels of time-ordered, non-overlapping pulses '
                          f'(channel {general[0]} overlaps)')
@@ -591,7 +593,8 @@ def pulse_train_batch(templates, tmpl_idx, t0, start, stop, sample_rate, params=
     parts, owners = [], []
     if plain:
         parts.append(_pulse_train_disjoint(templates, [tmpl_idx[c] for c in plain], [t0[c] for c in plain], start, stop,
-                                           sample_rate, {k: [v[c] for c in plain] for k, v in params.items()}, spot_check))
+                                           sample_rate, {k: [v[c] for c in plain] for k, v in params.items()}, spot_check,
+                                           align=align))
         owners.append(plain)
     grid = engine.arange_grid(start, stop, 1 / sample_rate)
     pair = bool(templates[0].pair)
@@ -607,13 +610,13 @@ def pulse_train_batch(templates, tmpl_idx, t0, start, stop, sample_rate, params=
                 rows[1].append((mat[0], mat[2]))
         chans = [Channel(members=r, clip=None, offset=0, pre_shift=0, real_only=True) for r in rows[:2 if pair else 1]]
         items.append(((chans[0], chans[1]), grid) if pair else (chans[0], grid))
-    parts.append(lower(items))
+    parts.append(lower(items, align))
     owners.append(general)
-    return merge_batches(parts, owners)
+    return merge_batches(parts, owners, align)
 
 
 def _pulse_train_disjoint(templates, tmpl_idx, t0, start, stop, sample_rate, params=None,
-                          spot_check=4, compact=False) -> LoweredBatch:
+                          spot_check=4, compact=False, align=4) -> LoweredBatch:
     """Channels of time-ordered, NON-overlapping pulses, sampled on
     ``np.arange(start, stop, 1/sample_rate)`` — the ``LoweredBatch`` that
     ``lower([channel_grid(WaveVStack([fn(t, ...) for ...]))])`` yields, built with NumPy.
@@ -735,7 +738,7 @@ def _pulse_train_disjoint(templates, tmpl_idx, t0, start, stop, sample_rate, par
     if any(bool(t.pair) != pair for t in templates):
         raise ValueError('pair templates (fn returns (I, Q)) and single-output templates cannot share a batch')
     rows = 2 if pair else 1
-    pitch = (grid.n + 3) & ~3
+    pitch = row_pitch(grid.n, align)
     waves = np.zeros(n_ch, dtype=WAVE_DT)
     waves['t0'], waves['delta'], waves['n'] = grid.t0, grid.delta, grid.n
     waves['out_off'] = np.arange(n_ch, dtype=np.int64) * (rows * pitch)

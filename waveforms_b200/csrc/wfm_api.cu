@@ -205,6 +205,7 @@ struct WfmProgram {
   int64_t launches = 0;
   bool any_complex = false;
   bool gapless = false;
+  bool rows_aligned8 = true;  // every row starts at a multiple of 8 samples: WFM_I16 output (16-byte stores of 2-byte codes)
   // complex128 output: a planar twin (channels [0, n) = real parts, [n, 2n) = imaginary parts,
   // both real-valued programs for the fast kernel) and the scratch the two planes are sampled into
   WfmProgram* planar = nullptr;
@@ -470,9 +471,11 @@ int wfm_program_create(const WfmProgramDesc* d, int device, wfm_program_t* out) 
     rows += d->waves[w].n * ((d->waves[w].flags & WFM_WAVE_PAIR) ? 2 : 1);
     total = std::max(total, d->waves[w].out_off + d->waves[w].n);
     if (d->waves[w].flags & WFM_WAVE_COMPLEX) p->any_complex = true;
+    if (d->waves[w].out_off % 8) p->rows_aligned8 = false;
     if (d->waves[w].flags & WFM_WAVE_PAIR) {
       p->dev.planes = 2;
       total = std::max(total, d->waves[w].out_off2 + d->waves[w].n);
+      if (d->waves[w].out_off2 % 8) p->rows_aligned8 = false;
     }
   }
   p->total_samples = total;
@@ -784,7 +787,8 @@ static int check_launch(wfm_program_t prog, const WfmLaunch* l, int64_t* first, 
   *first = l->first_wave;
   *count = l->n_wave == 0 ? nw - l->first_wave : l->n_wave;
   if (*first < 0 || *count < 0 || *first + *count > nw) return fail(WFM_EINVAL, "channel range out of bounds");
-  if (l->dtype != WFM_F64 && l->dtype != WFM_F32 && l->dtype != WFM_F32_FAST && l->dtype != WFM_C128) return fail(WFM_EINVAL, "bad dtype");
+  if (l->dtype != WFM_F64 && l->dtype != WFM_F32 && l->dtype != WFM_F32_FAST && l->dtype != WFM_C128 && l->dtype != WFM_I16)
+    return fail(WFM_EINVAL, "bad dtype");
   if (prog->any_complex && l->dtype != WFM_C128)
     for (int64_t w = *first; w < *first + *count; ++w)
       if (prog->waves[w].flags & WFM_WAVE_COMPLEX)
@@ -802,10 +806,10 @@ static int check_launch(wfm_program_t prog, const WfmLaunch* l, int64_t* first, 
 
 // the launch(es) of one sampling request: channels [first, first + count) -> out (device)
 static int launch_request(wfm_program_t prog, int64_t first, int64_t count, int dtype, int accumulate, void* out,
-                          cudaStream_t st) {
+                          cudaStream_t st, const double* quant = nullptr) {
   const int64_t t0 = prog->tile_prefix[first], t1 = prog->tile_prefix[first + count];
   if (dtype != WFM_C128) {
-    WFM_CUDA(wfm::launch_sample(prog->dev, prog->d_tiles, t0, t1 - t0, dtype, accumulate, out, st));
+    WFM_CUDA(wfm::launch_sample(prog->dev, prog->d_tiles, t0, t1 - t0, dtype, accumulate, out, st, quant));
     return WFM_OK;
   }
   // complex128: real and imaginary plane by the real-valued kernel into scratch, then
@@ -836,14 +840,22 @@ static int launch_request(wfm_program_t prog, int64_t first, int64_t count, int 
   return WFM_OK;
 }
 
-int wfm_sample(wfm_program_t prog, const WfmLaunch* l, void* stream) {
-  int64_t first, count, need;
-  int rc = check_launch(prog, l, &first, &count, &need);
-  if (rc != WFM_OK) return rc;
+// the WFM_I16 requirements of a launch (wfm_sample_quant / wfm_sample_quant_host), after check_launch
+static int check_quant(wfm_program_t prog, const WfmLaunch* l, const WfmQuant* q) {
+  if (l->dtype != WFM_I16) return fail(WFM_EINVAL, "wfm_sample_quant writes WFM_I16 codes only (dtype %d)", l->dtype);
+  if (l->accumulate) return fail(WFM_EINVAL, "DAC codes cannot be accumulated");
+  if (!q || !q->row_gain_offset) return fail(WFM_EINVAL, "null gain / offset table");
+  if (!prog->rows_aligned8)
+    return fail(WFM_EINVAL, "WFM_I16 output needs every row at a multiple of 8 samples (lower the batch with align=8)");
+  return WFM_OK;
+}
+
+static int sample_device(wfm_program_t prog, const WfmLaunch* l, const double* quant, void* stream, int64_t first,
+                         int64_t count) {
   if ((uintptr_t)l->out % 16) return fail(WFM_EINVAL, "output buffer must be 16-byte aligned");
   DeviceGuard g(prog->device);
   const int64_t t0 = prog->tile_prefix[first], t1 = prog->tile_prefix[first + count];
-  rc = launch_request(prog, first, count, l->dtype, l->accumulate, l->out, (cudaStream_t)stream);
+  int rc = launch_request(prog, first, count, l->dtype, l->accumulate, l->out, (cudaStream_t)stream, quant);
   if (rc != WFM_OK) return rc;
   if (t1 > t0) {
     prog->launches += 1;
@@ -860,15 +872,29 @@ int wfm_sample(wfm_program_t prog, const WfmLaunch* l, void* stream) {
   return WFM_OK;
 }
 
-int wfm_sample_host(wfm_program_t prog, const WfmLaunch* l) {
+int wfm_sample(wfm_program_t prog, const WfmLaunch* l, void* stream) {
   int64_t first, count, need;
   int rc = check_launch(prog, l, &first, &count, &need);
   if (rc != WFM_OK) return rc;
+  if (l->dtype == WFM_I16) return fail(WFM_EINVAL, "WFM_I16 output takes a gain / offset table: call wfm_sample_quant");
+  return sample_device(prog, l, nullptr, stream, first, count);
+}
+
+int wfm_sample_quant(wfm_program_t prog, const WfmLaunch* l, const WfmQuant* q, void* stream) {
+  int64_t first, count, need;
+  int rc = check_launch(prog, l, &first, &count, &need);
+  if (rc == WFM_OK) rc = check_quant(prog, l, q);
+  if (rc != WFM_OK) return rc;
+  return sample_device(prog, l, q->row_gain_offset, stream, first, count);
+}
+
+static int sample_host(wfm_program_t prog, const WfmLaunch* l, const double* quant, int64_t first, int64_t count,
+                       int64_t need) {
   if (l->accumulate) return fail(WFM_EUNSUPPORTED, "accumulate is not available with host buffers");
   StageTimer tm("sample_host");
   const cudaStream_t ST = cudaStreamPerThread;  // see wfm_program_create
   DeviceGuard g(prog->device);
-  const size_t esz = l->dtype == WFM_F64 ? 8 : ((l->dtype == WFM_F32 || l->dtype == WFM_F32_FAST) ? 4 : 16);
+  const size_t esz = l->dtype == WFM_F64 ? 8 : ((l->dtype == WFM_F32 || l->dtype == WFM_F32_FAST) ? 4 : (l->dtype == WFM_I16 ? 2 : 16));
   // only the extent actually covered by the requested channels is staged/copied
   int64_t lo = INT64_MAX;
   for (int64_t w = first; w < first + count; ++w) lo = std::min(lo, prog->waves[w].out_off);
@@ -885,7 +911,7 @@ int wfm_sample_host(wfm_program_t prog, const WfmLaunch* l) {
   if (!(prog->gapless && first == 0 && count == (int64_t)prog->waves.size())) WFM_CUDA(cudaMemsetAsync((char*)prog->stage.p + (size_t)lo * esz, 0, (size_t)(need - lo) * esz, ST));
   const int64_t t0 = prog->tile_prefix[first], t1 = prog->tile_prefix[first + count];
   {
-    const int rc2 = launch_request(prog, first, count, l->dtype, 0, prog->stage.p, ST);
+    const int rc2 = launch_request(prog, first, count, l->dtype, 0, prog->stage.p, ST, quant);
     if (rc2 != WFM_OK) return rc2;
   }
   if (t1 > t0) prog->launches += 1;
@@ -908,6 +934,32 @@ int wfm_sample_host(wfm_program_t prog, const WfmLaunch* l) {
     WFM_CUDA(cudaStreamSynchronize(ST));
   }
   tm.lap("memset+kernel+D2H");
+  return WFM_OK;
+}
+
+int wfm_sample_host(wfm_program_t prog, const WfmLaunch* l) {
+  int64_t first, count, need;
+  int rc = check_launch(prog, l, &first, &count, &need);
+  if (rc != WFM_OK) return rc;
+  if (l->dtype == WFM_I16) return fail(WFM_EINVAL, "WFM_I16 output takes a gain / offset table: call wfm_sample_quant_host");
+  return sample_host(prog, l, nullptr, first, count, need);
+}
+
+int wfm_sample_quant_host(wfm_program_t prog, const WfmLaunch* l, const WfmQuant* q) {
+  int64_t first, count, need;
+  int rc = check_launch(prog, l, &first, &count, &need);
+  if (rc == WFM_OK) rc = check_quant(prog, l, q);
+  if (rc != WFM_OK) return rc;
+  return sample_host(prog, l, q->row_gain_offset, first, count, need);
+}
+
+int wfm_quantize(const double* x, int16_t* y, int64_t n_sig, int64_t n, int64_t x_stride, int64_t y_stride,
+                 const double* gain_offset, void* stream) {
+  if (n_sig < 0 || n < 0) return fail(WFM_EINVAL, "negative size");
+  if (n_sig == 0 || n == 0) return WFM_OK;
+  if (!x || !y || !gain_offset) return fail(WFM_EINVAL, "null pointer");
+  if (n_sig > 1 && (x_stride < n || y_stride < n)) return fail(WFM_EINVAL, "row stride smaller than the row");
+  WFM_CUDA(wfm::launch_quantize(x, y, n_sig, n, x_stride, y_stride, gain_offset, (cudaStream_t)stream));
   return WFM_OK;
 }
 

@@ -2,6 +2,7 @@
 // NumPy / SciPy evaluate a*b+c as two rounded operations; these wrappers keep
 // the compiler from fusing them (see wfm_basis.cuh, wfm_iir.cu).
 #pragma once
+#include <stdint.h>
 
 namespace wfm {
 
@@ -143,6 +144,18 @@ __device__ __forceinline__ void sincos_cw_n(const double (&a)[N], double (&s_out
     s_out[u] = __longlong_as_double(__double_as_longlong(ss) ^ sbit);
     c_out[u] = __longlong_as_double(__double_as_longlong(cc) ^ cbit);
   }
+}
+
+// The 16-bit DAC code of a sample v on a row with gain g and offset o (WFM_I16 output, wfm_quantize):
+//   clamp(rint(v * g + o), -32768, 32767)   multiply, then add (never fused); rint rounds half to even
+// NaN -> 0 (tested here, not left to the conversion instruction); +-inf saturate like any out-of-range value.
+// The clamp runs on the integer: cvt.rni.s32.f64 saturates at the int32 range (PTX: float-to-integer conversions
+// clamp to the destination range), and the two fp64 min / max it saves are issue slots of the FP64 pipe, which the
+// dense kernel is bound by.
+__device__ __forceinline__ int16_t dac_code(double v, double g, double o) {
+  const double y = add(mul(v, g), o);
+  if (y != y) return 0;
+  return (int16_t)min(max(__double2int_rn(y), -32768), 32767);
 }
 
 }  // namespace wfm

@@ -42,7 +42,7 @@
 //      are spent on the output, and the store drains while the warp is already in
 //      the prologue of its next tile.
 //
-// Algorithmic traffic: 8 B (4 B) per sample, write-only.
+// Algorithmic traffic: 8 B (4 B, 2 B) per sample, write-only.
 #include <cuda_runtime.h>
 #include <mutex>
 #include <cstdlib>
@@ -62,6 +62,20 @@ constexpr int kWarpsPerCta = kThreads / 32;
 template <typename T> struct OutVec;
 template <> struct OutVec<double> { static constexpr int N = 2; };
 template <> struct OutVec<float> { static constexpr int N = 4; };
+template <> struct OutVec<int16_t> { static constexpr int N = 8; };
+
+// WFM_I16 output: 16-bit DAC codes (dac_code, wfm_math.cuh) with the gain and offset of each output row
+template <typename OutT> constexpr bool kCodes = std::is_same_v<OutT, int16_t>;
+// (gain, offset) of row `plane` of channel `wave` in the WfmQuant table; read where a conversion needs them, not held
+// in registers across the tile loop (the sparse kernel sits at its register budget)
+__device__ __forceinline__ const double* row_quant(const double* quant, int wave, int plane) {
+  return quant + ((size_t)wave * 2 + plane) * 2;
+}
+// eight codes in one 16-byte word
+__device__ __forceinline__ uint4 code_pattern(int16_t c) {
+  const uint32_t w = (uint32_t)(uint16_t)c * 0x10001u;
+  return make_uint4(w, w, w, w);
+}
 
 // ---- shared-memory vector stores ---------------------------------------------------
 __device__ __forceinline__ void fill_vec(double* p, double v) { *reinterpret_cast<double2*>(p) = make_double2(v, v); }
@@ -69,6 +83,7 @@ __device__ __forceinline__ void fill_vec(float* p, double v) {
   const float f = (float)v;
   *reinterpret_cast<float4*>(p) = make_float4(f, f, f, f);
 }
+__device__ __forceinline__ void fill_vec(int16_t* p, int16_t c) { *reinterpret_cast<uint4*>(p) = code_pattern(c); }
 // ---- mbarrier + TMA bulk copies ------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
@@ -1065,8 +1080,8 @@ __global__ void __launch_bounds__(256) fill_packets_kernel(DevProgram P, const T
 
 // ---- the sampling kernel ------------------------------------------------------------------
 // [a, b) of the warp's shared tile <- val
-template <typename OutT>
-__device__ __forceinline__ void fill_run(OutT* __restrict__ s_out, int a, int b, double val, int lane) {
+template <typename OutT, typename T>
+__device__ __forceinline__ void fill_run_value(OutT* __restrict__ s_out, int a, int b, T val, int lane) {
   constexpr int V = OutVec<OutT>::N;
   const int a_al = (a + V - 1) & ~(V - 1), b_al = b & ~(V - 1);
   if (a_al >= b_al) {
@@ -1078,6 +1093,13 @@ __device__ __forceinline__ void fill_run(OutT* __restrict__ s_out, int a, int b,
 #pragma unroll 1
   for (int p = a_al + lane * V; p < b_al; p += 32 * V) fill_vec(s_out + p, val);
 }
+// (int16 output: the code of val with the row's (gain, offset) q)
+template <typename OutT>
+__device__ __forceinline__ void fill_run(OutT* __restrict__ s_out, int a, int b, double val, int lane,
+                                         const double* q = nullptr) {
+  if constexpr (kCodes<OutT>) fill_run_value(s_out, a, b, dac_code(val, q[0], q[1]), lane);
+  else fill_run_value(s_out, a, b, val, lane);
+}
 
 // n_rows 512-byte rows of the warp's tile buffer <- val: every lane stores 16 bytes per
 // row, fully unrolled per size so that the fill is n_rows stores and nothing else
@@ -1086,7 +1108,8 @@ __device__ __forceinline__ void fill_rows(unsigned char* p, uint4 v) {
 #pragma unroll
   for (int r = 0; r < R; ++r) *reinterpret_cast<uint4*>(p + r * 512) = v;
 }
-__device__ __forceinline__ void fill_tile(unsigned char* p, int n_rows, double val, bool f32) {
+// the 16-byte pattern of a float / double tile buffer holding val
+__device__ __forceinline__ uint4 fill_pattern(double val, bool f32) {
   uint4 v = make_uint4(0u, 0u, 0u, 0u);
   if (__double_as_longlong(val) != 0) {
     if (f32) {
@@ -1096,8 +1119,11 @@ __device__ __forceinline__ void fill_tile(unsigned char* p, int n_rows, double v
       v.y = v.w = (uint32_t)__double2hiint(val);
     }
   }
+  return v;
+}
+__device__ __forceinline__ void fill_tile(unsigned char* p, int n_rows, uint4 v) {
   static_assert(kMaxTileSamples * 8 / 512 == 24, "the largest tile (fp64) is the first case");
-  switch (n_rows) {  // tile_samples is a multiple of 128: 2 rows each in fp64, 1 row in fp32
+  switch (n_rows) {  // tile_samples is a multiple of 128: 2 rows each in fp64, 1 row in fp32, half a row in int16
     case 24: fill_rows<24>(p, v); break;
     case 22: fill_rows<22>(p, v); break;
     case 20: fill_rows<20>(p, v); break;
@@ -1127,13 +1153,22 @@ __device__ __forceinline__ unsigned char* lane_slots(unsigned char* s_slots, int
 }
 
 // the cold path of a tile (its packet would not fit the warp's buffers): per-sample
-// search, tables in global memory, direct stores
+// search, tables in global memory, direct stores (int16 output: codes with the rows' (gain, offset) from quant)
 template <typename OutT, bool kAccumulate, bool kPair>
-__device__ __noinline__ void sample_tile_cold(const DevProgram& P, const TileDesc& td, OutT* __restrict__ out, int lane) {
+__device__ __forceinline__ void cold_tile(const DevProgram& P, const TileDesc& td, OutT* __restrict__ out, int lane,
+                                          const double* quant) {
   OutT* __restrict__ dst = out + td.out0;
   const WfmWave w = P.waves[td.wave];
   const WaveEval we{w.offset, w.flags, td.wave};
   const int32_t* __restrict__ st = P.seg_start + td.seg0;
+  auto store = [&](OutT* __restrict__ row, int jj, double re, int plane) {
+    if constexpr (kCodes<OutT>) {
+      const double* q = row_quant(quant, td.wave, plane);
+      row[jj] = dac_code(re, q[0], q[1]);
+    } else {
+      row[jj] = kAccumulate ? (OutT)add((double)row[jj], re) : (OutT)re;
+    }
+  };
   for (int jj = lane; jj < td.cnt; jj += 32) {
     int lo = 0, hi = td.nb - 1;
     while (lo < hi) {
@@ -1145,14 +1180,23 @@ __device__ __noinline__ void sample_tile_cold(const DevProgram& P, const TileDes
     if (kPair && (w.flags & WFM_WAVE_PAIR)) {
       OutT* __restrict__ dst1 = out + w.out_off2 + td.j0;
       re = eval_segment_slow_row(P, td.seg0 + lo, we.offset, we.flags, we.wave, xv, 0, 0.0);
-      dst[jj] = kAccumulate ? (OutT)add((double)dst[jj], re) : (OutT)re;
+      store(dst, jj, re, 0);
       re = eval_segment_slow_row(P, td.seg0 + lo, we.offset, we.flags, we.wave, xv, 1, w.offset2);
-      dst1[jj] = kAccumulate ? (OutT)add((double)dst1[jj], re) : (OutT)re;
+      store(dst1, jj, re, 1);
     } else {
       re = eval_segment_slow(P, td.seg0 + lo, we.offset, we.flags, we.wave, xv);
-      dst[jj] = kAccumulate ? (OutT)add((double)dst[jj], re) : (OutT)re;
+      store(dst, jj, re, 0);
     }
   }
+}
+template <typename OutT, bool kAccumulate, bool kPair>
+__device__ __noinline__ void sample_tile_cold(const DevProgram& P, const TileDesc& td, OutT* __restrict__ out, int lane) {
+  cold_tile<OutT, kAccumulate, kPair>(P, td, out, lane, nullptr);
+}
+template <bool kPair>
+__device__ __noinline__ void sample_tile_cold_codes(const DevProgram& P, const TileDesc& td, int16_t* __restrict__ out,
+                                                    const double* quant, int lane) {
+  cold_tile<int16_t, false, kPair>(P, td, out, lane, quant);
 }
 
 // batch size of the dynamic deal (WFM_K1_DEAL=dynamic at run time, or a large launch: dynamic_deal)
@@ -1173,7 +1217,7 @@ extern __shared__ __align__(128) unsigned char k1_smem[];
 // the packet pipeline can still look two tiles on
 template <int kCtaWarps, int kBatch, int U, bool kF32Eval, typename OutT, bool kAccumulate, bool kPair, typename Body>
 __device__ __forceinline__ void for_each_tile(const DevProgram& P, const TileDesc* tiles, int tile_begin, int tile_end,
-                                              OutT* out, unsigned int* tile_counter,
+                                              OutT* out, const double* quant, unsigned int* tile_counter,
                                               unsigned char* s_slots, unsigned char* s_pkt, uint64_t* s_bar, const Body& body) {
   static_assert(kBatch == 0 || (kBatch >= 2 && (kBatch & (kBatch - 1)) == 0), "batch: 0 or a power of two >= 2");
   const int lane = threadIdx.x & 31;
@@ -1277,7 +1321,8 @@ __device__ __forceinline__ void for_each_tile(const DevProgram& P, const TileDes
     // of spills at its 128-register budget, ptxas -v)
     const uint32_t flags = reinterpret_cast<const PacketHeader*>(pk)->flags;
     if (flags & kPacketCold) {
-      sample_tile_cold<OutT, kAccumulate, kPair>(P, tiles[t], out, lane);
+      if constexpr (kCodes<OutT>) sample_tile_cold_codes<kPair>(P, tiles[t], out, quant, lane);
+      else sample_tile_cold<OutT, kAccumulate, kPair>(P, tiles[t], out, lane);
       __syncwarp();
       ++it;
       continue;
@@ -1359,7 +1404,7 @@ __device__ __forceinline__ void eval_units(const DevProgram& P, const unsigned c
 template <typename OutT, bool kAccumulate, int U, int kBatch, bool kPair, bool kF32Eval>
 __global__ void __launch_bounds__(kThreads, kMinBlocks)
     sample_kernel(const __grid_constant__ DevProgram P, const TileDesc* __restrict__ tiles, int tile_begin, int tile_end,
-                  OutT* __restrict__ out, unsigned int* __restrict__ tile_counter) {
+                  OutT* __restrict__ out, unsigned int* __restrict__ tile_counter, const double* __restrict__ quant) {
   constexpr int V = OutVec<OutT>::N;
   const int lane = threadIdx.x & 31;
   // this warp's private slice
@@ -1377,7 +1422,7 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks)
       if (u < n_valid) row_buf[jj + u] = (OutT)r.v[u];
   };
   for_each_tile<kWarpsPerCta, kBatch, U, kF32Eval, OutT, kAccumulate, kPair>(
-      P, tiles, tile_begin, tile_end, out, tile_counter, s_slots, slice + ws.packets(),
+      P, tiles, tile_begin, tile_end, out, quant, tile_counter, s_slots, slice + ws.packets(),
       reinterpret_cast<uint64_t*>(slice + ws.barriers()), [&](const unsigned char* pk, uint32_t flags) {
         const PacketHeader* __restrict__ h = reinterpret_cast<const PacketHeader*>(pk);
         const int cnt = h->cnt;
@@ -1391,24 +1436,53 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks)
 
         // base fill: the whole tile BUFFER (tile_samples, a multiple of 128) <- the zero-segment
         // value; flat segments with another value and the active samples overwrite it below
-        fill_tile(reinterpret_cast<unsigned char*>(s_out) + lane * 16, P.tile_samples * (int)sizeof(OutT) / 512, base,
-                  sizeof(OutT) == 4);
+        const int tile_bytes = P.tile_samples * (int)sizeof(OutT);
+        auto base_fill = [&](OutT* buf, double val, int plane) {
+          unsigned char* p = reinterpret_cast<unsigned char*>(buf) + lane * 16;
+          if constexpr (kCodes<OutT>) {
+            const double* q = row_quant(quant, h->wave, plane);
+            const uint4 v = code_pattern(dac_code(val, q[0], q[1]));
+            fill_tile(p, tile_bytes / 512, v);
+            // an odd multiple of 128 samples ends in half a 512-byte row
+            if ((tile_bytes & 511) && lane < 16) *reinterpret_cast<uint4*>(p + (tile_bytes & ~511)) = v;
+          } else {
+            fill_tile(p, tile_bytes / 512, fill_pattern(val, sizeof(OutT) == 4));
+          }
+        };
+        base_fill(s_out, base, 0);
         if constexpr (kPair) {
-          if (flags & WFM_WAVE_PAIR)
-            fill_tile(reinterpret_cast<unsigned char*>(s_out + P.tile_samples) + lane * 16,
-                      P.tile_samples * (int)sizeof(OutT) / 512, h->base1, sizeof(OutT) == 4);
+          if (flags & WFM_WAVE_PAIR) base_fill(s_out + P.tile_samples, h->base1, 1);
         }
         __syncwarp();
 
         const ARow* __restrict__ arows = reinterpret_cast<const ARow*>(pk + sizeof(PacketHeader));
         const PatchRow* __restrict__ patches = reinterpret_cast<const PatchRow*>(arows + (n_arows ? n_arows + 1 : 0));
         // ---- flat segments with their own value ----------------------------------------------
-        for (int i = 0; i < n_patch; ++i)
-          fill_run(kPair && patches[i].plane ? s_out + P.tile_samples : s_out, (int)patches[i].a, (int)patches[i].b,
-                   patches[i].val, lane);
+        for (int i = 0; i < n_patch; ++i) {
+          if constexpr (kCodes<OutT>) {
+            const int plane = kPair && patches[i].plane;
+            fill_run(plane ? s_out + P.tile_samples : s_out, (int)patches[i].a, (int)patches[i].b, patches[i].val, lane,
+                     row_quant(quant, h->wave, plane));
+          } else {
+            fill_run(kPair && patches[i].plane ? s_out + P.tile_samples : s_out, (int)patches[i].a, (int)patches[i].b,
+                     patches[i].val, lane);
+          }
+        }
 
         // ---- the tile's ACTIVE samples ---------------------------------------------------------
-        eval_units<U, kPair, kF32Eval>(P, pk, base, flags, cnt, n_units, s_slots, sl, lane, to_tile);
+        if constexpr (kCodes<OutT>) {
+          // a unit's codes -> the tile buffer of its row
+          eval_units<U, kPair, kF32Eval>(P, pk, base, flags, cnt, n_units, s_slots, sl, lane,
+                                         [&](bool plane1, int jj, int n_valid, const Val<U>& r) {
+                                           const double* q = row_quant(quant, h->wave, plane1);
+                                           OutT* row_buf = plane1 ? s_out + P.tile_samples : s_out;
+#pragma unroll
+                                           for (int u = 0; u < U; ++u)
+                                             if (u < n_valid) row_buf[jj + u] = dac_code(r.v[u], q[0], q[1]);
+                                         });
+        } else {
+          eval_units<U, kPair, kF32Eval>(P, pk, base, flags, cnt, n_units, s_slots, sl, lane, to_tile);
+        }
 
         // ---- store ---------------------------------------------------------------------------
         if (kAccumulate) {
@@ -1425,7 +1499,7 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks)
           // the whole tile as one TMA bulk copy (an I/Q pair: one per row)
           fence_proxy_async_smem();
           __syncwarp();
-          const int n_bulk = cnt & ~(V - 1);  // 16-byte multiple; the ragged tail goes out as scalars
+          const int n_bulk = cnt & ~(V - 1);  // 16-byte multiple (8 codes, 4 floats, 2 doubles); the ragged tail goes out as scalars
           if (lane == 0 && n_bulk > 0) {
             const uint64_t policy = l2_evict_first_policy();
             bulk_s2g_evict_first(dst, s_out, (uint32_t)n_bulk * sizeof(OutT), policy);
@@ -1459,9 +1533,24 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks)
 // Packets, the pre-pass, the deal of the tiles and the evaluator are the sparse kernel's.
 constexpr int kDenseThreads = 32 * kDenseWarps;
 
-// U consecutive results -> global memory (16-byte stores when the address allows)
+// U consecutive results -> global memory (16-byte stores when the address allows; int16 output: the codes with the
+// row's (gain, offset) q, one 8-byte store)
 template <typename OutT, bool kAccumulate, int U>
-__device__ __forceinline__ void store_unit(OutT* __restrict__ p, const Val<U>& r, int n_valid) {
+__device__ __forceinline__ void store_unit(OutT* __restrict__ p, const Val<U>& r, int n_valid, const double* q = nullptr) {
+  if constexpr (kCodes<OutT>) {
+    static_assert(U == 4 && !kAccumulate, "int16 dense stores are one short4, never accumulated");
+    int16_t c[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) c[u] = dac_code(r.v[u], q[0], q[1]);
+    if (n_valid == U && ((uintptr_t)p & 7) == 0) {
+      *reinterpret_cast<short4*>(p) = make_short4(c[0], c[1], c[2], c[3]);
+    } else {
+#pragma unroll
+      for (int u = 0; u < U; ++u)
+        if (u < n_valid) p[u] = c[u];
+    }
+    return;
+  }
   if (kAccumulate) {
 #pragma unroll
     for (int u = 0; u < U; ++u)
@@ -1483,9 +1572,23 @@ __device__ __forceinline__ void store_unit(OutT* __restrict__ p, const Val<U>& r
   }
 }
 
-// [a, b) of a channel row <- val, by the whole warp
+// [a, b) of a channel row <- val, by the whole warp (int16 output: its code with the row's (gain, offset) q)
 template <typename OutT, bool kAccumulate>
-__device__ __forceinline__ void fill_global(OutT* __restrict__ row, int a, int b, double val, int lane) {
+__device__ __forceinline__ void fill_global(OutT* __restrict__ row, int a, int b, double val, int lane,
+                                            const double* q = nullptr) {
+  if constexpr (kCodes<OutT>) {
+    static_assert(!kAccumulate, "codes are never accumulated");
+    const int16_t c = dac_code(val, q[0], q[1]);
+    const int mis = (int)(((uintptr_t)(row + a) & 15) / sizeof(OutT));
+    const int head = min(b - a, mis ? 8 - mis : 0);
+    if (lane < head) row[a + lane] = c;
+    const int a2 = a + head, nvec = (b - a2) / 8;
+    const uint4 v = code_pattern(c);
+    for (int k = lane; k < nvec; k += 32) *reinterpret_cast<uint4*>(row + a2 + k * 8) = v;
+    const int t0 = a2 + nvec * 8;
+    if (t0 + lane < b) row[t0 + lane] = c;
+    return;
+  }
   if (kAccumulate) {
     if (val != 0.0)
       for (int p = a + lane; p < b; p += 32) row[p] = (OutT)add((double)row[p], val);
@@ -1511,7 +1614,7 @@ __device__ __forceinline__ void fill_global(OutT* __restrict__ row, int a, int b
 template <typename OutT, bool kAccumulate, int kBatch, bool kPair, bool kF32Eval>
 __global__ void __launch_bounds__(kDenseThreads, 1)
     sample_dense_kernel(const __grid_constant__ DevProgram P, const TileDesc* __restrict__ tiles, int tile_begin, int tile_end,
-                        OutT* __restrict__ out, unsigned int* __restrict__ tile_counter) {
+                        OutT* __restrict__ out, unsigned int* __restrict__ tile_counter, const double* __restrict__ quant) {
   constexpr int U = kDenseUnit;
   const int lane = threadIdx.x & 31;
   const WarpSlice ws = warp_slice(0, 0, 0, P.n_slots, U, P.pkt_cap);
@@ -1519,7 +1622,7 @@ __global__ void __launch_bounds__(kDenseThreads, 1)
   unsigned char* s_slots = slice + ws.slots();
   unsigned char* sl = lane_slots<U>(s_slots, lane);
   for_each_tile<kDenseWarps, kBatch, U, kF32Eval, OutT, kAccumulate, kPair>(
-      P, tiles, tile_begin, tile_end, out, tile_counter, s_slots, slice + ws.packets(),
+      P, tiles, tile_begin, tile_end, out, quant, tile_counter, s_slots, slice + ws.packets(),
       reinterpret_cast<uint64_t*>(slice + ws.barriers()), [&](const unsigned char* pk, uint32_t flags) {
         const PacketHeader* __restrict__ h = reinterpret_cast<const PacketHeader*>(pk);
         const int n_arows = h->n_arows, n_patch = h->n_patch, n_units = h->n_units;
@@ -1529,13 +1632,24 @@ __global__ void __launch_bounds__(kDenseThreads, 1)
         const ARow* __restrict__ arows = reinterpret_cast<const ARow*>(pk + sizeof(PacketHeader));
         const PatchRow* __restrict__ patches = reinterpret_cast<const PatchRow*>(arows + (n_arows ? n_arows + 1 : 0));
         // ---- flat runs: every zero / constant segment of the tile is listed (dense programs) --------------------------
-        for (int i = 0; i < n_patch; ++i)
-          fill_global<OutT, kAccumulate>((kPair && patches[i].plane) ? dst1 : dst0, (int)patches[i].a, (int)patches[i].b,
-                                         patches[i].val, lane);
+        for (int i = 0; i < n_patch; ++i) {
+          if constexpr (kCodes<OutT>) {
+            const int plane = kPair && patches[i].plane;
+            fill_global<OutT, false>(plane ? dst1 : dst0, (int)patches[i].a, (int)patches[i].b, patches[i].val, lane,
+                                     row_quant(quant, h->wave, plane));
+          } else {
+            fill_global<OutT, kAccumulate>((kPair && patches[i].plane) ? dst1 : dst0, (int)patches[i].a, (int)patches[i].b,
+                                           patches[i].val, lane);
+          }
+        }
         // ---- active samples: units of four, results straight to global memory ----------------------------------------
         eval_units<U, kPair, kF32Eval>(P, pk, h->base, flags, h->cnt, n_units, s_slots, sl, lane,
                                        [&](bool plane1, int jj, int n_valid, const Val<U>& r) {
-                                         store_unit<OutT, kAccumulate, U>((plane1 ? dst1 : dst0) + jj, r, n_valid);
+                                         if constexpr (kCodes<OutT>)
+                                           store_unit<OutT, false, U>((plane1 ? dst1 : dst0) + jj, r, n_valid,
+                                                                      row_quant(quant, h->wave, plane1));
+                                         else
+                                           store_unit<OutT, kAccumulate, U>((plane1 ? dst1 : dst0) + jj, r, n_valid);
                                        });
       });
 }
@@ -1635,7 +1749,8 @@ cudaError_t launch_fill_packets(const DevProgram& P, const TileDesc* tiles, int6
 }
 
 size_t sample_smem_bytes(const DevProgram& P, int dtype) {
-  return (size_t)(P.dense ? kDenseWarps : kWarpsPerCta) * program_slice(P, P.tile_samples, dtype == WFM_F32 ? 4 : 8, P.pkt_cap).bytes();
+  const int elem = dtype == WFM_F32 ? 4 : (dtype == WFM_I16 ? 2 : 8);
+  return (size_t)(P.dense ? kDenseWarps : kWarpsPerCta) * program_slice(P, P.tile_samples, elem, P.pkt_cap).bytes();
 }
 
 // tile counters of the dynamic deal: one ring per device, never freed
@@ -1704,7 +1819,7 @@ static cudaError_t launch_cfg(K k, LaunchCfg* table, std::mutex& mu, size_t smem
 // tiles), at most one warp per tile.  The shared-memory attribute and occupancy table is per kernel instantiation.
 template <auto kKernel, int kThreadsPerCta, int kBatch, typename OutT>
 static cudaError_t launch_kernel(const DevProgram& P, const TileDesc* tiles, int64_t tile_begin, int64_t n_tiles, int dtype,
-                                 void* out, cudaStream_t stream) {
+                                 void* out, const double* quant, cudaStream_t stream) {
   static LaunchCfg cfg_table[64];
   static std::mutex cfg_mu;
   const int warps = kThreadsPerCta / 32;
@@ -1715,7 +1830,8 @@ static cudaError_t launch_kernel(const DevProgram& P, const TileDesc* tiles, int
   if (per_sm < 1) return cudaErrorInvalidConfiguration;
   const unsigned grid = (unsigned)std::min<int64_t>((n_tiles + warps - 1) / warps, (int64_t)sms * per_sm);
   if (kBatch == 0) {
-    kKernel<<<grid, kThreadsPerCta, smem, stream>>>(P, tiles, (int)tile_begin, (int)(tile_begin + n_tiles), (OutT*)out, nullptr);
+    kKernel<<<grid, kThreadsPerCta, smem, stream>>>(P, tiles, (int)tile_begin, (int)(tile_begin + n_tiles), (OutT*)out, nullptr,
+                                                    quant);
     return cudaGetLastError();
   }
   // the tile counter of this launch: the next slot of a per-device ring (allocated once), zeroed on the launch's
@@ -1734,7 +1850,8 @@ static cudaError_t launch_kernel(const DevProgram& P, const TileDesc* tiles, int
   }
   unsigned int* counter = ring->counters + slot;
   if ((e = cudaMemsetAsync(counter, 0, sizeof(unsigned int), stream)) != cudaSuccess) return e;
-  kKernel<<<grid, kThreadsPerCta, smem, stream>>>(P, tiles, (int)tile_begin, (int)(tile_begin + n_tiles), (OutT*)out, counter);
+  kKernel<<<grid, kThreadsPerCta, smem, stream>>>(P, tiles, (int)tile_begin, (int)(tile_begin + n_tiles), (OutT*)out, counter,
+                                                  quant);
   if ((e = cudaGetLastError()) != cudaSuccess) return e;
   return cudaEventRecord(ring->used[slot], stream);
 }
@@ -1759,10 +1876,38 @@ static cudaError_t with_bool(bool b, F&& f) {
   return b ? f(std::true_type{}) : f(std::false_type{});
 }
 
+// the kernel for one output type: dense or sparse (unit 1 / 2), I/Q pairs or not, static or dynamic deal
+template <typename OutT, bool kAcc, bool kFast>
+static cudaError_t launch_typed(const DevProgram& P, const TileDesc* tiles, int64_t tile_begin, int64_t n_tiles, int dtype,
+                                bool dynamic, void* out, const double* quant, cudaStream_t stream) {
+  return with_bool(P.planes == 2, [&](auto pair) {
+    return with_bool(dynamic, [&](auto dyn) {
+      constexpr bool kPair = decltype(pair)::value;
+      if (P.dense) {
+        constexpr int kBatch = decltype(dyn)::value ? kDenseDealBatch : 0;
+        return launch_kernel<sample_dense_kernel<OutT, kAcc, kBatch, kPair, kFast>, kDenseThreads, kBatch, OutT>(
+            P, tiles, tile_begin, n_tiles, dtype, out, quant, stream);
+      }
+      constexpr int kBatch = decltype(dyn)::value ? kDealBatch : 0;
+      return with_bool(P.unit == 2, [&](auto u2) {
+        constexpr int U = decltype(u2)::value ? 2 : 1;
+        return launch_kernel<sample_kernel<OutT, kAcc, U, kBatch, kPair, kFast>, kThreads, kBatch, OutT>(
+            P, tiles, tile_begin, n_tiles, dtype, out, quant, stream);
+      });
+    });
+  });
+}
+
 cudaError_t launch_sample(const DevProgram& P, const TileDesc* tiles, int64_t tile_begin, int64_t n_tiles, int dtype,
-                          int accumulate, void* out, cudaStream_t stream) {
+                          int accumulate, void* out, cudaStream_t stream, const double* quant) {
   if (n_tiles == 0) return cudaSuccess;
   if (tile_begin + n_tiles > INT32_MAX) return cudaErrorInvalidValue;
+  // WFM_I16: codes from the fp64 evaluator, never accumulated
+  if (dtype == WFM_I16) {
+    if (accumulate || !quant) return cudaErrorInvalidValue;
+    return launch_typed<int16_t, false, false>(P, tiles, tile_begin, n_tiles, dtype, dynamic_deal(P, n_tiles, dtype), out,
+                                               quant, stream);
+  }
   // WFM_F32_FAST: float output by the fp32 evaluator (not with accumulate: that is the careful path anyway)
   const bool fast32 = dtype == WFM_F32_FAST && !accumulate;
   if (dtype == WFM_F32_FAST) dtype = WFM_F32;
@@ -1771,31 +1916,60 @@ cudaError_t launch_sample(const DevProgram& P, const TileDesc* tiles, int64_t ti
   return with_bool(fast32, [&](auto fast) {
     return with_bool(dtype == WFM_F64 && !fast32, [&](auto f64) {
       return with_bool(accumulate && !fast32, [&](auto acc) {
-        return with_bool(P.planes == 2, [&](auto pair) {
-          return with_bool(dynamic, [&](auto dyn) {
-            constexpr bool kFast = decltype(fast)::value, kAcc = decltype(acc)::value;
-            using OutT = std::conditional_t<decltype(f64)::value, double, float>;
-            if constexpr (kFast && (sizeof(OutT) == 8 || kAcc)) {
-              return cudaErrorInvalidValue;  // not reached: the fp32 evaluator writes float and never accumulates
-            } else {
-              constexpr bool kPair = decltype(pair)::value;
-              if (P.dense) {
-                constexpr int kBatch = decltype(dyn)::value ? kDenseDealBatch : 0;
-                return launch_kernel<sample_dense_kernel<OutT, kAcc, kBatch, kPair, kFast>, kDenseThreads, kBatch, OutT>(
-                    P, tiles, tile_begin, n_tiles, dtype, out, stream);
-              }
-              constexpr int kBatch = decltype(dyn)::value ? kDealBatch : 0;
-              return with_bool(P.unit == 2, [&](auto u2) {
-                constexpr int U = decltype(u2)::value ? 2 : 1;
-                return launch_kernel<sample_kernel<OutT, kAcc, U, kBatch, kPair, kFast>, kThreads, kBatch, OutT>(
-                    P, tiles, tile_begin, n_tiles, dtype, out, stream);
-              });
-            }
-          });
-        });
+        constexpr bool kFast = decltype(fast)::value, kAcc = decltype(acc)::value;
+        using OutT = std::conditional_t<decltype(f64)::value, double, float>;
+        if constexpr (kFast && (sizeof(OutT) == 8 || kAcc)) {
+          return cudaErrorInvalidValue;  // not reached: the fp32 evaluator writes float and never accumulates
+        } else {
+          return launch_typed<OutT, kAcc, kFast>(P, tiles, tile_begin, n_tiles, dtype, dynamic, out, nullptr, stream);
+        }
       });
     });
   });
+}
+
+// ---- wfm_quantize: f64 rows -> 16-bit DAC codes -----------------------------------------------------------------
+// One thread per 8 consecutive samples of a row: four 16-byte loads and one 16-byte store when both rows allow it
+// (kVec), scalar accesses otherwise.  Grid: x over the row, y over the rows.
+constexpr int kQuantThreads = 256;
+template <bool kVec>
+__global__ void __launch_bounds__(kQuantThreads) quantize_kernel(const double* __restrict__ x, int16_t* __restrict__ y,
+                                                                  int64_t n_sig, int64_t n, int64_t x_stride, int64_t y_stride,
+                                                                  const double* __restrict__ gain_offset) {
+  const int64_t j = ((int64_t)blockIdx.x * kQuantThreads + threadIdx.x) * 8;
+  if (j >= n) return;
+  for (int64_t s = blockIdx.y; s < n_sig; s += gridDim.y) {
+    const double g = gain_offset[2 * s], o = gain_offset[2 * s + 1];
+    const double* __restrict__ xr = x + s * x_stride + j;
+    int16_t* __restrict__ yr = y + s * y_stride + j;
+    if (kVec && j + 8 <= n) {
+      int16_t c[8];
+#pragma unroll
+      for (int k = 0; k < 8; k += 2) {
+        const double2 v = __ldcs(reinterpret_cast<const double2*>(xr + k));
+        c[k] = dac_code(v.x, g, o);
+        c[k + 1] = dac_code(v.y, g, o);
+      }
+      uint4 w;
+      w.x = (uint32_t)(uint16_t)c[0] | ((uint32_t)(uint16_t)c[1] << 16);
+      w.y = (uint32_t)(uint16_t)c[2] | ((uint32_t)(uint16_t)c[3] << 16);
+      w.z = (uint32_t)(uint16_t)c[4] | ((uint32_t)(uint16_t)c[5] << 16);
+      w.w = (uint32_t)(uint16_t)c[6] | ((uint32_t)(uint16_t)c[7] << 16);
+      *reinterpret_cast<uint4*>(yr) = w;
+    } else {
+      for (int k = 0; k < 8 && j + k < n; ++k) yr[k] = dac_code(xr[k], g, o);
+    }
+  }
+}
+
+cudaError_t launch_quantize(const double* x, int16_t* y, int64_t n_sig, int64_t n, int64_t x_stride, int64_t y_stride,
+                            const double* gain_offset, cudaStream_t stream) {
+  if (n_sig <= 0 || n <= 0) return cudaSuccess;
+  const bool vec = ((uintptr_t)x % 16) == 0 && ((uintptr_t)y % 16) == 0 && (x_stride % 2) == 0 && (y_stride % 8) == 0;
+  const dim3 grid((unsigned)((n + 8 * kQuantThreads - 1) / (8 * kQuantThreads)), (unsigned)std::min<int64_t>(n_sig, 65535));
+  if (vec) quantize_kernel<true><<<grid, kQuantThreads, 0, stream>>>(x, y, n_sig, n, x_stride, y_stride, gain_offset);
+  else quantize_kernel<false><<<grid, kQuantThreads, 0, stream>>>(x, y, n_sig, n, x_stride, y_stride, gain_offset);
+  return cudaGetLastError();
 }
 
 }  // namespace wfm

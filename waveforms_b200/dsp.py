@@ -134,6 +134,58 @@ def apply_channel_filters(out, batch, waveforms, mode=None):
                 sosfilt_device(sos, out[off:off + n], initial=initial, mode=mode)
 
 
+def quantize_device(x, gain, offset=0.0, out=None):
+    """16-bit DAC codes of a CUDA float64 tensor ``x`` of shape (n,) or (n_sig, n) (row stride
+    ``x.stride(0)``): ``clamp(rint(x * gain + offset), -32768, 32767)`` (multiply, then add; half
+    to even; NaN -> 0, +-inf saturate) — the conversion of ``sample_batch(dtype=np.int16)``
+    (``wfm_quantize``), e.g. for the outputs of ``predistort`` / ``correct_reflection``.  ``gain``,
+    ``offset``: scalars or one value per row.  Returns an int16 tensor of x's shape, or ``out``
+    (int16, same shape, unit stride along a row)."""
+    import torch
+    lib = engine.require_gpu()
+    x2 = x if x.dim() == 2 else x.unsqueeze(0)
+    if x2.dtype != torch.float64 or not x2.is_cuda or x2.stride(1) != 1:
+        raise TypeError('quantize_device: x must be a CUDA float64 tensor with unit stride along a row')
+    n_sig, n = x2.shape
+    go = np.stack([np.broadcast_to(np.asarray(gain, dtype=np.float64), (n_sig,)),
+                   np.broadcast_to(np.asarray(offset, dtype=np.float64), (n_sig,))], 1)
+    table = torch.from_numpy(np.ascontiguousarray(go)).to(x.device)
+    if out is None:
+        y = torch.empty((n_sig, n), dtype=torch.int16, device=x.device)
+    else:
+        y = out if out.dim() == 2 else out.unsqueeze(0)
+        if y.dtype != torch.int16 or y.shape != x2.shape or y.stride(1) != 1 or y.device != x.device:
+            raise TypeError('quantize_device: out must be an int16 tensor of x\'s shape on its device')
+    rc = lib.wfm_quantize(x2.data_ptr(), y.data_ptr(), n_sig, n, x2.stride(0), y.stride(0), table.data_ptr(),
+                          _stream(torch, x.device))
+    engine._check(rc)
+    if out is not None:
+        return out
+    return y if x.dim() == 2 else y[0]
+
+
+def quantize_batch(x, batch, gain, offset):
+    """The DAC codes of a flat float64 batch buffer ``x`` (channel k at ``batch.chan_off[k]``, ``batch.chan_n[k]``
+    samples) with per-channel ``gain`` / ``offset``, in a flat int16 buffer of the same layout (the padding between
+    rows is not written).  Consecutive channels of one length at one pitch go through one call."""
+    import torch
+    y = torch.empty(x.shape, dtype=torch.int16, device=x.device)
+    offs, ns = [int(v) for v in batch.chan_off], [int(v) for v in batch.chan_n]
+    k = 0
+    while k < len(offs):
+        e, pitch = k + 1, max(ns[k], 1)
+        if e < len(offs) and ns[e] == ns[k] and offs[e] - offs[k] >= ns[k]:
+            pitch = offs[e] - offs[k]
+            while e < len(offs) and ns[e] == ns[k] and offs[e] - offs[e - 1] == pitch:
+                e += 1
+        if ns[k] > 0:
+            shape, stride = (e - k, ns[k]), (pitch, 1)
+            quantize_device(x.as_strided(shape, stride, offs[k]), gain[k:e], offset[k:e],
+                            out=y.as_strided(shape, stride, offs[k]))
+        k = e
+    return y
+
+
 LFILTER_SCAN_MAX_ORDER = 4
 
 

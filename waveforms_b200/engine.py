@@ -15,8 +15,8 @@ from pathlib import Path
 import numpy as np
 
 from . import _algebra as A
-from .lowering import (FACTOR_DT, REF_DT, SEGPTR_DT, TERM_DT, WAVE_DT, Channel,
-                       Grid, LoweredBatch, lower)
+from .lowering import (FACTOR_DT, REF_DT, SEGPTR_DT, TERM_DT, WAVE_DT, WAVE_PAIR,
+                       Channel, Grid, LoweredBatch, lower)
 
 import os
 
@@ -24,8 +24,9 @@ import os
 _LIB_PATH = Path(os.environ.get('WFM_LIB') or
                  Path(__file__).resolve().parent / 'csrc' / 'libwfmb200.so')
 
-WFM_F64, WFM_F32, WFM_C128, WFM_F32_FAST = 0, 1, 2, 3
-_NP_DTYPE = {WFM_F64: np.float64, WFM_F32: np.float32, WFM_C128: np.complex128, WFM_F32_FAST: np.float32}
+WFM_F64, WFM_F32, WFM_C128, WFM_F32_FAST, WFM_I16 = 0, 1, 2, 3, 4
+_NP_DTYPE = {WFM_F64: np.float64, WFM_F32: np.float32, WFM_C128: np.complex128, WFM_F32_FAST: np.float32,
+             WFM_I16: np.int16}
 
 
 class EngineUnavailable(RuntimeError):
@@ -65,13 +66,18 @@ class _Launch(C.Structure):
                 ('out', C.c_void_p), ('out_elems', C.c_int64)]
 
 
+class _Quant(C.Structure):
+    _fields_ = [('row_gain_offset', C.c_void_p)]
+
+
 _lib = None
 _lib_lock = threading.Lock()
 
 EXPORTS = [
     'wfm_abi_version', 'wfm_last_error', 'wfm_device_count', 'wfm_trim',
     'wfm_program_create', 'wfm_program_destroy', 'wfm_program_total_samples',
-    'wfm_program_launch_count', 'wfm_program_info', 'wfm_sample', 'wfm_sample_host', 'wfm_sosfilt',
+    'wfm_program_launch_count', 'wfm_program_info', 'wfm_sample', 'wfm_sample_host', 'wfm_sample_quant',
+    'wfm_sample_quant_host', 'wfm_quantize', 'wfm_sosfilt',
     'wfm_lfilter', 'wfm_lfilter_mode', 'wfm_expand_templates', 'wfm_fft_filter', 'wfm_fft_response_create', 'wfm_fft_response_destroy',
     'wfm_fft_filter_prepared', 'wfm_reflection_filter', 'wfm_fft_c2c', 'wfm_calibrate_fp64', 'wfm_calibrate_copy'
 ]
@@ -103,6 +109,10 @@ def load_library():
         lib.wfm_program_info.argtypes = [C.c_void_p, C.POINTER(C.c_int64), C.c_int32]
         lib.wfm_sample.argtypes = [C.c_void_p, C.POINTER(_Launch), C.c_void_p]
         lib.wfm_sample_host.argtypes = [C.c_void_p, C.POINTER(_Launch)]
+        lib.wfm_sample_quant.argtypes = [C.c_void_p, C.POINTER(_Launch), C.POINTER(_Quant), C.c_void_p]
+        lib.wfm_sample_quant_host.argtypes = [C.c_void_p, C.POINTER(_Launch), C.POINTER(_Quant)]
+        lib.wfm_quantize.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
+                                     C.c_void_p]
         lib.wfm_sosfilt.argtypes = [
             C.c_void_p, C.c_int32, C.c_double, C.c_void_p, C.c_void_p,
             C.c_int64, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p,
@@ -323,14 +333,16 @@ class Program:
         return WFM_C128 if self.batch.any_complex else WFM_F64
 
     def sample_device(self, dtype=None, out=None, accumulate=False,
-                      first_wave=0, n_wave=0, stream=None):
+                      first_wave=0, n_wave=0, stream=None, quant=None):
         """Launch K1; returns a torch tensor on ``self.device`` holding the
-        whole batch back to back (channel w at ``waves['out_off'][w]``)."""
+        whole batch back to back (channel w at ``waves['out_off'][w]``).
+        ``dtype=WFM_I16``: 16-bit DAC codes, ``quant`` = the (n_waves, 2, 2) float64
+        (gain, offset) table of every output row on this device (``quant_table``)."""
         torch = _torch()
         if dtype is None:
             dtype = self.default_dtype()
         tdt = {WFM_F64: torch.float64, WFM_F32: torch.float32, WFM_F32_FAST: torch.float32,
-               WFM_C128: torch.complex128}[dtype]
+               WFM_C128: torch.complex128, WFM_I16: torch.int16}[dtype]
         if out is None:
             alloc = torch.zeros if accumulate else torch.empty
             out = alloc(self.total_samples, dtype=tdt,
@@ -340,20 +352,51 @@ class Program:
             stream = torch.cuda.current_stream(self.device).cuda_stream
         l = _Launch(first_wave, n_wave, dtype, int(bool(accumulate)),
                     out.data_ptr(), out.numel())
-        _check(self._lib.wfm_sample(self._h, C.byref(l), C.c_void_p(stream)))
+        if quant is None:
+            _check(self._lib.wfm_sample(self._h, C.byref(l), C.c_void_p(stream)))
+        else:
+            q = self._quant(quant)
+            _check(self._lib.wfm_sample_quant(self._h, C.byref(l), C.byref(q), C.c_void_p(stream)))
         return out
 
-    def sample_host(self, dtype=None, out=None, first_wave=0, n_wave=0):
+    def sample_host(self, dtype=None, out=None, first_wave=0, n_wave=0, quant=None):
         """End-to-end: kernel + device->host copy into a NumPy buffer through
-        ``wfm_sample_host``."""
+        ``wfm_sample_host`` (``wfm_sample_quant_host`` with ``quant``, see ``sample_device``)."""
         if dtype is None:
             dtype = self.default_dtype()
         if out is None:
             out = np.empty(self.total_samples, dtype=_NP_DTYPE[dtype])
         assert out.dtype == _NP_DTYPE[dtype] and out.flags.c_contiguous
         l = _Launch(first_wave, n_wave, dtype, 0, out.ctypes.data, out.size)
-        _check(self._lib.wfm_sample_host(self._h, C.byref(l)))
+        if quant is None:
+            _check(self._lib.wfm_sample_host(self._h, C.byref(l)))
+        else:
+            q = self._quant(quant)
+            _check(self._lib.wfm_sample_quant_host(self._h, C.byref(l), C.byref(q)))
         return out
+
+    def _quant(self, table):
+        torch = _torch()
+        if not (isinstance(table, torch.Tensor) and table.dtype == torch.float64 and table.is_contiguous()
+                and table.device == torch.device('cuda', self.device) and table.shape == (len(self.batch.waves), 2, 2)):
+            raise ValueError('quant: a contiguous float64 CUDA tensor of shape (n_waves, 2, 2) on the program\'s device')
+        return _Quant(table.data_ptr())
+
+
+def quant_table(batch, gain, offset=0.0):
+    """The (n_waves, 2, 2) float64 (gain, offset) table of ``wfm_sample_quant`` from per-CHANNEL values in the
+    batch's channel order (``batch.chan_off``: an I/Q pair is two channels, its rows 0 and 1).  ``gain`` /
+    ``offset``: scalars or arrays of ``batch.n_channels`` values.  Rows no channel owns stay 0."""
+    n = batch.n_channels
+    g = np.broadcast_to(np.asarray(gain, dtype=np.float64), (n,))
+    o = np.broadcast_to(np.asarray(offset, dtype=np.float64), (n,))
+    pair = (np.asarray(batch.waves['flags']) & WAVE_PAIR) != 0
+    keep = np.stack([np.ones(len(pair), bool), pair], 1)
+    if int(keep.sum()) != n:
+        raise ValueError('batch channels do not match its rows')
+    table = np.zeros((len(pair), 2, 2), dtype=np.float64)
+    table[keep] = np.stack([g, o], 1)
+    return table
 
 
 # -- single-channel helpers used by Waveform.__call__/sample -------------------

@@ -540,11 +540,18 @@ def find_pairs(items, min_shared=0.5):
     return out
 
 
-def lower(items) -> LoweredBatch:
+def row_pitch(n, align=4):
+    """Samples an output row of ``n`` samples occupies: ``n`` rounded up to a multiple of ``align`` (a power of two).
+    Rows start at multiples of ``align``: 4 keeps the 16-byte stores of fp32 and fp64 output aligned, 16-bit DAC
+    codes (``WFM_I16``) need 8."""
+    return (n + align - 1) & ~(align - 1)
+
+
+def lower(items, align=4) -> LoweredBatch:
     """items: iterable of (Channel, Grid), or ((Channel, Channel), Grid) for two
     channels evaluated as one I/Q pair (``find_pairs``).  Output offsets are
-    assigned back-to-back, each channel's start padded to a multiple of 4 samples
-    so 16-byte vector stores stay aligned for fp32 and fp64 output."""
+    assigned back-to-back, each channel's start padded to a multiple of ``align``
+    samples (``row_pitch``)."""
     pools = _Pools()
     items = list(items)
     waves = np.zeros(len(items), dtype=WAVE_DT)
@@ -588,7 +595,7 @@ def lower(items) -> LoweredBatch:
         w['n_seg'] = n_seg
         chan_off.append(out_off)
         chan_n.append(grid.n)
-        out_off += (grid.n + 3) & ~3
+        out_off += row_pitch(grid.n, align)
         if partner is not None:
             if cplx or _clipped(chan) or _clipped(partner):
                 raise ValueError('an I/Q pair must be real-valued and unclipped (see can_pair)')
@@ -598,7 +605,7 @@ def lower(items) -> LoweredBatch:
             w['out_off2'] = out_off
             chan_off.append(out_off)
             chan_n.append(grid.n)
-            out_off += (grid.n + 3) & ~3
+            out_off += row_pitch(grid.n, align)
         w['flags'] = flags
     n_segs = len(pools.bound)
     seg_ptr = np.zeros(n_segs + 1, dtype=SEGPTR_DT)
@@ -624,10 +631,10 @@ def lower(items) -> LoweredBatch:
         chan_n=np.asarray(chan_n, dtype=np.int64))
 
 
-def merge_batches(parts, owners) -> LoweredBatch:
+def merge_batches(parts, owners, align=4) -> LoweredBatch:
     """Several lowered batches as ONE, their waves interleaved back into an original order: ``owners[k][i]`` is
     the position (0 .. n-1, every position exactly once) of wave ``i`` of ``parts[k]``.  Tables are concatenated
-    with rebased indices; output rows are re-assigned back to back in the merged order."""
+    with rebased indices; output rows are re-assigned back to back in the merged order (``row_pitch(n, align)``)."""
     n = sum(len(o) for o in owners)
     waves = np.zeros(n, dtype=WAVE_DT)
     seg_base = fac_base = term_base = ref_base = arg_base = x_base = 0
@@ -666,7 +673,7 @@ def merge_batches(parts, owners) -> LoweredBatch:
     seg_ptr['fac'][seg_base], seg_ptr['term'][seg_base] = fac_base, term_base
     out_off = 0
     for i in range(n):
-        pitch = (int(waves['n'][i]) + 3) & ~3
+        pitch = row_pitch(int(waves['n'][i]), align)
         waves['out_off'][i] = out_off
         out_off += pitch
         if waves['flags'][i] & WAVE_PAIR:
