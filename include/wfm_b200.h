@@ -226,10 +226,15 @@ typedef struct WfmLaunch {
   int64_t first_wave;  /* channels [first_wave, first_wave + n_wave) */
   int64_t n_wave;      /* 0 = all from first_wave                    */
   int32_t dtype;       /* WFM_F64 | WFM_F32 | WFM_F32_FAST | WFM_C128 | WFM_I16 */
-  int32_t accumulate;  /* 0: out = value; 1: out += value            */
+  int32_t accumulate;  /* 0: out = value; 1: out += value (see below) */
   void*   out;         /* DEVICE pointer (wfm_sample) / HOST pointer (wfm_sample_host) */
   int64_t out_elems;   /* capacity of out, in elements of dtype      */
 } WfmLaunch;
+/* accumulate = 1 writes out = (OutT)((double)out + v) with ONE rounding, where v is, bit for bit, the value the WFM_F64
+ * launch of the same program writes; WFM_F32_FAST then evaluates in fp64 like WFM_F32.  WFM_C128 adds the real and
+ * the imaginary part separately.  Flat runs of value 0.0 in programs laid out for the dense kernel may be skipped
+ * (out + 0.0 == out), so an out of -0.0 can stay -0.0 there.  Only the samples of the launched channels are read and
+ * written.  Host buffers (wfm_sample_host) refuse accumulate (WFM_EUNSUPPORTED); WFM_I16 codes are never accumulated. */
 
 int  wfm_abi_version(void);
 const char* wfm_last_error(void);

@@ -98,3 +98,88 @@ def rel_err(got, want):
     assert got.shape == want.shape, (got.shape, want.shape)
     scale = max(float(np.max(np.abs(want))) if want.size else 0.0, 1e-300)
     return float(np.max(np.abs(got - want))) / scale if want.size else 0.0
+
+
+def oracle_sample(w):
+    """Oracle evaluation of a waveforms_b200 object on its own sample() grid."""
+    from oracle import wfm_oracle as O
+    x = O.sample_grid(w.start, w.stop, w.sample_rate)
+    if hasattr(w, 'wlist'):
+        return O.stack_call(list(w.wlist), x, getattr(w, 'offset', 0), getattr(w, 'shift', 0))
+    return O.waveform_call(w.bounds, w.seq, x, w.min, w.max)
+
+
+# ---- channels that steer the sampling kernels onto particular paths ---------------------------------------------------
+def cold_tiles_waveform(ns):
+    """Hundreds of tiny active segments inside one tile: the tile's packet does not fit a warp's buffer (kPacketCold)
+    and the tile is evaluated from the global tables."""
+    rng = np.random.default_rng(3)
+    w = ns.zero()
+    for k in range(300):
+        w = w + rng.uniform(0.1, 1) * (ns.gaussian(1.5e-9) >> (2e-9 + 3e-9 * k))
+    w.start, w.stop, w.sample_rate = 0.0, 1e-6, 4e9
+    return w
+
+
+def wide_segments_stack(ns):
+    """A stack whose members overlap with 9 different carrier frequencies: the merged segments need more than 12 value
+    slots (kSegWide) and are evaluated from the ABI tables."""
+    pulses = []
+    for k in range(9):
+        I, _ = ns.mixing(0.1 * (k + 1) * ns.cosPulse(200e-9) >> (150e-9 + 5e-9 * k), freq=(20 + 7 * k) * 1e6, phase=0.1 * k,
+                         DRAGScaling=3e-10)
+        pulses.append(I)
+    w = ns.WaveVStack(pulses)
+    w.start, w.stop, w.sample_rate = 0.0, 400e-9, 4e9
+    return w
+
+
+def iq_pair_waveforms(ns):
+    """Six I/Q pairs of DRAG pulses (I, Q, I, Q, ...); every Q row has its own constant 0.25, so the two rows of a
+    pair have different zero-segment values."""
+    rng = np.random.default_rng(31)
+    ws = []
+    for k in range(6):
+        I, Q = ns.mixing(rng.uniform(0.2, 1) * ns.cosPulse(30e-9) >> (40e-9 + 37e-9 * k), freq=rng.uniform(-200e6, 200e6),
+                         phase=rng.uniform(0, 6), DRAGScaling=rng.uniform(2e-10, 1e-9))
+        Q = Q + 0.25
+        for w in (I, Q):
+            w.start, w.stop, w.sample_rate = 0, 0.45e-6, 2e9
+        ws += [I, Q]
+    return ws
+
+
+def small_batch_waveforms(ns, n=6):
+    """n short mixed channels of ragged lengths."""
+    rng = np.random.default_rng(21)
+    ws = []
+    for k in range(n):
+        I, Q = ns.mixing(rng.uniform(0.2, 1) * ns.cosPulse(30e-9) >> (60e-9 + 41e-9 * k), freq=rng.uniform(-150e6, 150e6),
+                         phase=rng.uniform(0, 6), DRAGScaling=3e-10)
+        w = I if k % 2 else Q
+        w.start, w.stop, w.sample_rate = 0.0, 0.5e-6 + 7e-9 * k, 2e9
+        ws.append(w)
+    return ws
+
+
+def ragged_waveforms(ns):
+    """Channels of 1, 0, 7, 9, 127, 129, 1000 and 2001 samples."""
+    ws = []
+    for n in (1, 0, 7, 9, 127, 129, 1000, 2001):
+        w = 0.7 * ns.gaussian(3e-9) >> (n / 2 * 0.25e-9)
+        w.start, w.stop, w.sample_rate = 0.0, n * 0.25e-9, 4e9
+        ws.append(w)
+    return ws
+
+
+def uneven_waveforms(ns):
+    """37 channels of 40 k - 140 k samples with 0 - 5 pulses each: thousands of tiles of uneven work."""
+    rng = np.random.default_rng(99)
+    ws = []
+    for k in range(37):
+        w = ns.zero()
+        for j in range(int(rng.integers(0, 6))):
+            w = w + rng.uniform(-1, 1) * (ns.gaussian(40e-9) >> float(rng.uniform(1e-6, 60e-6)))
+        w.start, w.stop, w.sample_rate = 0.0, float(rng.uniform(20e-6, 70e-6)), 2e9
+        ws.append(w)
+    return ws

@@ -8,7 +8,7 @@ import ctypes
 import numpy as np
 import pytest
 
-from helpers import b200_object, load_golden
+from helpers import b200_object, cold_tiles_waveform, load_golden, ragged_waveforms, wide_segments_stack
 
 
 def q(v, g=1.0, o=0.0):
@@ -234,11 +234,7 @@ def test_saturation_clip_and_flat_segments(ns):
 @pytest.mark.gpu
 def test_ragged_short_and_empty_channels(ns):
     from waveforms_b200 import sample_batch
-    ws = []
-    for n in (1, 0, 7, 9, 127, 129, 1000, 2001):
-        w = 0.7 * ns.gaussian(3e-9) >> (n / 2 * 0.25e-9)
-        w.start, w.stop, w.sample_rate = 0.0, n * 0.25e-9, 4e9
-        ws.append(w)
+    ws = ragged_waveforms(ns)
     rng = np.random.default_rng(11)
     g, o = _gain_offset(rng, len(ws))
     f64 = sample_batch(ws, pair_iq=False).numpy()
@@ -253,18 +249,7 @@ def test_cold_tiles_and_wide_segments(ns):
     """Hundreds of tiny segments in one tile (cold path: global tables) and a stack whose merged segments exceed
     the value slots (wide segments: the slow evaluator)."""
     from waveforms_b200 import sample_batch
-    rng = np.random.default_rng(3)
-    cold = ns.zero()
-    for k in range(300):
-        cold = cold + rng.uniform(0.1, 1) * (ns.gaussian(1.5e-9) >> (2e-9 + 3e-9 * k))
-    cold.start, cold.stop, cold.sample_rate = 0.0, 1e-6, 4e9
-    pulses = []
-    for k in range(9):
-        I, _ = ns.mixing(0.1 * (k + 1) * ns.cosPulse(200e-9) >> (150e-9 + 5e-9 * k), freq=(20 + 7 * k) * 1e6, phase=0.1 * k,
-                         DRAGScaling=3e-10)
-        pulses.append(I)
-    wide = ns.WaveVStack(pulses)
-    wide.start, wide.stop, wide.sample_rate = 0.0, 400e-9, 4e9
+    cold, wide = cold_tiles_waveform(ns), wide_segments_stack(ns)
     for w, g, o in ((cold, 9000.0, 17.0), (wide, 6000.0, -5.5)):
         f64 = sample_batch([w]).numpy()[0]
         codes = sample_batch([w], dtype=np.int16, dac_gain=g, dac_offset=o).numpy()[0]

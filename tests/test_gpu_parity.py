@@ -4,7 +4,8 @@ wire-format program.  fp64 tolerance 1e-12 relative, fp32 1e-6."""
 import numpy as np
 import pytest
 
-from helpers import FP32_TOL, FP64_TOL, b200_eval, b200_object, load_golden, oracle_eval, rel_err
+from helpers import (FP32_TOL, FP64_TOL, b200_eval, b200_object, cold_tiles_waveform, iq_pair_waveforms, load_golden, oracle_eval,
+                     oracle_sample, rel_err, small_batch_waveforms, uneven_waveforms, wide_segments_stack)
 
 pytestmark = pytest.mark.gpu
 
@@ -88,41 +89,22 @@ def test_unsupported_basis_raises(ns):
         w(np.linspace(0, 1, 5))
 
 
-def _oracle_sample(w):
-    """Oracle evaluation of a waveforms_b200 object on its own sample() grid."""
-    from oracle import wfm_oracle as O
-    x = O.sample_grid(w.start, w.stop, w.sample_rate)
-    if hasattr(w, 'wlist'):
-        return O.stack_call(list(w.wlist), x, getattr(w, 'offset', 0), getattr(w, 'shift', 0))
-    return O.waveform_call(w.bounds, w.seq, x, w.min, w.max)
-
-
 def test_wide_segments_take_the_slow_evaluator(ns):
     """A stack whose members overlap with 9 different carrier frequencies: the merged segments
     need more than 12 value slots (kSegWide) and are evaluated from the ABI tables."""
     from waveforms_b200.lowering import lower
     from waveforms_b200.batch import channel_grid
-    pulses = []
-    for k in range(9):
-        I, _ = ns.mixing(0.1 * (k + 1) * ns.cosPulse(200e-9) >> (150e-9 + 5e-9 * k), freq=(20 + 7 * k) * 1e6, phase=0.1 * k,
-                         DRAGScaling=3e-10)
-        pulses.append(I)
-    w = ns.WaveVStack(pulses)
-    w.start, w.stop, w.sample_rate = 0.0, 400e-9, 4e9
+    w = wide_segments_stack(ns)
     b = lower([channel_grid(w)])
     assert np.diff(b.seg_ptr['fac']).max() > 12
     got = w.sample()
-    assert rel_err(got, _oracle_sample(w)) <= FP64_TOL
+    assert rel_err(got, oracle_sample(w)) <= FP64_TOL
 
 
 def test_cold_tiles_take_the_global_path(ns):
     """Hundreds of tiny active segments inside one tile: the tile's packet does not fit a
     warp's buffer (kPacketCold) and the tile is evaluated from the global tables."""
-    rng = np.random.default_rng(3)
-    w = ns.zero()
-    for k in range(300):
-        w = w + rng.uniform(0.1, 1) * (ns.gaussian(1.5e-9) >> (2e-9 + 3e-9 * k))
-    w.start, w.stop, w.sample_rate = 0.0, 1e-6, 4e9
+    w = cold_tiles_waveform(ns)
     from waveforms_b200 import engine
     from waveforms_b200.lowering import lower
     from waveforms_b200.batch import channel_grid
@@ -131,7 +113,7 @@ def test_cold_tiles_take_the_global_path(ns):
     prog.close()
     got = w.sample()
     assert got.shape == (4000, )
-    assert rel_err(got, _oracle_sample(w)) <= FP64_TOL
+    assert rel_err(got, oracle_sample(w)) <= FP64_TOL
     assert info['tile_samples'] >= 128
 
 
@@ -158,7 +140,7 @@ def test_single_sample_and_tile_edges(ns):
     w = 0.3 * ns.cosPulse(40e-9) >> 30e-9
     for n in (1, 2, 3, 127, 1023, 1024, 1025, 2049):
         w.start, w.stop, w.sample_rate = 0.0, n * 1e-10, 1e10
-        got, want = w.sample(), _oracle_sample(w)
+        got, want = w.sample(), oracle_sample(w)
         assert got.shape == want.shape and abs(len(got) - n) <= 1  # np.arange's length rule, fp rounding included
         if np.max(np.abs(want)) > 0:
             assert rel_err(got, want) <= FP64_TOL
@@ -189,18 +171,6 @@ def test_program_info_and_pool_trim(ns):
             assert engine.load_library().wfm_trim() == 0
 
 
-def _small_batch(ns, n=6):
-    rng = np.random.default_rng(21)
-    ws = []
-    for k in range(n):
-        I, Q = ns.mixing(rng.uniform(0.2, 1) * ns.cosPulse(30e-9) >> (60e-9 + 41e-9 * k), freq=rng.uniform(-150e6, 150e6),
-                         phase=rng.uniform(0, 6), DRAGScaling=3e-10)
-        w = I if k % 2 else Q
-        w.start, w.stop, w.sample_rate = 0.0, 0.5e-6 + 7e-9 * k, 2e9
-        ws.append(w)
-    return ws
-
-
 def test_channel_subrange_and_stream(ns):
     """wfm_sample over a sub-range of the program's channels, on a non-default stream, writes
     exactly those channels' samples."""
@@ -208,7 +178,7 @@ def test_channel_subrange_and_stream(ns):
     from waveforms_b200 import engine
     from waveforms_b200.batch import channel_grid
     from waveforms_b200.lowering import lower
-    ws = _small_batch(ns)
+    ws = small_batch_waveforms(ns)
     batch = lower([channel_grid(w) for w in ws])
     prog = engine.Program(batch)
     full = prog.sample_device().cpu().numpy()
@@ -232,7 +202,7 @@ def test_sample_batch_over_two_devices(ns):
     if torch.cuda.device_count() < 2:
         pytest.skip('needs two GPUs')
     from waveforms_b200 import sample_batch
-    ws = _small_batch(ns, 9)
+    ws = small_batch_waveforms(ns, 9)
     one = sample_batch(ws, devices=[0]).numpy()
     two = sample_batch(ws, devices=[0, 1])
     assert {t.device.index for t in two.tensors} == {0, 1}
@@ -316,23 +286,15 @@ def test_both_unit_sizes(name, unit, golden, monkeypatch):
 
 @pytest.mark.parametrize('unit', ['1', '2', '4'])
 def test_unit_sizes_on_pairs_and_accumulate(unit, ns, monkeypatch):
-    """I/Q pairs and the accumulate epilogue through every kernel variant (small programs take the one-sample
-    sparse kernel by default, so the other variants are forced here)."""
-    from test_gpu_parity import _oracle_sample
+    """I/Q pairs through every kernel variant (small programs take the one-sample sparse kernel by default, so the
+    other variants are forced here), and Waveform.__call__(..., accumulate=True), which adds on the host.  The
+    kernels' accumulate epilogue (WfmLaunch.accumulate) is checked in test_gpu_store.py."""
     from waveforms_b200 import sample_batch
     monkeypatch.setenv('WFM_K1_UNIT', unit)
-    rng = np.random.default_rng(31)
-    ws = []
-    for k in range(6):
-        I, Q = ns.mixing(rng.uniform(0.2, 1) * ns.cosPulse(30e-9) >> (40e-9 + 37e-9 * k), freq=rng.uniform(-200e6, 200e6),
-                         phase=rng.uniform(0, 6), DRAGScaling=rng.uniform(2e-10, 1e-9))
-        Q = Q + 0.25
-        for w in (I, Q):
-            w.start, w.stop, w.sample_rate = 0, 0.45e-6, 2e9
-        ws += [I, Q]
+    ws = iq_pair_waveforms(ns)
     got = sample_batch(ws, pair_iq=True).numpy()
     for w, y in zip(ws, got):
-        assert rel_err(y, _oracle_sample(w)) <= FP64_TOL
+        assert rel_err(y, oracle_sample(w)) <= FP64_TOL
     x = np.linspace(-50e-9, 0.5e-6, 1201)
     acc = np.full_like(x, 0.5)
     ws[0](x, out=acc, accumulate=True)
@@ -375,14 +337,7 @@ def test_dynamic_deal_many_tiles_and_subranges(ns, monkeypatch):
     """A batch with thousands of tiles of uneven work, whole and as channel sub-ranges (tile_begin
     not a multiple of the batch size): both deals agree bit for bit."""
     from waveforms_b200 import sample_batch
-    rng = np.random.default_rng(99)
-    chans = []
-    for k in range(37):
-        w = ns.zero()
-        for j in range(int(rng.integers(0, 6))):
-            w = w + rng.uniform(-1, 1) * (ns.gaussian(40e-9) >> float(rng.uniform(1e-6, 60e-6)))
-        w.start, w.stop, w.sample_rate = 0.0, float(rng.uniform(20e-6, 70e-6)), 2e9
-        chans.append(w)
+    chans = uneven_waveforms(ns)
     monkeypatch.setenv('WFM_K1_DEAL', 'static')
     want = sample_batch(chans).numpy()
     monkeypatch.setenv('WFM_K1_DEAL', 'dynamic')
@@ -424,4 +379,4 @@ def test_fast_create_of_small_programs_falls_back_when_tiles_would_be_cold(ns, m
             prog.close()
         assert res['fast'][0]['tile_samples'] == res['slow'][0]['tile_samples']
         assert np.array_equal(res['fast'][1], res['slow'][1])
-        assert rel_err(res['fast'][1], _oracle_sample(wav)) <= FP64_TOL
+        assert rel_err(res['fast'][1], oracle_sample(wav)) <= FP64_TOL

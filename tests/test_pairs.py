@@ -9,7 +9,7 @@ the oracle / the reference's golden vectors."""
 import numpy as np
 import pytest
 
-from helpers import FP32_TOL, FP64_TOL, b200_object, rel_err
+from helpers import FP32_TOL, FP64_TOL, b200_object, oracle_sample, rel_err
 from waveforms_b200.batch import channel_grid
 from waveforms_b200.builder import PulseTemplate, pulse_train_batch
 from waveforms_b200.lowering import (TERM_PLANE1, WAVE_PAIR, can_pair, find_pairs, lower)
@@ -148,7 +148,6 @@ def test_builder_pair_templates_match_lowered_object_pairs(ns):
 def test_paired_sampling_equals_unpaired_and_the_oracle(ns):
     """Mixed batch: DRAG cosPulse / gaussian I/Q pairs, an unrelated channel between them,
     ragged lengths; paired == unpaired to a few ulp, both within 1e-12 of the oracle."""
-    from test_gpu_parity import _oracle_sample
     from waveforms_b200 import sample_batch
     rng = np.random.default_rng(21)
     ws = []
@@ -165,7 +164,7 @@ def test_paired_sampling_equals_unpaired_and_the_oracle(ns):
     single = sample_batch(ws, pair_iq=False).numpy()
     for w, a, b in zip(ws, paired, single):
         assert rel_err(a, b) <= PAIR_TOL
-        assert rel_err(a, _oracle_sample(w)) <= FP64_TOL
+        assert rel_err(a, oracle_sample(w)) <= FP64_TOL
     f32 = sample_batch(ws, pair_iq='auto', dtype=np.float32).numpy()
     for a, b in zip(f32, single):
         assert a.dtype == np.float32 and rel_err(a.astype(np.float64), b) <= FP32_TOL
@@ -189,7 +188,6 @@ def test_rb_stack_pair_against_golden(ns, golden):
 def test_pair_rows_with_own_offsets_constants_and_gaps(ns):
     """Rows that differ in structure: different stack offsets, a constant plateau in one row only,
     a pulse present in one row only, a pre-shift; dense enough for two-sample units."""
-    from test_gpu_parity import _oracle_sample
     from waveforms_b200 import sample_batch
     I, Q = rb_pair(ns, 9, 40)
     extra = 0.25 * (ns.square(300e-9) >> 500e-9)
@@ -203,13 +201,12 @@ def test_pair_rows_with_own_offsets_constants_and_gaps(ns):
     single = sample_batch([I2, Q2], pair_iq=False).numpy()
     for w, a, b in zip((I2, Q2), got, single):
         assert rel_err(a, b) <= PAIR_TOL
-        assert rel_err(a, _oracle_sample(w)) <= FP64_TOL
+        assert rel_err(a, oracle_sample(w)) <= FP64_TOL
 
 
 @pytest.mark.gpu
 def test_pair_cold_tiles_and_wide_segments(ns):
     """The slow evaluators (packet larger than a buffer; more than 12 value slots) on pairs."""
-    from test_gpu_parity import _oracle_sample
     from waveforms_b200 import sample_batch
     rng = np.random.default_rng(4)
     Is, Qs = [], []
@@ -236,7 +233,7 @@ def test_pair_cold_tiles_and_wide_segments(ns):
     single = sample_batch(chans, pair_iq=False).numpy()
     for w, a, b in zip(chans, got, single):
         assert rel_err(a, b) <= PAIR_TOL
-        assert rel_err(a, _oracle_sample(w)) <= FP64_TOL
+        assert rel_err(a, oracle_sample(w)) <= FP64_TOL
 
 
 @pytest.mark.gpu

@@ -776,7 +776,7 @@ int wfm_program_info(wfm_program_t prog, int64_t* out, int32_t n) {
   if (!prog || !out) return fail(WFM_EINVAL, "null program or output");
   const int64_t v[8] = {prog->dev.tile_samples, prog->dev.pkt_cap, prog->dev.n_slots, prog->n_tiles,
                         (int64_t)prog->packets.bytes, (int64_t)(prog->arena.bytes + prog->tile_tables.bytes), prog->dev.unit,
-                        (int64_t)wfm::sample_smem_bytes(prog->dev, WFM_F64)};
+                        (int64_t)wfm::sample_smem_bytes(prog->dev, WFM_F64, false)};
   for (int i = 0; i < n && i < 8; ++i) out[i] = v[i];
   return WFM_OK;
 }
@@ -836,7 +836,8 @@ static int launch_request(wfm_program_t prog, int64_t first, int64_t count, int 
   } else {
     WFM_CUDA(wfm::launch_sample(prog->dev, prog->d_tiles, t0, t1 - t0, WFM_F64, 0, re, st));
   }
-  WFM_CUDA(wfm::launch_interleave_c128(prog->d_tiles + t0, t1 - t0, re, im, out, accumulate, st));
+  WFM_CUDA(wfm::launch_interleave_c128(prog->d_tiles + t0, t1 - t0, prog->dev.waves, prog->dev.planes == 2, re, im, out,
+                                       accumulate, st));
   return WFM_OK;
 }
 

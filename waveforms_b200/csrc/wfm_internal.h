@@ -238,11 +238,12 @@ inline WarpSlice program_slice(const DevProgram& P, int tile_samples, int elem_b
   return warp_slice(P.planes == 2 ? 2 : 1, tile_samples, elem_bytes, P.n_slots, P.unit, pkt_cap);
 }
 // the packet buffer capacity of tiles of tile_samples: the largest that fits the kernel's warp slice when the
-// tile buffers hold fp64 (fp32 and int16 output use a smaller slice with the same buffers)
+// tile buffers hold fp64 (fp32 and int16 output use a smaller slice with the same buffers, fp32 accumulate this one)
 inline int packet_capacity(const DevProgram& P, int tile_samples) {
   return program_slice(P, tile_samples, 8, 0).max_pkt_cap(P.dense ? kDenseSliceBytes : kWarpSliceBytes);
 }
-size_t sample_smem_bytes(const DevProgram& P, int dtype);
+// dynamic shared memory of a sampling launch (accumulate: fp64 tile buffers whatever the output type)
+size_t sample_smem_bytes(const DevProgram& P, int dtype, bool accumulate);
 
 // quant: WFM_I16 only, the DEVICE [n_waves][2][2] (gain, offset) table of WfmQuant
 cudaError_t launch_sample(const DevProgram& P, const TileDesc* tiles, int64_t tile_begin, int64_t n_tiles, int dtype,
@@ -250,8 +251,9 @@ cudaError_t launch_sample(const DevProgram& P, const TileDesc* tiles, int64_t ti
 // y[s][j] = dac_code(x[s][j], gain_offset[s][0], gain_offset[s][1])
 cudaError_t launch_quantize(const double* x, int16_t* y, int64_t n_sig, int64_t n, int64_t x_stride, int64_t y_stride,
                             const double* gain_offset, cudaStream_t stream);
-// out[tile samples] = (re, im) (+ out when accumulate); im may be NULL (zero imaginary part)
-cudaError_t launch_interleave_c128(const TileDesc* tiles, int64_t n_tiles, const double* re, const double* im, void* out,
-                                   int accumulate, cudaStream_t stream);
+// out[tile samples] = (re, im) (+ out when accumulate), and the same for the second row of the tiles of I/Q pairs
+// (pairs: the program holds any, waves: its DEVICE channel table); im may be NULL (zero imaginary part)
+cudaError_t launch_interleave_c128(const TileDesc* tiles, int64_t n_tiles, const WfmWave* waves, bool pairs, const double* re,
+                                   const double* im, void* out, int accumulate, cudaStream_t stream);
 
 }  // namespace wfm

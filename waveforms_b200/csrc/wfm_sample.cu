@@ -1406,20 +1406,23 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks)
     sample_kernel(const __grid_constant__ DevProgram P, const TileDesc* __restrict__ tiles, int tile_begin, int tile_end,
                   OutT* __restrict__ out, unsigned int* __restrict__ tile_counter, const double* __restrict__ quant) {
   constexpr int V = OutVec<OutT>::N;
+  // an accumulating launch keeps its tile buffer in fp64, so that the epilogue adds the fp64 value to out and rounds
+  // once (an fp32 buffer would round twice); packet_capacity sizes every program's slice for fp64 tile buffers
+  using TileT = std::conditional_t<kAccumulate, double, OutT>;
   const int lane = threadIdx.x & 31;
   // this warp's private slice
-  const WarpSlice ws = warp_slice(kPair ? 2 : 1, P.tile_samples, sizeof(OutT), P.n_slots, U, P.pkt_cap);
+  const WarpSlice ws = warp_slice(kPair ? 2 : 1, P.tile_samples, sizeof(TileT), P.n_slots, U, P.pkt_cap);
   unsigned char* slice = k1_smem + (size_t)(threadIdx.x >> 5) * ws.bytes();
-  OutT* s_out = reinterpret_cast<OutT*>(slice);
+  TileT* s_out = reinterpret_cast<TileT*>(slice);
   unsigned char* s_slots = slice + ws.slots();
   unsigned char* sl = lane_slots<U>(s_slots, lane);
 
   // a unit's results -> the tile buffer of its row
   auto to_tile = [&](bool plane1, int jj, int n_valid, const Val<U>& r) {
-    OutT* row_buf = plane1 ? s_out + P.tile_samples : s_out;
+    TileT* row_buf = plane1 ? s_out + P.tile_samples : s_out;
 #pragma unroll
     for (int u = 0; u < U; ++u)
-      if (u < n_valid) row_buf[jj + u] = (OutT)r.v[u];
+      if (u < n_valid) row_buf[jj + u] = (TileT)r.v[u];
   };
   for_each_tile<kWarpsPerCta, kBatch, U, kF32Eval, OutT, kAccumulate, kPair>(
       P, tiles, tile_begin, tile_end, out, quant, tile_counter, s_slots, slice + ws.packets(),
@@ -1436,8 +1439,8 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks)
 
         // base fill: the whole tile BUFFER (tile_samples, a multiple of 128) <- the zero-segment
         // value; flat segments with another value and the active samples overwrite it below
-        const int tile_bytes = P.tile_samples * (int)sizeof(OutT);
-        auto base_fill = [&](OutT* buf, double val, int plane) {
+        const int tile_bytes = P.tile_samples * (int)sizeof(TileT);
+        auto base_fill = [&](TileT* buf, double val, int plane) {
           unsigned char* p = reinterpret_cast<unsigned char*>(buf) + lane * 16;
           if constexpr (kCodes<OutT>) {
             const double* q = row_quant(quant, h->wave, plane);
@@ -1446,7 +1449,7 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks)
             // an odd multiple of 128 samples ends in half a 512-byte row
             if ((tile_bytes & 511) && lane < 16) *reinterpret_cast<uint4*>(p + (tile_bytes & ~511)) = v;
           } else {
-            fill_tile(p, tile_bytes / 512, fill_pattern(val, sizeof(OutT) == 4));
+            fill_tile(p, tile_bytes / 512, fill_pattern(val, sizeof(TileT) == 4));
           }
         };
         base_fill(s_out, base, 0);
@@ -1486,7 +1489,7 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks)
 
         // ---- store ---------------------------------------------------------------------------
         if (kAccumulate) {
-          // out += tile (Waveform.__call__(..., accumulate=True)): read-modify-write epilogue
+          // out += tile (WfmLaunch::accumulate): read-modify-write epilogue, one rounding to OutT
           __syncwarp();
           for (int p = lane; p < cnt; p += 32) dst[p] = (OutT)add((double)dst[p], (double)s_out[p]);
           if constexpr (kPair) {
@@ -1656,15 +1659,22 @@ __global__ void __launch_bounds__(kDenseThreads, 1)
 
 // complex128 output: the real and the imaginary PLANE are sampled by the real-valued kernel
 // (a planar twin of the program, wfm_api.cu) into scratch; this kernel interleaves them
-// tile by tile (exactly the samples of the requested channels, no padding touched).
-// im == nullptr: a real program read as complex.
+// tile by tile (exactly the samples of the requested channels, no padding touched), both
+// rows of an I/Q pair (blockIdx.y = row).  im == nullptr: a real program read as complex.
 template <bool kAccumulate>
-__global__ void __launch_bounds__(256) interleave_c128_kernel(const TileDesc* __restrict__ tiles, const double* __restrict__ re,
-                                                              const double* __restrict__ im, double2* __restrict__ out) {
+__global__ void __launch_bounds__(256) interleave_c128_kernel(const TileDesc* __restrict__ tiles, const WfmWave* __restrict__ waves,
+                                                              const double* __restrict__ re, const double* __restrict__ im,
+                                                              double2* __restrict__ out) {
   const TileDesc td = tiles[blockIdx.x];
-  const double* __restrict__ r = re + td.out0;
-  const double* __restrict__ i = im ? im + td.out0 : nullptr;
-  double2* __restrict__ dst = out + td.out0;
+  int64_t off = td.out0;
+  if (blockIdx.y) {
+    const WfmWave& w = waves[td.wave];
+    if (!(w.flags & WFM_WAVE_PAIR)) return;
+    off = w.out_off2 + td.j0;
+  }
+  const double* __restrict__ r = re + off;
+  const double* __restrict__ i = im ? im + off : nullptr;
+  double2* __restrict__ dst = out + off;
   for (int j = threadIdx.x; j < td.cnt; j += blockDim.x) {
     double2 v = make_double2(r[j], i ? i[j] : 0.0);
     if (kAccumulate) {
@@ -1676,11 +1686,12 @@ __global__ void __launch_bounds__(256) interleave_c128_kernel(const TileDesc* __
   }
 }
 
-cudaError_t launch_interleave_c128(const TileDesc* tiles, int64_t n_tiles, const double* re, const double* im, void* out,
-                                   int accumulate, cudaStream_t stream) {
+cudaError_t launch_interleave_c128(const TileDesc* tiles, int64_t n_tiles, const WfmWave* waves, bool pairs, const double* re,
+                                   const double* im, void* out, int accumulate, cudaStream_t stream) {
   if (n_tiles == 0) return cudaSuccess;
-  if (accumulate) interleave_c128_kernel<true><<<(unsigned)n_tiles, 256, 0, stream>>>(tiles, re, im, (double2*)out);
-  else interleave_c128_kernel<false><<<(unsigned)n_tiles, 256, 0, stream>>>(tiles, re, im, (double2*)out);
+  const dim3 grid((unsigned)n_tiles, pairs ? 2 : 1);
+  if (accumulate) interleave_c128_kernel<true><<<grid, 256, 0, stream>>>(tiles, waves, re, im, (double2*)out);
+  else interleave_c128_kernel<false><<<grid, 256, 0, stream>>>(tiles, waves, re, im, (double2*)out);
   return cudaGetLastError();
 }
 
@@ -1748,8 +1759,8 @@ cudaError_t launch_fill_packets(const DevProgram& P, const TileDesc* tiles, int6
   return cudaGetLastError();
 }
 
-size_t sample_smem_bytes(const DevProgram& P, int dtype) {
-  const int elem = dtype == WFM_F32 ? 4 : (dtype == WFM_I16 ? 2 : 8);
+size_t sample_smem_bytes(const DevProgram& P, int dtype, bool accumulate) {
+  const int elem = dtype == WFM_F32 && !accumulate ? 4 : (dtype == WFM_I16 ? 2 : 8);
   return (size_t)(P.dense ? kDenseWarps : kWarpsPerCta) * program_slice(P, P.tile_samples, elem, P.pkt_cap).bytes();
 }
 
@@ -1819,11 +1830,11 @@ static cudaError_t launch_cfg(K k, LaunchCfg* table, std::mutex& mu, size_t smem
 // tiles), at most one warp per tile.  The shared-memory attribute and occupancy table is per kernel instantiation.
 template <auto kKernel, int kThreadsPerCta, int kBatch, typename OutT>
 static cudaError_t launch_kernel(const DevProgram& P, const TileDesc* tiles, int64_t tile_begin, int64_t n_tiles, int dtype,
-                                 void* out, const double* quant, cudaStream_t stream) {
+                                 bool accumulate, void* out, const double* quant, cudaStream_t stream) {
   static LaunchCfg cfg_table[64];
   static std::mutex cfg_mu;
   const int warps = kThreadsPerCta / 32;
-  const size_t smem = sample_smem_bytes(P, dtype);
+  const size_t smem = sample_smem_bytes(P, dtype, accumulate);
   int dev = 0, sms = 0, per_sm = 0;
   cudaError_t e = launch_cfg(kKernel, cfg_table, cfg_mu, smem, &sms, &per_sm, kThreadsPerCta);
   if (e != cudaSuccess) return e;
@@ -1886,13 +1897,13 @@ static cudaError_t launch_typed(const DevProgram& P, const TileDesc* tiles, int6
       if (P.dense) {
         constexpr int kBatch = decltype(dyn)::value ? kDenseDealBatch : 0;
         return launch_kernel<sample_dense_kernel<OutT, kAcc, kBatch, kPair, kFast>, kDenseThreads, kBatch, OutT>(
-            P, tiles, tile_begin, n_tiles, dtype, out, quant, stream);
+            P, tiles, tile_begin, n_tiles, dtype, kAcc, out, quant, stream);
       }
       constexpr int kBatch = decltype(dyn)::value ? kDealBatch : 0;
       return with_bool(P.unit == 2, [&](auto u2) {
         constexpr int U = decltype(u2)::value ? 2 : 1;
         return launch_kernel<sample_kernel<OutT, kAcc, U, kBatch, kPair, kFast>, kThreads, kBatch, OutT>(
-            P, tiles, tile_begin, n_tiles, dtype, out, quant, stream);
+            P, tiles, tile_begin, n_tiles, dtype, kAcc, out, quant, stream);
       });
     });
   });
