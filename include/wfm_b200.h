@@ -9,6 +9,10 @@
  *                          waveforms/_waveform.pyx:155-169 (calc_parts) does
  *                          per call; here the piecewise program is uploaded
  *                          once as a flat IR and reused.
+ *   wfm_program_create_windows
+ *                        – Waveform.__call__(x, frag=True) batched: a program
+ *                          that samples and stores only given windows of its
+ *                          channels (the non-zero runs), packed.
  *   wfm_sample           – Waveform.sample / Waveform.__call__ /
  *                          WaveVStack.__call__  (waveforms/waveform.py:173-207,
  *                          :529-563, :679-693) = np.arange + calc_parts +
@@ -247,6 +251,29 @@ int  wfm_trim(void);
  * wfm_program_destroy returns it to (no cudaMalloc / cudaFree in a scheduler's steady
  * state); wfm_trim() hands the cached blocks back to the driver. */
 int  wfm_program_create(const WfmProgramDesc* host_ir, int device, wfm_program_t* out);
+
+/* ---- windowed programs: only some samples of each channel -------------------------------------------------------
+ * A window is the samples [j_begin, j_end) of channel `wave`; its sample j goes to out[out_off + (j - j_begin)] (and,
+ * for a WFM_WAVE_PAIR channel, the second row's to out[out_off2 + (j - j_begin)]).  The program is laid out as the
+ * unwindowed program of the same tables (the same samples per lane, the same tile size, its tiles clipped to the
+ * windows) and only the window samples are computed and stored, with the same abscissae and segment ownership.  The
+ * values are bit for bit those of the unwindowed program when it evaluates one sample per lane (sparse programs), and
+ * otherwise for every window that starts in a segment without factors, at the first sample of a segment or at a tile
+ * boundary (the windows of lowering.nonzero_windows): two- and four-sample units rotate a unit's later samples from its first, and a window starting
+ * inside a segment starts its units there (the last bits may then differ).  The channel rows' own out_off / out_off2
+ * are not used.  Windows must be sorted by (wave, j_begin), must not overlap within a channel, must satisfy
+ * 0 <= j_begin < j_end <= n, and their output ranges (both rows of a pair) must be disjoint; j_begin, out_off and
+ * out_off2 are multiples of 4 samples (8 for WFM_I16 launches: a window's tiles start at j_begin and at multiples of
+ * the tile size, and their stores are 16-byte aligned).  Checked on the host before any device work (WFM_EINVAL).  Complex channels are refused at create, WFM_C128 output and accumulate at launch
+ * (WFM_EUNSUPPORTED).  wfm_program_total_samples returns the extent of the windows; first_wave / n_wave of a launch
+ * select the windows of those channels.  (The non-zero runs of a batch: lowering.nonzero_windows.) */
+typedef struct WfmWindow {  /* 40 bytes */
+  int64_t wave, j_begin, j_end;
+  int64_t out_off;   /* first output sample of the window */
+  int64_t out_off2;  /* WFM_WAVE_PAIR channels: first output sample of the window's second row */
+} WfmWindow;
+int  wfm_program_create_windows(const WfmProgramDesc* host_ir, const WfmWindow* windows, int64_t n_windows, int device,
+                                wfm_program_t* out);
 int  wfm_program_destroy(wfm_program_t prog);
 int64_t wfm_program_total_samples(wfm_program_t prog);
 /* number of kernel launches issued through this program so far */

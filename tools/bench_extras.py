@@ -438,13 +438,15 @@ def pipeline_cfg4(ns, torch, engine, peak, quick=False):
     return res
 
 
-def cfg2_frame_from_arrays(ns, torch, engine, seed, channels, xy_pulses, z_pulses, t_end, rate, chans=None):
+def cfg2_frame_from_arrays(ns, torch, engine, seed, channels, xy_pulses, z_pulses, t_end, rate, chans=None,
+                           batch_only=False, align=4):
     """The bench's cfg2 frame (bench.build_frame: cases.xy_channel / z_channel) built from PARAMETER ARRAYS with
     waveforms_b200.builder instead of one Python object per pulse: the same random draws in the same order, one template
     per (channel carrier, envelope) and one for the flux squares; templates are traced with strict=False (random carriers
     between -200 and 200 MHz: the reference algebra's structure depends on the phase value for some of them), so the
     batch equals the object API's to rounding instead of bit for bit.  Returns timings and the parity of the sampled
-    frame against the object-API frame's channels ``chans`` (sampled by the same kernels)."""
+    frame against the object-API frame's channels ``chans`` (sampled by the same kernels).  ``batch_only``: return the
+    builder.CompactBatch itself (rows at multiples of ``align`` samples) instead."""
     from waveforms_b200.builder import PulseTemplate, pulse_train_batch
     rng = np.random.default_rng(seed)
     half = channels // 2
@@ -488,7 +490,10 @@ def cfg2_frame_from_arrays(ns, torch, engine, seed, channels, xy_pulses, z_pulse
         one = lambda rows, n: [[1.0] * n for _ in range(rows)]
         params = {'amp': AMP + ZA, 'phase': PH + one(half, z_pulses), 'drag': DR + one(half, z_pulses),
                   'width': one(half, xy_pulses) + ZW}
-        return pulse_train_batch(templates, idx, t0, 0.0, t_end, rate, params=params, compact=True, spot_check=1)
+        return pulse_train_batch(templates, idx, t0, 0.0, t_end, rate, params=params, compact=True, spot_check=1,
+                                 align=align)
+    if batch_only:
+        return build()
     build()
     ts = []
     for _ in range(3):

@@ -11,7 +11,7 @@ from __future__ import annotations
 import numpy as np
 
 from . import engine
-from .lowering import can_pair, find_pairs, lower
+from .lowering import can_pair, find_pairs, lower, nonzero_windows
 
 
 PAIR_MIN_SAMPLES = 4_000_000  # 'auto' pairing of I/Q channels starts at this batch size (per device)
@@ -80,6 +80,95 @@ class BatchResult:
         return [host[dev][off:off + n] for dev, off, n in self.table]
 
 
+PARTS_RUN_DT = np.dtype([('slot', '<i8'), ('channel', '<i8'), ('start', '<i8'), ('stop', '<i8'), ('offset', '<i8')])
+
+
+class BatchParts:
+    """Device-resident result of ``sample_batch(..., parts=True)``: only the samples of each channel's non-zero runs
+    (maximal ranges of samples owned by segments with at least one term), packed in one flat tensor per device.
+
+    ``runs``: ``PARTS_RUN_DT`` rows ``(slot, channel, start, stop, offset)`` in channel order: samples
+    ``[start, stop)`` of ``channel`` are ``tensors[slot][offset:offset + stop - start]``.  ``base[i]``: the value of
+    every other sample of channel ``i`` (its ``WaveVStack`` offset, else 0; for int16 output its DAC code).
+    ``lengths[i]``: the channel's samples."""
+
+    def __init__(self, tensors, runs, base, lengths, dtype):
+        self.tensors = tensors
+        self.runs = runs
+        self.base = base
+        self.lengths = lengths
+        self.dtype = dtype
+        self._first = np.searchsorted(runs['channel'], np.arange(len(lengths) + 1))
+
+    def __len__(self):
+        return len(self.lengths)
+
+    def channel(self, i):
+        """The runs of channel ``i``: a list of ``(start, stop, tensor view)``."""
+        rs = self.runs[self._first[i]:self._first[i + 1]]
+        return [(int(r['start']), int(r['stop']), self.tensors[r['slot']][r['offset']:r['offset'] + r['stop'] - r['start']])
+                for r in rs]
+
+    def dense(self, i):
+        """Channel ``i`` as a full NumPy row: its runs, ``base[i]`` everywhere else (the packed tensors are copied to
+        the host once)."""
+        if getattr(self, '_host', None) is None:
+            self._host = [t.cpu().numpy() for t in self.tensors]
+        row = np.full(int(self.lengths[i]), self.base[i], dtype=self.dtype)
+        for r in self.runs[self._first[i]:self._first[i + 1]]:
+            row[r['start']:r['stop']] = self._host[r['slot']][r['offset']:r['offset'] + r['stop'] - r['start']]
+        return row
+
+
+def dac_code(v, gain, offset):
+    """``clamp(rint(v * gain + offset), -32768, 32767)`` with NaN -> 0 (multiply, then add): the conversion of
+    ``dtype=np.int16``, on the host."""
+    with np.errstate(invalid='ignore', over='ignore'):
+        y = np.asarray(v, dtype=np.float64) * np.asarray(gain, dtype=np.float64) + np.asarray(offset, dtype=np.float64)
+        c = np.clip(np.rint(y), -32768, 32767)
+    return np.where(np.isnan(y), 0, c).astype(np.int16)
+
+
+def _check_parts(np_dtype, filtered):
+    """The requests ``parts=True`` refuses, before any device work."""
+    if np_dtype == np.dtype(np.complex128):
+        raise TypeError('parts=True returns real samples: complex128 output is not available as parts')
+    if filtered:
+        raise ValueError("parts=True: channels with .filters under filters='own' have no zero runs "
+                         '(the IIR response fills the gaps); pass filters=None or parts=False')
+
+
+def _sample_parts(prog_batch, dev, code, align, gain=None, offset=None):
+    """One device's share of a parts request: (program, packed tensor, NonzeroWindows)."""
+    nz = nonzero_windows(prog_batch, align)
+    if prog_batch.any_complex:
+        raise TypeError('parts=True: a channel with complex amplitudes has no real parts')
+    prog = engine.Program(prog_batch, dev, windows=nz.windows)
+    if code == engine.WFM_I16:
+        return prog, _codes(prog, prog_batch, dev, gain, offset), nz
+    return prog, prog.sample_device(dtype=code), nz
+
+
+def _parts_result(shard_parts, dtype, dac=None):
+    """A ``BatchParts`` from per-device (first channel, batch, tensor, NonzeroWindows)."""
+    tensors, runs, base, lengths = [], [], [], []
+    for slot, (c0, batch, out, nz) in enumerate(shard_parts):
+        tensors.append(out)
+        r = np.zeros(len(nz.runs), dtype=PARTS_RUN_DT)
+        r['slot'] = slot
+        r['channel'] = nz.runs['channel'] + c0
+        for k in ('start', 'stop', 'offset'):
+            r[k] = nz.runs[k]
+        runs.append(r)
+        base.append(nz.base)
+        lengths.append(np.asarray(batch.chan_n, dtype=np.int64))
+    base = np.concatenate(base) if base else np.zeros(0)
+    if dac is not None:
+        base = dac_code(base, dac[0], dac[1])
+    return BatchParts(tensors, np.concatenate(runs) if runs else np.zeros(0, PARTS_RUN_DT), base,
+                      np.concatenate(lengths) if lengths else np.zeros(0, np.int64), np.dtype(dtype))
+
+
 def dac_rows(dtype, dac_gain, dac_offset, n, fast_fp32=False):
     """The per-channel (gain, offset) arrays of a request for 16-bit DAC codes (``dtype=np.int16``), or None for
     any other dtype.  Checked on the host before any device work: ``dac_gain`` is required for int16 and refused
@@ -109,7 +198,7 @@ def _codes(prog, batch, dev, gain, offset):
 
 def sample_batch(waveforms, sample_rate=None, dtype=np.float64, devices=None,
                  filters='own', iir_mode='auto', pair_iq='auto', fast_fp32=False,
-                 dac_gain=None, dac_offset=0.0):
+                 dac_gain=None, dac_offset=0.0, parts=False):
     """Sample every waveform in ``waveforms`` on its own start/stop/sample_rate
     grid.  ``dtype``: np.float64 (reference parity, 1e-12) or np.float32
     (fp32 output, 1e-6).  ``devices``: list of CUDA device indices to shard the
@@ -144,8 +233,16 @@ def sample_batch(waveforms, sample_rate=None, dtype=np.float64, devices=None,
     (waveform.py:1487-1527) — as one I/Q pair: every cos / envelope factor is
     computed once and feeds both outputs (the second row's cosines are rotated from
     the shared sincos: equal to unpaired sampling to a few ulp); ``False`` keeps every channel
-    on its own; ``True`` requires channels (0, 1), (2, 3) ... to pair."""
+    on its own; ``True`` requires channels (0, 1), (2, 3) ... to pair.
+
+    ``parts=True``: compute and return only the samples of each channel's non-zero runs (``BatchParts``; the
+    batched ``Waveform.__call__(x, frag=True)``): a control frame is mostly zeros between pulses, and only the
+    pulses are sampled and leave the GPU.  Every value equals, bit for bit, the one ``parts=False`` returns.  Not for complex
+    output or channels filtered under ``filters='own'``."""
     dac = dac_rows(dtype, dac_gain, dac_offset, len(waveforms), fast_fp32)
+    filtered = filters == 'own' and any(w.filters is not None for w in waveforms)
+    if parts:
+        _check_parts(np.dtype(dtype), filtered)
     import torch
     engine.require_gpu()
     items = [channel_grid(w, sample_rate) for w in waveforms]
@@ -156,7 +253,6 @@ def sample_batch(waveforms, sample_rate=None, dtype=np.float64, devices=None,
             np.dtype(np.float32): engine.WFM_F32,
             np.dtype(np.complex128): engine.WFM_C128,
             np.dtype(np.int16): engine.WFM_I16}[np_dtype]
-    filtered = filters == 'own' and any(w.filters is not None for w in waveforms)
     if filtered and code == engine.WFM_C128:
         raise TypeError('sample_batch(filters=\'own\') filters real channels; sample complex '
                         'channels one by one (Waveform.sample) or pass filters=None')
@@ -176,8 +272,22 @@ def sample_batch(waveforms, sample_rate=None, dtype=np.float64, devices=None,
     # 16-bit codes: rows at multiples of 8 samples (16-byte bulk stores of 2-byte samples)
     align = 8 if dac is not None else 4
     shards = [(dev, lo, hi, lower(plan_pairs(items[lo:hi], pair_iq), align)) for dev, (lo, hi) in zip(devices, ranges)]
+    if parts and any(batch.any_complex for _, _, _, batch in shards):
+        raise TypeError('parts=True: a channel with complex amplitudes has no real parts')
     if dac is not None and any(batch.any_complex for _, _, _, batch in shards):
         raise ValueError('dtype=np.int16: a channel with complex amplitudes has no single DAC code')
+
+    if parts:
+        def run_parts(shard):
+            dev, lo, hi, batch = shard
+            with torch.cuda.device(dev):
+                return _sample_parts(batch, dev, run_code, align, *((dac[0][lo:hi], dac[1][lo:hi]) if dac else ()))
+
+        results = _run_shards(run_parts, shards)
+        for prog, _, _ in results:
+            prog.close()
+        return _parts_result([(lo, batch, out, nz) for (_, lo, _, batch), (_, out, nz) in zip(shards, results)], dtype,
+                             dac)
 
     def run(shard):
         # one host thread per device: upload, pre-pass, K1 and the filters of every device run
@@ -247,7 +357,7 @@ def sample_wire(records, kinds=None, **kw):
 
 def sample_pulse_trains(templates, tmpl_idx, t0, start, stop, sample_rate,
                         dtype=np.float64, devices=None, params=None, compact='auto',
-                        dac_gain=None, dac_offset=0.0):
+                        dac_gain=None, dac_offset=0.0, parts=False):
     """Channels given as PARAMETER ARRAYS instead of objects: channel ``c`` is the
     stack of pulses ``templates[tmpl_idx[c][k]]`` started at ``t0[c][k]``
     (``builder.PulseTemplate.trace`` / ``builder.pulse_train_batch``), sampled on
@@ -258,9 +368,12 @@ def sample_pulse_trains(templates, tmpl_idx, t0, start, stop, sample_rate,
     on the device (``builder.CompactBatch``, ``wfm_expand_templates``) — 'auto' = whenever the channels allow it
     (time-ordered, non-overlapping pulses), True = insist, False = build the full tables on the host.
     ``dtype=np.int16`` with ``dac_gain`` / ``dac_offset``: 16-bit DAC codes as in ``sample_batch``; per-channel
-    values follow the result's channels (pair templates: the I and Q rows of every ``t0`` row)."""
+    values follow the result's channels (pair templates: the I and Q rows of every ``t0`` row).
+    ``parts=True``: only the samples of the non-zero runs, as a ``BatchParts`` (see ``sample_batch``)."""
     rows = 2 if templates and templates[0].pair else 1
     dac = dac_rows(dtype, dac_gain, dac_offset, len(t0) * rows)
+    if parts:
+        _check_parts(np.dtype(dtype), False)
     import torch
     from .builder import pulse_train_batch
     engine.require_gpu()
@@ -288,6 +401,10 @@ def sample_pulse_trains(templates, tmpl_idx, t0, start, stop, sample_rate,
             batch = pulse_train_batch(*args, compact=bool(compact), **kw)
         if dac is not None and batch.any_complex:
             raise ValueError('dtype=np.int16: a channel with complex amplitudes has no single DAC code')
+        if parts:
+            with torch.cuda.device(dev):
+                return _sample_parts(batch, dev, code, kw['align'],
+                                     *((dac[0][lo * rows:hi * rows], dac[1][lo * rows:hi * rows]) if dac else ())) + (batch,)
         with torch.cuda.device(dev):
             prog = engine.Program(batch, dev)
             if dac is not None:
@@ -296,6 +413,11 @@ def sample_pulse_trains(templates, tmpl_idx, t0, start, stop, sample_rate,
         return prog, out, batch
 
     results = _run_shards(run, shards)
+    if parts:
+        for res in results:
+            res[0].close()
+        return _parts_result([(lo * rows, batch, out, nz) for (_, lo, _), (_, out, nz, batch) in zip(shards, results)],
+                             dtype, dac)
     tensors, table = [], []
     for slot, ((dev, lo, hi), (prog, out, batch)) in enumerate(zip(shards, results)):
         tensors.append(out)

@@ -200,6 +200,10 @@ struct WfmProgram {
   pool::Block stage{nullptr, 0};    // device staging buffer of wfm_sample_host
   wfm::TileDesc* d_tiles = nullptr;
   std::vector<int64_t> tile_prefix;  // tiles before channel w
+  // windowed programs (wfm_program_create_windows): the windows and, per channel, its first window ([n_waves + 1])
+  bool windowed = false;
+  std::vector<WfmWindow> windows;
+  std::vector<int64_t> win_first;
   int64_t n_tiles = 0;
   int64_t total_samples = 0;  // extent of the output buffer in samples
   int64_t launches = 0;
@@ -415,6 +419,66 @@ static int validate(const WfmProgramDesc* d, int* max_rows_out) {
   return WFM_OK;
 }
 
+// the windows of wfm_program_create_windows, checked against the (validated) channel table; win_first[w] = first window
+// of channel w, win_first[n_waves] = n_windows
+static int validate_windows(const WfmProgramDesc* d, const WfmWindow* win, int64_t n, std::vector<int64_t>* win_first) {
+  if (n < 0 || (n > 0 && !win)) return fail(WFM_EINVAL, "bad window table");
+  win_first->assign(d->n_waves + 1, n);
+  std::vector<std::pair<int64_t, int64_t>> ranges;  // output ranges of every window row
+  ranges.reserve(n);
+  for (int64_t i = n - 1; i >= 0; --i) {
+    const WfmWindow& v = win[i];
+    if (v.wave < 0 || v.wave >= d->n_waves) return fail(WFM_EINVAL, "window %lld: channel %lld out of range", (long long)i, (long long)v.wave);
+    const WfmWave& w = d->waves[v.wave];
+    if (!(0 <= v.j_begin && v.j_begin < v.j_end && v.j_end <= w.n))
+      return fail(WFM_EINVAL, "window %lld: [%lld, %lld) is not inside [0, %lld) or is empty", (long long)i, (long long)v.j_begin,
+                  (long long)v.j_end, (long long)w.n);
+    if (i + 1 < n && (win[i + 1].wave < v.wave || (win[i + 1].wave == v.wave && win[i + 1].j_begin < v.j_end)))
+      return fail(WFM_EINVAL, "window %lld: windows must be sorted by (wave, j_begin) and must not overlap", (long long)i + 1);
+    (*win_first)[v.wave] = i;
+    if (v.out_off < 0 || v.out_off % 4) return fail(WFM_EINVAL, "window %lld: out_off must be a non-negative multiple of 4", (long long)i);
+    // a window's tiles start at j_begin and at multiples of the tile size: their outputs stay 16-byte aligned
+    if (v.j_begin % 4) return fail(WFM_EINVAL, "window %lld: j_begin must be a multiple of 4", (long long)i);
+    ranges.emplace_back(v.out_off, v.out_off + (v.j_end - v.j_begin));
+    if (w.flags & WFM_WAVE_PAIR) {
+      if (v.out_off2 < 0 || v.out_off2 % 4) return fail(WFM_EINVAL, "window %lld: out_off2 must be a non-negative multiple of 4", (long long)i);
+      ranges.emplace_back(v.out_off2, v.out_off2 + (v.j_end - v.j_begin));
+    }
+  }
+  for (int64_t w = d->n_waves - 1; w >= 0; --w) (*win_first)[w] = std::min((*win_first)[w], (*win_first)[w + 1]);
+  std::sort(ranges.begin(), ranges.end());
+  for (size_t k = 1; k < ranges.size(); ++k)
+    if (ranges[k].first < ranges[k - 1].second)
+      return fail(WFM_EINVAL, "window output ranges intersect at sample %lld", (long long)ranges[k].first);
+  return WFM_OK;
+}
+
+// [lo, hi): the output samples the channels [first, first + count) write (lo = INT64_MAX, hi = 0 if none)
+static void output_extent(const WfmProgram* prog, int64_t first, int64_t count, int64_t* lo, int64_t* hi) {
+  *lo = INT64_MAX;
+  *hi = 0;
+  if (!prog->windowed) {
+    for (int64_t w = first; w < first + count; ++w) {
+      *lo = std::min(*lo, prog->waves[w].out_off);
+      *hi = std::max(*hi, prog->waves[w].out_off + prog->waves[w].n);
+      if (prog->waves[w].flags & WFM_WAVE_PAIR) *hi = std::max(*hi, prog->waves[w].out_off2 + prog->waves[w].n);
+    }
+    return;
+  }
+  for (int64_t i = prog->win_first[first]; i < prog->win_first[first + count]; ++i) {
+    const WfmWindow& v = prog->windows[i];
+    const int64_t len = v.j_end - v.j_begin;
+    *lo = std::min(*lo, v.out_off);
+    *hi = std::max(*hi, v.out_off + len);
+    if (prog->waves[v.wave].flags & WFM_WAVE_PAIR) {
+      *lo = std::min(*lo, v.out_off2);
+      *hi = std::max(*hi, v.out_off2 + len);
+    }
+  }
+}
+
+static int create_program(const WfmProgramDesc* d, const WfmWindow* windows, int64_t n_windows, int device, wfm_program_t* out);
+
 extern "C" {
 
 int wfm_abi_version(void) { return WFM_ABI_VERSION; }
@@ -444,9 +508,23 @@ int wfm_trim(void) {
 }
 
 int wfm_program_create(const WfmProgramDesc* d, int device, wfm_program_t* out) {
+  return create_program(d, nullptr, -1, device, out);
+}
+
+int wfm_program_create_windows(const WfmProgramDesc* d, const WfmWindow* windows, int64_t n_windows, int device,
+                               wfm_program_t* out) {
+  if (n_windows < 0) return fail(WFM_EINVAL, "negative window count");
+  return create_program(d, windows, n_windows, device, out);
+}
+
+}  // extern "C"
+
+// n_windows < 0: the plain program (every sample of every channel)
+static int create_program(const WfmProgramDesc* d, const WfmWindow* windows, int64_t n_windows, int device, wfm_program_t* out) {
   if (!out) return fail(WFM_EINVAL, "null output handle");
   *out = nullptr;
   StageTimer tm("program_create");
+  const bool windowed = n_windows >= 0;
   // all device work of this call runs on the calling thread's own stream: two host threads
   // (a scheduler double-buffering its batches) overlap one batch's upload and pre-pass with
   // the other's device->host copy instead of serialising on the legacy default stream
@@ -454,6 +532,14 @@ int wfm_program_create(const WfmProgramDesc* d, int device, wfm_program_t* out) 
   int max_rows = 0;
   int rc = validate(d, &max_rows);
   if (rc != WFM_OK) return rc;
+  std::vector<int64_t> win_first;
+  if (windowed) {
+    rc = validate_windows(d, windows, n_windows, &win_first);
+    if (rc != WFM_OK) return rc;
+    for (int64_t w = 0; w < d->n_waves; ++w)
+      if (d->waves[w].flags & WFM_WAVE_COMPLEX)
+        return fail(WFM_EUNSUPPORTED, "channel %lld: a windowed program samples real channels only", (long long)w);
+  }
   tm.lap("validate");
   DeviceGuard g(device);
   if (!g.ok) return fail(WFM_ECUDA, "cannot select CUDA device %d: %s", device, cudaGetErrorString(cudaGetLastError()));
@@ -461,6 +547,11 @@ int wfm_program_create(const WfmProgramDesc* d, int device, wfm_program_t* out) 
   if (!p) return fail(WFM_ENOMEM, "out of host memory");
   p->device = device;
   p->waves.assign(d->waves, d->waves + d->n_waves);
+  if (windowed) {
+    p->windowed = true;
+    p->windows.assign(windows, windows + n_windows);
+    p->win_first = std::move(win_first);
+  }
   p->dev.n_slots = 1 + std::max(1, std::min(max_rows, wfm::kMaxSlots));
   p->dev.planes = 1;
   p->dev.dense = 0;
@@ -477,6 +568,20 @@ int wfm_program_create(const WfmProgramDesc* d, int device, wfm_program_t* out) 
       total = std::max(total, d->waves[w].out_off2 + d->waves[w].n);
       if (d->waves[w].out_off2 % 8) p->rows_aligned8 = false;
     }
+  }
+  // A windowed program is laid out as the plain program of the same channels: the same unit and tile size (decided
+  // from the channels' samples), its tiles the plain tiles clipped to the windows.  Two- and four-sample units pair
+  // the samples of a segment from the start of its tile and rotate the second sample's sines from the first's, so only
+  // the plain program's tiles give the plain program's values.  Only the output rows are the windows'.
+  if (windowed) {
+    rows = 0;
+    for (const WfmWindow& v : p->windows)
+      rows += (v.j_end - v.j_begin) * ((d->waves[v.wave].flags & WFM_WAVE_PAIR) ? 2 : 1);
+    int64_t lo;
+    output_extent(p, 0, d->n_waves, &lo, &total);
+    p->rows_aligned8 = true;
+    for (const WfmWindow& v : p->windows)
+      if (v.j_begin % 8 || v.out_off % 8 || ((d->waves[v.wave].flags & WFM_WAVE_PAIR) && v.out_off2 % 8)) p->rows_aligned8 = false;
   }
   p->total_samples = total;
   p->gapless = rows == total;  // the channels' rows tile the output: nothing between them that the kernel leaves unwritten
@@ -496,7 +601,8 @@ int wfm_program_create(const WfmProgramDesc* d, int device, wfm_program_t* out) 
                o_segval = reserve(sizeof(double) * d->n_segs),
                o_segval1 = reserve(p->dev.planes == 2 ? sizeof(double) * d->n_segs : 0), o_plan = reserve(sizeof(wfm::SegPlan) * d->n_segs),
                o_rowslot = reserve((size_t)d->n_facs), o_cterms = reserve(sizeof(wfm::CTerm) * d->n_terms),
-               o_prefix = reserve(sizeof(int64_t) * (d->n_waves + 1)), o_stats = reserve(sizeof(uint64_t) * 2);
+               o_prefix = reserve(sizeof(int64_t) * (std::max<int64_t>(d->n_waves, windowed ? n_windows : 0) + 1)), o_stats = reserve(sizeof(uint64_t) * 2),
+               o_windows = reserve(windowed ? sizeof(WfmWindow) * n_windows : 0);
   cudaError_t e = pool::alloc(device, arena_bytes, &p->arena);
   if (e != cudaSuccess) {
     delete p;
@@ -507,8 +613,9 @@ int wfm_program_create(const WfmProgramDesc* d, int device, wfm_program_t* out) 
   const bool small_program = samples <= (int64_t)1 << 20;
   const char* force_unit = std::getenv("WFM_K1_UNIT");
   const bool unit_forced = force_unit && (force_unit[0] == '1' || force_unit[0] == '2' || force_unit[0] == '4');
-  // the fast path of small programs: the whole arena staged and sent in one copy, no sizing round trip
-  unsigned char* stg = (small_program && !g_no_fast_create && !(d->flags & WFM_DESC_DEVICE_TABLES) && !p->any_complex &&
+  // the fast path of small programs: the whole arena staged and sent in one copy, no sizing round trip (a windowed
+  // program measures the plain tiles to take their size)
+  unsigned char* stg = (small_program && !windowed && !g_no_fast_create && !(d->flags & WFM_DESC_DEVICE_TABLES) && !p->any_complex &&
                         arena_bytes <= kStageBytes && d->n_waves > 0 && !std::getenv("WFM_NO_FAST_CREATE"))
                            ? stage_buffer() : nullptr;
   auto up = [&](size_t off, const void* host, size_t bytes) {
@@ -539,6 +646,7 @@ int wfm_program_create(const WfmProgramDesc* d, int device, wfm_program_t* out) 
     up(o_args, d->args, sizeof(double) * d->n_args);
   }
   up(o_x, d->x, sizeof(double) * d->n_x);
+  if (windowed) up(o_windows, windows, sizeof(WfmWindow) * n_windows);
   p->dev.waves = (const WfmWave*)(base + o_waves);
   p->dev.seg_bound = (const double*)(base + o_bound);
   p->dev.seg_ptr = (const WfmSegPtr*)(base + o_segptr);
@@ -560,8 +668,9 @@ int wfm_program_create(const WfmProgramDesc* d, int device, wfm_program_t* out) 
   // values, segment plans
   wfm::PrepareBuffers pb{(int32_t*)(base + o_segwave), (int32_t*)(base + o_segstart), (double*)(base + o_segval),
                          p->dev.planes == 2 ? (double*)(base + o_segval1) : nullptr, (wfm::SegPlan*)(base + o_plan), (uint8_t*)(base + o_rowslot), (wfm::CTerm*)(base + o_cterms),
-                         nullptr, (const int64_t*)(base + o_prefix), nullptr};
-  wfm::PrepareCounts pc{d->n_waves, d->n_segs, d->n_facs, d->n_terms, 0};
+                         nullptr, windowed ? (const WfmWindow*)(base + o_windows) : nullptr, (const int64_t*)(base + o_prefix),
+                         nullptr};
+  wfm::PrepareCounts pc{d->n_waves, d->n_segs, d->n_facs, d->n_terms, 0, windowed ? n_windows : 0};
   p->dev.unit = 1;
   uint32_t* d_stats = (uint32_t*)(base + o_stats);
   auto cap_of = [&](int ts) { return wfm::packet_capacity(p->dev, ts); };
@@ -574,24 +683,46 @@ int wfm_program_create(const WfmProgramDesc* d, int device, wfm_program_t* out) 
     while (ts > wfm::kMinTileSamples && !(cap_of(ts) >= 256 && 64.0 + ir * ts <= cap_of(ts))) ts -= 128;
     return ts;
   };
-  int64_t n_tiles = 0;
+  // n_plain / plain_prefix: the plain program's tiles (what the tile size is measured on); n_tiles / p->tile_prefix: this
+  // program's (a windowed program's: per window the grid cells it intersects, range_prefix; per channel, tile_prefix)
+  int64_t n_tiles = 0, n_plain = 0;
+  std::vector<int64_t> plain_prefix, range_prefix;
   auto set_tile = [&](int ts) {
     p->dev.tile_samples = ts;
     p->dev.pkt_cap = std::max(cap_of(ts), 64);
-    p->tile_prefix.resize(d->n_waves + 1);
-    n_tiles = 0;
+    plain_prefix.resize(d->n_waves + 1);
+    n_plain = 0;
     for (int64_t w = 0; w < d->n_waves; ++w) {
-      p->tile_prefix[w] = n_tiles;
-      n_tiles += (d->waves[w].n + ts - 1) / ts;
+      plain_prefix[w] = n_plain;
+      n_plain += (d->waves[w].n + ts - 1) / ts;
     }
-    p->tile_prefix[d->n_waves] = n_tiles;
+    plain_prefix[d->n_waves] = n_plain;
+    if (!windowed) {
+      p->tile_prefix = plain_prefix;
+      n_tiles = n_plain;
+      return;
+    }
+    range_prefix.resize(n_windows + 1);
+    n_tiles = 0;
+    for (int64_t i = 0; i < n_windows; ++i) {
+      range_prefix[i] = n_tiles;
+      n_tiles += (p->windows[i].j_end - 1) / ts - p->windows[i].j_begin / ts + 1;
+    }
+    range_prefix[n_windows] = n_tiles;
+    p->tile_prefix.resize(d->n_waves + 1);
+    for (int64_t w = 0; w <= d->n_waves; ++w) p->tile_prefix[w] = range_prefix[p->win_first[w]];
+  };
+  // the device's tile_prefix: this program's tiles, or (plain = true) the plain program's
+  auto upload_prefix = [&](bool plain) {
+    if (windowed && !plain) up(o_prefix, range_prefix.data(), sizeof(int64_t) * (n_windows + 1));
+    else up(o_prefix, plain_prefix.data(), sizeof(int64_t) * (d->n_waves + 1));
   };
   if (stg) {
     // everything the device needs is known on the host: unit, tile size, tile prefix; zeroed statistics ride along
     if (unit_forced) p->dev.unit = force_unit[0] - '0';
     p->dev.dense = p->dev.unit == wfm::kDenseUnit ? 1 : 0;
     set_tile(estimate_tile());
-    up(o_prefix, p->tile_prefix.data(), sizeof(int64_t) * (d->n_waves + 1));
+    upload_prefix(false);
     memset(stg + o_stats, 0, sizeof(uint64_t) * 2);
     e = cudaMemcpyAsync(base, stg, arena_bytes, cudaMemcpyHostToDevice, ST);
   }
@@ -627,20 +758,23 @@ int wfm_program_create(const WfmProgramDesc* d, int device, wfm_program_t* out) 
   int sizing_passes = 0;
   for (; !stg; ts -= 128) {
     set_tile(ts);
-    if (n_tiles >= INT32_MAX) {
+    if (std::max(n_tiles, n_plain) >= INT32_MAX) {
       delete p;
-      return fail(WFM_EINVAL, "too many tiles (%lld)", (long long)n_tiles);
+      return fail(WFM_EINVAL, "too many tiles (%lld)", (long long)std::max(n_tiles, n_plain));
     }
-    if (e != cudaSuccess || ts <= wfm::kMinTileSamples || n_tiles == 0) break;
-    // sizing pass: statistics only
+    if (e != cudaSuccess || ts <= wfm::kMinTileSamples || n_plain == 0) break;
+    // sizing pass on the plain tiles: statistics only
     uint32_t stats[2] = {0, 0};
     e = cudaMemsetAsync(d_stats, 0, sizeof(stats), ST);
-    up(o_prefix, p->tile_prefix.data(), sizeof(int64_t) * (d->n_waves + 1));
-    pc.n_tiles = n_tiles;
-    if (e == cudaSuccess) e = wfm::launch_prepare_tiles(p->dev, pc, pb, d_stats, ST);
+    upload_prefix(true);
+    wfm::PrepareBuffers pb_plain = pb;
+    pb_plain.windows = nullptr;
+    wfm::PrepareCounts pc_plain = pc;
+    pc_plain.n_tiles = n_plain;
+    if (e == cudaSuccess) e = wfm::launch_prepare_tiles(p->dev, pc_plain, pb_plain, d_stats, ST);
     if (e == cudaSuccess) e = read_words(stats, d_stats, 2, ST);  // synchronises: tile_prefix may be rewritten now
     ++sizing_passes;
-    if (e != cudaSuccess || (int64_t)stats[1] * 4096 <= n_tiles) break;
+    if (e != cudaSuccess || (int64_t)stats[1] * 4096 <= n_plain) break;
   }
   p->n_tiles = n_tiles;
   p->sizing_passes = sizing_passes;
@@ -665,7 +799,7 @@ int wfm_program_create(const WfmProgramDesc* d, int device, wfm_program_t* out) 
     pb.tiles = p->d_tiles;
     pb.pkt_size = (uint32_t*)(base2 + o_pktsize);
     pc.n_tiles = n_tiles;
-    if (!stg) up(o_prefix, p->tile_prefix.data(), sizeof(int64_t) * (d->n_waves + 1));
+    if (!stg) upload_prefix(false);
     // pre-pass 1b: the tile rows with their packet sizes (fast path: and the statistics the sizing pass would have
     // taken); then the packet offsets
     if (e == cudaSuccess) e = wfm::launch_prepare_tiles(p->dev, pc, pb, stg ? d_stats : nullptr, ST);
@@ -682,7 +816,7 @@ int wfm_program_create(const WfmProgramDesc* d, int device, wfm_program_t* out) 
   // pass 2: the packets themselves
   if (e == cudaSuccess) e = pool::alloc(device, std::max<size_t>((size_t)total16 * 16, 16), &p->packets);
   p->dev.packets = (const unsigned char*)p->packets.p;
-  if (e == cudaSuccess) e = wfm::launch_fill_packets(p->dev, p->d_tiles, n_tiles, (unsigned char*)p->packets.p, ST);
+  if (e == cudaSuccess) e = wfm::launch_fill_packets(p->dev, p->d_tiles, n_tiles, pc, pb, (unsigned char*)p->packets.p, ST);
   if (stg && n_tiles > 0 && ts > wfm::kMinTileSamples) {
     // the one synchronisation of the fast path also brings the statistics: tiles whose packet does not fit their buffer
     // (they would take the kernel's cold path) send the program through the measured sizing loop instead
@@ -691,7 +825,7 @@ int wfm_program_create(const WfmProgramDesc* d, int device, wfm_program_t* out) 
     if (e == cudaSuccess && (int64_t)stats[1] * 4096 > n_tiles) {
       delete p;
       g_no_fast_create = true;
-      const int rc2 = wfm_program_create(d, device, out);
+      const int rc2 = create_program(d, windows, n_windows, device, out);
       g_no_fast_create = false;
       return rc2;
     }
@@ -761,6 +895,8 @@ int wfm_program_create(const WfmProgramDesc* d, int device, wfm_program_t* out) 
   return WFM_OK;
 }
 
+extern "C" {
+
 int wfm_program_destroy(wfm_program_t prog) {
   StageTimer tm("program_destroy");
   delete prog;
@@ -793,11 +929,10 @@ static int check_launch(wfm_program_t prog, const WfmLaunch* l, int64_t* first, 
     for (int64_t w = *first; w < *first + *count; ++w)
       if (prog->waves[w].flags & WFM_WAVE_COMPLEX)
         return fail(WFM_EINVAL, "channel %lld has complex amplitudes: request WFM_C128 output", (long long)w);
-  int64_t ext = 0;
-  for (int64_t w = *first; w < *first + *count; ++w) {
-    ext = std::max(ext, prog->waves[w].out_off + prog->waves[w].n);
-    if (prog->waves[w].flags & WFM_WAVE_PAIR) ext = std::max(ext, prog->waves[w].out_off2 + prog->waves[w].n);
-  }
+  if (prog->windowed && (l->dtype == WFM_C128 || l->accumulate))
+    return fail(WFM_EUNSUPPORTED, "a windowed program writes real samples only: no WFM_C128 output, no accumulate");
+  int64_t lo, ext;
+  output_extent(prog, *first, *count, &lo, &ext);
   *need = ext;
   if (!l->out && ext > 0) return fail(WFM_EINVAL, "null output buffer");
   if (l->out_elems < ext) return fail(WFM_EINVAL, "output buffer too small: %lld < %lld", (long long)l->out_elems, (long long)ext);
@@ -897,8 +1032,8 @@ static int sample_host(wfm_program_t prog, const WfmLaunch* l, const double* qua
   DeviceGuard g(prog->device);
   const size_t esz = l->dtype == WFM_F64 ? 8 : ((l->dtype == WFM_F32 || l->dtype == WFM_F32_FAST) ? 4 : (l->dtype == WFM_I16 ? 2 : 16));
   // only the extent actually covered by the requested channels is staged/copied
-  int64_t lo = INT64_MAX;
-  for (int64_t w = first; w < first + count; ++w) lo = std::min(lo, prog->waves[w].out_off);
+  int64_t lo, hi;
+  output_extent(prog, first, count, &lo, &hi);
   if (count == 0 || need == 0) return WFM_OK;
   const size_t bytes = (size_t)need * esz;
   if (prog->stage.bytes < bytes) {

@@ -201,6 +201,7 @@ static_assert(sizeof(TileDesc) == 32, "TileDesc layout");
 
 struct PrepareCounts {
   int64_t n_waves, n_segs, n_facs, n_terms, n_tiles;
+  int64_t n_windows;  // windowed program (wfm_program_create_windows): tiles per window; 0: tiles per channel
 };
 
 // tables the pre-pass writes (device pointers into the program's arena)
@@ -213,7 +214,8 @@ struct PrepareBuffers {
   uint8_t* row_slot;
   CTerm* cterms;
   TileDesc* tiles;
-  const int64_t* tile_prefix;  // [n_waves + 1] tiles before channel w (host-built)
+  const WfmWindow* windows;    // [n_windows] (windowed programs; NULL otherwise)
+  const int64_t* tile_prefix;  // [n_waves + 1] tiles before channel w, or [n_windows + 1] before window w (host-built)
   uint32_t* pkt_size;          // [n_tiles + 1]
 };
 
@@ -229,9 +231,9 @@ cudaError_t launch_prepare_tiles(const DevProgram& P, const PrepareCounts& n, co
                                  cudaStream_t stream);
 // exclusive scan: pkt_size[n] -> pkt_off[n + 1] (pkt_off[n] = total); scratch holds ceil(n / 4096) + 1 words
 cudaError_t launch_scan(const uint32_t* pkt_size, uint32_t* pkt_off, uint32_t* scratch, int64_t n, cudaStream_t stream);
-// pass 2: write the packets
-cudaError_t launch_fill_packets(const DevProgram& P, const TileDesc* tiles, int64_t n_tiles, unsigned char* packets,
-                                cudaStream_t stream);
+// pass 2: write the packets (windowed programs: b.windows / b.tile_prefix give a pair tile's second row)
+cudaError_t launch_fill_packets(const DevProgram& P, const TileDesc* tiles, int64_t n_tiles, const PrepareCounts& n,
+                                const PrepareBuffers& b, unsigned char* packets, cudaStream_t stream);
 // a warp's shared-memory slice for the program's kernel, with tiles of tile_samples elements of elem_bytes
 inline WarpSlice program_slice(const DevProgram& P, int tile_samples, int elem_bytes, int pkt_cap) {
   if (P.dense) return warp_slice(0, 0, 0, P.n_slots, kDenseUnit, pkt_cap);

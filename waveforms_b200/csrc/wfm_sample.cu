@@ -836,27 +836,39 @@ __device__ TileLayout measure_tile(const DevProgram& P, const TileDesc& td, cons
   return L;
 }
 
+// the tile range t falls in: last r in [0, n_ranges) with tile_prefix[r] <= t (ranges without samples own no tile)
+__device__ __forceinline__ int64_t tile_range(const int64_t* __restrict__ tile_prefix, int64_t n_ranges, int64_t t) {
+  int64_t lo = 0, hi = n_ranges - 1;
+  while (lo < hi) {
+    const int64_t mid = (lo + hi + 1) >> 1;
+    if (tile_prefix[mid] <= t) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+
 // one thread per tile: the tile row itself (channel, sample range), the segment rows it
 // spans, its packet size.  tiles / pkt_size may be NULL (sizing pass: only the statistics);
-// stats[0] = largest packet (16-byte units), stats[1] = tiles whose packet does not fit
+// stats[0] = largest packet (16-byte units), stats[1] = tiles whose packet does not fit.
+// Tiles cover each channel from sample 0, or (windows != NULL) each window on the same grid: a window's tiles are the
+// cells [k * tile_samples, (k + 1) * tile_samples) it intersects, clipped to it.  Two- and four-sample units pair the
+// samples of a segment from max(segment start, tile start), so the plain program's tile grid gives the same pairs.
 __global__ void prepare_tiles_kernel(DevProgram P, TileDesc* __restrict__ tiles, const int64_t* __restrict__ tile_prefix,
-                                     int64_t n_waves, int64_t n_tiles, uint32_t* __restrict__ pkt_size,
-                                     uint32_t* __restrict__ stats) {
+                                     const WfmWindow* __restrict__ windows, int64_t n_ranges, int64_t n_tiles,
+                                     uint32_t* __restrict__ pkt_size, uint32_t* __restrict__ stats) {
   const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   uint32_t full16 = 0, cold = 0;
   if (t < n_tiles) {
-    // the channel whose tile range holds t: last w with tile_prefix[w] <= t (channels without samples own no tile)
-    int64_t lo_w = 0, hi_w = n_waves - 1;
-    while (lo_w < hi_w) {
-      const int64_t mid = (lo_w + hi_w + 1) >> 1;
-      if (tile_prefix[mid] <= t) lo_w = mid; else hi_w = mid - 1;
-    }
-    const WfmWave w = P.waves[lo_w];
+    const int64_t r = tile_range(tile_prefix, n_ranges, t);
+    const int64_t wave = windows ? windows[r].wave : r;
+    const WfmWave w = P.waves[wave];
+    const int64_t j_begin = windows ? windows[r].j_begin : 0, j_end = windows ? windows[r].j_end : w.n;
+    const int64_t out_off = windows ? windows[r].out_off : w.out_off;
     TileDesc td;
-    td.j0 = (t - tile_prefix[lo_w]) * (int64_t)P.tile_samples;
-    td.out0 = w.out_off + td.j0;
-    td.wave = (int32_t)lo_w;
-    td.cnt = (int32_t)min((int64_t)P.tile_samples, w.n - td.j0);
+    const int64_t ts = P.tile_samples, cell = j_begin / ts + (t - tile_prefix[r]);
+    td.j0 = max(j_begin, cell * ts);
+    td.out0 = out_off + (td.j0 - j_begin);
+    td.wave = (int32_t)wave;
+    td.cnt = (int32_t)(min((cell + 1) * ts, j_end) - td.j0);
     const int32_t* st = P.seg_start + w.seg_begin;
     const int lo = owning_segment(st, w.n_seg, td.j0);
     const int hi = max(lo, owning_segment(st, w.n_seg, td.j0 + td.cnt - 1));
@@ -954,7 +966,9 @@ __global__ void __launch_bounds__(kScanBlock) scan_apply_kernel(const uint32_t* 
 
 // ---- pass 2: one warp per tile writes its packet --------------------------------------------
 __global__ void __launch_bounds__(256) fill_packets_kernel(DevProgram P, const TileDesc* __restrict__ tiles,
-                                                           int64_t n_tiles, unsigned char* __restrict__ packets) {
+                                                           int64_t n_tiles, const WfmWindow* __restrict__ windows,
+                                                           const int64_t* __restrict__ tile_prefix, int64_t n_windows,
+                                                           unsigned char* __restrict__ packets) {
   const int64_t t = (int64_t)blockIdx.x * (blockDim.x / 32) + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   if (t >= n_tiles) return;
@@ -979,7 +993,15 @@ __global__ void __launch_bounds__(256) fill_packets_kernel(DevProgram P, const T
     h.n_patch = L.cold ? 0 : (uint16_t)L.n_patch;
     h.n_units = L.cold ? 0 : (uint16_t)L.n_units;
     h.reserved[0] = h.reserved[1] = 0;
-    h.out1 = (w.flags & WFM_WAVE_PAIR) ? w.out_off2 + td.j0 : td.out0;
+    h.out1 = td.out0;
+    if (w.flags & WFM_WAVE_PAIR) {  // the second row of the tile: the channel's, or its window's
+      if (windows) {
+        const WfmWindow win = windows[tile_range(tile_prefix, n_windows, t)];
+        h.out1 = win.out_off2 + (td.j0 - win.j_begin);
+      } else {
+        h.out1 = w.out_off2 + td.j0;
+      }
+    }
     h.base1 = w.offset2;
     *reinterpret_cast<PacketHeader*>(pk) = h;
   }
@@ -1154,9 +1176,10 @@ __device__ __forceinline__ unsigned char* lane_slots(unsigned char* s_slots, int
 
 // the cold path of a tile (its packet would not fit the warp's buffers): per-sample
 // search, tables in global memory, direct stores (int16 output: codes with the rows' (gain, offset) from quant)
+// out1: the tile's second row (kPair: the packet header's out1, the channel's or its window's)
 template <typename OutT, bool kAccumulate, bool kPair>
-__device__ __forceinline__ void cold_tile(const DevProgram& P, const TileDesc& td, OutT* __restrict__ out, int lane,
-                                          const double* quant) {
+__device__ __forceinline__ void cold_tile(const DevProgram& P, const TileDesc& td, int64_t out1, OutT* __restrict__ out,
+                                          int lane, const double* quant) {
   OutT* __restrict__ dst = out + td.out0;
   const WfmWave w = P.waves[td.wave];
   const WaveEval we{w.offset, w.flags, td.wave};
@@ -1178,7 +1201,7 @@ __device__ __forceinline__ void cold_tile(const DevProgram& P, const TileDesc& t
     double re;
     const double xv = abscissa(w, P.x, td.j0 + jj);
     if (kPair && (w.flags & WFM_WAVE_PAIR)) {
-      OutT* __restrict__ dst1 = out + w.out_off2 + td.j0;
+      OutT* __restrict__ dst1 = out + out1;
       re = eval_segment_slow_row(P, td.seg0 + lo, we.offset, we.flags, we.wave, xv, 0, 0.0);
       store(dst, jj, re, 0);
       re = eval_segment_slow_row(P, td.seg0 + lo, we.offset, we.flags, we.wave, xv, 1, w.offset2);
@@ -1191,12 +1214,22 @@ __device__ __forceinline__ void cold_tile(const DevProgram& P, const TileDesc& t
 }
 template <typename OutT, bool kAccumulate, bool kPair>
 __device__ __noinline__ void sample_tile_cold(const DevProgram& P, const TileDesc& td, OutT* __restrict__ out, int lane) {
-  cold_tile<OutT, kAccumulate, kPair>(P, td, out, lane, nullptr);
+  cold_tile<OutT, kAccumulate, kPair>(P, td, 0, out, lane, nullptr);
 }
 template <bool kPair>
 __device__ __noinline__ void sample_tile_cold_codes(const DevProgram& P, const TileDesc& td, int16_t* __restrict__ out,
                                                     const double* quant, int lane) {
-  cold_tile<int16_t, false, kPair>(P, td, out, lane, quant);
+  cold_tile<int16_t, false, kPair>(P, td, 0, out, lane, quant);
+}
+// I/Q pairs: the second row's position comes with the call
+template <typename OutT, bool kAccumulate>
+__device__ __noinline__ void sample_tile_cold_pair(const DevProgram& P, const TileDesc& td, int64_t out1,
+                                                   OutT* __restrict__ out, int lane) {
+  cold_tile<OutT, kAccumulate, true>(P, td, out1, out, lane, nullptr);
+}
+__device__ __noinline__ void sample_tile_cold_pair_codes(const DevProgram& P, const TileDesc& td, int64_t out1,
+                                                         int16_t* __restrict__ out, const double* quant, int lane) {
+  cold_tile<int16_t, false, true>(P, td, out1, out, lane, quant);
 }
 
 // batch size of the dynamic deal (WFM_K1_DEAL=dynamic at run time, or a large launch: dynamic_deal)
@@ -1321,8 +1354,14 @@ __device__ __forceinline__ void for_each_tile(const DevProgram& P, const TileDes
     // of spills at its 128-register budget, ptxas -v)
     const uint32_t flags = reinterpret_cast<const PacketHeader*>(pk)->flags;
     if (flags & kPacketCold) {
-      if constexpr (kCodes<OutT>) sample_tile_cold_codes<kPair>(P, tiles[t], out, quant, lane);
-      else sample_tile_cold<OutT, kAccumulate, kPair>(P, tiles[t], out, lane);
+      if constexpr (kPair) {
+        const int64_t out1 = reinterpret_cast<const PacketHeader*>(pk)->out1;
+        if constexpr (kCodes<OutT>) sample_tile_cold_pair_codes(P, tiles[t], out1, out, quant, lane);
+        else sample_tile_cold_pair<OutT, kAccumulate>(P, tiles[t], out1, out, lane);
+      } else {
+        if constexpr (kCodes<OutT>) sample_tile_cold_codes<kPair>(P, tiles[t], out, quant, lane);
+        else sample_tile_cold<OutT, kAccumulate, kPair>(P, tiles[t], out, lane);
+      }
       __syncwarp();
       ++it;
       continue;
@@ -1715,9 +1754,8 @@ cudaError_t launch_prepare_tiles(const DevProgram& P, const PrepareCounts& n, co
                                  cudaStream_t stream) {
   if (n.n_tiles <= 0) return cudaSuccess;
   const int threads = 128;
-  prepare_tiles_kernel<<<(unsigned)((n.n_tiles + threads - 1) / threads), threads, 0, stream>>>(P, b.tiles, b.tile_prefix,
-                                                                                              n.n_waves, n.n_tiles,
-                                                                                              b.pkt_size, stats);
+  prepare_tiles_kernel<<<(unsigned)((n.n_tiles + threads - 1) / threads), threads, 0, stream>>>(
+      P, b.tiles, b.tile_prefix, b.windows, b.windows ? n.n_windows : n.n_waves, n.n_tiles, b.pkt_size, stats);
   return cudaGetLastError();
 }
 
@@ -1752,10 +1790,11 @@ cudaError_t launch_scan(const uint32_t* pkt_size, uint32_t* pkt_off, uint32_t* s
   return cudaGetLastError();
 }
 
-cudaError_t launch_fill_packets(const DevProgram& P, const TileDesc* tiles, int64_t n_tiles, unsigned char* packets,
-                                cudaStream_t stream) {
+cudaError_t launch_fill_packets(const DevProgram& P, const TileDesc* tiles, int64_t n_tiles, const PrepareCounts& n,
+                                const PrepareBuffers& b, unsigned char* packets, cudaStream_t stream) {
   if (n_tiles == 0) return cudaSuccess;
-  fill_packets_kernel<<<(unsigned)((n_tiles + 7) / 8), 256, 0, stream>>>(P, tiles, n_tiles, packets);
+  fill_packets_kernel<<<(unsigned)((n_tiles + 7) / 8), 256, 0, stream>>>(P, tiles, n_tiles, b.windows, b.tile_prefix,
+                                                                         n.n_windows, packets);
   return cudaGetLastError();
 }
 

@@ -15,7 +15,7 @@ from pathlib import Path
 import numpy as np
 
 from . import _algebra as A
-from .lowering import (FACTOR_DT, REF_DT, SEGPTR_DT, TERM_DT, WAVE_DT, WAVE_PAIR,
+from .lowering import (FACTOR_DT, REF_DT, SEGPTR_DT, TERM_DT, WAVE_DT, WAVE_PAIR, WINDOW_DT,
                        Channel, Grid, LoweredBatch, lower)
 
 import os
@@ -75,7 +75,7 @@ _lib_lock = threading.Lock()
 
 EXPORTS = [
     'wfm_abi_version', 'wfm_last_error', 'wfm_device_count', 'wfm_trim',
-    'wfm_program_create', 'wfm_program_destroy', 'wfm_program_total_samples',
+    'wfm_program_create', 'wfm_program_create_windows', 'wfm_program_destroy', 'wfm_program_total_samples',
     'wfm_program_launch_count', 'wfm_program_info', 'wfm_sample', 'wfm_sample_host', 'wfm_sample_quant',
     'wfm_sample_quant_host', 'wfm_quantize', 'wfm_sosfilt',
     'wfm_lfilter', 'wfm_lfilter_mode', 'wfm_expand_templates', 'wfm_fft_filter', 'wfm_fft_response_create', 'wfm_fft_response_destroy',
@@ -99,6 +99,10 @@ def load_library():
         lib.wfm_last_error.restype = C.c_char_p
         lib.wfm_program_create.argtypes = [
             C.POINTER(_ProgramDesc), C.c_int,
+            C.POINTER(C.c_void_p)
+        ]
+        lib.wfm_program_create_windows.argtypes = [
+            C.POINTER(_ProgramDesc), C.c_void_p, C.c_int64, C.c_int,
             C.POINTER(C.c_void_p)
         ]
         lib.wfm_program_destroy.argtypes = [C.c_void_p]
@@ -233,9 +237,11 @@ def explicit_grid(x) -> Grid:
 
 # -- program -----------------------------------------------------------------
 class Program:
-    """A lowered batch resident on one GPU."""
+    """A lowered batch resident on one GPU.  ``windows`` (a ``lowering.WINDOW_DT`` array, e.g.
+    ``lowering.nonzero_windows(batch).windows``): sample and store only those windows of the channels, packed at
+    their own offsets (``wfm_program_create_windows``); real-valued output without accumulate."""
 
-    def __init__(self, batch: LoweredBatch, device: int | None = None):
+    def __init__(self, batch: LoweredBatch, device: int | None = None, windows=None):
         lib = require_gpu()
         torch = _torch()
         if device is None:
@@ -256,7 +262,14 @@ class Program:
                 except AttributeError:
                     pass
         h = C.c_void_p()
-        _check(lib.wfm_program_create(C.byref(d), self.device, C.byref(h)))
+        if windows is None:
+            _check(lib.wfm_program_create(C.byref(d), self.device, C.byref(h)))
+            self._total_samples = batch.total_samples
+        else:
+            win = np.ascontiguousarray(windows, dtype=WINDOW_DT)
+            _check(lib.wfm_program_create_windows(C.byref(d), win.ctypes.data if len(win) else None, len(win), self.device,
+                                                  C.byref(h)))
+            self._total_samples = int(lib.wfm_program_total_samples(h))
         self._h = h
 
     def _describe(self, batch, lib):
@@ -315,7 +328,7 @@ class Program:
 
     @property
     def total_samples(self):
-        return self.batch.total_samples
+        return self._total_samples
 
     @property
     def launch_count(self):

@@ -44,7 +44,9 @@ FACTOR_DT = np.dtype([('func', '<i4'), ('arg_off', '<i4'), ('shift', '<f8'),
 TERM_DT = np.dtype([('amp_re', '<f8'), ('amp_im', '<f8'), ('ref_begin', '<i4'),
                     ('n_ref', '<i4'), ('flags', '<u4'), ('reserved', '<u4')])
 REF_DT = np.dtype([('expo', '<f8'), ('slot', '<i4'), ('kind', '<i4')])
-assert WAVE_DT.itemsize == 112 and FACTOR_DT.itemsize == 32
+WINDOW_DT = np.dtype([('wave', '<i8'), ('j_begin', '<i8'), ('j_end', '<i8'), ('out_off', '<i8'), ('out_off2', '<i8')])
+RUN_DT = np.dtype([('channel', '<i8'), ('start', '<i8'), ('stop', '<i8'), ('offset', '<i8')])
+assert WAVE_DT.itemsize == 112 and FACTOR_DT.itemsize == 32 and WINDOW_DT.itemsize == 40
 assert TERM_DT.itemsize == 32 and REF_DT.itemsize == 16
 
 WAVE_EXPLICIT_X = 0x1
@@ -725,3 +727,153 @@ def replicate(batch: LoweredBatch, copies: int, amp_scale=None) -> LoweredBatch:
                         chan_off=(np.tile(batch.chan_off, R) +
                                   np.repeat(np.arange(R), len(batch.chan_off)) * batch.total_samples),
                         chan_n=np.tile(batch.chan_n, R))
+
+
+# ---------------------------------------------------------------------------
+# non-zero runs: the samples a windowed program (wfm_program_create_windows) computes
+# ---------------------------------------------------------------------------
+def _abscissa(w, x, j):
+    """The device's abscissa of sample ``j`` (csrc/wfm_sample.cu ``abscissa``), vectorised: ``w`` holds one channel
+    row per query."""
+    flags = w['flags']
+    j_c = np.clip(j, 0, np.maximum(w['n'] - 1, 0))
+    v = w['t0'] + j_c.astype(np.float64) * w['delta']
+    v = np.where(((flags & WAVE_LAST_OVERRIDE) != 0) & (j_c == w['n'] - 1), w['x_last'], v)
+    explicit = (flags & WAVE_EXPLICIT_X) != 0
+    if explicit.any():
+        v = np.where(explicit, x[np.where(explicit, w['x_off'] + j_c, 0)] if len(x) else 0.0, v)
+    return np.where((flags & WAVE_PRESHIFT) != 0, v - w['pre_shift'], v)
+
+
+def _first_sample_at_or_after(w, x, bound):
+    """The device's ``first_sample_at_or_after``, vectorised: per query, the first sample ``j`` in [0, n] whose
+    abscissa (after the pre-shift) is >= ``bound``: on an affine grid a division for the guess and an exact fix-up
+    against the rounded abscissae, otherwise a binary search."""
+    n = w['n'].astype(np.int64)
+    affine = ((w['flags'] & WAVE_EXPLICIT_X) == 0) & (w['delta'] > 0)
+    out = np.zeros(len(w), dtype=np.int64)
+    a = np.nonzero(affine)[0]
+    if len(a):
+        wa, ba, na = w[a], bound[a], n[a]
+        b = np.where((wa['flags'] & WAVE_PRESHIFT) != 0, ba + wa['pre_shift'], ba)
+        with np.errstate(invalid='ignore', over='ignore'):
+            g = np.ceil((b - wa['t0']) / wa['delta'])
+            j = np.where(g <= 0, 0, np.where(g >= na, na, np.where(np.isnan(g), na, g))).astype(np.int64)
+        while True:
+            m = (j > 0) & (_abscissa(wa, x, j - 1) >= ba)
+            if not m.any():
+                break
+            j -= m
+        while True:
+            m = (j < na) & (_abscissa(wa, x, j) < ba)
+            if not m.any():
+                break
+            j += m
+        out[a] = j
+    g = np.nonzero(~affine)[0]
+    if len(g):
+        wg, bg = w[g], bound[g]
+        lo, hi = np.zeros(len(g), np.int64), n[g].copy()
+        while (lo < hi).any():
+            act = lo < hi
+            mid = (lo + hi) >> 1
+            less = _abscissa(wg, x, mid) < bg
+            lo = np.where(act & less, mid + 1, lo)
+            hi = np.where(act & ~less, mid, hi)
+        out[g] = lo
+    return out
+
+
+@dataclass
+class NonzeroWindows:
+    """The non-zero runs of a batch and their packed layout (``nonzero_windows``).
+
+    ``windows``: the ``WfmWindow`` table (``WINDOW_DT``) of ``wfm_program_create_windows``: the runs, each widened
+    down to a multiple of ``align`` samples (runs closer than that share a window);
+    ``total_samples``: extent of the packed output (``wfm_program_total_samples`` of the windowed program);
+    ``runs``: ``RUN_DT`` rows ``(channel, start, stop, offset)`` in channel order (the batch's channels, ``chan_off``
+    order; the I and Q of a pair have the same runs at their own offsets): samples ``[start, stop)`` are at ``offset``
+    of the packed output;
+    ``base``: per channel, the value of every sample outside its runs."""
+    windows: np.ndarray
+    total_samples: int
+    runs: np.ndarray
+    base: np.ndarray
+
+
+def nonzero_windows(batch, align=4) -> NonzeroWindows:
+    """The runs of a ``LoweredBatch`` or ``builder.CompactBatch``: maximal ranges of consecutive samples owned by
+    segments with at least one term (adjacent non-zero segments merge; an I/Q pair shares one segment table and so
+    its runs), with segment ownership computed as the device computes it.  Outside the runs a channel holds its base
+    (the ``WaveVStack`` offset, else 0; clipping acts on non-zero segments only).  The windows are packed channel
+    by channel, each at a multiple of ``align`` samples (``row_pitch``)."""
+    waves = batch.waves
+    nw = len(waves)
+    pair = (waves['flags'] & WAVE_PAIR) != 0
+    rows = 1 + pair.astype(np.int64)
+    first_chan = np.concatenate([[0], np.cumsum(rows)[:-1]]).astype(np.int64) if nw else np.zeros(0, np.int64)
+    base = np.zeros(int(rows.sum()), dtype=np.float64)
+    base[first_chan] = waves['offset']
+    base[first_chan[pair] + 1] = waves['offset2'][pair]
+
+    # every segment row in channel order: its channel and its position k in the channel
+    n_seg = waves['n_seg'].astype(np.int64)
+    seg_wave = np.repeat(np.arange(nw, dtype=np.int64), n_seg)
+    k = np.arange(len(seg_wave), dtype=np.int64) - np.repeat(np.cumsum(n_seg) - n_seg, n_seg)
+    seg = waves['seg_begin'].astype(np.int64)[seg_wave] + k
+    w = waves[seg_wave]
+    start = np.zeros(len(seg), dtype=np.int64)
+    later = np.nonzero(k > 0)[0]
+    bounds = np.asarray(batch.seg_bound, dtype=np.float64)
+    start[later] = _first_sample_at_or_after(w[later], np.asarray(batch.x, dtype=np.float64), bounds[seg[later] - 1])
+    last = np.ones(len(seg), dtype=bool)
+    last[:-1] = seg_wave[1:] != seg_wave[:-1]
+    stop = np.where(last, w['n'], np.roll(start, -1))
+    terms = batch.seg_ptr['term'].astype(np.int64)
+    keep = (terms[seg + 1] > terms[seg]) & (stop > start)
+    rw, ra, rb = seg_wave[keep], start[keep], stop[keep]
+    # merge runs that touch: a new run starts at a new channel or after a gap
+    new = np.ones(len(rw), dtype=bool)
+    new[1:] = (rw[1:] != rw[:-1]) | (ra[1:] != rb[:-1])
+    heads = np.nonzero(new)[0]
+    rw, ra = rw[heads], ra[heads]
+    rb = rb[np.concatenate([heads[1:] - 1, [len(new) - 1]])] if len(heads) else rb[:0]
+
+    # windows: the runs, each started at the multiple of ``align`` samples at or before it (every tile of a window then
+    # starts at an aligned output sample: the window's start or a multiple of the tile size); runs whose windows would
+    # overlap share one (the few samples between them hold the base)
+    wa = ra & ~(align - 1)
+    head = np.ones(len(rw), dtype=bool)
+    head[1:] = (rw[1:] != rw[:-1]) | (wa[1:] >= rb[:-1])
+    grp = np.cumsum(head) - 1  # window of every run
+    heads = np.nonzero(head)[0]
+    ww, wb = rw[heads], wa[heads]
+    we = rb[np.concatenate([heads[1:] - 1, [len(rw) - 1]])] if len(heads) else rb[:0]
+
+    # packed layout: per channel its first row's windows, then (pairs) its second row's
+    pitch = (we - wb + align - 1) & ~(align - 1)
+    pr = pair[ww]
+    per_wave = np.bincount(ww, weights=pitch * (1 + pr.astype(np.int64)), minlength=nw).astype(np.int64)
+    wave_off = np.concatenate([[0], np.cumsum(per_wave)]).astype(np.int64)
+    row0 = np.bincount(ww, weights=pitch, minlength=nw).astype(np.int64)
+    before = np.cumsum(pitch) - pitch  # first-row samples of the windows before this one
+    off0 = wave_off[ww] + before - before[np.searchsorted(ww, ww)]
+    off1 = np.where(pr, off0 + row0[ww], 0)
+    windows = np.zeros(len(ww), dtype=WINDOW_DT)
+    windows['wave'], windows['j_begin'], windows['j_end'] = ww, wb, we
+    windows['out_off'], windows['out_off2'] = off0, off1
+
+    # the runs in channel order: for each wave, the first row's, then the second row's
+    rpr = pair[rw]
+    order_key = np.concatenate([wave_off[rw] * 2, (wave_off[rw] * 2 + 1)[rpr]])
+    idx = np.concatenate([np.arange(len(rw)), np.arange(len(rw))[rpr]])
+    sec = np.concatenate([np.zeros(len(rw), bool), np.ones(int(rpr.sum()), bool)])
+    perm = np.lexsort((idx, order_key))
+    idx, sec = idx[perm], sec[perm]
+    runs = np.zeros(len(idx), dtype=RUN_DT)
+    runs['channel'] = first_chan[rw[idx]] + sec
+    runs['start'], runs['stop'] = ra[idx], rb[idx]
+    g = grp[idx]
+    runs['offset'] = np.where(sec, off1[g], off0[g]) + (ra[idx] - wb[g])
+    total = int(max((off0 + we - wb).max(initial=0), (off1 + we - wb)[pr].max(initial=0)))
+    return NonzeroWindows(windows=windows, total_samples=total, runs=runs, base=base)
